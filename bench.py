@@ -8,8 +8,10 @@ HeightCompression (K9) -> backward to voxel_features and every parameter (K6/K7/
 (N>1 only).  `value` = frames/s with the points resident in HBM; `e2e` = the same step fed from pinned HOST
 memory through the plugin modules, H2D copy and a D2H read of the loss inside the timed region.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--precision fp32|bf16]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--precision fp32|bf16] [--dump-outputs DIR]
 Under torchrun every rank runs its own 4 frames (weak scaling); rank 0 prints the line.
+--dump-outputs DIR writes what the last timed step of the device-resident arm computed (rank 0) as DIR/<name>.npy, so that
+two builds can be compared output for output on identical seeded inputs (see dump_outputs()).
 """
 import argparse
 import gc
@@ -341,6 +343,8 @@ def run_ours(args, rank, world, local_rank):
     e1.record()
     barrier()                       # (also drains the side stream: torch.cuda.synchronize)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, bd, net)
     per_step = [marks[i].elapsed_time(marks[i + 1]) for i in range(args.steps)]
     if rank == 0:
         print("per-step ms (device arm, main stream): " + " ".join("%.2f" % t for t in per_step), file=sys.stderr)
@@ -416,6 +420,38 @@ def run_ours(args, rank, world, local_rank):
                 host_ms_detail=dict(fwd_bwd=round(host_ms["fwd_bwd"], 3), front_incl_device_waits=round(host_ms["front"], 3)),
                 roofline=roof, roofline_layers=layers)
     return line
+
+
+DUMP_BYTES = 64 << 20       # cap on everything dump_outputs() writes
+
+
+def dump_outputs(out_dir, loss, bd, net):
+    """What a caller of the timed step receives, as float32 / float64 .npy files in `out_dir`:
+      loss.npy                          the step's scalar loss (float64)
+      grad.<parameter name>.npy         every parameter gradient of the backbone (train workloads), full
+      spatial_features_channel_sum.npy  the dense BEV map summed over H x W per (frame, channel), float64, full coverage
+      spatial_features_sample.npy       the dense BEV map [B, C, H, W] at a fixed sample of flat positions (drawn with
+                                        numpy.random.default_rng(0), sorted), as many as fit in what is left of DUMP_BYTES
+    The sparse tensors are left out: their row order is an implementation detail, the dense BEV map is not."""
+    os.makedirs(out_dir, exist_ok=True)
+    sf = bd["spatial_features"].detach()
+    arrays = {"loss": np.asarray(float(loss.item()), dtype=np.float64),
+              "spatial_features_channel_sum": sf.double().sum(dim=(2, 3)).cpu().numpy()}
+    for name, p in net.named_parameters():
+        if p.grad is not None:
+            arrays["grad." + name] = p.grad.detach().float().cpu().numpy()
+    left = (DUMP_BYTES - (1 << 20) - sum(a.nbytes for a in arrays.values())) // 4     # 1 MB kept for the .npy headers
+    if left <= 0:
+        raise RuntimeError("dump_outputs: gradients alone exceed %d bytes" % DUMP_BYTES)
+    n = sf.numel()
+    if n <= left:
+        arrays["spatial_features_sample"] = sf.float().reshape(-1).cpu().numpy()
+    else:
+        idx = np.sort(np.random.default_rng(0).choice(n, size=left, replace=False))
+        arrays["spatial_features_sample"] = sf.float().reshape(-1)[torch.from_numpy(idx).to(sf.device)].cpu().numpy()
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    print("dumped %d arrays (%.1f MB) to %s" % (len(arrays), sum(a.nbytes for a in arrays.values()) / 2**20, out_dir), file=sys.stderr)
 
 
 def roofline_from_profile(prof, bd, peaks, step_ms):
@@ -581,7 +617,11 @@ def main():
     ap.add_argument("--data-rank", type=int, default=None, help="debug: use the synthetic frames rank R of a multi-GPU run would get")
     ap.add_argument("--workload", default="nus_0075", choices=sorted(WORKLOADS),
                     help="default = BASELINE.json configs[2]; waymo_second = configs[1]; toda_stage2 = configs[3]")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl ours)")
     global WORKLOAD, METRIC
     WORKLOAD = args.workload
     METRIC = WORKLOADS[WORKLOAD]["metric"]

@@ -2,8 +2,8 @@
 
 `oracle/_ref/` (a compile of the *reference's own* sources) is not produced:
 the reference's arithmetic for this path lives in the third-party `spconv` /
-`cumm` packages, which are absent from /root/reference (SURVEY.md fact 2), so
-there is nothing under /root/reference to compile.  DESIGN.md records this.
+`cumm` packages, which are absent from the reference repository (SURVEY.md fact 2),
+so there is nothing of the reference to compile.  DESIGN.md records this.
 """
 import os
 import subprocess

@@ -14,15 +14,16 @@ compiled ops are absent), so a synthetic package skeleton is created and only th
 The arithmetic they call (`spconv`, `cumm`) is supplied by a provider: the CPU oracle
 (oracle.spconv_oracle.make_modules()) when generating goldens.
 
-/root/reference exists only in the build container, never on the GPU box: nothing that runs
-under `-m gpu`, smoke() or bench.py may call this.
+The reference is a checkout of rasd3/TODA named by the TODA_REFERENCE environment variable; it is not part of
+this repository.  Nothing that runs under `-m gpu`, smoke() or bench.py may call this, and the tests that need it
+skip when TODA_REFERENCE is unset.
 """
 import importlib.util
 import os
 import sys
 import types
 
-REF_ROOT = "/root/reference"
+REF_ROOT = os.environ.get("TODA_REFERENCE", "")
 
 
 class Cfg(dict):
@@ -34,7 +35,7 @@ class Cfg(dict):
 
 
 def available(root=REF_ROOT):
-    return os.path.isfile(os.path.join(root, "pcdet/models/backbones_3d/spconv_backbone.py"))
+    return bool(root) and os.path.isfile(os.path.join(root, "pcdet/models/backbones_3d/spconv_backbone.py"))
 
 
 def _pkg(name, path=None):

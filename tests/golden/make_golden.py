@@ -1,11 +1,11 @@
 """Generates the committed golden fixtures in tests/golden/*.npz.
 
-Run in the build container only:   python tests/golden/make_golden.py
-It drives the REFERENCE'S OWN files under /root/reference (data_processor.py, mean_vfe.py,
+Run with a reference checkout:   TODA_REFERENCE=<rasd3/TODA clone> python tests/golden/make_golden.py
+It drives the REFERENCE'S OWN files of that checkout (data_processor.py, mean_vfe.py,
 spconv_backbone.py, height_compression.py -- loaded by path, oracle/reference_loader.py) with the
 CPU oracle standing in for the absent third-party `spconv`/`cumm` packages, on small seeded inputs,
 and records inputs + outputs.  The GPU parity tests replay the inputs through the CUDA path and
-compare.  /root/reference does not exist on the GPU box; the fixtures are what travels.
+compare.  The reference is not part of this repository; the fixtures are what travels.
 """
 import os
 import sys
@@ -168,6 +168,8 @@ def golden_backbone(ns, cls_name, fname, frame_cfg, crop, vs, k, f):
 
 
 def main():
+    from tests import parity_utils as PU
+    torch.set_num_threads(PU.GOLDEN_THREADS)      # the replay in tests/test_plugin_topology.py runs at the same count
     ns = R.load(S.make_modules())
     if "--stage2" in sys.argv:
         # TODA stage-1/2 grid: z range -5 .. 4.8 -> 49 bins -> sparse_shape [50, ., .] (shape chain 50 -> 25 -> 13 -> 6 -> 2), F = 4

@@ -1,7 +1,7 @@
 """Generates tests/golden/points.npz: outputs of the REFERENCE'S OWN point pre-steps and mixers on small seeded inputs.
 
-Run in the build container only:   python tests/golden/make_golden_points.py
-Functions driven (loaded by path from /root/reference, oracle/reference_loader.py):
+Run with a reference checkout:   TODA_REFERENCE=<rasd3/TODA clone> python tests/golden/make_golden_points.py
+Functions driven (loaded by path from that checkout, oracle/reference_loader.py):
   * common_utils.mask_points_by_range + DataProcessor.mask_points_and_boxes_outside_range / shuffle_points
     (pcdet/utils/common_utils.py L60-63, pcdet/datasets/processor/data_processor.py L78-103)
   * inter_domain_point_cutmix (inter_domain_point_cutmix.py L10-90): points output; the crop rectangle it drew is

@@ -1,5 +1,6 @@
 """Shared helpers for the parity tests and __graft_entry__.smoke(): run the CPU oracle and the CUDA path on the
 same inputs and compare (bit-exact for integers, rtol 1e-4 for fp32)."""
+import contextlib
 import os
 
 import numpy as np
@@ -11,6 +12,19 @@ from toda_b200.pcdet_plugin.backbones import make_backbones
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 RTOL = 1e-4     # north-star tolerance for fp32 features / activations / gradients
+# The backbone goldens were generated with 8 torch intra-op threads.  The oracle's fp32 results depend on the thread count
+# (BatchNorm statistics and the GEMMs split their sums by thread), so a golden replays bit for bit only at that count.
+GOLDEN_THREADS = 8
+
+
+@contextlib.contextmanager
+def golden_threads():
+    prev = torch.get_num_threads()
+    torch.set_num_threads(GOLDEN_THREADS)
+    try:
+        yield
+    finally:
+        torch.set_num_threads(prev)
 
 
 class Cfg(dict):

@@ -22,7 +22,8 @@ def test_twin_reproduces_reference_golden(cls, fname):
     vf, vc = torch.from_numpy(g["voxel_features"]), torch.from_numpy(g["voxel_coords"]).float()
     gen = torch.Generator().manual_seed(int(g["seed"]))
     cot = torch.randn(tuple(g["bev_shape"]), generator=gen)
-    r = PU.run_backbone(net, PU._oracle_hc, vf, vc, 2, cot=cot, train=True)
+    with PU.golden_threads():
+        r = PU.run_backbone(net, PU._oracle_hc, vf, vc, 2, cot=cot, train=True)
     assert np.array_equal(r["enc_indices"], g["train_enc_indices"])
     np.testing.assert_allclose(r["enc_features"], g["train_enc_features"], rtol=1e-5, atol=1e-6)
     np.testing.assert_allclose(r["dvoxel_features"], g["train_dvoxel_features"], rtol=1e-4, atol=1e-6)
@@ -36,10 +37,25 @@ def test_twin_reproduces_reference_golden(cls, fname):
         np.testing.assert_allclose(r[k + "_features"], g[f"train_{k}_features"], rtol=1e-5, atol=1e-6)
 
 
+@pytest.mark.parametrize("cls,fname", [("VoxelResBackBone8x", "backbone_res.npz"), ("VoxelBackBone8x", "backbone_voxel.npz")])
+def test_cuda_plugin_parameters_match_reference_golden(cls, fname):
+    """The CUDA plugin module (constructed on the CPU) has the reference's parameter names, order and seeded initial
+    values, as recorded in the golden built through the reference's own spconv_backbone.py."""
+    import toda_b200.pcdet_plugin as P
+    g = PU.load_golden(fname)
+    torch.manual_seed(int(g["seed"]))
+    net = getattr(P, cls)(PU.Cfg(), int(g["voxel_features"].shape[1]), g["grid_size"])
+    assert [n for n, _ in net.named_parameters()] == [str(n) for n in g["grad_names"]]
+    wsum = float(sum(p.detach().double().abs().sum() for p in net.parameters()))
+    assert abs(wsum - float(g["weight_abs_sum"])) < 1e-6 * wsum
+    assert net.conv_input[0].weight.shape == g["grad_conv_input_weight"].shape
+    assert net.conv_out[0].weight.shape == g["grad_conv_out_weight"].shape
+
+
 def test_state_dict_matches_reference_when_present():
     from oracle import reference_loader as R, spconv_oracle as S
     if not R.available():
-        pytest.skip("/root/reference not present (GPU box)")
+        pytest.skip("needs a rasd3/TODA checkout named by TODA_REFERENCE")
     ns = R.load(S.make_modules())
     for cls in ["VoxelResBackBone8x", "VoxelBackBone8x"]:
         ref = getattr(ns, cls)(R.Cfg(), 5, np.array([1440, 1440, 40]))
