@@ -227,7 +227,8 @@ int toda_spconv_wgrad(const float *x, const void *x_bf16, int n_in, int cin, con
  * K8 BatchNorm1d(eps, momentum) + ReLU (+ residual) over (N_active, C) rows
  * (spconv_backbone.py L23-24, L54-64, L73/L187).
  *   stats : per-channel mean / biased var of y -> scale = gamma*rstd, shift = beta - mean*scale,
- *           save_mean, save_rstd, running stats update (unbiased var, momentum).
+ *           save_mean, save_rstd, running stats update (unbiased var, momentum).  An empty batch (n = 0) leaves the
+ *           running stats unchanged, as torch.nn.BatchNorm1d does.
  *   apply : a = act(y*scale + shift (+ residual)).
  *   bwd   : g = da * (a>0 if relu); dgamma = sum g*xhat; dbeta = sum g;
  *           dy = scale*(g - dbeta/N - xhat*dgamma/N); dresidual = g.
@@ -265,7 +266,8 @@ int toda_col_sum(const float *dy, int n, int channels, float *out, void *workspa
  * individual entry points above, sequenced in C so that the Python host pays one call per layer.
  *   stats: float[4*cout] = scale, shift, save_mean, save_rstd (mean / rstd rows unused in eval mode)
  *   sums : double[2*cout] scratch for the conv epilogue's statistics (training mode, tensor-core kernel)
- * Pointers marked optional may be NULL.
+ * Pointers marked optional may be NULL; with n_out = 0 the output pointers may be NULL too (the forward then leaves the
+ * running statistics unchanged, the backward writes zero parameter gradients).
  * ------------------------------------------------------------------------------------------ */
 typedef struct {
     const float *x; const void *x_bf16; int n_in, cin; const int32_t *nbr; int n_out, kvol;

@@ -213,7 +213,8 @@ def test_conv_empty_and_tiny_inputs():
 # ------------------------------------------------------------------------------------------ K8 / K9
 @pytest.mark.parametrize("c,n,res,relu,train", [(16, 5000, False, True, True), (128, 3001, True, True, True),
                                                 (64, 1, False, True, True), (32, 4000, True, False, True),
-                                                (16, 2000, False, True, False), (5, 777, True, True, True)])
+                                                (16, 2000, False, True, False), (5, 777, True, True, True),
+                                                (32, 0, True, True, True)])
 def test_bn_act_vs_torch(c, n, res, relu, train):
     from toda_b200 import ops
     torch.manual_seed(1)
@@ -250,6 +251,8 @@ def test_bn_act_vs_torch(c, n, res, relu, train):
         PU.assert_close(rb.grad.cpu().numpy(), ra.grad.numpy(), what="dresidual")
     PU.assert_close(bn_b.running_mean.cpu().numpy(), bn_a.running_mean.numpy(), what="running_mean")
     PU.assert_close(bn_b.running_var.cpu().numpy(), bn_a.running_var.numpy(), what="running_var")
+    # (n = 0: empty output, zero parameter gradients, running statistics unchanged, the batch still counted -- as torch)
+    assert int(bn_b.num_batches_tracked) == int(bn_a.num_batches_tracked)
 
 
 def test_bev_scatter_bit_exact_and_backward():

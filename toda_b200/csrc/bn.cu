@@ -389,8 +389,10 @@ extern "C" int toda_bn_stats(const float *y, int n, int c, const float *gamma, c
     double *partial = (double *)workspace;
     launch_col_reduce<0>(y, nullptr, nullptr, n, c, nullptr, nullptr, 0, partial, st);
     TODA_LAUNCH_OK();
-    bn_finalize_kernel<<<ceil_div(c * 32, 128), 128, 0, st>>>(partial, kPartials, n, c, gamma, beta, eps, momentum, running_mean,
-                                                        running_var, scale, shift, save_mean, save_rstd);
+    // an empty batch has no statistics: the running statistics stay as they are (torch.nn.BatchNorm1d does the same)
+    bn_finalize_kernel<<<ceil_div(c * 32, 128), 128, 0, st>>>(partial, kPartials, n, c, gamma, beta, eps, momentum,
+                                                        n > 0 ? running_mean : nullptr, n > 0 ? running_var : nullptr,
+                                                        scale, shift, save_mean, save_rstd);
     TODA_LAUNCH_OK();
     return TODA_OK;
 }
@@ -399,10 +401,12 @@ extern "C" int toda_bn_finalize_sums(const double *sums, int n, int c, const flo
                                      float momentum, float *running_mean, float *running_var, float *scale, float *shift,
                                      float *save_mean, float *save_rstd, void *stream) {
     TODA_CHECK_ARG(n >= 0 && c > 0 && sums && scale && shift, "bn_finalize_sums: bad args");
-    // `sums` = [sum(y) per channel | sum(y*y) per channel]: the layout of one partial block of toda_bn_stats
+    // `sums` = [sum(y) per channel | sum(y*y) per channel]: the layout of one partial block of toda_bn_stats.  An empty
+    // batch leaves the running statistics unchanged, as in toda_bn_stats.
     bn_finalize_kernel<<<ceil_div(c * 32, 128), 128, 0, (cudaStream_t)stream>>>(sums, 1, n, c, gamma, beta, eps, momentum,
-                                                                            running_mean, running_var, scale, shift, save_mean,
-                                                                            save_rstd);
+                                                                            n > 0 ? running_mean : nullptr,
+                                                                            n > 0 ? running_var : nullptr, scale, shift,
+                                                                            save_mean, save_rstd);
     TODA_LAUNCH_OK();
     return TODA_OK;
 }
@@ -458,7 +462,7 @@ extern "C" int toda_bn_apply_sums(const float *y, int n, int c, const double *su
     TODA_CHECK_ARG(n >= 0 && c > 0 && sums && scale && shift, "bn_apply_sums: bad args");
     cudaStream_t st = (cudaStream_t)stream;
     // the fused kernel needs a thread to keep its four channels over the grid stride; other shapes (none in these backbones)
-    // and empty inputs (the running statistics are still updated) take the two-launch route
+    // and empty inputs (coefficients only: the running statistics are left unchanged) take the two-launch route
     if (n == 0 || c % 4 != 0 || kThreads % (c / 4) != 0) {
         int rc = toda_bn_finalize_sums(sums, n, c, gamma, beta, eps, momentum, running_mean, running_var, scale, shift, save_mean,
                                        save_rstd, stream);

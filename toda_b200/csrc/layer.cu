@@ -8,14 +8,15 @@
 extern "C" int toda_layer_fwd(const toda_layer_fwd_args *p, void *stream) {
     TODA_CHECK_ARG(p, "layer_fwd: null args");
     const int c = p->cout, n = p->n_out;
-    TODA_CHECK_ARG(c > 0 && n >= 0 && p->stats && p->y && p->a, "layer_fwd: bad sizes / null outputs");
+    // an empty tensor's storage pointer is NULL: y and a are only required when there are rows to write
+    TODA_CHECK_ARG(c > 0 && n >= 0 && p->stats && (n == 0 || (p->y && p->a)), "layer_fwd: bad sizes / null outputs");
     float *scale = p->stats, *shift = p->stats + c, *mean = p->stats + 2 * c, *rstd = p->stats + 3 * c;
     const bool tc = p->training && n > 0 && p->sums && toda_spconv_uses_tensor_cores(p->cin, c, p->kvol, p->precision);
     int rc = toda_spconv_fwd_plan(p->x, p->x_bf16, p->n_in, p->cin, p->nbr, n, p->kvol, p->w, c, p->bias, nullptr, p->y, nullptr,
                                   p->tile_masks, p->plan_lidx, p->plan_rows, p->plan_cnt, p->plan_groups, p->plan_cap,
                                   tc ? p->sums : nullptr, p->w_bf16, p->precision, p->conv_ws, p->conv_ws_bytes, stream);
     if (rc) return rc;
-    if (n == 0) return TODA_OK;
+    if (n == 0) return TODA_OK;     // empty batch: no rows, running statistics unchanged (torch.nn.BatchNorm1d does the same)
     if (tc)   // statistics from the convolution's epilogue: coefficients and apply in one launch
         return toda_bn_apply_sums(p->y, n, c, p->sums, p->gamma, p->beta, p->eps, p->momentum, p->running_mean, p->running_var, scale,
                                   shift, mean, rstd, p->residual, p->relu, p->a, p->a_bf16, stream);

@@ -173,6 +173,10 @@ class SparseSequential(SparseModule):
                 i += 1
             elif isinstance(x, SparseConvTensor):
                 if x.indices.shape[0] == 0:
+                    # spconv skips the feature modules on an empty tensor; a training BatchNorm1d still counts the batch
+                    # (torch.nn.BatchNorm1d on zero rows: running statistics unchanged, num_batches_tracked + 1)
+                    if isinstance(m, nn.modules.batchnorm._BatchNorm) and m.training and m.num_batches_tracked is not None:
+                        m.num_batches_tracked += 1
                     i += 1
                     continue
                 # BatchNorm1d [+ ReLU] after a conv: one fused pass of libtoda_b200 instead of ATen's
