@@ -255,6 +255,30 @@ int toda_bn_apply_sums(const float *y, int n, int channels, const double *sums, 
 int toda_bn_bwd(const float *da, const float *a, const float *y, int n, int channels, const float *gamma,
                 const float *save_mean, const float *save_rstd, int relu, int training, float *dy, void *dy_bf16,
                 float *dresidual, float *dgamma, float *dbeta, void *workspace, size_t workspace_bytes, void *stream);
+/* BatchNorm over a batch split across processes (torch.nn.SyncBatchNorm, training mode): each statistic that needs the
+ * other ranks is produced locally, all-reduced (SUM) by the caller, and consumed by a second call.
+ *   forward : toda_bn_local_sums -> all-reduce local_sums -> toda_bn_apply_global
+ *   backward: toda_bn_bwd_reduce -> all-reduce local_red  -> toda_bn_bwd_finish
+ * local_sums / global_sums: double[2*channels+1] = sum(y) per channel | sum(y*y) per channel | row count; the count is
+ * written on the device.  epilogue_sums (optional): the convolution epilogue's double[2*channels] sums of y (then y is not
+ * read; it may be local_sums itself).  global_sums gives mean, biased variance (coefficients, save_mean / save_rstd) and
+ * the running statistics' update (unbiased variance, global count; unchanged when the global count is 0).
+ * local_red / global_red: double[2*channels] = sum g | sum g*xhat (g = da after the ReLU mask); dgamma / dbeta are
+ * this process's own sums (torch leaves their averaging to the gradient all-reduce).  global_count: &global_sums[2*channels]
+ * of the forward.  A process with no rows still makes every call.  With its own buffers passed through unreduced, each
+ * pair computes what toda_bn_stats + toda_bn_apply (or toda_bn_apply_sums) and toda_bn_bwd compute, bit for bit. */
+int toda_bn_local_sums(const float *y, const double *epilogue_sums, int n, int channels, double *local_sums, void *workspace,
+                       size_t workspace_bytes, void *stream);
+int toda_bn_apply_global(const float *y, int n, int channels, const double *global_sums, const float *gamma, const float *beta,
+                         float eps, float momentum, float *running_mean, float *running_var, float *scale, float *shift,
+                         float *save_mean, float *save_rstd, const float *residual, int relu, float *a, void *a_bf16,
+                         void *stream);
+int toda_bn_bwd_reduce(const float *da, const float *a, const float *y, int n, int channels, const float *save_mean,
+                       const float *save_rstd, int relu, double *local_red, float *dgamma, float *dbeta, void *workspace,
+                       size_t workspace_bytes, void *stream);
+int toda_bn_bwd_finish(const float *da, const float *a, const float *y, int n, int channels, const float *gamma,
+                       const float *save_mean, const float *save_rstd, int relu, const double *global_red,
+                       const double *global_count, float *dy, void *dy_bf16, float *dresidual, void *stream);
 /* column sums: dbias[c] = sum_rows dy[:,c] */
 int toda_col_sum(const float *dy, int n, int channels, float *out, void *workspace, size_t workspace_bytes,
                  void *stream);
@@ -295,6 +319,16 @@ typedef struct {
 } toda_layer_bwd_args;
 int toda_layer_fwd(const toda_layer_fwd_args *args, void *stream);
 int toda_layer_bwd(const toda_layer_bwd_args *args, void *stream);
+/* The same layer with a BatchNorm synchronized across processes (training mode), split at the all-reduces as the
+ * toda_bn_* calls above: toda_layer_fwd_stats (conv + local_sums, double[2*cout+1]) -> all-reduce ->
+ * toda_layer_fwd_apply (stats, a, a_bf16, running statistics from global_sums); toda_layer_bwd_reduce (local_red,
+ * double[2*cout], and this process's dgamma / dbeta) -> all-reduce -> toda_layer_bwd_finish (dy, dres, dgrad, wgrad,
+ * bias gradient; global_count = &global_sums[2*cout] of the forward).  `sums` of the forward args is not used.  Unreduced,
+ * fwd_stats + fwd_apply = toda_layer_fwd and bwd_reduce + bwd_finish = toda_layer_bwd, bit for bit. */
+int toda_layer_fwd_stats(const toda_layer_fwd_args *args, double *local_sums, void *stream);
+int toda_layer_fwd_apply(const toda_layer_fwd_args *args, const double *global_sums, void *stream);
+int toda_layer_bwd_reduce(const toda_layer_bwd_args *args, double *local_red, void *stream);
+int toda_layer_bwd_finish(const toda_layer_bwd_args *args, const double *global_red, const double *global_count, void *stream);
 
 /* ------------------------------------------------------------------------------------------
  * K9 HeightCompression: pcdet/models/backbones_2d/map_to_bev/height_compression.py L20-25

@@ -51,6 +51,10 @@ SIGNATURES = {
     "toda_weight_kmajor_bf16": (c_int, [c_vp, c_int, c_int, c_int, c_vp, c_vp]),
     "toda_layer_fwd": (c_int, [c_vp, c_vp]),
     "toda_layer_bwd": (c_int, [c_vp, c_vp]),
+    "toda_layer_fwd_stats": (c_int, [c_vp, c_vp, c_vp]),
+    "toda_layer_fwd_apply": (c_int, [c_vp, c_vp, c_vp]),
+    "toda_layer_bwd_reduce": (c_int, [c_vp, c_vp, c_vp]),
+    "toda_layer_bwd_finish": (c_int, [c_vp, c_vp, c_vp, c_vp]),
     "toda_spconv_wgrad_workspace_bytes": (c_sz, [c_int] * 6),
     "toda_spconv_wgrad": (c_int, [c_vp, c_vp, c_int, c_int, c_vp, c_int, c_int, c_vp, c_vp, c_int, c_vp, c_vp, c_sz, c_int, c_vp]),
     "toda_bn_workspace_bytes": (c_sz, [c_int]),
@@ -63,6 +67,11 @@ SIGNATURES = {
                                    c_int, c_vp, c_vp, c_vp]),
     "toda_bn_bwd": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp,
                             c_vp, c_sz, c_vp]),
+    "toda_bn_local_sums": (c_int, [c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_sz, c_vp]),
+    "toda_bn_apply_global": (c_int, [c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_f32, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
+                                     c_int, c_vp, c_vp, c_vp]),
+    "toda_bn_bwd_reduce": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
+    "toda_bn_bwd_finish": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "toda_col_sum": (c_int, [c_vp, c_int, c_int, c_vp, c_vp, c_sz, c_vp]),
     "toda_bev_scatter_fwd": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp]),
     "toda_bev_scatter_bwd": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp]),

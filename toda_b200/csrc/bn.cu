@@ -186,6 +186,22 @@ __global__ void bn_finalize_kernel(const double *__restrict__ partial, int nbloc
     bn_update_running(running_mean, running_var, ch, momentum, meanf, var, n);
 }
 
+// Local statistics of a BatchNorm whose batch spans several processes: out = [sum(y) | sum(y*y) | n], the fp64 buffer
+// that is all-reduced across ranks.  From the per-CTA partials (partial != NULL: the same fixed-order sums as
+// bn_finalize_kernel) or copied from `src` (the convolution epilogue's sums; src == out: count only; NULL: zeros).
+// The count is written here, on the device, so the host never has to provide or read it.
+__global__ void bn_local_sums_kernel(const double *partial, int nblocks, const double *src, int n, int c, double *out) {
+    if (blockIdx.x == 0 && threadIdx.x == 0) out[2 * c] = (double)n;
+    int ch = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (ch >= c) return;
+    double s = 0.0, ss = 0.0;
+    if (partial) warp_sum_partials(partial, nblocks, c, ch, s, ss);
+    else if (src) { s = src[ch]; ss = src[c + ch]; }
+    if ((threadIdx.x & 31) != 0) return;
+    out[ch] = s;
+    out[c + ch] = ss;
+}
+
 __global__ void bn_eval_coeffs_kernel(const float *gamma, const float *beta, const float *rm, const float *rv, float eps,
                                       int c, float *scale, float *shift) {
     int ch = blockIdx.x * blockDim.x + threadIdx.x;
@@ -284,8 +300,72 @@ __global__ void __launch_bounds__(kThreads) bn_apply_sums_kernel(const float *__
     }
 }
 
+// Training-mode BatchNorm from statistics all-reduced over several processes: sums = [sum(y) | sum(y*y) | n] of the
+// union batch (bn_local_sums_kernel's layout).  Every CTA derives the coefficients of all channels into shared memory
+// (the same bn_coeffs as the finalize kernels, so the same bits), block 0 publishes scale / shift / mean / rstd and
+// updates the running statistics with the global count; then the rows of this process stream as in bn_apply_kernel.
+// A process with no rows still runs block 0: its running statistics must follow the other ranks'.
+template <bool VEC>
+__global__ void __launch_bounds__(kThreads) bn_apply_global_kernel(const float *__restrict__ y, long long total, int c,
+                                                                   const double *__restrict__ sums, const float *__restrict__ gamma,
+                                                                   const float *__restrict__ beta, float eps, float momentum,
+                                                                   float *running_mean, float *running_var, float *scale_out,
+                                                                   float *shift_out, float *save_mean, float *save_rstd,
+                                                                   const float *__restrict__ residual, int relu, float *__restrict__ a,
+                                                                   __nv_bfloat16 *__restrict__ a_bf16) {
+    __shared__ __align__(16) float s_sc[256], s_sh[256];
+    const int n = (int)sums[2 * c];
+    for (int ch = threadIdx.x; ch < c; ch += blockDim.x) {
+        float meanf, rstd;
+        double var;
+        bn_coeffs(sums[ch], sums[c + ch], n, gamma ? gamma[ch] : 1.f, beta ? beta[ch] : 0.f, eps, s_sc[ch], s_sh[ch], meanf, rstd, var);
+        if (blockIdx.x == 0) {
+            scale_out[ch] = s_sc[ch];
+            shift_out[ch] = s_sh[ch];
+            if (save_mean) save_mean[ch] = meanf;
+            if (save_rstd) save_rstd[ch] = rstd;
+            if (n > 0) bn_update_running(running_mean, running_var, ch, momentum, meanf, var, n);
+        }
+    }
+    __syncthreads();
+    if (VEC) {
+        const long long tv = total >> 2;
+        for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < tv; e += (long long)gridDim.x * blockDim.x) {
+            const int ch = (int)((e << 2) % c);
+            const float4 v = __ldg((const float4 *)y + e);
+            const float4 sc = *(const float4 *)(s_sc + ch), sh = *(const float4 *)(s_sh + ch);
+            float4 o = make_float4(fmaf(v.x, sc.x, sh.x), fmaf(v.y, sc.y, sh.y), fmaf(v.z, sc.z, sh.z), fmaf(v.w, sc.w, sh.w));
+            if (residual) {
+                const float4 r = __ldg((const float4 *)residual + e);
+                o.x += r.x; o.y += r.y; o.z += r.z; o.w += r.w;
+            }
+            if (relu) { o.x = fmaxf(o.x, 0.f); o.y = fmaxf(o.y, 0.f); o.z = fmaxf(o.z, 0.f); o.w = fmaxf(o.w, 0.f); }
+            ((float4 *)a)[e] = o;
+            if (a_bf16) {
+                __nv_bfloat162 lo = __floats2bfloat162_rn(o.x, o.y), hi = __floats2bfloat162_rn(o.z, o.w);
+                uint2 pk;
+                pk.x = *(uint32_t *)&lo;
+                pk.y = *(uint32_t *)&hi;
+                ((uint2 *)a_bf16)[e] = pk;
+            }
+        }
+    } else {
+        for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+            const int ch = (int)(e % c);
+            float o = fmaf(__ldg(y + e), s_sc[ch], s_sh[ch]);
+            if (residual) o += __ldg(residual + e);
+            if (relu) o = fmaxf(o, 0.f);
+            a[e] = o;
+            if (a_bf16) a_bf16[e] = __float2bfloat16_rn(o);
+        }
+    }
+}
+
+// T = float: the sums bn_bwd_apply_kernel reads in the same call; T = double: the local sums a multi-process BatchNorm
+// all-reduces before its bn_bwd_apply_kernel<., true> (which rounds them to float exactly as this kernel does for float).
+template <typename T>
 __global__ void bn_bwd_finalize_kernel(const double *__restrict__ partial, int nblocks, int c, float *dgamma, float *dbeta,
-                                       float *sums /* [2c]: sum_g, sum_g_xhat */) {
+                                       T *sums /* [2c]: sum_g, sum_g_xhat */) {
     int ch = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (ch >= c) return;
     double s, sx;
@@ -293,20 +373,25 @@ __global__ void bn_bwd_finalize_kernel(const double *__restrict__ partial, int n
     if ((threadIdx.x & 31) != 0) return;
     if (dbeta) dbeta[ch] = (float)s;
     if (dgamma) dgamma[ch] = (float)sx;
-    sums[ch] = (float)s;
-    sums[c + ch] = (float)sx;
+    sums[ch] = (T)s;
+    sums[c + ch] = (T)sx;
 }
 
 // dy = gamma*rstd*(g - sum_g/N - xhat*sum_gx/N)   (training)   |   dy = gamma*rstd*g   (eval)
 // Per channel this is dy = A*g + B*y + C with A = gamma*rstd, B = -gamma*rstd^2*sum_gx/N,
 // C = -A*sum_g/N - B*mean: coefficients are computed once per thread (4 channels), rows stream as float4.
-template <bool VEC>
+// GLOBAL: the sums are the fp64 ones all-reduced over the processes of a synchronized BatchNorm (`gsums`) and N is the
+// global count (`gcount`, device memory); both are rounded exactly as the single-process path rounds them.
+template <bool VEC, bool GLOBAL>
 __global__ void __launch_bounds__(kThreads) bn_bwd_apply_kernel(const float *__restrict__ da, const float *__restrict__ a,
-                                                                const float *__restrict__ y, long long total, int c, int n,
+                                                                const float *__restrict__ y, long long total, int c, int n_local,
                                                                 const float *__restrict__ gamma, const float *__restrict__ mean,
-                                                                const float *__restrict__ rstd, const float *__restrict__ sums,
+                                                                const float *__restrict__ rstd, const float *__restrict__ fsums,
+                                                                const double *__restrict__ gsums, const double *__restrict__ gcount,
                                                                 int relu, int training, float *__restrict__ dy,
                                                                 float *__restrict__ dres, __nv_bfloat16 *__restrict__ dy_bf16) {
+    const int n = GLOBAL ? (int)*gcount : n_local;
+    auto sums = [&](int i) -> float { return GLOBAL ? (float)gsums[i] : fsums[i]; };
     const float inv_n = n > 0 ? 1.0f / (float)n : 0.f;
     if (VEC) {
         const long long tv = total >> 2;
@@ -318,8 +403,8 @@ __global__ void __launch_bounds__(kThreads) bn_bwd_apply_kernel(const float *__r
         for (int q = 0; q < 4; ++q) {
             float gm = gamma ? gamma[ch + q] : 1.f, rs = rstd[ch + q];
             A[q] = gm * rs;
-            B[q] = training ? -gm * rs * rs * sums[c + ch + q] * inv_n : 0.f;
-            C[q] = training ? -A[q] * sums[ch + q] * inv_n - B[q] * mean[ch + q] : 0.f;
+            B[q] = training ? -gm * rs * rs * sums(c + ch + q) * inv_n : 0.f;
+            C[q] = training ? -A[q] * sums(ch + q) * inv_n - B[q] * mean[ch + q] : 0.f;
         }
         for (; e < tv; e += stride) {
             float4 g4 = __ldg((const float4 *)da + e);
@@ -355,7 +440,7 @@ __global__ void __launch_bounds__(kThreads) bn_bwd_apply_kernel(const float *__r
             float o;
             if (training) {
                 float xh = (__ldg(y + e) - mean[ch]) * rs;
-                o = gm * rs * (g - sums[ch] * inv_n - xh * sums[c + ch] * inv_n);
+                o = gm * rs * (g - sums(ch) * inv_n - xh * sums(c + ch) * inv_n);
             } else {
                 o = gm * rs * g;
             }
@@ -481,6 +566,33 @@ extern "C" int toda_bn_apply_sums(const float *y, int n, int c, const double *su
     return TODA_OK;
 }
 
+// The streaming pass of the BatchNorm backward (bn_bwd_apply_kernel) over n > 0 rows.  GLOBAL: the reductions and the
+// count come from device memory (fp64, all-reduced over the processes of a synchronized BatchNorm) instead of `fsums`/`n`.
+template <bool GLOBAL>
+static void launch_bn_bwd_apply(const float *da, const float *a, const float *y, int n, int c, const float *gamma,
+                                const float *save_mean, const float *save_rstd, const float *fsums, const double *gsums,
+                                const double *gcount, int relu, int training, float *dy, float *dresidual, void *dy_bf16,
+                                cudaStream_t st) {
+    long long total = (long long)n * c;
+    static int per_sm_vec = 0, per_sm_scalar = 0;
+    if (!per_sm_vec) {
+        per_sm_vec = resident_grid(bn_bwd_apply_kernel<true, GLOBAL>, (int64_t)1 << 40) / kNumSMs;
+        per_sm_scalar = resident_grid(bn_bwd_apply_kernel<false, GLOBAL>, (int64_t)1 << 40) / kNumSMs;
+    }
+    auto grid_for = [](int64_t items, int per_sm) {
+        int64_t need = (items + kThreads - 1) / kThreads, cap = (int64_t)per_sm * kNumSMs;
+        return (int)(need < 1 ? 1 : (need < cap ? need : cap));
+    };
+    if (c % 4 == 0 && kThreads % (c / 4) == 0)   // grid*block is then a multiple of c/4: a thread keeps its 4 channels
+        bn_bwd_apply_kernel<true, GLOBAL><<<grid_for(total / 4, per_sm_vec), kThreads, 0, st>>>(
+            da, a, y, total, c, n, gamma, save_mean, save_rstd, fsums, gsums, gcount, relu, training, dy, dresidual,
+            (__nv_bfloat16 *)dy_bf16);
+    else
+        bn_bwd_apply_kernel<false, GLOBAL><<<grid_for(total, per_sm_scalar), kThreads, 0, st>>>(
+            da, a, y, total, c, n, gamma, save_mean, save_rstd, fsums, gsums, gcount, relu, training, dy, dresidual,
+            (__nv_bfloat16 *)dy_bf16);
+}
+
 extern "C" int toda_bn_bwd(const float *da, const float *a, const float *y, int n, int c, const float *gamma,
                            const float *save_mean, const float *save_rstd, int relu, int training, float *dy, void *dy_bf16,
                            float *dresidual, float *dgamma, float *dbeta, void *workspace, size_t workspace_bytes, void *stream) {
@@ -495,27 +607,95 @@ extern "C" int toda_bn_bwd(const float *da, const float *a, const float *y, int 
     float *sums = (float *)((char *)workspace + (size_t)kPartials * 2 * c * sizeof(double));
     launch_col_reduce<1>(da, a, y, n, c, save_mean, save_rstd, relu, partial, st);
     TODA_LAUNCH_OK();
-    bn_bwd_finalize_kernel<<<ceil_div(c * 32, 128), 128, 0, st>>>(partial, kPartials, c, dgamma, dbeta, sums);
+    bn_bwd_finalize_kernel<float><<<ceil_div(c * 32, 128), 128, 0, st>>>(partial, kPartials, c, dgamma, dbeta, sums);
     TODA_LAUNCH_OK();
     if (n > 0) {
-        long long total = (long long)n * c;
-        static int per_sm_vec = 0, per_sm_scalar = 0;
-        if (!per_sm_vec) {
-            per_sm_vec = resident_grid(bn_bwd_apply_kernel<true>, (int64_t)1 << 40) / kNumSMs;
-            per_sm_scalar = resident_grid(bn_bwd_apply_kernel<false>, (int64_t)1 << 40) / kNumSMs;
-        }
-        auto grid_for = [](int64_t items, int per_sm) {
-            int64_t need = (items + kThreads - 1) / kThreads, cap = (int64_t)per_sm * kNumSMs;
-            return (int)(need < 1 ? 1 : (need < cap ? need : cap));
-        };
-        if (c % 4 == 0 && kThreads % (c / 4) == 0)   // grid*block is then a multiple of c/4: a thread keeps its 4 channels
-            bn_bwd_apply_kernel<true><<<grid_for(total / 4, per_sm_vec), kThreads, 0, st>>>(
-                da, a, y, total, c, n, gamma, save_mean, save_rstd, sums, relu, training, dy, dresidual, (__nv_bfloat16 *)dy_bf16);
-        else
-            bn_bwd_apply_kernel<false><<<grid_for(total, per_sm_scalar), kThreads, 0, st>>>(
-                da, a, y, total, c, n, gamma, save_mean, save_rstd, sums, relu, training, dy, dresidual, (__nv_bfloat16 *)dy_bf16);
+        launch_bn_bwd_apply<false>(da, a, y, n, c, gamma, save_mean, save_rstd, sums, nullptr, nullptr, relu, training, dy,
+                                   dresidual, dy_bf16, st);
         TODA_LAUNCH_OK();
     }
+    return TODA_OK;
+}
+
+// ---- BatchNorm over a batch split across processes (torch.nn.SyncBatchNorm): each phase that needs the other ranks'
+// statistics is split at the all-reduce.  Forward: toda_bn_local_sums -> all-reduce SUM -> toda_bn_apply_global.
+// Backward: toda_bn_bwd_reduce -> all-reduce SUM -> toda_bn_bwd_finish.  Given its own local buffers unreduced, each
+// pair computes exactly what the single-process call computes (toda_bn_stats + toda_bn_apply / toda_bn_apply_sums,
+// toda_bn_bwd), bit for bit.
+
+extern "C" int toda_bn_local_sums(const float *y, const double *epilogue_sums, int n, int c, double *local_sums, void *workspace,
+                                  size_t workspace_bytes, void *stream) {
+    TODA_CHECK_ARG(n >= 0 && c > 0 && c <= 256 && local_sums, "bn_local_sums: bad args n=%d c=%d", n, c);
+    cudaStream_t st = (cudaStream_t)stream;
+    const double *partial = nullptr;
+    if (n > 0 && !epilogue_sums) {
+        TODA_CHECK_ARG(y && workspace, "bn_local_sums: null pointer");
+        if (workspace_bytes < bn_ws_bytes(c)) { toda_set_error("bn_local_sums: workspace too small"); return TODA_ERR_WORKSPACE; }
+        launch_col_reduce<0>(y, nullptr, nullptr, n, c, nullptr, nullptr, 0, (double *)workspace, st);
+        TODA_LAUNCH_OK();
+        partial = (const double *)workspace;
+    }
+    bn_local_sums_kernel<<<ceil_div(c * 32, 128), 128, 0, st>>>(partial, kPartials, n > 0 ? epilogue_sums : nullptr, n, c,
+                                                              local_sums);
+    TODA_LAUNCH_OK();
+    return TODA_OK;
+}
+
+extern "C" int toda_bn_apply_global(const float *y, int n, int c, const double *global_sums, const float *gamma, const float *beta,
+                                    float eps, float momentum, float *running_mean, float *running_var, float *scale, float *shift,
+                                    float *save_mean, float *save_rstd, const float *residual, int relu, float *a, void *a_bf16,
+                                    void *stream) {
+    TODA_CHECK_ARG(n >= 0 && c > 0 && c <= 256 && global_sums && scale && shift, "bn_apply_global: bad args");
+    TODA_CHECK_ARG(n == 0 || (y && a), "bn_apply_global: null pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    const long long total = (long long)n * c;
+    static int per_sm_vec = 0, per_sm_scalar = 0;
+    if (!per_sm_vec) {
+        per_sm_vec = resident_grid(bn_apply_global_kernel<true>, (int64_t)1 << 40) / kNumSMs;
+        per_sm_scalar = resident_grid(bn_apply_global_kernel<false>, (int64_t)1 << 40) / kNumSMs;
+    }
+    auto grid_for = [](int64_t items, int per_sm) {
+        int64_t need = (items + kThreads - 1) / kThreads, cap = (int64_t)per_sm * kNumSMs;
+        return (int)(need < 1 ? 1 : (need < cap ? need : cap));
+    };
+    if (c % 4 == 0)
+        bn_apply_global_kernel<true><<<grid_for(total / 4, per_sm_vec), kThreads, 0, st>>>(
+            y, total, c, global_sums, gamma, beta, eps, momentum, running_mean, running_var, scale, shift, save_mean, save_rstd,
+            residual, relu, a, (__nv_bfloat16 *)a_bf16);
+    else
+        bn_apply_global_kernel<false><<<grid_for(total, per_sm_scalar), kThreads, 0, st>>>(
+            y, total, c, global_sums, gamma, beta, eps, momentum, running_mean, running_var, scale, shift, save_mean, save_rstd,
+            residual, relu, a, (__nv_bfloat16 *)a_bf16);
+    TODA_LAUNCH_OK();
+    return TODA_OK;
+}
+
+extern "C" int toda_bn_bwd_reduce(const float *da, const float *a, const float *y, int n, int c, const float *save_mean,
+                                  const float *save_rstd, int relu, double *local_red, float *dgamma, float *dbeta, void *workspace,
+                                  size_t workspace_bytes, void *stream) {
+    TODA_CHECK_ARG(n >= 0 && c > 0 && c <= 256, "bn_bwd_reduce: unsupported sizes n=%d c=%d", n, c);
+    TODA_CHECK_ARG(save_mean && save_rstd && workspace && local_red && (n == 0 || (da && y)) && (!relu || a || n == 0),
+                   "bn_bwd_reduce: null pointer");
+    if (workspace_bytes < bn_ws_bytes(c)) { toda_set_error("bn_bwd_reduce: workspace too small"); return TODA_ERR_WORKSPACE; }
+    cudaStream_t st = (cudaStream_t)stream;
+    double *partial = (double *)workspace;
+    launch_col_reduce<1>(da, a, y, n, c, save_mean, save_rstd, relu, partial, st);
+    TODA_LAUNCH_OK();
+    bn_bwd_finalize_kernel<double><<<ceil_div(c * 32, 128), 128, 0, st>>>(partial, kPartials, c, dgamma, dbeta, local_red);
+    TODA_LAUNCH_OK();
+    return TODA_OK;
+}
+
+extern "C" int toda_bn_bwd_finish(const float *da, const float *a, const float *y, int n, int c, const float *gamma,
+                                  const float *save_mean, const float *save_rstd, int relu, const double *global_red,
+                                  const double *global_count, float *dy, void *dy_bf16, float *dresidual, void *stream) {
+    TODA_CHECK_ARG(n >= 0 && c > 0 && c <= 256, "bn_bwd_finish: unsupported sizes n=%d c=%d", n, c);
+    TODA_CHECK_ARG(save_mean && save_rstd && global_red && global_count && (n == 0 || (da && y && (dy || dy_bf16))) &&
+                   (!relu || a || n == 0), "bn_bwd_finish: null pointer");
+    if (n == 0) return TODA_OK;
+    launch_bn_bwd_apply<true>(da, a, y, n, c, gamma, save_mean, save_rstd, nullptr, global_red, global_count, relu, 1, dy,
+                              dresidual, dy_bf16, (cudaStream_t)stream);
+    TODA_LAUNCH_OK();
     return TODA_OK;
 }
 

@@ -29,30 +29,33 @@ extern "C" int toda_layer_fwd(const toda_layer_fwd_args *p, void *stream) {
     return toda_bn_apply(p->y, n, c, scale, shift, p->residual, p->relu, p->a, p->a_bf16, stream);
 }
 
-extern "C" int toda_layer_bwd(const toda_layer_bwd_args *p, void *stream) {
-    TODA_CHECK_ARG(p, "layer_bwd: null args");
-    const int c = p->cout, n = p->n_out;
-    TODA_CHECK_ARG(c > 0 && n >= 0, "layer_bwd: bad sizes");
-    if (n == 0) {
-        cudaStream_t st = (cudaStream_t)stream;
-        if (p->dgamma) TODA_CUDA_OK(cudaMemsetAsync(p->dgamma, 0, sizeof(float) * c, st));
-        if (p->dbeta) TODA_CUDA_OK(cudaMemsetAsync(p->dbeta, 0, sizeof(float) * c, st));
-        if (p->need_db && p->db) TODA_CUDA_OK(cudaMemsetAsync(p->db, 0, sizeof(float) * c, st));
-        if (p->need_dw && p->dw) TODA_CUDA_OK(cudaMemsetAsync(p->dw, 0, sizeof(float) * (size_t)p->kvol * p->cin * c, st));
-        if (p->need_dx && p->dx && p->n_in > 0) {
-            if (p->addend) TODA_CUDA_OK(cudaMemcpyAsync(p->dx, p->addend, sizeof(float) * (size_t)p->n_in * p->cin, cudaMemcpyDeviceToDevice, st));
-            else TODA_CUDA_OK(cudaMemsetAsync(p->dx, 0, sizeof(float) * (size_t)p->n_in * p->cin, st));
-        }
-        return TODA_OK;
+// Backward of an empty layer: zero parameter gradients (BatchNorm's too when `bn_grads`), dx = the residual-branch addend.
+static int layer_bwd_empty(const toda_layer_bwd_args *p, bool bn_grads, cudaStream_t st) {
+    const int c = p->cout;
+    if (bn_grads && p->dgamma) TODA_CUDA_OK(cudaMemsetAsync(p->dgamma, 0, sizeof(float) * c, st));
+    if (bn_grads && p->dbeta) TODA_CUDA_OK(cudaMemsetAsync(p->dbeta, 0, sizeof(float) * c, st));
+    if (p->need_db && p->db) TODA_CUDA_OK(cudaMemsetAsync(p->db, 0, sizeof(float) * c, st));
+    if (p->need_dw && p->dw) TODA_CUDA_OK(cudaMemsetAsync(p->dw, 0, sizeof(float) * (size_t)p->kvol * p->cin * c, st));
+    if (p->need_dx && p->dx && p->n_in > 0) {
+        if (p->addend) TODA_CUDA_OK(cudaMemcpyAsync(p->dx, p->addend, sizeof(float) * (size_t)p->n_in * p->cin, cudaMemcpyDeviceToDevice, st));
+        else TODA_CUDA_OK(cudaMemsetAsync(p->dx, 0, sizeof(float) * (size_t)p->n_in * p->cin, st));
     }
-    // The fp32 copy of the gradient between BatchNorm and the convolution is only written when something reads it: the
-    // tensor-core dgrad / wgrad take the bf16 copy the same pass writes (4 of ~30 bytes per element of this HBM-bound pass).
-    const bool dy_f32_read = p->need_db || !p->dy_bf16 || p->precision != TODA_CONV_BF16 ||
-                             (p->need_dx && !toda_spconv_uses_tensor_cores(c, p->cin, p->kvol, p->precision)) ||
-                             (p->need_dw && !toda_spconv_wgrad_uses_tensor_cores(p->cin, c, p->kvol, p->precision));
-    int rc = toda_bn_bwd(p->da, p->a_mask, p->y, n, c, p->gamma, p->mean, p->rstd, p->relu, p->training, dy_f32_read ? p->dy : nullptr,
-                         p->dy_bf16, p->dres, p->dgamma, p->dbeta, p->bn_ws, p->bn_ws_bytes, stream);
-    if (rc) return rc;
+    return TODA_OK;
+}
+
+// The fp32 copy of the gradient between BatchNorm and the convolution is only written when something reads it: the
+// tensor-core dgrad / wgrad take the bf16 copy the same pass writes (4 of ~30 bytes per element of this HBM-bound pass).
+static bool layer_bwd_reads_dy_f32(const toda_layer_bwd_args *p) {
+    const int c = p->cout;
+    return p->need_db || !p->dy_bf16 || p->precision != TODA_CONV_BF16 ||
+           (p->need_dx && !toda_spconv_uses_tensor_cores(c, p->cin, p->kvol, p->precision)) ||
+           (p->need_dw && !toda_spconv_wgrad_uses_tensor_cores(p->cin, c, p->kvol, p->precision));
+}
+
+// The convolution's part of the layer backward, from dy: dgrad (+ residual-branch addend), wgrad, bias gradient.
+static int layer_bwd_conv(const toda_layer_bwd_args *p, void *stream) {
+    const int c = p->cout, n = p->n_out;
+    int rc;
     if (p->need_dx) {
         // dgrad = the forward kernel on the input-stationary table with transposed (SubM: mirrored) weights; `addend` is the
         // gradient that reaches the same tensor through the block's residual branch (spconv_backbone.py L63)
@@ -71,4 +74,62 @@ extern "C" int toda_layer_bwd(const toda_layer_bwd_args *p, void *stream) {
         if (rc) return rc;
     }
     return TODA_OK;
+}
+
+extern "C" int toda_layer_bwd(const toda_layer_bwd_args *p, void *stream) {
+    TODA_CHECK_ARG(p, "layer_bwd: null args");
+    const int c = p->cout, n = p->n_out;
+    TODA_CHECK_ARG(c > 0 && n >= 0, "layer_bwd: bad sizes");
+    if (n == 0) return layer_bwd_empty(p, true, (cudaStream_t)stream);
+    int rc = toda_bn_bwd(p->da, p->a_mask, p->y, n, c, p->gamma, p->mean, p->rstd, p->relu, p->training,
+                         layer_bwd_reads_dy_f32(p) ? p->dy : nullptr, p->dy_bf16, p->dres, p->dgamma, p->dbeta, p->bn_ws,
+                         p->bn_ws_bytes, stream);
+    if (rc) return rc;
+    return layer_bwd_conv(p, stream);
+}
+
+// ---- The same layer with its BatchNorm synchronized over several processes (torch.nn.SyncBatchNorm): each direction is
+// split at its all-reduce (include/toda_b200.h).  Training mode only; eval mode needs no exchange and uses the calls above.
+
+extern "C" int toda_layer_fwd_stats(const toda_layer_fwd_args *p, double *local_sums, void *stream) {
+    TODA_CHECK_ARG(p && local_sums, "layer_fwd_stats: null args");
+    const int c = p->cout, n = p->n_out;
+    TODA_CHECK_ARG(c > 0 && n >= 0 && p->training && (n == 0 || p->y), "layer_fwd_stats: bad sizes / not training / null y");
+    // in tensor-core mode the convolution's epilogue accumulates sum(y), sum(y*y) straight into the buffer
+    const bool tc = n > 0 && toda_spconv_uses_tensor_cores(p->cin, c, p->kvol, p->precision);
+    int rc = toda_spconv_fwd_plan(p->x, p->x_bf16, p->n_in, p->cin, p->nbr, n, p->kvol, p->w, c, p->bias, nullptr, p->y, nullptr,
+                                  p->tile_masks, p->plan_lidx, p->plan_rows, p->plan_cnt, p->plan_groups, p->plan_cap,
+                                  tc ? local_sums : nullptr, p->w_bf16, p->precision, p->conv_ws, p->conv_ws_bytes, stream);
+    if (rc) return rc;
+    return toda_bn_local_sums(p->y, tc ? local_sums : nullptr, n, c, local_sums, p->bn_ws, p->bn_ws_bytes, stream);
+}
+
+extern "C" int toda_layer_fwd_apply(const toda_layer_fwd_args *p, const double *global_sums, void *stream) {
+    TODA_CHECK_ARG(p && global_sums, "layer_fwd_apply: null args");
+    const int c = p->cout, n = p->n_out;
+    TODA_CHECK_ARG(c > 0 && n >= 0 && p->training && p->stats && (n == 0 || (p->y && p->a)),
+                   "layer_fwd_apply: bad sizes / not training / null outputs");
+    float *scale = p->stats, *shift = p->stats + c, *mean = p->stats + 2 * c, *rstd = p->stats + 3 * c;
+    return toda_bn_apply_global(p->y, n, c, global_sums, p->gamma, p->beta, p->eps, p->momentum, p->running_mean, p->running_var,
+                                scale, shift, mean, rstd, p->residual, p->relu, p->a, p->a_bf16, stream);
+}
+
+extern "C" int toda_layer_bwd_reduce(const toda_layer_bwd_args *p, double *local_red, void *stream) {
+    TODA_CHECK_ARG(p && local_red, "layer_bwd_reduce: null args");
+    const int c = p->cout, n = p->n_out;
+    TODA_CHECK_ARG(c > 0 && n >= 0 && p->training, "layer_bwd_reduce: bad sizes / not training");
+    return toda_bn_bwd_reduce(p->da, p->a_mask, p->y, n, c, p->mean, p->rstd, p->relu, local_red, p->dgamma, p->dbeta, p->bn_ws,
+                              p->bn_ws_bytes, stream);
+}
+
+extern "C" int toda_layer_bwd_finish(const toda_layer_bwd_args *p, const double *global_red, const double *global_count,
+                                     void *stream) {
+    TODA_CHECK_ARG(p && global_red && global_count, "layer_bwd_finish: null args");
+    const int c = p->cout, n = p->n_out;
+    TODA_CHECK_ARG(c > 0 && n >= 0 && p->training, "layer_bwd_finish: bad sizes / not training");
+    if (n == 0) return layer_bwd_empty(p, false, (cudaStream_t)stream);   // dgamma / dbeta: written by the reduce phase
+    int rc = toda_bn_bwd_finish(p->da, p->a_mask, p->y, n, c, p->gamma, p->mean, p->rstd, p->relu, global_red, global_count,
+                                layer_bwd_reads_dy_f32(p) ? p->dy : nullptr, p->dy_bf16, p->dres, stream);
+    if (rc) return rc;
+    return layer_bwd_conv(p, stream);
 }

@@ -9,6 +9,7 @@ from typing import List, Optional
 
 import numpy as np
 import torch
+import torch.distributed as dist
 
 from . import _C
 
@@ -743,10 +744,111 @@ def set_relu_mask_tape(tape):
     _relu_tape = tape
 
 
+# ------------------------------------------------------------------------------------------------
+# BatchNorm synchronized across processes (torch.nn.SyncBatchNorm)
+# ------------------------------------------------------------------------------------------------
+def sync_group(bn):
+    """The process group over which `bn` reduces its batch statistics in this call, or None for a local BatchNorm.
+    torch.nn.SyncBatchNorm's rule (torch 2.11): a SyncBatchNorm in training mode synchronizes when torch.distributed is
+    initialized and its process_group (None: WORLD) has more than one rank; otherwise it is an ordinary BatchNorm1d."""
+    if not isinstance(bn, torch.nn.SyncBatchNorm) or not bn.training:
+        return None
+    if bn.momentum is None:
+        raise NotImplementedError("toda_b200: SyncBatchNorm with momentum=None (cumulative moving average) is not supported; "
+                                  "set a momentum (these backbones use 0.01)")
+    if not (dist.is_available() and dist.is_initialized()):
+        return None
+    group = bn.process_group if bn.process_group is not None else dist.group.WORLD
+    return group if dist.get_world_size(group) > 1 else None
+
+
+def _run_phases(phases, group):
+    """Drives a phase generator of a synchronized BatchNorm: every buffer it yields is all-reduced (SUM over `group`, in
+    place, on the current stream: NCCL orders it after the local kernels without a host synchronisation) before the
+    generator continues.  Returns the generator's result."""
+    try:
+        buf = next(phases)
+        while True:
+            dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
+            buf = phases.send(None)
+    except StopIteration as stop:
+        return stop.value
+
+
+def _tape_mask(a, want_bf16):
+    """The ReluMaskTape's mask on a pre-activation `a` -> (a, a_bf16, mask as float32)."""
+    if _relu_tape.mode == "record":
+        mask = a > 0
+        _relu_tape.masks.append(mask)
+    else:
+        mask = _relu_tape.masks[_relu_tape.i]
+        _relu_tape.i += 1
+    a = a * mask
+    return a, (a.to(torch.bfloat16) if want_bf16 else None), mask.to(torch.float32)
+
+
+def _bn_forward_phases(y, gamma, beta, running_mean, running_var, eps, momentum, residual, relu, want_bf16, sums):
+    """Phase generator (see _run_phases) of a training-mode BatchNorm synchronized across processes: local sums (from the
+    conv epilogue's `sums` when given), yield them for the all-reduce, apply with the global statistics.
+    -> (a, a_bf16, y, mean, rstd, a_mask, global_sums) as _bn_forward_impl."""
+    y = _need(y.contiguous(), torch.float32, "bn input")
+    n, c = y.shape
+    dev = y.device
+    L = _C.lib()
+    scale, shift, mean, rstd = torch.empty((4, c), dtype=torch.float32, device=dev).unbind(0)
+    gsums = torch.empty((2 * c + 1,), dtype=torch.float64, device=dev)
+    ws = _workspace("bn", L.toda_bn_workspace_bytes(c), dev)
+    with _timed("bn_local_sums", n=n, c=c):
+        _C.check(L.toda_bn_local_sums(_p(y), _p(sums), n, c, _p(gsums), _p(ws), ws.numel(), _stream()), "toda_bn_local_sums")
+    _count(1 if (sums is not None or n == 0) else 2)
+    yield gsums
+    res = residual.contiguous() if residual is not None else None
+    a = torch.empty_like(y)
+    tape = _relu_tape is not None and relu
+    ab = torch.empty(y.shape, dtype=torch.bfloat16, device=dev) if (want_bf16 and not tape) else None
+    with _timed("bn_apply_global", n=n, c=c, residual=res is not None):
+        _C.check(L.toda_bn_apply_global(_p(y), n, c, _p(gsums), _p(gamma), _p(beta), float(eps), float(momentum),
+                                        _p(running_mean), _p(running_var), _p(scale), _p(shift), _p(mean), _p(rstd), _p(res),
+                                        0 if tape else int(relu), _p(a), _p(ab), _stream()), "toda_bn_apply_global")
+    _count(1)
+    if tape:
+        a, ab, mask = _tape_mask(a, want_bf16)
+        return a, ab, y, mean, rstd, mask, gsums
+    return a, ab, y, mean, rstd, a, gsums
+
+
+def _bn_backward_phases(da, y, a, gamma, mean, rstd, relu, has_res, want_bf16, gsums):
+    """Phase generator of the backward of _bn_forward_phases: local sums of g and g*xhat (and this process's dgamma /
+    dbeta), yield them for the all-reduce, dy from the global sums and the forward's global count.  da None = zeros (a
+    rank must join the collective even when no gradient reached it).  -> (dy, dy_bf16, dresidual, dgamma, dbeta)."""
+    n, c = y.shape
+    da = da.contiguous() if da is not None else torch.zeros_like(y)
+    L = _C.lib()
+    dy = torch.empty_like(y)
+    dyb = torch.empty(y.shape, dtype=torch.bfloat16, device=y.device) if want_bf16 else None
+    dres = torch.empty_like(y) if has_res else None
+    dgamma, dbeta = torch.empty((2, c), dtype=torch.float32, device=y.device).unbind(0)
+    red = torch.empty((2 * c,), dtype=torch.float64, device=y.device)
+    ws = _workspace("bn", L.toda_bn_workspace_bytes(c), y.device)
+    with _timed("bn_bwd_reduce", n=n, c=c):
+        _C.check(L.toda_bn_bwd_reduce(_p(da), _p(a), _p(y), n, c, _p(mean), _p(rstd), int(relu), _p(red), _p(dgamma), _p(dbeta),
+                                      _p(ws), ws.numel(), _stream()), "toda_bn_bwd_reduce")
+    _count(2)
+    yield red
+    with _timed("bn_bwd_finish", n=n, c=c, residual=has_res):
+        _C.check(L.toda_bn_bwd_finish(_p(da), _p(a), _p(y), n, c, _p(gamma), _p(mean), _p(rstd), int(relu), _p(red),
+                                      gsums.data_ptr() + 16 * c, _p(dy), _p(dyb), _p(dres), _stream()), "toda_bn_bwd_finish")
+    _count(1 if n > 0 else 0)
+    return dy, dyb, dres, dgamma, dbeta
+
+
 def _bn_forward_impl(y, gamma, beta, running_mean, running_var, eps, momentum, training, residual, relu, want_bf16, sums,
-                     need_grad):
-    """-> (a, a_bf16, y, mean, rstd, a_mask): a_mask is what the backward pass derives the ReLU mask from (`a` itself,
-    except under a ReluMaskTape)."""
+                     need_grad, group=None):
+    """-> (a, a_bf16, y, mean, rstd, a_mask, global_sums): a_mask is what the backward pass derives the ReLU mask from
+    (`a` itself, except under a ReluMaskTape); global_sums is None unless the statistics are synchronized over `group`."""
+    if group is not None:
+        return _run_phases(_bn_forward_phases(y, gamma, beta, running_mean, running_var, eps, momentum, residual, relu,
+                                              want_bf16, sums if training else None), group)
     y = _need(y.contiguous(), torch.float32, "bn input")
     n, c = y.shape
     dev = y.device
@@ -782,25 +884,20 @@ def _bn_forward_impl(y, gamma, beta, running_mean, running_var, eps, momentum, t
         # pre-activation z, then the recorded / replayed mask (test instrument, see ReluMaskTape)
         _C.check(L.toda_bn_apply(_p(y), n, c, _p(scale), _p(shift), _p(res), 0, _p(a), None, _stream()), "toda_bn_apply")
         _count(1)
-        if _relu_tape.mode == "record":
-            mask = a > 0
-            _relu_tape.masks.append(mask)
-        else:
-            mask = _relu_tape.masks[_relu_tape.i]
-            _relu_tape.i += 1
-        a = a * mask
-        if want_bf16:
-            ab = a.to(torch.bfloat16)
-        return a, ab, y, mean, rstd, mask.to(torch.float32)
+        a, ab, mask = _tape_mask(a, want_bf16)
+        return a, ab, y, mean, rstd, mask, None
     with _timed("bn_apply", n=n, c=c, residual=res is not None):
         _C.check(L.toda_bn_apply(_p(y), n, c, _p(scale), _p(shift), _p(res), int(relu), _p(a), _p(ab), _stream()),
                  "toda_bn_apply")
     _count(1)
-    return a, ab, y, mean, rstd, a
+    return a, ab, y, mean, rstd, a, None
 
 
-def _bn_backward_impl(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16):
-    """-> (dy, dy_bf16, dresidual, dgamma, dbeta)"""
+def _bn_backward_impl(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16, group=None, gsums=None):
+    """-> (dy, dy_bf16, dresidual, dgamma, dbeta).  group / gsums: the process group and the forward's global sums of a
+    synchronized BatchNorm (then da may be None)."""
+    if group is not None:
+        return _run_phases(_bn_backward_phases(da, y, a, gamma, mean, rstd, relu, has_res, want_bf16, gsums), group)
     n, c = y.shape
     da = da.contiguous()
     L = _C.lib()
@@ -820,26 +917,29 @@ def _bn_backward_impl(da, y, a, gamma, mean, rstd, training, relu, has_res, want
 
 class _BNAct(torch.autograd.Function):
     @staticmethod
-    def forward(ctx, y, gamma, beta, running_mean, running_var, eps, momentum, training, residual, relu, want_bf16, sums):
-        a, ab, y, mean, rstd, a_mask = _bn_forward_impl(y, gamma, beta, running_mean, running_var, eps, momentum, training,
-                                                        residual, relu, want_bf16, sums, y.requires_grad or gamma.requires_grad)
-        ctx.save_for_backward(y, a_mask, gamma, mean, rstd)
+    def forward(ctx, y, gamma, beta, running_mean, running_var, eps, momentum, training, residual, relu, want_bf16, sums, group):
+        a, ab, y, mean, rstd, a_mask, gsums = _bn_forward_impl(y, gamma, beta, running_mean, running_var, eps, momentum,
+                                                               training, residual, relu, want_bf16, sums,
+                                                               y.requires_grad or gamma.requires_grad, group)
+        ctx.save_for_backward(y, a_mask, gamma, mean, rstd, gsums)
         ctx.set_materialize_grads(False)      # the bf16 copy is non-differentiable: no zero tensor for it in backward
         ctx.cfg = (bool(training), bool(relu), residual is not None, bool(want_bf16))
+        ctx.group = group
         if ab is not None:
             ctx.mark_non_differentiable(ab)
         return a, ab
 
     @staticmethod
     def backward(ctx, da, _dab=None):
-        if da is None:
-            return (None,) * 12
-        y, a, gamma, mean, rstd = ctx.saved_tensors
+        if da is None and ctx.group is None:      # a synchronized BatchNorm still joins its peers' collective
+            return (None,) * 13
+        y, a, gamma, mean, rstd, gsums = ctx.saved_tensors
         training, relu, has_res, want_bf16 = ctx.cfg
-        dy, dyb, dres, dgamma, dbeta = _bn_backward_impl(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16)
+        dy, dyb, dres, dgamma, dbeta = _bn_backward_impl(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16,
+                                                         ctx.group, gsums)
         if dyb is not None:
             dy._toda_bf16 = (dyb, dy._version)     # picked up by the producing conv's backward (see _bf16_shadow_of)
-        return dy, dgamma, dbeta, None, None, None, None, None, dres, None, None, None
+        return dy, dgamma, dbeta, None, None, None, None, None, dres, None, None, None, None
 
 
 def _vp(t):
@@ -853,13 +953,55 @@ def _fused_ok(training, need_grad):
 
 
 def _layer_forward(x, x_bf16, weight, bias, rb, precision, gamma, beta, running_mean, running_var, eps, momentum, training,
-                   residual, relu, want_bf16, need_grad=True):
-    """conv -> BN (+residual) (+ReLU).  -> (a, a_bf16, saved) with saved = (x, x_bf16, weight, y, a_mask, gamma, mean, rstd)."""
+                   residual, relu, want_bf16, need_grad=True, group=None):
+    """conv -> BN (+residual) (+ReLU).  -> (a, a_bf16, saved) with saved = (x, x_bf16, weight, y, a_mask, gamma, mean, rstd,
+    global_sums).  group: the process group of a synchronized BatchNorm (sync_group), else None (global_sums is then None)."""
+    if group is not None:
+        return _run_phases(_layer_forward_phases(x, x_bf16, weight, bias, rb, precision, gamma, beta, running_mean, running_var,
+                                                 eps, momentum, residual, relu, want_bf16, need_grad), group)
     if not _fused_ok(training, need_grad):
         y, sums, x, weight, x_bf16 = _conv_forward_impl(x, x_bf16, weight, bias, rb, precision, bool(training))
-        a, ab, y, mean, rstd, a_mask = _bn_forward_impl(y, gamma, beta, running_mean, running_var, eps, momentum, training,
-                                                        residual, relu, want_bf16, sums, need_grad)
-        return a, ab, (x, x_bf16, weight, y, a_mask, gamma, mean, rstd)
+        a, ab, y, mean, rstd, a_mask, _ = _bn_forward_impl(y, gamma, beta, running_mean, running_var, eps, momentum, training,
+                                                           residual, relu, want_bf16, sums, need_grad)
+        return a, ab, (x, x_bf16, weight, y, a_mask, gamma, mean, rstd, None)
+    args, tc, x, x_bf16, weight, y, a, ab, small, _keep = _layer_fwd_args(
+        x, x_bf16, weight, bias, rb, precision, gamma, beta, running_mean, running_var, eps, momentum, training, residual, relu,
+        want_bf16)
+    cout, n_out = y.shape[1], y.shape[0]
+    _C.check(_C.lib().toda_layer_fwd(ctypes.byref(args), _stream()), "toda_layer_fwd")
+    _count(2 if (tc and training and n_out > 0) else (3 if tc else 4))
+    mean = small[2 * cout:3 * cout] if training else running_mean
+    rstd = small[3 * cout:4 * cout] if training else None
+    return a, ab, (x, x_bf16, weight, y, a, gamma, mean, rstd, None)
+
+
+def _layer_forward_phases(x, x_bf16, weight, bias, rb, precision, gamma, beta, running_mean, running_var, eps, momentum,
+                          residual, relu, want_bf16, need_grad=True):
+    """Phase generator (see _run_phases) of _layer_forward in training mode with a synchronized BatchNorm:
+    toda_layer_fwd_stats, yield the local sums (double[2C+1]) for the all-reduce, toda_layer_fwd_apply."""
+    if not _fused_ok(True, need_grad):
+        y, sums, x, weight, x_bf16 = _conv_forward_impl(x, x_bf16, weight, bias, rb, precision, True)
+        a, ab, y, mean, rstd, a_mask, gsums = yield from _bn_forward_phases(y, gamma, beta, running_mean, running_var, eps,
+                                                                            momentum, residual, relu, want_bf16, sums)
+        return a, ab, (x, x_bf16, weight, y, a_mask, gamma, mean, rstd, gsums)
+    args, tc, x, x_bf16, weight, y, a, ab, small, _keep = _layer_fwd_args(
+        x, x_bf16, weight, bias, rb, precision, gamma, beta, running_mean, running_var, eps, momentum, True, residual, relu,
+        want_bf16)
+    n_out, cout = y.shape
+    L = _C.lib()
+    gsums = torch.empty((2 * cout + 1,), dtype=torch.float64, device=y.device)
+    _C.check(L.toda_layer_fwd_stats(ctypes.byref(args), _p(gsums), _stream()), "toda_layer_fwd_stats")
+    _count(2 if tc else (1 if n_out == 0 else 3))
+    yield gsums
+    _C.check(L.toda_layer_fwd_apply(ctypes.byref(args), _p(gsums), _stream()), "toda_layer_fwd_apply")
+    _count(1)
+    return a, ab, (x, x_bf16, weight, y, a, gamma, small[2 * cout:3 * cout], small[3 * cout:4 * cout], gsums)
+
+
+def _layer_fwd_args(x, x_bf16, weight, bias, rb, precision, gamma, beta, running_mean, running_var, eps, momentum, training,
+                    residual, relu, want_bf16):
+    """Outputs and toda_layer_fwd_args of one fused layer -> (args, tc, x, x_bf16, weight, y, a, a_bf16, small, keep); keep
+    holds the other tensors the args point to: all of them must stay alive until the layer's calls are enqueued."""
     x = _need(x.contiguous(), torch.float32, "features")
     weight = _need(weight.contiguous(), torch.float32, "weight")
     cout, cin = weight.shape[0], weight.shape[4]
@@ -891,16 +1033,16 @@ def _layer_forward(x, x_bf16, weight, bias, rb, precision, gamma, beta, running_
         pl.ngroups if pl else 0, pl.cap if pl else 0, precision, _vp(ws), ws.numel() if ws is not None else 0,
         gamma.data_ptr(), beta.data_ptr(), float(eps), float(momentum), _vp(running_mean), _vp(running_var), int(bool(training)),
         _vp(res), int(bool(relu)), y.data_ptr(), sp + 16 * cout, sp, a.data_ptr(), _vp(ab), bws.data_ptr(), bws.numel())
-    _C.check(L.toda_layer_fwd(ctypes.byref(args), _stream()), "toda_layer_fwd")
-    _count(2 if (tc and training and n_out > 0) else (3 if tc else 4))
-    mean = small[2 * cout:3 * cout] if training else running_mean
-    rstd = small[3 * cout:4 * cout] if training else None
-    return a, ab, (x, x_bf16, weight, y, a, gamma, mean, rstd)
+    return args, tc, x, x_bf16, weight, y, a, ab, small, (w, wb, ws, bws, res, b)
 
 
-def _layer_backward(da, saved, rb, precision, training, relu, has_res, has_bias, need_dx, need_dw, addend=None):
-    """-> (dx, dw, db, dgamma, dbeta, dres).  addend: a gradient to be ADDED to dx (fused into the dgrad epilogue)."""
-    x, xb, weight, y, a_mask, gamma, mean, rstd = saved
+def _layer_backward(da, saved, rb, precision, training, relu, has_res, has_bias, need_dx, need_dw, addend=None, group=None):
+    """-> (dx, dw, db, dgamma, dbeta, dres).  addend: a gradient to be ADDED to dx (fused into the dgrad epilogue).
+    group: the process group of a synchronized BatchNorm (then da may be None: zeros)."""
+    if group is not None:
+        return _run_phases(_layer_backward_phases(da, saved, rb, precision, relu, has_res, has_bias, need_dx, need_dw, addend),
+                           group)
+    x, xb, weight, y, a_mask, gamma, mean, rstd, _ = saved
     if not _fused_ok(training, True):
         dy, dyb, dres, dgamma, dbeta = _bn_backward_impl(da, y, a_mask, gamma, mean, rstd, training, relu, has_res,
                                                          precision == CONV_BF16)
@@ -908,6 +1050,46 @@ def _layer_backward(da, saved, rb, precision, training, relu, has_res, has_bias,
         if addend is not None and dx is not None:
             dx = dx + addend
         return dx, dw, db, dgamma, dbeta, dres
+    args, dx, dw, dres, small, _keep = _layer_bwd_args(da, saved, rb, precision, training, relu, has_res, has_bias, need_dx,
+                                                       need_dw, addend)
+    cout = y.shape[1]
+    _C.check(_C.lib().toda_layer_bwd(ctypes.byref(args), _stream()), "toda_layer_bwd")
+    _count(3 + (1 if need_dx else 0) + (2 if need_dw else 0) + (2 if has_bias else 0))
+    return dx, dw, (small[2 * cout:] if has_bias else None), small[:cout], small[cout:2 * cout], dres
+
+
+def _layer_backward_phases(da, saved, rb, precision, relu, has_res, has_bias, need_dx, need_dw, addend=None):
+    """Phase generator of _layer_backward with a synchronized BatchNorm: toda_layer_bwd_reduce, yield the local sums of g
+    and g*xhat (double[2C]) for the all-reduce, toda_layer_bwd_finish with the forward's global count.  dgamma / dbeta
+    are this process's own (as torch.nn.SyncBatchNorm's; the gradient all-reduce averages them)."""
+    x, xb, weight, y, a_mask, gamma, mean, rstd, gsums = saved
+    if da is None:
+        da = torch.zeros_like(y)
+    if not _fused_ok(True, True):
+        dy, dyb, dres, dgamma, dbeta = yield from _bn_backward_phases(da, y, a_mask, gamma, mean, rstd, relu, has_res,
+                                                                      precision == CONV_BF16, gsums)
+        dx, dw, db = _conv_backward_impl(dy, dyb, x, weight, xb, rb, precision, need_dx, need_dw, has_bias)
+        if addend is not None and dx is not None:
+            dx = dx + addend
+        return dx, dw, db, dgamma, dbeta, dres
+    args, dx, dw, dres, small, _keep = _layer_bwd_args(da, saved, rb, precision, True, relu, has_res, has_bias, need_dx,
+                                                       need_dw, addend)
+    cout = y.shape[1]
+    L = _C.lib()
+    red = torch.empty((2 * cout,), dtype=torch.float64, device=y.device)
+    _C.check(L.toda_layer_bwd_reduce(ctypes.byref(args), _p(red), _stream()), "toda_layer_bwd_reduce")
+    _count(2)
+    yield red
+    _C.check(L.toda_layer_bwd_finish(ctypes.byref(args), _p(red), gsums.data_ptr() + 16 * cout, _stream()),
+             "toda_layer_bwd_finish")
+    _count(1 + (1 if need_dx else 0) + (2 if need_dw else 0) + (2 if has_bias else 0))
+    return dx, dw, (small[2 * cout:] if has_bias else None), small[:cout], small[cout:2 * cout], dres
+
+
+def _layer_bwd_args(da, saved, rb, precision, training, relu, has_res, has_bias, need_dx, need_dw, addend):
+    """Outputs and toda_layer_bwd_args of one fused layer's backward -> (args, dx, dw, dres, small, keep): small = dgamma,
+    dbeta, dbias; keep holds the other tensors the args point to."""
+    x, xb, weight, y, a_mask, gamma, mean, rstd, _ = saved
     L = _C.lib()
     da = da.contiguous()
     n_out, cout = y.shape
@@ -954,9 +1136,7 @@ def _layer_backward(da, saved, rb, precision, training, relu, has_res, has_bias,
         pl.cap if pl else 0, _vp(addend) if need_dx else None, _vp(dx),
         int(bool(need_dw)), rb.nbr_fwd.data_ptr(), _vp(dw), _vp(wws), wws.numel() if wws is not None else 0,
         int(bool(has_bias)), sp + 8 * cout, precision, _vp(ws), ws.numel() if ws is not None else 0)
-    _C.check(L.toda_layer_bwd(ctypes.byref(args), _stream()), "toda_layer_bwd")
-    _count(3 + (1 if need_dx else 0) + (2 if need_dw else 0) + (2 if has_bias else 0))
-    return dx, dw, (small[2 * cout:] if has_bias else None), small[:cout], small[cout:2 * cout], dres
+    return args, dx, dw, dres, small, (da, dy, dyb, addend, wt, wtb, ws, wws, bws)
 
 
 class _ConvBNAct(torch.autograd.Function):
@@ -965,14 +1145,14 @@ class _ConvBNAct(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, x, x_bf16, weight, bias, rb, precision, gamma, beta, running_mean, running_var, eps, momentum, training,
-                residual, relu, want_bf16):
+                residual, relu, want_bf16, group):
         need_grad = any(ctx.needs_input_grad)
         a, ab, saved = _layer_forward(x, x_bf16, weight, bias, rb, precision, gamma, beta, running_mean, running_var, eps, momentum,
-                                      training, residual, relu, want_bf16, need_grad)
+                                      training, residual, relu, want_bf16, need_grad, group)
         if need_grad:
             ctx.save_for_backward(*saved)
         ctx.set_materialize_grads(False)
-        ctx.rb, ctx.precision, ctx.has_bias = rb, precision, bias is not None
+        ctx.rb, ctx.precision, ctx.has_bias, ctx.group = rb, precision, bias is not None, group
         ctx.cfg = (bool(training), bool(relu), residual is not None, bool(want_bf16))
         if ab is not None:
             ctx.mark_non_differentiable(ab)
@@ -980,13 +1160,13 @@ class _ConvBNAct(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, da, _dab=None):
-        if da is None:
-            return (None,) * 16
+        if da is None and ctx.group is None:      # a synchronized BatchNorm still joins its peers' collective
+            return (None,) * 17
         training, relu, has_res, want_bf16 = ctx.cfg
         dx, dw, db, dgamma, dbeta, dres = _layer_backward(da, ctx.saved_tensors, ctx.rb, ctx.precision, training, relu, has_res,
                                                           ctx.has_bias and ctx.needs_input_grad[3], ctx.needs_input_grad[0],
-                                                          ctx.needs_input_grad[2])
-        return dx, None, dw, db, None, None, dgamma, dbeta, None, None, None, None, None, dres, None, None
+                                                          ctx.needs_input_grad[2], group=ctx.group)
+        return dx, None, dw, db, None, None, dgamma, dbeta, None, None, None, None, None, dres, None, None, None
 
 
 class _ResBlock(torch.autograd.Function):
@@ -995,16 +1175,18 @@ class _ResBlock(torch.autograd.Function):
     no autograd accumulation of the two branches)."""
 
     @staticmethod
-    def forward(ctx, x, x_bf16, w1, b1, g1, be1, rm1, rv1, w2, b2, g2, be2, rm2, rv2, rb, precision, eps, momentum, training, want_bf16):
+    def forward(ctx, x, x_bf16, w1, b1, g1, be1, rm1, rv1, w2, b2, g2, be2, rm2, rv2, rb, precision, eps, momentum, training, want_bf16,
+                group1, group2):
         need_grad = any(ctx.needs_input_grad)
         h, hb, s1 = _layer_forward(x, x_bf16, w1, b1, rb, precision, g1, be1, rm1, rv1, eps, momentum, training, None, True,
-                                   want_bf16, need_grad)
+                                   want_bf16, need_grad, group1)
         out, outb, s2 = _layer_forward(h, hb, w2, b2, rb, precision, g2, be2, rm2, rv2, eps, momentum, training, s1[0], True,
-                                       want_bf16, need_grad)
+                                       want_bf16, need_grad, group2)
         if need_grad:
             ctx.save_for_backward(*s1, *s2)
         ctx.set_materialize_grads(False)
         ctx.rb, ctx.precision, ctx.training = rb, precision, bool(training)
+        ctx.groups = (group1, group2)
         ctx.has_bias = (b1 is not None, b2 is not None)
         if outb is not None:
             ctx.mark_non_differentiable(outb)
@@ -1012,20 +1194,24 @@ class _ResBlock(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, dout, _db=None):
-        if dout is None:
-            return (None,) * 20
+        if dout is None and ctx.groups == (None, None):      # a synchronized BatchNorm still joins its peers' collectives
+            return (None,) * 22
         sv = ctx.saved_tensors
-        s1, s2 = sv[:8], sv[8:]
+        s1, s2 = sv[:9], sv[9:]
         ng = ctx.needs_input_grad
         dh, dw2, db2, dg2, dbe2, dres = _layer_backward(dout, s2, ctx.rb, ctx.precision, ctx.training, True, True,
-                                                        ctx.has_bias[1] and ng[9], True, ng[8])
+                                                        ctx.has_bias[1] and ng[9], True, ng[8], group=ctx.groups[1])
         dx, dw1, db1, dg1, dbe1, _ = _layer_backward(dh, s1, ctx.rb, ctx.precision, ctx.training, True, False,
-                                                     ctx.has_bias[0] and ng[3], ng[0], ng[2], addend=dres if ng[0] else None)
-        return (dx, None, dw1, db1, dg1, dbe1, None, None, dw2, db2, dg2, dbe2, None, None, None, None, None, None, None, None)
+                                                     ctx.has_bias[0] and ng[3], ng[0], ng[2], addend=dres if ng[0] else None,
+                                                     group=ctx.groups[0])
+        return (dx, None, dw1, db1, dg1, dbe1, None, None, dw2, db2, dg2, dbe2, None, None, None, None, None, None, None, None,
+                None, None)
 
 
 def res_block(x, x_bf16, conv1_w, conv1_b, bn1, conv2_w, conv2_b, bn2, rb, precision, want_bf16=False):
-    """SparseBasicBlock on feature rows; bn1 / bn2 are the nn.BatchNorm1d modules.  -> (out, out_bf16 or None)"""
+    """SparseBasicBlock on feature rows; bn1 / bn2 are the nn.BatchNorm1d (or nn.SyncBatchNorm) modules.
+    -> (out, out_bf16 or None)"""
+    group1, group2 = sync_group(bn1), sync_group(bn2)
     training = bn1.training or bn1.running_mean is None
     if training:
         for bn in (bn1, bn2):
@@ -1034,27 +1220,31 @@ def res_block(x, x_bf16, conv1_w, conv1_b, bn1, conv2_w, conv2_b, bn2, rb, preci
     assert bn1.eps == bn2.eps and bn1.momentum == bn2.momentum
     return _ResBlock.apply(x, x_bf16, conv1_w, conv1_b, bn1.weight, bn1.bias, bn1.running_mean, bn1.running_var, conv2_w, conv2_b,
                            bn2.weight, bn2.bias, bn2.running_mean, bn2.running_var, rb, precision, bn1.eps, bn1.momentum, training,
-                           want_bf16)
+                           want_bf16, group1, group2)
 
 
 def conv_bn_act(x, weight, bias, rb, precision, bn: torch.nn.BatchNorm1d, residual=None, relu=True, x_bf16=None, want_bf16=False):
-    """Fused-node version of bn_act(sparse_conv(x, ...), bn, residual, relu).  -> (a, a_bf16 or None)"""
+    """Fused-node version of bn_act(sparse_conv(x, ...), bn, residual, relu).  -> (a, a_bf16 or None).  An nn.SyncBatchNorm
+    in training mode reduces its statistics over its process group (sync_group)."""
+    group = sync_group(bn)
     training = bn.training or bn.running_mean is None
     if training and bn.running_mean is not None and bn.num_batches_tracked is not None:
         bn.num_batches_tracked += 1
     return _ConvBNAct.apply(x, x_bf16, weight, bias, rb, precision, bn.weight, bn.bias, bn.running_mean, bn.running_var, bn.eps,
-                            bn.momentum, training, residual, relu, want_bf16)
+                            bn.momentum, training, residual, relu, want_bf16, group)
 
 
 def bn_act(y, bn: torch.nn.BatchNorm1d, residual=None, relu=True, want_bf16=False, sums=None):
     """BatchNorm1d (+ residual) (+ ReLU) with the module's parameters / running stats
     (spconv_backbone.py L23-24, L54-64).  want_bf16: also return the bf16 copy written by the same pass.
-    sums: per-channel (sum, sum of squares) of y from the producing convolution's epilogue (skips the statistics pass)."""
+    sums: per-channel (sum, sum of squares) of y from the producing convolution's epilogue (skips the statistics pass).
+    An nn.SyncBatchNorm in training mode reduces its statistics over its process group (sync_group)."""
+    group = sync_group(bn)
     training = bn.training or bn.running_mean is None
     if training and bn.running_mean is not None and bn.num_batches_tracked is not None:
         bn.num_batches_tracked += 1
     a, ab = _BNAct.apply(y, bn.weight, bn.bias, bn.running_mean, bn.running_var, bn.eps, bn.momentum, training, residual,
-                         relu, want_bf16, sums if training else None)
+                         relu, want_bf16, sums if training else None, group)
     return (a, ab) if want_bf16 else a
 
 

@@ -20,6 +20,8 @@ import torch.nn as nn
 from .. import ops
 
 _precision = ops.CONV_FP32
+# BatchNorm modules SparseSequential runs on libtoda_b200 (nn.SyncBatchNorm: what convert_sync_batchnorm makes of the former)
+_FUSED_BN = (nn.BatchNorm1d, nn.SyncBatchNorm)
 
 
 def set_conv_precision(p):
@@ -162,9 +164,9 @@ class SparseSequential(SparseModule):
         while i < len(mods):
             m = mods[i]
             if (isinstance(m, SparseConvolution) and isinstance(x, SparseConvTensor) and i + 1 < len(mods)
-                    and type(mods[i + 1]) is nn.BatchNorm1d and mods[i + 1].affine and mods[i + 1].track_running_stats
+                    and type(mods[i + 1]) in _FUSED_BN and mods[i + 1].affine and mods[i + 1].track_running_stats
                     and x.features.is_cuda and x.indices.shape[0] > 0):
-                # conv + BatchNorm1d [+ ReLU]: one fused autograd node
+                # conv + BatchNorm1d / SyncBatchNorm [+ ReLU]: one fused autograd node
                 relu = i + 2 < len(mods) and type(mods[i + 2]) is nn.ReLU
                 x = conv_bn_act_tensor(x, m, mods[i + 1], None, relu)
                 i += 3 if relu else 2
@@ -172,6 +174,13 @@ class SparseSequential(SparseModule):
                 x = m(x)
                 i += 1
             elif isinstance(x, SparseConvTensor):
+                if x.indices.shape[0] == 0 and ops.sync_group(m) is not None and x.features.is_cuda:
+                    # a synchronized BatchNorm on an empty tensor: this rank joins its peers' collectives (forward and
+                    # backward) with a zero contribution, and takes the running statistics of the union batch
+                    relu = i + 1 < len(mods) and type(mods[i + 1]) is nn.ReLU
+                    x = bn_act_tensor(x, m, None, relu)
+                    i += 2 if relu else 1
+                    continue
                 if x.indices.shape[0] == 0:
                     # spconv skips the feature modules on an empty tensor; a training BatchNorm1d still counts the batch
                     # (torch.nn.BatchNorm1d on zero rows: running statistics unchanged, num_batches_tracked + 1)
@@ -179,8 +188,8 @@ class SparseSequential(SparseModule):
                         m.num_batches_tracked += 1
                     i += 1
                     continue
-                # BatchNorm1d [+ ReLU] after a conv: one fused pass of libtoda_b200 instead of ATen's
-                if type(m) is nn.BatchNorm1d and m.affine and m.track_running_stats and x.features.is_cuda:
+                # BatchNorm1d / SyncBatchNorm [+ ReLU] after a conv: one fused pass of libtoda_b200 instead of ATen's
+                if type(m) in _FUSED_BN and m.affine and m.track_running_stats and x.features.is_cuda:
                     relu = i + 1 < len(mods) and type(mods[i + 1]) is nn.ReLU
                     x = bn_act_tensor(x, m, None, relu)
                     i += 2 if relu else 1
