@@ -179,7 +179,7 @@ size_t toda_spconv_fwd_workspace_bytes(int n_in, int cin, int cout, int kvol, in
 /* x_bf16 / dy_bf16 (optional, may be NULL): an existing bf16 copy of x / dy ([rows][channels], same values rounded to
  * nearest) that the TODA_CONV_BF16 kernels use instead of converting x / dy themselves. */
 /* bn_sums (optional, may be NULL; tensor-core kernel only, see toda_spconv_uses_tensor_cores): double[2*cout] receiving
- * sum(y) and sum(y*y) per output channel, accumulated in the epilogue, for toda_bn_finalize_sums -- the BatchNorm that
+ * sum(y) and sum(y*y) per output channel, accumulated in the epilogue, for toda_bn_apply_sums -- the BatchNorm that
  * follows the convolution (spconv_backbone.py L23-24) then needs no statistics pass over y. */
 /* out_rows (optional, may be NULL): int32[n_out]; output row o of this call is written to y[out_rows[o], :] instead of
  * y[o, :].  Used by the dgrad of strided convolutions: with stride s only the offsets k = (in + pad) mod s (per axis) can
@@ -226,59 +226,50 @@ int toda_spconv_wgrad(const float *x, const void *x_bf16, int n_in, int cin, con
 /* ------------------------------------------------------------------------------------------
  * K8 BatchNorm1d(eps, momentum) + ReLU (+ residual) over (N_active, C) rows
  * (spconv_backbone.py L23-24, L54-64, L73/L187).
- *   stats : per-channel mean / biased var of y -> scale = gamma*rstd, shift = beta - mean*scale,
- *           save_mean, save_rstd, running stats update (unbiased var, momentum).  An empty batch (n = 0) leaves the
- *           running stats unchanged, as torch.nn.BatchNorm1d does.
- *   apply : a = act(y*scale + shift (+ residual)).
- *   bwd   : g = da * (a>0 if relu); dgamma = sum g*xhat; dbeta = sum g;
- *           dy = scale*(g - dbeta/N - xhat*dgamma/N); dresidual = g.
+ *   training: fp64 sums of y (sum(y) | sum(y*y) per channel), all-reduced across processes when the BatchNorm is
+ *             synchronized (torch.nn.SyncBatchNorm), then one apply pass that derives from them scale = gamma*rstd,
+ *             shift = beta - mean*scale, save_mean, save_rstd and the running stats update (unbiased var, momentum).
+ *             An empty batch (count 0) leaves the running stats unchanged, as torch.nn.BatchNorm1d does.
+ *   eval    : scale / shift from the running stats (toda_bn_eval_coeffs), then the same apply pass (toda_bn_apply).
+ *   apply   : a = act(y*scale + shift (+ residual)).
+ *   bwd     : g = da * (a>0 if relu); dgamma = sum g*xhat; dbeta = sum g;
+ *             dy = scale*(g - dbeta/N - xhat*dgamma/N); dresidual = g.
+ * Each phase that needs the other processes' statistics is split at the all-reduce (SUM, done by the caller):
+ *   forward : toda_bn_local_sums -> all-reduce sums (+ count) -> toda_bn_apply_sums
+ *   backward: toda_bn_bwd_reduce -> all-reduce red            -> toda_bn_bwd_finish
+ * A single process passes its own buffers through and the row count n (count = NULL); toda_bn_bwd is its backward in
+ * one call.  A process of a synchronized BatchNorm with no rows still makes every call.
  * ------------------------------------------------------------------------------------------ */
 size_t toda_bn_workspace_bytes(int channels);
-int toda_bn_stats(const float *y, int n, int channels, const float *gamma, const float *beta, float eps,
-                  float momentum, float *running_mean, float *running_var, float *scale, float *shift,
-                  float *save_mean, float *save_rstd, void *workspace, size_t workspace_bytes, void *stream);
-int toda_bn_finalize_sums(const double *sums, int n, int channels, const float *gamma, const float *beta, float eps,
-                          float momentum, float *running_mean, float *running_var, float *scale, float *shift,
-                          float *save_mean, float *save_rstd, void *stream);
+/* sums: double[2*channels] = sum(y) | sum(y*y) per channel, from the per-CTA fixed-order partials of y, or from the
+ * convolution epilogue's `epilogue_sums` (optional; y is then not read, and it may be `sums` itself).  count (optional):
+ * receives the row count, written on the device (&sums[2*channels] when the count is all-reduced with the sums). */
+int toda_bn_local_sums(const float *y, const double *epilogue_sums, int n, int channels, double *sums, double *count,
+                       void *workspace, size_t workspace_bytes, void *stream);
 int toda_bn_eval_coeffs(const float *gamma, const float *beta, const float *running_mean, const float *running_var,
                         float eps, int channels, float *scale, float *shift, void *stream);
 /* a_bf16 / dy_bf16 (optional, may be NULL): bf16 copies written by the same pass, consumed as tensor-core operands. */
 int toda_bn_apply(const float *y, int n, int channels, const float *scale, const float *shift, const float *residual,
                   int relu, float *a, void *a_bf16, void *stream);
-/* finalize_sums + apply in ONE launch (training mode, statistics from the convolution's epilogue): every thread derives the
- * coefficients of its four channels from `sums`; scale / shift / save_mean / save_rstd are still written for the backward
- * pass and the running statistics updated.  Same results, bit for bit, as the two calls it replaces. */
-int toda_bn_apply_sums(const float *y, int n, int channels, const double *sums, const float *gamma, const float *beta,
-                       float eps, float momentum, float *running_mean, float *running_var, float *scale, float *shift,
-                       float *save_mean, float *save_rstd, const float *residual, int relu, float *a, void *a_bf16,
-                       void *stream);
+/* Training-mode apply: coefficients, save_mean / save_rstd and the running statistics from `sums` (toda_bn_local_sums'
+ * layout, all-reduced or not) and the row count *count (the global count of a synchronized BatchNorm) or n when count is
+ * NULL, applied in the same launch; scale / shift are written for the backward pass. */
+int toda_bn_apply_sums(const float *y, int n, int channels, const double *sums, const double *count, const float *gamma,
+                       const float *beta, float eps, float momentum, float *running_mean, float *running_var, float *scale,
+                       float *shift, float *save_mean, float *save_rstd, const float *residual, int relu, float *a,
+                       void *a_bf16, void *stream);
+/* red: double[2*channels] = sum g | sum g*xhat (g = da after the ReLU mask); dgamma / dbeta are this process's own sums
+ * (torch leaves their averaging to the gradient all-reduce).  count: as in toda_bn_apply_sums (the forward's).  training
+ * = 0 (eval-mode gradient): dy = scale*g, red is not read. */
+int toda_bn_bwd_reduce(const float *da, const float *a, const float *y, int n, int channels, const float *save_mean,
+                       const float *save_rstd, int relu, double *red, float *dgamma, float *dbeta, void *workspace,
+                       size_t workspace_bytes, void *stream);
+int toda_bn_bwd_finish(const float *da, const float *a, const float *y, int n, int channels, const float *gamma,
+                       const float *save_mean, const float *save_rstd, int relu, int training, const double *red,
+                       const double *count, float *dy, void *dy_bf16, float *dresidual, void *stream);
 int toda_bn_bwd(const float *da, const float *a, const float *y, int n, int channels, const float *gamma,
                 const float *save_mean, const float *save_rstd, int relu, int training, float *dy, void *dy_bf16,
                 float *dresidual, float *dgamma, float *dbeta, void *workspace, size_t workspace_bytes, void *stream);
-/* BatchNorm over a batch split across processes (torch.nn.SyncBatchNorm, training mode): each statistic that needs the
- * other ranks is produced locally, all-reduced (SUM) by the caller, and consumed by a second call.
- *   forward : toda_bn_local_sums -> all-reduce local_sums -> toda_bn_apply_global
- *   backward: toda_bn_bwd_reduce -> all-reduce local_red  -> toda_bn_bwd_finish
- * local_sums / global_sums: double[2*channels+1] = sum(y) per channel | sum(y*y) per channel | row count; the count is
- * written on the device.  epilogue_sums (optional): the convolution epilogue's double[2*channels] sums of y (then y is not
- * read; it may be local_sums itself).  global_sums gives mean, biased variance (coefficients, save_mean / save_rstd) and
- * the running statistics' update (unbiased variance, global count; unchanged when the global count is 0).
- * local_red / global_red: double[2*channels] = sum g | sum g*xhat (g = da after the ReLU mask); dgamma / dbeta are
- * this process's own sums (torch leaves their averaging to the gradient all-reduce).  global_count: &global_sums[2*channels]
- * of the forward.  A process with no rows still makes every call.  With its own buffers passed through unreduced, each
- * pair computes what toda_bn_stats + toda_bn_apply (or toda_bn_apply_sums) and toda_bn_bwd compute, bit for bit. */
-int toda_bn_local_sums(const float *y, const double *epilogue_sums, int n, int channels, double *local_sums, void *workspace,
-                       size_t workspace_bytes, void *stream);
-int toda_bn_apply_global(const float *y, int n, int channels, const double *global_sums, const float *gamma, const float *beta,
-                         float eps, float momentum, float *running_mean, float *running_var, float *scale, float *shift,
-                         float *save_mean, float *save_rstd, const float *residual, int relu, float *a, void *a_bf16,
-                         void *stream);
-int toda_bn_bwd_reduce(const float *da, const float *a, const float *y, int n, int channels, const float *save_mean,
-                       const float *save_rstd, int relu, double *local_red, float *dgamma, float *dbeta, void *workspace,
-                       size_t workspace_bytes, void *stream);
-int toda_bn_bwd_finish(const float *da, const float *a, const float *y, int n, int channels, const float *gamma,
-                       const float *save_mean, const float *save_rstd, int relu, const double *global_red,
-                       const double *global_count, float *dy, void *dy_bf16, float *dresidual, void *stream);
 /* column sums: dbias[c] = sum_rows dy[:,c] */
 int toda_col_sum(const float *dy, int n, int channels, float *out, void *workspace, size_t workspace_bytes,
                  void *stream);
@@ -289,7 +280,8 @@ int toda_col_sum(const float *dy, int n, int channels, float *out, void *workspa
  * `SparseBasicBlock` (spconv_backbone.py L8-27, L30-66) as the host sees them.  Same kernels as the
  * individual entry points above, sequenced in C so that the Python host pays one call per layer.
  *   stats: float[4*cout] = scale, shift, save_mean, save_rstd (mean / rstd rows unused in eval mode)
- *   sums : double[2*cout] scratch for the conv epilogue's statistics (training mode, tensor-core kernel)
+ *   sums : double[2*cout] scratch for the BatchNorm's sums of y (training mode): accumulated by the conv epilogue
+ *          (tensor-core kernel) or by toda_bn_local_sums (FFMA kernel)
  * Pointers marked optional may be NULL; with n_out = 0 the output pointers may be NULL too (the forward then leaves the
  * running statistics unchanged, the backward writes zero parameter gradients).
  * ------------------------------------------------------------------------------------------ */
@@ -319,12 +311,12 @@ typedef struct {
 } toda_layer_bwd_args;
 int toda_layer_fwd(const toda_layer_fwd_args *args, void *stream);
 int toda_layer_bwd(const toda_layer_bwd_args *args, void *stream);
-/* The same layer with a BatchNorm synchronized across processes (training mode), split at the all-reduces as the
- * toda_bn_* calls above: toda_layer_fwd_stats (conv + local_sums, double[2*cout+1]) -> all-reduce ->
- * toda_layer_fwd_apply (stats, a, a_bf16, running statistics from global_sums); toda_layer_bwd_reduce (local_red,
+/* The same layer split at the all-reduces of a BatchNorm synchronized across processes (training mode), as the
+ * toda_bn_* calls above: toda_layer_fwd_stats (conv + sums, double[2*cout+1] with the row count) -> all-reduce ->
+ * toda_layer_fwd_apply (stats, a, a_bf16, running statistics from global_sums); toda_layer_bwd_reduce (red,
  * double[2*cout], and this process's dgamma / dbeta) -> all-reduce -> toda_layer_bwd_finish (dy, dres, dgrad, wgrad,
- * bias gradient; global_count = &global_sums[2*cout] of the forward).  `sums` of the forward args is not used.  Unreduced,
- * fwd_stats + fwd_apply = toda_layer_fwd and bwd_reduce + bwd_finish = toda_layer_bwd, bit for bit. */
+ * bias gradient; global_count = &global_sums[2*cout] of the forward).  `sums` of the forward args is not used.
+ * toda_layer_fwd / toda_layer_bwd are the two phases back to back on the layer's own buffers, with the count n_out. */
 int toda_layer_fwd_stats(const toda_layer_fwd_args *args, double *local_sums, void *stream);
 int toda_layer_fwd_apply(const toda_layer_fwd_args *args, const double *global_sums, void *stream);
 int toda_layer_bwd_reduce(const toda_layer_bwd_args *args, double *local_red, void *stream);

@@ -21,10 +21,10 @@ for n in names[:12] + names[-6:]:
     print("%-40s gpu-vs-oracle %.2e   norm %.3e" % (n, rl2(r["grads"][n], ro["grads"][n]), np.linalg.norm(ro["grads"][n])))
 # ---- which BN backward call produces a wrong dbeta?
 from toda_b200 import ops
-orig = ops._bn_backward_impl
+orig = ops._bn_backward_phases
 log = []
-def spy(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16):
-    out = orig(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16)
+def spy(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16, gsums=None):
+    out = yield from orig(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16, gsums)
     dy, dyb, dres, dgamma, dbeta = out
     g = da * (a > 0) if relu else da
     ref_db = g.double().sum(0)
@@ -33,16 +33,16 @@ def spy(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16):
     log.append((y.shape, has_res, float((dbeta.double() - ref_db).norm() / ref_db.norm()), float((dgamma.double() - ref_dg).norm() / ref_dg.norm()),
                 bool(torch.isfinite(da).all()), float(da.abs().max())))
     return out
-ops._bn_backward_impl = spy
+ops._bn_backward_phases = spy
 twin, net = PU.build_pair("VoxelResBackBone8x", nf, g["grid_size"], seed=int(g["seed"]))
 r = PU.run_backbone(net, hc, vf, vc, 2, cot=cot, train=True)
 for l in log[:8]: print(l)
 # ---- compare d(x_conv4) between oracle and GPU
 das = []
-def spy2(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16):
+def spy2(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16, gsums=None):
     das.append((da.detach().cpu().numpy().copy(), a.detach().cpu().numpy().copy()))
-    return orig(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16)
-ops._bn_backward_impl = spy2
+    return (yield from orig(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16, gsums))
+ops._bn_backward_phases = spy2
 twin, net = PU.build_pair("VoxelResBackBone8x", nf, g["grid_size"], seed=int(g["seed"]))
 net.train(); twin.train()
 bd_g = hc(net({"voxel_features": vf.clone().requires_grad_(True), "voxel_coords": vc, "batch_size": 2}))

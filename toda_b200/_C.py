@@ -58,20 +58,16 @@ SIGNATURES = {
     "toda_spconv_wgrad_workspace_bytes": (c_sz, [c_int] * 6),
     "toda_spconv_wgrad": (c_int, [c_vp, c_vp, c_int, c_int, c_vp, c_int, c_int, c_vp, c_vp, c_int, c_vp, c_vp, c_sz, c_int, c_vp]),
     "toda_bn_workspace_bytes": (c_sz, [c_int]),
-    "toda_bn_stats": (c_int, [c_vp, c_int, c_int, c_vp, c_vp, c_f32, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
-                              c_sz, c_vp]),
-    "toda_bn_finalize_sums": (c_int, [c_vp, c_int, c_int, c_vp, c_vp, c_f32, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "toda_bn_local_sums": (c_int, [c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "toda_bn_eval_coeffs": (c_int, [c_vp, c_vp, c_vp, c_vp, c_f32, c_int, c_vp, c_vp, c_vp]),
     "toda_bn_apply": (c_int, [c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_vp, c_vp, c_vp]),
-    "toda_bn_apply_sums": (c_int, [c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_f32, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
-                                   c_int, c_vp, c_vp, c_vp]),
+    "toda_bn_apply_sums": (c_int, [c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_f32, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
+                                   c_vp, c_int, c_vp, c_vp, c_vp]),
     "toda_bn_bwd": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp,
                             c_vp, c_sz, c_vp]),
-    "toda_bn_local_sums": (c_int, [c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_sz, c_vp]),
-    "toda_bn_apply_global": (c_int, [c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_f32, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
-                                     c_int, c_vp, c_vp, c_vp]),
     "toda_bn_bwd_reduce": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
-    "toda_bn_bwd_finish": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "toda_bn_bwd_finish": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp,
+                                   c_vp]),
     "toda_col_sum": (c_int, [c_vp, c_int, c_int, c_vp, c_vp, c_sz, c_vp]),
     "toda_bev_scatter_fwd": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp]),
     "toda_bev_scatter_bwd": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp]),

@@ -113,10 +113,14 @@ __global__ void __launch_bounds__(kThreads) col_reduce_kernel(const float *__res
     }
 }
 
+// A thread of the float4 kernels owns four channels; with kThreads a multiple of C/4, so is every grid stride, and a
+// thread keeps its channels over the whole grid-stride loop.
+static bool vec_channels(int c) { return c % 4 == 0 && kThreads % (c / 4) == 0; }
+
 template <int MODE>
 static void launch_col_reduce(const float *p0, const float *p1, const float *p2, int n, int c, const float *mean,
                               const float *rstd, int relu, double *partial, cudaStream_t st) {
-    if (c % 4 == 0 && kThreads % (c / 4) == 0)
+    if (vec_channels(c))
         col_reduce_vec_kernel<MODE><<<kPartials, kThreads, 0, st>>>(p0, p1, p2, n, c, mean, rstd, relu, partial);
     else
         col_reduce_kernel<MODE><<<kPartials, kThreads, 0, st>>>(p0, p1, p2, n, c, mean, rstd, relu, partial);
@@ -145,8 +149,8 @@ __device__ __forceinline__ void warp_sum_partials(const double *__restrict__ par
     s = a; ss = b;
 }
 
-// BatchNorm coefficients of one channel from its sums (fp64).  One definition for the finalize kernel and for the fused
-// statistics+apply kernel below, with explicit roundings so that both produce the same bits.
+// BatchNorm coefficients of one channel from its sums (fp64), with explicit roundings: every training-mode coefficient
+// of the library is derived here.
 __device__ __forceinline__ void bn_coeffs(double s, double ss, int n, float g, float bt, float eps, float &scale, float &shift,
                                           float &meanf, float &rstd, double &var) {
     const double mean = n > 0 ? s / n : 0.0;
@@ -167,31 +171,12 @@ __device__ __forceinline__ void bn_update_running(float *running_mean, float *ru
     }
 }
 
-__global__ void bn_finalize_kernel(const double *__restrict__ partial, int nblocks, int n, int c,
-                                   const float *__restrict__ gamma, const float *__restrict__ beta, float eps, float momentum,
-                                   float *running_mean, float *running_var, float *scale, float *shift, float *save_mean,
-                                   float *save_rstd) {
-    int ch = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (ch >= c) return;
-    double s, ss;
-    warp_sum_partials(partial, nblocks, c, ch, s, ss);
-    if ((threadIdx.x & 31) != 0) return;
-    float sc, sh, meanf, rstd;
-    double var;
-    bn_coeffs(s, ss, n, gamma ? gamma[ch] : 1.f, beta ? beta[ch] : 0.f, eps, sc, sh, meanf, rstd, var);
-    scale[ch] = sc;
-    shift[ch] = sh;
-    if (save_mean) save_mean[ch] = meanf;
-    if (save_rstd) save_rstd[ch] = rstd;
-    bn_update_running(running_mean, running_var, ch, momentum, meanf, var, n);
-}
-
-// Local statistics of a BatchNorm whose batch spans several processes: out = [sum(y) | sum(y*y) | n], the fp64 buffer
-// that is all-reduced across ranks.  From the per-CTA partials (partial != NULL: the same fixed-order sums as
-// bn_finalize_kernel) or copied from `src` (the convolution epilogue's sums; src == out: count only; NULL: zeros).
-// The count is written here, on the device, so the host never has to provide or read it.
-__global__ void bn_local_sums_kernel(const double *partial, int nblocks, const double *src, int n, int c, double *out) {
-    if (blockIdx.x == 0 && threadIdx.x == 0) out[2 * c] = (double)n;
+// out = [sum(y) | sum(y*y)] per channel: from the per-CTA partials (partial != NULL), copied from `src` (the convolution
+// epilogue's sums; src == out: in place) or zeros (no rows).  `count` (optional) receives the row count: written here, on
+// the device, so that a count all-reduced with the sums never has to pass through the host.
+__global__ void bn_local_sums_kernel(const double *partial, int nblocks, const double *src, int n, int c, double *out,
+                                     double *count) {
+    if (count && blockIdx.x == 0 && threadIdx.x == 0) *count = (double)n;
     int ch = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (ch >= c) return;
     double s = 0.0, ss = 0.0;
@@ -212,128 +197,62 @@ __global__ void bn_eval_coeffs_kernel(const float *gamma, const float *beta, con
     shift[ch] = bt - rm[ch] * g * rstd;
 }
 
-// a = act(y*scale + shift (+ residual)); C % 4 == 0 -> float4 path
+// bf16 copy of four consecutive outputs (element group e of a float4 stream): the next convolution's tensor-core operand
+__device__ __forceinline__ void store_bf16x4(__nv_bfloat16 *__restrict__ dst, long long e, float4 o) {
+    __nv_bfloat162 lo = __floats2bfloat162_rn(o.x, o.y), hi = __floats2bfloat162_rn(o.z, o.w);
+    uint2 pk;
+    pk.x = *(uint32_t *)&lo;
+    pk.y = *(uint32_t *)&hi;
+    ((uint2 *)dst)[e] = pk;
+}
+
+// Where the coefficients of an apply pass come from.  Training (sums != NULL): sums = [sum(y) | sum(y*y)] (fp64) of the
+// whole batch and its row count (*count, or n when count is NULL); block 0 publishes scale / shift / save_mean /
+// save_rstd and updates the running statistics (not on an empty batch).  Eval (sums == NULL): scale / shift as
+// toda_bn_eval_coeffs wrote them.
+struct BnCoeffs {
+    const double *sums; const double *count; int n;
+    const float *gamma, *beta; float eps, momentum;
+    float *running_mean, *running_var, *scale, *shift, *save_mean, *save_rstd;
+};
+
+// a = act(y*scale + shift (+ residual)): every CTA first fills the coefficients of all channels into shared memory
+// (scale[c] | shift[c]), then streams its rows.  VEC (vec_channels(c)): float4 rows, a thread's four coefficients held
+// in registers.  A process with no rows still runs block 0: its running statistics must follow the other ranks'.
 template <bool VEC>
-__global__ void __launch_bounds__(kThreads) bn_apply_kernel(const float *__restrict__ y, long long total, int c,
-                                                            const float *__restrict__ scale, const float *__restrict__ shift,
+__global__ void __launch_bounds__(kThreads) bn_apply_kernel(const float *__restrict__ y, long long total, int c, BnCoeffs k,
                                                             const float *__restrict__ residual, int relu, float *__restrict__ a,
                                                             __nv_bfloat16 *__restrict__ a_bf16) {
-    if (VEC) {
-        long long tv = total >> 2;
-        for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < tv; e += (long long)gridDim.x * blockDim.x) {
-            int ch = (int)((e << 2) % c);
-            float4 v = __ldg((const float4 *)y + e);
-            float4 sc = __ldg((const float4 *)(scale + ch)), sh = __ldg((const float4 *)(shift + ch));
-            float4 o = make_float4(fmaf(v.x, sc.x, sh.x), fmaf(v.y, sc.y, sh.y), fmaf(v.z, sc.z, sh.z), fmaf(v.w, sc.w, sh.w));
-            if (residual) {
-                float4 r = __ldg((const float4 *)residual + e);
-                o.x += r.x; o.y += r.y; o.z += r.z; o.w += r.w;
-            }
-            if (relu) { o.x = fmaxf(o.x, 0.f); o.y = fmaxf(o.y, 0.f); o.z = fmaxf(o.z, 0.f); o.w = fmaxf(o.w, 0.f); }
-            ((float4 *)a)[e] = o;
-            if (a_bf16) {   // bf16 shadow for the tensor-core operands of the next convolution
-                __nv_bfloat162 lo = __floats2bfloat162_rn(o.x, o.y), hi = __floats2bfloat162_rn(o.z, o.w);
-                uint2 pk;
-                pk.x = *(uint32_t *)&lo;
-                pk.y = *(uint32_t *)&hi;
-                ((uint2 *)a_bf16)[e] = pk;
-            }
-        }
-    } else {
-        for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
-            int ch = (int)(e % c);
-            float o = fmaf(__ldg(y + e), scale[ch], shift[ch]);
-            if (residual) o += __ldg(residual + e);
-            if (relu) o = fmaxf(o, 0.f);
-            a[e] = o;
-            if (a_bf16) a_bf16[e] = __float2bfloat16_rn(o);
-        }
-    }
-}
-
-// Training-mode BatchNorm whose statistics arrive as per-channel sums from the producing convolution's epilogue: every
-// thread derives the coefficients of its four channels itself (grid x block is a multiple of C/4: a thread keeps its
-// channels over the grid stride), so the finalize launch between the convolution and this pass disappears; the first C/4
-// threads of block 0 also publish scale / shift / mean / rstd for the backward pass and update the running statistics.
-__global__ void __launch_bounds__(kThreads) bn_apply_sums_kernel(const float *__restrict__ y, long long total, int c, int n,
-                                                                 const double *__restrict__ sums, const float *__restrict__ gamma,
-                                                                 const float *__restrict__ beta, float eps, float momentum,
-                                                                 float *running_mean, float *running_var, float *scale_out,
-                                                                 float *shift_out, float *save_mean, float *save_rstd,
-                                                                 const float *__restrict__ residual, int relu, float *__restrict__ a,
-                                                                 __nv_bfloat16 *__restrict__ a_bf16) {
-    const long long tv = total >> 2;
-    const long long stride = (long long)gridDim.x * blockDim.x;
-    long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
-    const int ch = (int)((e << 2) % c);
-    float sc[4], sh[4];
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-        float meanf, rstd;
-        double var;
-        bn_coeffs(sums[ch + q], sums[c + ch + q], n, gamma ? gamma[ch + q] : 1.f, beta ? beta[ch + q] : 0.f, eps, sc[q], sh[q], meanf,
-                  rstd, var);
-        if (e < (c >> 2)) {          // block 0, one thread per group of four channels
-            scale_out[ch + q] = sc[q];
-            shift_out[ch + q] = sh[q];
-            if (save_mean) save_mean[ch + q] = meanf;
-            if (save_rstd) save_rstd[ch + q] = rstd;
-            bn_update_running(running_mean, running_var, ch + q, momentum, meanf, var, n);
-        }
-    }
-    for (; e < tv; e += stride) {
-        const float4 v = __ldg((const float4 *)y + e);
-        float4 o = make_float4(fmaf(v.x, sc[0], sh[0]), fmaf(v.y, sc[1], sh[1]), fmaf(v.z, sc[2], sh[2]), fmaf(v.w, sc[3], sh[3]));
-        if (residual) {
-            const float4 r = __ldg((const float4 *)residual + e);
-            o.x += r.x; o.y += r.y; o.z += r.z; o.w += r.w;
-        }
-        if (relu) { o.x = fmaxf(o.x, 0.f); o.y = fmaxf(o.y, 0.f); o.z = fmaxf(o.z, 0.f); o.w = fmaxf(o.w, 0.f); }
-        ((float4 *)a)[e] = o;
-        if (a_bf16) {
-            __nv_bfloat162 lo = __floats2bfloat162_rn(o.x, o.y), hi = __floats2bfloat162_rn(o.z, o.w);
-            uint2 pk;
-            pk.x = *(uint32_t *)&lo;
-            pk.y = *(uint32_t *)&hi;
-            ((uint2 *)a_bf16)[e] = pk;
-        }
-    }
-}
-
-// Training-mode BatchNorm from statistics all-reduced over several processes: sums = [sum(y) | sum(y*y) | n] of the
-// union batch (bn_local_sums_kernel's layout).  Every CTA derives the coefficients of all channels into shared memory
-// (the same bn_coeffs as the finalize kernels, so the same bits), block 0 publishes scale / shift / mean / rstd and
-// updates the running statistics with the global count; then the rows of this process stream as in bn_apply_kernel.
-// A process with no rows still runs block 0: its running statistics must follow the other ranks'.
-template <bool VEC>
-__global__ void __launch_bounds__(kThreads) bn_apply_global_kernel(const float *__restrict__ y, long long total, int c,
-                                                                   const double *__restrict__ sums, const float *__restrict__ gamma,
-                                                                   const float *__restrict__ beta, float eps, float momentum,
-                                                                   float *running_mean, float *running_var, float *scale_out,
-                                                                   float *shift_out, float *save_mean, float *save_rstd,
-                                                                   const float *__restrict__ residual, int relu, float *__restrict__ a,
-                                                                   __nv_bfloat16 *__restrict__ a_bf16) {
-    __shared__ __align__(16) float s_sc[256], s_sh[256];
-    const int n = (int)sums[2 * c];
+    extern __shared__ __align__(16) float s_coef[];
+    float *s_sc = s_coef, *s_sh = s_coef + c;
+    const int n = k.count ? (int)*k.count : k.n;
     for (int ch = threadIdx.x; ch < c; ch += blockDim.x) {
+        if (!k.sums) {
+            s_sc[ch] = k.scale[ch];
+            s_sh[ch] = k.shift[ch];
+            continue;
+        }
         float meanf, rstd;
         double var;
-        bn_coeffs(sums[ch], sums[c + ch], n, gamma ? gamma[ch] : 1.f, beta ? beta[ch] : 0.f, eps, s_sc[ch], s_sh[ch], meanf, rstd, var);
+        bn_coeffs(k.sums[ch], k.sums[c + ch], n, k.gamma ? k.gamma[ch] : 1.f, k.beta ? k.beta[ch] : 0.f, k.eps, s_sc[ch], s_sh[ch],
+                  meanf, rstd, var);
         if (blockIdx.x == 0) {
-            scale_out[ch] = s_sc[ch];
-            shift_out[ch] = s_sh[ch];
-            if (save_mean) save_mean[ch] = meanf;
-            if (save_rstd) save_rstd[ch] = rstd;
-            if (n > 0) bn_update_running(running_mean, running_var, ch, momentum, meanf, var, n);
+            k.scale[ch] = s_sc[ch];
+            k.shift[ch] = s_sh[ch];
+            if (k.save_mean) k.save_mean[ch] = meanf;
+            if (k.save_rstd) k.save_rstd[ch] = rstd;
+            if (n > 0) bn_update_running(k.running_mean, k.running_var, ch, k.momentum, meanf, var, n);
         }
     }
     __syncthreads();
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     if (VEC) {
         const long long tv = total >> 2;
-        for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < tv; e += (long long)gridDim.x * blockDim.x) {
-            const int ch = (int)((e << 2) % c);
+        const int ch = (int)((e << 2) % c);
+        const float4 sc = *(const float4 *)(s_sc + ch), sh = *(const float4 *)(s_sh + ch);
+        for (; e < tv; e += stride) {
             const float4 v = __ldg((const float4 *)y + e);
-            const float4 sc = *(const float4 *)(s_sc + ch), sh = *(const float4 *)(s_sh + ch);
             float4 o = make_float4(fmaf(v.x, sc.x, sh.x), fmaf(v.y, sc.y, sh.y), fmaf(v.z, sc.z, sh.z), fmaf(v.w, sc.w, sh.w));
             if (residual) {
                 const float4 r = __ldg((const float4 *)residual + e);
@@ -341,16 +260,10 @@ __global__ void __launch_bounds__(kThreads) bn_apply_global_kernel(const float *
             }
             if (relu) { o.x = fmaxf(o.x, 0.f); o.y = fmaxf(o.y, 0.f); o.z = fmaxf(o.z, 0.f); o.w = fmaxf(o.w, 0.f); }
             ((float4 *)a)[e] = o;
-            if (a_bf16) {
-                __nv_bfloat162 lo = __floats2bfloat162_rn(o.x, o.y), hi = __floats2bfloat162_rn(o.z, o.w);
-                uint2 pk;
-                pk.x = *(uint32_t *)&lo;
-                pk.y = *(uint32_t *)&hi;
-                ((uint2 *)a_bf16)[e] = pk;
-            }
+            if (a_bf16) store_bf16x4(a_bf16, e, o);
         }
     } else {
-        for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+        for (; e < total; e += stride) {
             const int ch = (int)(e % c);
             float o = fmaf(__ldg(y + e), s_sc[ch], s_sh[ch]);
             if (residual) o += __ldg(residual + e);
@@ -361,11 +274,9 @@ __global__ void __launch_bounds__(kThreads) bn_apply_global_kernel(const float *
     }
 }
 
-// T = float: the sums bn_bwd_apply_kernel reads in the same call; T = double: the local sums a multi-process BatchNorm
-// all-reduces before its bn_bwd_apply_kernel<., true> (which rounds them to float exactly as this kernel does for float).
-template <typename T>
+// sums = [sum g | sum g*xhat] (fp64) of the per-CTA partials, and the same rounded to float as dbeta / dgamma
 __global__ void bn_bwd_finalize_kernel(const double *__restrict__ partial, int nblocks, int c, float *dgamma, float *dbeta,
-                                       T *sums /* [2c]: sum_g, sum_g_xhat */) {
+                                       double *sums) {
     int ch = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (ch >= c) return;
     double s, sx;
@@ -373,38 +284,38 @@ __global__ void bn_bwd_finalize_kernel(const double *__restrict__ partial, int n
     if ((threadIdx.x & 31) != 0) return;
     if (dbeta) dbeta[ch] = (float)s;
     if (dgamma) dgamma[ch] = (float)sx;
-    sums[ch] = (T)s;
-    sums[c + ch] = (T)sx;
+    sums[ch] = s;
+    sums[c + ch] = sx;
 }
 
 // dy = gamma*rstd*(g - sum_g/N - xhat*sum_gx/N)   (training)   |   dy = gamma*rstd*g   (eval)
 // Per channel this is dy = A*g + B*y + C with A = gamma*rstd, B = -gamma*rstd^2*sum_gx/N,
 // C = -A*sum_g/N - B*mean: coefficients are computed once per thread (4 channels), rows stream as float4.
-// GLOBAL: the sums are the fp64 ones all-reduced over the processes of a synchronized BatchNorm (`gsums`) and N is the
-// global count (`gcount`, device memory); both are rounded exactly as the single-process path rounds them.
-template <bool VEC, bool GLOBAL>
+// The sums are bn_bwd_finalize_kernel's (all-reduced over the processes of a synchronized BatchNorm), rounded to float;
+// N is *count (the global count of a synchronized BatchNorm, device memory) or n when count is NULL.
+template <bool VEC>
 __global__ void __launch_bounds__(kThreads) bn_bwd_apply_kernel(const float *__restrict__ da, const float *__restrict__ a,
-                                                                const float *__restrict__ y, long long total, int c, int n_local,
-                                                                const float *__restrict__ gamma, const float *__restrict__ mean,
-                                                                const float *__restrict__ rstd, const float *__restrict__ fsums,
-                                                                const double *__restrict__ gsums, const double *__restrict__ gcount,
-                                                                int relu, int training, float *__restrict__ dy,
-                                                                float *__restrict__ dres, __nv_bfloat16 *__restrict__ dy_bf16) {
-    const int n = GLOBAL ? (int)*gcount : n_local;
-    auto sums = [&](int i) -> float { return GLOBAL ? (float)gsums[i] : fsums[i]; };
+                                                                const float *__restrict__ y, long long total, int c, int n,
+                                                                const double *__restrict__ count, const float *__restrict__ gamma,
+                                                                const float *__restrict__ mean, const float *__restrict__ rstd,
+                                                                const double *__restrict__ sums, int relu, int training,
+                                                                float *__restrict__ dy, float *__restrict__ dres,
+                                                                __nv_bfloat16 *__restrict__ dy_bf16) {
+    if (count) n = (int)*count;
+    auto sum = [&](int i) -> float { return (float)sums[i]; };
     const float inv_n = n > 0 ? 1.0f / (float)n : 0.f;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     if (VEC) {
         const long long tv = total >> 2;
-        const long long stride = (long long)gridDim.x * blockDim.x;      // multiple of c/4 (host guarantees it)
-        long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
         const int ch = (int)((e << 2) % c);
         float A[4], B[4], C[4];
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
             float gm = gamma ? gamma[ch + q] : 1.f, rs = rstd[ch + q];
             A[q] = gm * rs;
-            B[q] = training ? -gm * rs * rs * sums(c + ch + q) * inv_n : 0.f;
-            C[q] = training ? -A[q] * sums(ch + q) * inv_n - B[q] * mean[ch + q] : 0.f;
+            B[q] = training ? -gm * rs * rs * sum(c + ch + q) * inv_n : 0.f;
+            C[q] = training ? -A[q] * sum(ch + q) * inv_n - B[q] * mean[ch + q] : 0.f;
         }
         for (; e < tv; e += stride) {
             float4 g4 = __ldg((const float4 *)da + e);
@@ -421,16 +332,10 @@ __global__ void __launch_bounds__(kThreads) bn_bwd_apply_kernel(const float *__r
             o.z = fmaf(A[2], g4.z, fmaf(B[2], y4.z, C[2]));
             o.w = fmaf(A[3], g4.w, fmaf(B[3], y4.w, C[3]));
             if (dy) ((float4 *)dy)[e] = o;
-            if (dy_bf16) {
-                __nv_bfloat162 lo = __floats2bfloat162_rn(o.x, o.y), hi = __floats2bfloat162_rn(o.z, o.w);
-                uint2 pk;
-                pk.x = *(uint32_t *)&lo;
-                pk.y = *(uint32_t *)&hi;
-                ((uint2 *)dy_bf16)[e] = pk;
-            }
+            if (dy_bf16) store_bf16x4(dy_bf16, e, o);
         }
     } else {
-        for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+        for (; e < total; e += stride) {
             int ch = (int)(e % c);
             float g = __ldg(da + e);
             if (relu && !(__ldg(a + e) > 0.f)) g = 0.f;
@@ -440,7 +345,7 @@ __global__ void __launch_bounds__(kThreads) bn_bwd_apply_kernel(const float *__r
             float o;
             if (training) {
                 float xh = (__ldg(y + e) - mean[ch]) * rs;
-                o = gm * rs * (g - sums(ch) * inv_n - xh * sums(c + ch) * inv_n);
+                o = gm * rs * (g - sum(ch) * inv_n - xh * sum(c + ch) * inv_n);
             } else {
                 o = gm * rs * g;
             }
@@ -458,40 +363,58 @@ __global__ void col_sum_finalize_kernel(const double *__restrict__ partial, int 
     if ((threadIdx.x & 31) == 0) out[ch] = (float)s;
 }
 
-size_t bn_ws_bytes(int c) { return align_up((size_t)kPartials * 2 * c * sizeof(double) + 2 * c * sizeof(float), 256); }
+// workspace: the per-CTA partials, then the 2c reduced backward sums of toda_bn_bwd
+size_t partials_bytes(int c) { return (size_t)kPartials * 2 * c * sizeof(double); }
+size_t bn_ws_bytes(int c) { return align_up(partials_bytes(c) + 2 * c * sizeof(double), 256); }
+
+// Grid of a grid-stride streaming kernel over `items` work items: exactly the CTAs that are resident at once (occupancy x
+// SMs, queried once per kernel), never more than the work.  A grid that is 1.3-1.6 waves (what a fixed 8 CTAs/SM gave for
+// the 34- and 41-register kernels) leaves most SMs idle during the second, partial wave.
+template <auto Kernel> int resident_grid(int64_t items) {
+    static const int64_t cap = [] {
+        int per_sm = 0;
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, Kernel, kThreads, 0) != cudaSuccess || per_sm < 1) per_sm = 4;
+        return (int64_t)per_sm * kNumSMs;
+    }();
+    const int64_t need = (items + kThreads - 1) / kThreads;
+    return (int)(need < 1 ? 1 : (need < cap ? need : cap));
+}
+
+int launch_bn_apply(const float *y, int n, int c, const BnCoeffs &k, const float *residual, int relu, float *a, void *a_bf16,
+                    cudaStream_t st) {
+    const long long total = (long long)n * c;
+    const size_t smem = 2 * (size_t)c * sizeof(float);
+    if (vec_channels(c))
+        bn_apply_kernel<true><<<resident_grid<bn_apply_kernel<true>>(total / 4), kThreads, smem, st>>>(
+            y, total, c, k, residual, relu, a, (__nv_bfloat16 *)a_bf16);
+    else
+        bn_apply_kernel<false><<<resident_grid<bn_apply_kernel<false>>(total), kThreads, smem, st>>>(
+            y, total, c, k, residual, relu, a, (__nv_bfloat16 *)a_bf16);
+    TODA_LAUNCH_OK();
+    return TODA_OK;
+}
 
 }  // namespace
 
 extern "C" size_t toda_bn_workspace_bytes(int channels) { return channels > 0 ? bn_ws_bytes(channels) : 0; }
 
-extern "C" int toda_bn_stats(const float *y, int n, int c, const float *gamma, const float *beta, float eps, float momentum,
-                             float *running_mean, float *running_var, float *scale, float *shift, float *save_mean,
-                             float *save_rstd, void *workspace, size_t workspace_bytes, void *stream) {
-    TODA_CHECK_ARG(n >= 0 && c > 0 && c <= 256, "bn_stats: unsupported sizes n=%d c=%d", n, c);
-    TODA_CHECK_ARG((y || n == 0) && scale && shift && workspace, "bn_stats: null pointer");
-    if (workspace_bytes < bn_ws_bytes(c)) { toda_set_error("bn_stats: workspace too small"); return TODA_ERR_WORKSPACE; }
-    cudaStream_t st = (cudaStream_t)stream;
-    double *partial = (double *)workspace;
-    launch_col_reduce<0>(y, nullptr, nullptr, n, c, nullptr, nullptr, 0, partial, st);
-    TODA_LAUNCH_OK();
-    // an empty batch has no statistics: the running statistics stay as they are (torch.nn.BatchNorm1d does the same)
-    bn_finalize_kernel<<<ceil_div(c * 32, 128), 128, 0, st>>>(partial, kPartials, n, c, gamma, beta, eps, momentum,
-                                                        n > 0 ? running_mean : nullptr, n > 0 ? running_var : nullptr,
-                                                        scale, shift, save_mean, save_rstd);
-    TODA_LAUNCH_OK();
-    return TODA_OK;
-}
+double *bn_workspace_red(void *workspace, int c) { return (double *)((char *)workspace + partials_bytes(c)); }
 
-extern "C" int toda_bn_finalize_sums(const double *sums, int n, int c, const float *gamma, const float *beta, float eps,
-                                     float momentum, float *running_mean, float *running_var, float *scale, float *shift,
-                                     float *save_mean, float *save_rstd, void *stream) {
-    TODA_CHECK_ARG(n >= 0 && c > 0 && sums && scale && shift, "bn_finalize_sums: bad args");
-    // `sums` = [sum(y) per channel | sum(y*y) per channel]: the layout of one partial block of toda_bn_stats.  An empty
-    // batch leaves the running statistics unchanged, as in toda_bn_stats.
-    bn_finalize_kernel<<<ceil_div(c * 32, 128), 128, 0, (cudaStream_t)stream>>>(sums, 1, n, c, gamma, beta, eps, momentum,
-                                                                            n > 0 ? running_mean : nullptr,
-                                                                            n > 0 ? running_var : nullptr, scale, shift,
-                                                                            save_mean, save_rstd);
+extern "C" int toda_bn_local_sums(const float *y, const double *epilogue_sums, int n, int c, double *sums, double *count,
+                                  void *workspace, size_t workspace_bytes, void *stream) {
+    TODA_CHECK_ARG(n >= 0 && c > 0 && c <= 256 && sums, "bn_local_sums: bad args n=%d c=%d", n, c);
+    if (n > 0 && epilogue_sums == sums && !count) return TODA_OK;      // already in place, and no count wanted
+    cudaStream_t st = (cudaStream_t)stream;
+    const double *partial = nullptr;
+    if (n > 0 && !epilogue_sums) {
+        TODA_CHECK_ARG(y && workspace, "bn_local_sums: null pointer");
+        if (workspace_bytes < bn_ws_bytes(c)) { toda_set_error("bn_local_sums: workspace too small"); return TODA_ERR_WORKSPACE; }
+        launch_col_reduce<0>(y, nullptr, nullptr, n, c, nullptr, nullptr, 0, (double *)workspace, st);
+        TODA_LAUNCH_OK();
+        partial = (const double *)workspace;
+    }
+    bn_local_sums_kernel<<<ceil_div(c * 32, 128), 128, 0, st>>>(partial, kPartials, n > 0 ? epilogue_sums : nullptr, n, c, sums,
+                                                              count);
     TODA_LAUNCH_OK();
     return TODA_OK;
 }
@@ -505,169 +428,25 @@ extern "C" int toda_bn_eval_coeffs(const float *gamma, const float *beta, const 
     return TODA_OK;
 }
 
-// Grid of a grid-stride streaming kernel: exactly the CTAs that are resident at once (occupancy x SMs), never more than
-// the work.  A grid that is 1.3-1.6 waves (what a fixed 8 CTAs/SM gave for the 34- and 41-register kernels) leaves most
-// SMs idle during the second, partial wave.
-template <typename K> static int resident_grid(K kernel, int64_t items) {
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, 0) != cudaSuccess || per_sm < 1) per_sm = 4;
-    int64_t need = (items + kThreads - 1) / kThreads;
-    int64_t cap = (int64_t)per_sm * kNumSMs;
-    return (int)(need < 1 ? 1 : (need < cap ? need : cap));
-}
-
 extern "C" int toda_bn_apply(const float *y, int n, int c, const float *scale, const float *shift, const float *residual,
                              int relu, float *a, void *a_bf16, void *stream) {
     TODA_CHECK_ARG(n >= 0 && c > 0, "bn_apply: bad sizes");
     if (n == 0) return TODA_OK;
     TODA_CHECK_ARG(y && scale && shift && a, "bn_apply: null pointer");
-    long long total = (long long)n * c;
-    cudaStream_t st = (cudaStream_t)stream;
-    static int per_sm_vec = 0, per_sm_scalar = 0;     // resident CTAs per SM of the two variants (queried once)
-    if (!per_sm_vec) {
-        per_sm_vec = resident_grid(bn_apply_kernel<true>, (int64_t)1 << 40) / kNumSMs;
-        per_sm_scalar = resident_grid(bn_apply_kernel<false>, (int64_t)1 << 40) / kNumSMs;
-    }
-    auto grid_for = [](int64_t items, int per_sm) {
-        int64_t need = (items + kThreads - 1) / kThreads, cap = (int64_t)per_sm * kNumSMs;
-        return (int)(need < 1 ? 1 : (need < cap ? need : cap));
-    };
-    if (c % 4 == 0)
-        bn_apply_kernel<true><<<grid_for(total / 4, per_sm_vec), kThreads, 0, st>>>(y, total, c, scale, shift, residual, relu, a, (__nv_bfloat16 *)a_bf16);
-    else
-        bn_apply_kernel<false><<<grid_for(total, per_sm_scalar), kThreads, 0, st>>>(y, total, c, scale, shift, residual, relu, a, (__nv_bfloat16 *)a_bf16);
-    TODA_LAUNCH_OK();
-    return TODA_OK;
+    BnCoeffs k{};
+    k.scale = (float *)scale;
+    k.shift = (float *)shift;
+    return launch_bn_apply(y, n, c, k, residual, relu, a, a_bf16, (cudaStream_t)stream);
 }
 
-extern "C" int toda_bn_apply_sums(const float *y, int n, int c, const double *sums, const float *gamma, const float *beta, float eps,
-                                  float momentum, float *running_mean, float *running_var, float *scale, float *shift,
-                                  float *save_mean, float *save_rstd, const float *residual, int relu, float *a, void *a_bf16,
-                                  void *stream) {
+extern "C" int toda_bn_apply_sums(const float *y, int n, int c, const double *sums, const double *count, const float *gamma,
+                                  const float *beta, float eps, float momentum, float *running_mean, float *running_var,
+                                  float *scale, float *shift, float *save_mean, float *save_rstd, const float *residual, int relu,
+                                  float *a, void *a_bf16, void *stream) {
     TODA_CHECK_ARG(n >= 0 && c > 0 && sums && scale && shift, "bn_apply_sums: bad args");
-    cudaStream_t st = (cudaStream_t)stream;
-    // the fused kernel needs a thread to keep its four channels over the grid stride; other shapes (none in these backbones)
-    // and empty inputs (coefficients only: the running statistics are left unchanged) take the two-launch route
-    if (n == 0 || c % 4 != 0 || kThreads % (c / 4) != 0) {
-        int rc = toda_bn_finalize_sums(sums, n, c, gamma, beta, eps, momentum, running_mean, running_var, scale, shift, save_mean,
-                                       save_rstd, stream);
-        if (rc) return rc;
-        return toda_bn_apply(y, n, c, scale, shift, residual, relu, a, a_bf16, stream);
-    }
-    TODA_CHECK_ARG(y && a, "bn_apply_sums: null pointer");
-    const long long total = (long long)n * c;
-    static int per_sm = 0;
-    if (!per_sm) per_sm = resident_grid(bn_apply_sums_kernel, (int64_t)1 << 40) / kNumSMs;
-    const int64_t need = (total / 4 + kThreads - 1) / kThreads, cap = (int64_t)per_sm * kNumSMs;
-    const int grid = (int)(need < 1 ? 1 : (need < cap ? need : cap));
-    bn_apply_sums_kernel<<<grid, kThreads, 0, st>>>(y, total, c, n, sums, gamma, beta, eps, momentum, running_mean, running_var, scale,
-                                                    shift, save_mean, save_rstd, residual, relu, a, (__nv_bfloat16 *)a_bf16);
-    TODA_LAUNCH_OK();
-    return TODA_OK;
-}
-
-// The streaming pass of the BatchNorm backward (bn_bwd_apply_kernel) over n > 0 rows.  GLOBAL: the reductions and the
-// count come from device memory (fp64, all-reduced over the processes of a synchronized BatchNorm) instead of `fsums`/`n`.
-template <bool GLOBAL>
-static void launch_bn_bwd_apply(const float *da, const float *a, const float *y, int n, int c, const float *gamma,
-                                const float *save_mean, const float *save_rstd, const float *fsums, const double *gsums,
-                                const double *gcount, int relu, int training, float *dy, float *dresidual, void *dy_bf16,
-                                cudaStream_t st) {
-    long long total = (long long)n * c;
-    static int per_sm_vec = 0, per_sm_scalar = 0;
-    if (!per_sm_vec) {
-        per_sm_vec = resident_grid(bn_bwd_apply_kernel<true, GLOBAL>, (int64_t)1 << 40) / kNumSMs;
-        per_sm_scalar = resident_grid(bn_bwd_apply_kernel<false, GLOBAL>, (int64_t)1 << 40) / kNumSMs;
-    }
-    auto grid_for = [](int64_t items, int per_sm) {
-        int64_t need = (items + kThreads - 1) / kThreads, cap = (int64_t)per_sm * kNumSMs;
-        return (int)(need < 1 ? 1 : (need < cap ? need : cap));
-    };
-    if (c % 4 == 0 && kThreads % (c / 4) == 0)   // grid*block is then a multiple of c/4: a thread keeps its 4 channels
-        bn_bwd_apply_kernel<true, GLOBAL><<<grid_for(total / 4, per_sm_vec), kThreads, 0, st>>>(
-            da, a, y, total, c, n, gamma, save_mean, save_rstd, fsums, gsums, gcount, relu, training, dy, dresidual,
-            (__nv_bfloat16 *)dy_bf16);
-    else
-        bn_bwd_apply_kernel<false, GLOBAL><<<grid_for(total, per_sm_scalar), kThreads, 0, st>>>(
-            da, a, y, total, c, n, gamma, save_mean, save_rstd, fsums, gsums, gcount, relu, training, dy, dresidual,
-            (__nv_bfloat16 *)dy_bf16);
-}
-
-extern "C" int toda_bn_bwd(const float *da, const float *a, const float *y, int n, int c, const float *gamma,
-                           const float *save_mean, const float *save_rstd, int relu, int training, float *dy, void *dy_bf16,
-                           float *dresidual, float *dgamma, float *dbeta, void *workspace, size_t workspace_bytes, void *stream) {
-    TODA_CHECK_ARG(n >= 0 && c > 0 && c <= 256, "bn_bwd: unsupported sizes n=%d c=%d", n, c);
-    // dy may be NULL when dy_bf16 is given: the fp32 gradient is then not stored (a caller whose consumers -- tensor-core
-    // dgrad and wgrad -- only read the bf16 copy saves 4 of the ~30 bytes per element this pass moves)
-    TODA_CHECK_ARG(save_mean && save_rstd && workspace && (n == 0 || (da && y && (dy || dy_bf16))) && (!relu || a || n == 0),
-                   "bn_bwd: null pointer");
-    if (workspace_bytes < bn_ws_bytes(c)) { toda_set_error("bn_bwd: workspace too small"); return TODA_ERR_WORKSPACE; }
-    cudaStream_t st = (cudaStream_t)stream;
-    double *partial = (double *)workspace;
-    float *sums = (float *)((char *)workspace + (size_t)kPartials * 2 * c * sizeof(double));
-    launch_col_reduce<1>(da, a, y, n, c, save_mean, save_rstd, relu, partial, st);
-    TODA_LAUNCH_OK();
-    bn_bwd_finalize_kernel<float><<<ceil_div(c * 32, 128), 128, 0, st>>>(partial, kPartials, c, dgamma, dbeta, sums);
-    TODA_LAUNCH_OK();
-    if (n > 0) {
-        launch_bn_bwd_apply<false>(da, a, y, n, c, gamma, save_mean, save_rstd, sums, nullptr, nullptr, relu, training, dy,
-                                   dresidual, dy_bf16, st);
-        TODA_LAUNCH_OK();
-    }
-    return TODA_OK;
-}
-
-// ---- BatchNorm over a batch split across processes (torch.nn.SyncBatchNorm): each phase that needs the other ranks'
-// statistics is split at the all-reduce.  Forward: toda_bn_local_sums -> all-reduce SUM -> toda_bn_apply_global.
-// Backward: toda_bn_bwd_reduce -> all-reduce SUM -> toda_bn_bwd_finish.  Given its own local buffers unreduced, each
-// pair computes exactly what the single-process call computes (toda_bn_stats + toda_bn_apply / toda_bn_apply_sums,
-// toda_bn_bwd), bit for bit.
-
-extern "C" int toda_bn_local_sums(const float *y, const double *epilogue_sums, int n, int c, double *local_sums, void *workspace,
-                                  size_t workspace_bytes, void *stream) {
-    TODA_CHECK_ARG(n >= 0 && c > 0 && c <= 256 && local_sums, "bn_local_sums: bad args n=%d c=%d", n, c);
-    cudaStream_t st = (cudaStream_t)stream;
-    const double *partial = nullptr;
-    if (n > 0 && !epilogue_sums) {
-        TODA_CHECK_ARG(y && workspace, "bn_local_sums: null pointer");
-        if (workspace_bytes < bn_ws_bytes(c)) { toda_set_error("bn_local_sums: workspace too small"); return TODA_ERR_WORKSPACE; }
-        launch_col_reduce<0>(y, nullptr, nullptr, n, c, nullptr, nullptr, 0, (double *)workspace, st);
-        TODA_LAUNCH_OK();
-        partial = (const double *)workspace;
-    }
-    bn_local_sums_kernel<<<ceil_div(c * 32, 128), 128, 0, st>>>(partial, kPartials, n > 0 ? epilogue_sums : nullptr, n, c,
-                                                              local_sums);
-    TODA_LAUNCH_OK();
-    return TODA_OK;
-}
-
-extern "C" int toda_bn_apply_global(const float *y, int n, int c, const double *global_sums, const float *gamma, const float *beta,
-                                    float eps, float momentum, float *running_mean, float *running_var, float *scale, float *shift,
-                                    float *save_mean, float *save_rstd, const float *residual, int relu, float *a, void *a_bf16,
-                                    void *stream) {
-    TODA_CHECK_ARG(n >= 0 && c > 0 && c <= 256 && global_sums && scale && shift, "bn_apply_global: bad args");
-    TODA_CHECK_ARG(n == 0 || (y && a), "bn_apply_global: null pointer");
-    cudaStream_t st = (cudaStream_t)stream;
-    const long long total = (long long)n * c;
-    static int per_sm_vec = 0, per_sm_scalar = 0;
-    if (!per_sm_vec) {
-        per_sm_vec = resident_grid(bn_apply_global_kernel<true>, (int64_t)1 << 40) / kNumSMs;
-        per_sm_scalar = resident_grid(bn_apply_global_kernel<false>, (int64_t)1 << 40) / kNumSMs;
-    }
-    auto grid_for = [](int64_t items, int per_sm) {
-        int64_t need = (items + kThreads - 1) / kThreads, cap = (int64_t)per_sm * kNumSMs;
-        return (int)(need < 1 ? 1 : (need < cap ? need : cap));
-    };
-    if (c % 4 == 0)
-        bn_apply_global_kernel<true><<<grid_for(total / 4, per_sm_vec), kThreads, 0, st>>>(
-            y, total, c, global_sums, gamma, beta, eps, momentum, running_mean, running_var, scale, shift, save_mean, save_rstd,
-            residual, relu, a, (__nv_bfloat16 *)a_bf16);
-    else
-        bn_apply_global_kernel<false><<<grid_for(total, per_sm_scalar), kThreads, 0, st>>>(
-            y, total, c, global_sums, gamma, beta, eps, momentum, running_mean, running_var, scale, shift, save_mean, save_rstd,
-            residual, relu, a, (__nv_bfloat16 *)a_bf16);
-    TODA_LAUNCH_OK();
-    return TODA_OK;
+    TODA_CHECK_ARG(n == 0 || (y && a), "bn_apply_sums: null pointer");
+    const BnCoeffs k{sums, count, n, gamma, beta, eps, momentum, running_mean, running_var, scale, shift, save_mean, save_rstd};
+    return launch_bn_apply(y, n, c, k, residual, relu, a, a_bf16, (cudaStream_t)stream);
 }
 
 extern "C" int toda_bn_bwd_reduce(const float *da, const float *a, const float *y, int n, int c, const float *save_mean,
@@ -681,22 +460,41 @@ extern "C" int toda_bn_bwd_reduce(const float *da, const float *a, const float *
     double *partial = (double *)workspace;
     launch_col_reduce<1>(da, a, y, n, c, save_mean, save_rstd, relu, partial, st);
     TODA_LAUNCH_OK();
-    bn_bwd_finalize_kernel<double><<<ceil_div(c * 32, 128), 128, 0, st>>>(partial, kPartials, c, dgamma, dbeta, local_red);
+    bn_bwd_finalize_kernel<<<ceil_div(c * 32, 128), 128, 0, st>>>(partial, kPartials, c, dgamma, dbeta, local_red);
     TODA_LAUNCH_OK();
     return TODA_OK;
 }
 
 extern "C" int toda_bn_bwd_finish(const float *da, const float *a, const float *y, int n, int c, const float *gamma,
-                                  const float *save_mean, const float *save_rstd, int relu, const double *global_red,
-                                  const double *global_count, float *dy, void *dy_bf16, float *dresidual, void *stream) {
+                                  const float *save_mean, const float *save_rstd, int relu, int training, const double *red,
+                                  const double *count, float *dy, void *dy_bf16, float *dresidual, void *stream) {
     TODA_CHECK_ARG(n >= 0 && c > 0 && c <= 256, "bn_bwd_finish: unsupported sizes n=%d c=%d", n, c);
-    TODA_CHECK_ARG(save_mean && save_rstd && global_red && global_count && (n == 0 || (da && y && (dy || dy_bf16))) &&
+    // dy may be NULL when dy_bf16 is given: the fp32 gradient is then not stored (a caller whose consumers -- tensor-core
+    // dgrad and wgrad -- only read the bf16 copy saves 4 of the ~30 bytes per element this pass moves)
+    TODA_CHECK_ARG(save_mean && save_rstd && (red || !training) && (n == 0 || (da && y && (dy || dy_bf16))) &&
                    (!relu || a || n == 0), "bn_bwd_finish: null pointer");
     if (n == 0) return TODA_OK;
-    launch_bn_bwd_apply<true>(da, a, y, n, c, gamma, save_mean, save_rstd, nullptr, global_red, global_count, relu, 1, dy,
-                              dresidual, dy_bf16, (cudaStream_t)stream);
+    const long long total = (long long)n * c;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (vec_channels(c))
+        bn_bwd_apply_kernel<true><<<resident_grid<bn_bwd_apply_kernel<true>>(total / 4), kThreads, 0, st>>>(
+            da, a, y, total, c, n, count, gamma, save_mean, save_rstd, red, relu, training, dy, dresidual, (__nv_bfloat16 *)dy_bf16);
+    else
+        bn_bwd_apply_kernel<false><<<resident_grid<bn_bwd_apply_kernel<false>>(total), kThreads, 0, st>>>(
+            da, a, y, total, c, n, count, gamma, save_mean, save_rstd, red, relu, training, dy, dresidual, (__nv_bfloat16 *)dy_bf16);
     TODA_LAUNCH_OK();
     return TODA_OK;
+}
+
+extern "C" int toda_bn_bwd(const float *da, const float *a, const float *y, int n, int c, const float *gamma,
+                           const float *save_mean, const float *save_rstd, int relu, int training, float *dy, void *dy_bf16,
+                           float *dresidual, float *dgamma, float *dbeta, void *workspace, size_t workspace_bytes, void *stream) {
+    TODA_CHECK_ARG(workspace, "bn_bwd: null workspace");
+    double *red = bn_workspace_red(workspace, c);
+    int rc = toda_bn_bwd_reduce(da, a, y, n, c, save_mean, save_rstd, relu, red, dgamma, dbeta, workspace, workspace_bytes, stream);
+    if (rc) return rc;
+    return toda_bn_bwd_finish(da, a, y, n, c, gamma, save_mean, save_rstd, relu, training, red, nullptr, dy, dy_bf16, dresidual,
+                              stream);
 }
 
 extern "C" int toda_col_sum(const float *dy, int n, int c, float *out, void *workspace, size_t workspace_bytes, void *stream) {

@@ -47,6 +47,10 @@ static inline int wave_grid(int64_t n, int block, int waves = 8) {
     return (int)(rounded < cap ? rounded : cap);
 }
 
+// The 2*c doubles that follow the per-CTA partials in a BatchNorm workspace (toda_bn_workspace_bytes): where a one-call
+// backward (toda_bn_bwd, toda_layer_bwd) keeps its reduced sums between the reduce and the finish phase.
+double *bn_workspace_red(void *workspace, int c);
+
 // ---------------------------------------------------------------------------------------------
 // Occupancy index: two-level bitmap + per-word rank.  See include/toda_b200.h.
 //   cell id = b * frame_stride + (z*H + y)*W + x      frame_stride = D*H*W rounded up to 4096

@@ -34,9 +34,6 @@ def reset_launches():
     _launch_base = int(_C.lib().toda_launch_count())
 
 
-def _count(n):
-    pass
-
 
 # optional per-call device timing (bench.py's roofline pass): list of (name, meta, start_event, end_event)
 _prof = None
@@ -159,7 +156,6 @@ def points_select(points, frame_offsets, mode, params, invert=False, add_batch_c
         _C.check(L.toda_points_select(_p(points), n, stride, int(x_col), _p(frame_offsets), batch, int(mode), _C.doubles(p),
                                       int(bool(invert)), int(bool(add_batch_col)), _p(out), _p(out_offsets), _p(ws),
                                       ws.numel(), _stream()), "toda_points_select")
-    _count(2)
     if trim:
         return out[:int(out_offsets[-1].item())], out_offsets
     return out, out_offsets
@@ -172,7 +168,6 @@ def gather_point_rows(points, rows):
     n, c = rows.shape[0], points.shape[1]
     out = torch.empty((n, c), dtype=torch.float32, device=points.device)
     _C.check(_C.lib().toda_gather_rows(_p(points), _p(rows), n, c, _p(out), _stream()), "toda_gather_rows")
-    _count(1)
     return out
 
 
@@ -222,7 +217,6 @@ def voxelize(points, frame_offsets, pc_range, voxel_size, max_points, max_voxels
                                   _C.floats(np.asarray(voxel_size, dtype=np.float32)), grid_c, max_points, max_voxels,
                                   order, _p(voxels), _p(coords), _p(num), _p(counts), _p(ws), ws.numel(), _stream())
     _C.check(rc, "toda_voxelize_hard")
-    _count(16 if order == ORDER_FIRST_APPEARANCE else 19)
     if trim:
         v = int(counts[batch].item())
         return voxels[:v], coords[:v], num[:v], counts
@@ -242,7 +236,6 @@ class _MeanVFE(torch.autograd.Function):
         with _timed("mean_vfe_fwd", V=v, K=k, F=f):
             _C.check(_C.lib().toda_mean_vfe_fwd(_p(voxels), _p(num_points), int(is_float), v, k, f, _p(out), _stream()),
                      "toda_mean_vfe_fwd")
-        _count(1)
         ctx.save_for_backward(num_points)
         ctx.shape = (v, k, f, is_float)
         return out
@@ -255,7 +248,6 @@ class _MeanVFE(torch.autograd.Function):
         dv = torch.empty((v, k, f), dtype=torch.float32, device=dout.device)
         _C.check(_C.lib().toda_mean_vfe_bwd(_p(dout), _p(num_points), int(is_float), v, k, f, _p(dv), _stream()),
                  "toda_mean_vfe_bwd")
-        _count(1)
         return dv, None
 
 
@@ -305,7 +297,6 @@ class OccupancyIndex:
         if self.coords is not None and self.n > 0:
             _C.check(_C.lib().toda_index_release(_p(self.buf), *self._dims(), _p(self.coords), self.n, _stream()),
                      "toda_index_release")
-            _count(1)
         if _index_occupant.get(self.key) is self:
             del _index_occupant[self.key]
 
@@ -314,7 +305,6 @@ class OccupancyIndex:
         coords = _need(coords, torch.int32, "coords")
         _C.check(_C.lib().toda_index_insert(_p(self.buf), *self._dims(), _p(coords), coords.shape[0], _stream()),
                  "toda_index_insert")
-        _count(1)
 
     def insert_strided(self, in_coords, ksize, stride, padding):
         self._acquire()
@@ -322,7 +312,6 @@ class OccupancyIndex:
         _C.check(_C.lib().toda_index_insert_strided(_p(self.buf), *self._dims(), _p(in_coords), in_coords.shape[0],
                                                     _C.ints(ksize), _C.ints(stride), _C.ints(padding), _stream()),
                  "toda_index_insert_strided")
-        _count(1)
 
     def build(self, cap, known_n=None):
         """Ranks the marked cells; returns canonical coords (n,4).  Host sync to read n unless known_n."""
@@ -332,7 +321,6 @@ class OccupancyIndex:
         with _timed("index_build", cells=self.batch * self.shape[0] * self.shape[1] * self.shape[2]):
             _C.check(_C.lib().toda_index_build(_p(self.buf), *self._dims(), _p(coords), cap, _p(n_out), _stream()),
                      "toda_index_build")
-        _count(5)
         self.n = int(n_out[0].item()) if known_n is None else int(known_n)
         self.coords = coords[:self.n]
         self.frame_counts = n_out
@@ -354,7 +342,6 @@ class OccupancyIndex:
         rows = torch.empty((coords.shape[0],), dtype=torch.int32, device=coords.device)
         _C.check(_C.lib().toda_index_rows(_p(self.buf), *self._dims(), _p(coords), coords.shape[0], _p(rows), _stream()),
                  "toda_index_rows")
-        _count(1)
         return rows
 
     def release(self):
@@ -423,7 +410,6 @@ def table_tile_plan(nbr, ksize, channels):
     with _timed("tile_plan", n=n, kvol=kvol):
         _C.check(L.toda_table_tile_plan(_p(nbr), n, kvol, ngroups, cap, _p(lidx), _p(rows), _p(cnt), _stream()),
                  "toda_table_tile_plan")
-    _count(1)
     return TilePlan(lidx, rows, cnt, ngroups, cap)
 
 
@@ -441,7 +427,6 @@ def rulebook_subm(index: OccupancyIndex, ksize, channels=None):
     with _timed("rulebook_subm", n=n, kvol=kvol):
         _C.check(_C.lib().toda_rulebook_subm(_p(index.buf), index.batch, *index.shape, _p(index.coords), n, _C.ints(ksize),
                                              _p(nbr), _stream()), "toda_rulebook_subm")
-    _count(1)
     rb = Rulebook(True, list(ksize), [1, 1, 1], [k // 2 for k in ksize], index.shape, index.shape, n, n, index.coords,
                   nbr, None)
     # even in raster order a 128-row tile often has no neighbour at all under whole groups of offsets (e.g. no dz = -1 /
@@ -479,7 +464,6 @@ def rulebook_sparse(index_in: OccupancyIndex, ksize, stride, padding, tag, cin=N
                                                index_in.batch, _p(index_in.coords), n_in, _p(out_coords), n_out,
                                                _C.ints(ksize), _C.ints(stride), _C.ints(padding), _p(nbr_fwd), _p(nbr_bwd),
                                                _stream()), "toda_rulebook_sparse")
-    _count(2)
     rb = Rulebook(False, list(ksize), list(stride), list(padding), index_in.shape, out_shape, n_in, n_out, out_coords,
                   nbr_fwd, nbr_bwd)
     rb.tile_masks = table_tile_masks(nbr_fwd) if (n_out > 0 and kvol <= 32) else None
@@ -517,7 +501,6 @@ def table_tile_masks(nbr):
     kvol, n = nbr.shape
     masks = torch.empty(((n + 127) // 128,), dtype=torch.int32, device=nbr.device)
     _C.check(_C.lib().toda_table_tile_masks(_p(nbr), n, kvol, _p(masks), _stream()), "toda_table_tile_masks")
-    _count(1)
     return masks
 
 
@@ -539,7 +522,6 @@ def _dgrad_parity_order(in_coords, nbr_bwd, stride, padding):
     order = torch.empty((n,), dtype=torch.int32, device=in_coords.device)
     _C.check(L.toda_parity_order(_p(in_coords), n, _C.ints(stride), _C.ints(padding), _p(order), None, _p(ws), ws.numel(),
                                  _stream()), "toda_parity_order")
-    _count(2)
     return order, nbr_bwd.index_select(1, order).contiguous()
 
 
@@ -569,7 +551,6 @@ def _repack(weight, transpose, mirror, want_bf16=False):
         out = torch.empty((kvol, cout, cin) if transpose else (kvol, cin, cout), dtype=torch.float32, device=weight.device)
         _C.check(_C.lib().toda_weight_repack(_p(weight), kvol, cin, cout, int(transpose), int(mirror), _p(out), _stream()),
                  "toda_weight_repack")
-        _count(1)
         if len(_repack_cache) > 512:
             _repack_cache.clear()
         hit = [weight._version, out, weakref.ref(weight), weight.data_ptr(), None]
@@ -580,7 +561,6 @@ def _repack(weight, transpose, mirror, want_bf16=False):
         kvol, ci, co = out.shape
         wb = torch.empty((co, kvol * max(ci, 16)), dtype=torch.bfloat16, device=out.device)
         _C.check(_C.lib().toda_weight_kmajor_bf16(_p(out), kvol, ci, co, _p(wb), _stream()), "toda_weight_kmajor_bf16")
-        _count(1)
         hit[4] = wb
     return out, hit[4]
 
@@ -616,7 +596,6 @@ def _conv_call(x, xb, cin, nbr, n_out, kvol, w, cout, bias, precision, what="con
                                             _p(pl.rows) if pl else None, _p(pl.cnt) if pl else None, pl.ngroups if pl else 0,
                                             pl.cap if pl else 0, _p(bn_sums), _p(w_bf16), precision, _p(ws),
                                             ws.numel() if ws is not None else 0, _stream()), "toda_spconv_fwd_plan")
-    _count(1)
     return y
 
 
@@ -674,7 +653,6 @@ def _conv_backward_impl(dy, dyb, x, weight, xb, rb, precision, need_dx, need_dw,
                     rb=id(rb)):
             _C.check(L.toda_spconv_wgrad(_p(x), _p(xb), rb.n_in, cin, _p(rb.nbr_fwd), rb.n_out, rb.kvol, _p(dy), _p(dyb),
                                          cout, _p(dw), _p(ws), ws.numel(), precision, _stream()), "toda_spconv_wgrad")
-        _count(2)
     if need_db:
         db = col_sum(dy)
     return dx, dw, db
@@ -715,7 +693,6 @@ def col_sum(t):
     L = _C.lib()
     ws = _workspace("bn", L.toda_bn_workspace_bytes(c), t.device)
     _C.check(L.toda_col_sum(_p(t), n, c, _p(out), _p(ws), ws.numel(), _stream()), "toda_col_sum")
-    _count(2)
     return out
 
 
@@ -763,9 +740,9 @@ def sync_group(bn):
 
 
 def _run_phases(phases, group):
-    """Drives a phase generator of a synchronized BatchNorm: every buffer it yields is all-reduced (SUM over `group`, in
-    place, on the current stream: NCCL orders it after the local kernels without a host synchronisation) before the
-    generator continues.  Returns the generator's result."""
+    """Drives a phase generator (_bn_forward_phases, _bn_backward_phases, _layer_forward_phases, _layer_backward_phases):
+    every buffer it yields -- only a synchronized BatchNorm's do -- is all-reduced (SUM over `group`, in place, on the current stream: NCCL orders it after
+    the local kernels without a host synchronisation) before the generator continues.  Returns the generator's result."""
     try:
         buf = next(phases)
         while True:
@@ -787,40 +764,59 @@ def _tape_mask(a, want_bf16):
     return a, (a.to(torch.bfloat16) if want_bf16 else None), mask.to(torch.float32)
 
 
-def _bn_forward_phases(y, gamma, beta, running_mean, running_var, eps, momentum, residual, relu, want_bf16, sums):
-    """Phase generator (see _run_phases) of a training-mode BatchNorm synchronized across processes: local sums (from the
-    conv epilogue's `sums` when given), yield them for the all-reduce, apply with the global statistics.
-    -> (a, a_bf16, y, mean, rstd, a_mask, global_sums) as _bn_forward_impl."""
+def _bn_forward_phases(y, gamma, beta, running_mean, running_var, eps, momentum, training, residual, relu, want_bf16, sums,
+                       need_grad, sync=False):
+    """Phase generator (see _run_phases) of BatchNorm (+ residual) (+ ReLU) over y.  Training: the fp64 sums of y (the conv
+    epilogue's `sums` when given), yielded with the row count for the all-reduce when `sync`, then one apply that derives
+    the coefficients and running statistics from them.  -> (a, a_bf16, y, mean, rstd, a_mask, global_sums): a_mask is what
+    the backward pass derives the ReLU mask from (`a` itself, except under a ReluMaskTape); global_sums is the all-reduced
+    buffer (None unless sync)."""
     y = _need(y.contiguous(), torch.float32, "bn input")
     n, c = y.shape
     dev = y.device
     L = _C.lib()
     scale, shift, mean, rstd = torch.empty((4, c), dtype=torch.float32, device=dev).unbind(0)
-    gsums = torch.empty((2 * c + 1,), dtype=torch.float64, device=dev)
-    ws = _workspace("bn", L.toda_bn_workspace_bytes(c), dev)
-    with _timed("bn_local_sums", n=n, c=c):
-        _C.check(L.toda_bn_local_sums(_p(y), _p(sums), n, c, _p(gsums), _p(ws), ws.numel(), _stream()), "toda_bn_local_sums")
-    _count(1 if (sums is not None or n == 0) else 2)
-    yield gsums
+    gsums = count = None
+    if training:
+        if sync or sums is None:
+            buf = torch.empty((2 * c + 1 if sync else 2 * c,), dtype=torch.float64, device=dev)
+            count = buf.data_ptr() + 16 * c if sync else None
+            ws = _workspace("bn", L.toda_bn_workspace_bytes(c), dev)
+            with _timed("bn_stats", n=n, c=c):
+                _C.check(L.toda_bn_local_sums(_p(y), _p(sums), n, c, _p(buf), count, _p(ws), ws.numel(), _stream()),
+                         "toda_bn_local_sums")
+            sums = buf
+        if sync:
+            yield sums
+            gsums = sums
+    else:
+        _C.check(L.toda_bn_eval_coeffs(_p(gamma), _p(beta), _p(running_mean), _p(running_var), float(eps), c, _p(scale),
+                                       _p(shift), _stream()), "toda_bn_eval_coeffs")
+        mean = running_mean
+        rstd = torch.rsqrt(running_var + eps) if need_grad else None
     res = residual.contiguous() if residual is not None else None
     a = torch.empty_like(y)
-    tape = _relu_tape is not None and relu
+    tape = _relu_tape is not None and relu      # pre-activation z, then the recorded / replayed mask (see ReluMaskTape)
     ab = torch.empty(y.shape, dtype=torch.bfloat16, device=dev) if (want_bf16 and not tape) else None
-    with _timed("bn_apply_global", n=n, c=c, residual=res is not None):
-        _C.check(L.toda_bn_apply_global(_p(y), n, c, _p(gsums), _p(gamma), _p(beta), float(eps), float(momentum),
-                                        _p(running_mean), _p(running_var), _p(scale), _p(shift), _p(mean), _p(rstd), _p(res),
-                                        0 if tape else int(relu), _p(a), _p(ab), _stream()), "toda_bn_apply_global")
-    _count(1)
+    act = 0 if tape else int(relu)
+    with _timed("bn_apply", n=n, c=c, residual=res is not None):
+        if training:
+            _C.check(L.toda_bn_apply_sums(_p(y), n, c, _p(sums), count, _p(gamma), _p(beta), float(eps), float(momentum),
+                                          _p(running_mean), _p(running_var), _p(scale), _p(shift), _p(mean), _p(rstd), _p(res),
+                                          act, _p(a), _p(ab), _stream()), "toda_bn_apply_sums")
+        else:
+            _C.check(L.toda_bn_apply(_p(y), n, c, _p(scale), _p(shift), _p(res), act, _p(a), _p(ab), _stream()), "toda_bn_apply")
     if tape:
         a, ab, mask = _tape_mask(a, want_bf16)
         return a, ab, y, mean, rstd, mask, gsums
     return a, ab, y, mean, rstd, a, gsums
 
 
-def _bn_backward_phases(da, y, a, gamma, mean, rstd, relu, has_res, want_bf16, gsums):
-    """Phase generator of the backward of _bn_forward_phases: local sums of g and g*xhat (and this process's dgamma /
-    dbeta), yield them for the all-reduce, dy from the global sums and the forward's global count.  da None = zeros (a
-    rank must join the collective even when no gradient reached it).  -> (dy, dy_bf16, dresidual, dgamma, dbeta)."""
+def _bn_backward_phases(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16, gsums=None):
+    """Phase generator of the backward of _bn_forward_phases -> (dy, dy_bf16, dresidual, dgamma, dbeta).  gsums: the forward's
+    global sums of a synchronized BatchNorm: the local sums of g and g*xhat (and this process's dgamma / dbeta) are then
+    yielded for the all-reduce, and dy follows from the global sums and the forward's global count.  da None = zeros (a
+    rank must join the collective even when no gradient reached it)."""
     n, c = y.shape
     da = da.contiguous() if da is not None else torch.zeros_like(y)
     L = _C.lib()
@@ -828,99 +824,27 @@ def _bn_backward_phases(da, y, a, gamma, mean, rstd, relu, has_res, want_bf16, g
     dyb = torch.empty(y.shape, dtype=torch.bfloat16, device=y.device) if want_bf16 else None
     dres = torch.empty_like(y) if has_res else None
     dgamma, dbeta = torch.empty((2, c), dtype=torch.float32, device=y.device).unbind(0)
+    ws = _workspace("bn", L.toda_bn_workspace_bytes(c), y.device)
+    if gsums is None:
+        with _timed("bn_bwd", n=n, c=c, residual=has_res):
+            _C.check(L.toda_bn_bwd(_p(da), _p(a), _p(y), n, c, _p(gamma), _p(mean), _p(rstd), int(relu), int(training),
+                                   _p(dy), _p(dyb), _p(dres), _p(dgamma), _p(dbeta), _p(ws), ws.numel(), _stream()), "toda_bn_bwd")
+        return dy, dyb, dres, dgamma, dbeta
     red = torch.empty((2 * c,), dtype=torch.float64, device=y.device)
-    ws = _workspace("bn", L.toda_bn_workspace_bytes(c), y.device)
-    with _timed("bn_bwd_reduce", n=n, c=c):
-        _C.check(L.toda_bn_bwd_reduce(_p(da), _p(a), _p(y), n, c, _p(mean), _p(rstd), int(relu), _p(red), _p(dgamma), _p(dbeta),
-                                      _p(ws), ws.numel(), _stream()), "toda_bn_bwd_reduce")
-    _count(2)
+    _C.check(L.toda_bn_bwd_reduce(_p(da), _p(a), _p(y), n, c, _p(mean), _p(rstd), int(relu), _p(red), _p(dgamma), _p(dbeta),
+                                  _p(ws), ws.numel(), _stream()), "toda_bn_bwd_reduce")
     yield red
-    with _timed("bn_bwd_finish", n=n, c=c, residual=has_res):
-        _C.check(L.toda_bn_bwd_finish(_p(da), _p(a), _p(y), n, c, _p(gamma), _p(mean), _p(rstd), int(relu), _p(red),
-                                      gsums.data_ptr() + 16 * c, _p(dy), _p(dyb), _p(dres), _stream()), "toda_bn_bwd_finish")
-    _count(1 if n > 0 else 0)
-    return dy, dyb, dres, dgamma, dbeta
-
-
-def _bn_forward_impl(y, gamma, beta, running_mean, running_var, eps, momentum, training, residual, relu, want_bf16, sums,
-                     need_grad, group=None):
-    """-> (a, a_bf16, y, mean, rstd, a_mask, global_sums): a_mask is what the backward pass derives the ReLU mask from
-    (`a` itself, except under a ReluMaskTape); global_sums is None unless the statistics are synchronized over `group`."""
-    if group is not None:
-        return _run_phases(_bn_forward_phases(y, gamma, beta, running_mean, running_var, eps, momentum, residual, relu,
-                                              want_bf16, sums if training else None), group)
-    y = _need(y.contiguous(), torch.float32, "bn input")
-    n, c = y.shape
-    dev = y.device
-    L = _C.lib()
-    scale = torch.empty((c,), dtype=torch.float32, device=dev)
-    shift = torch.empty_like(scale)
-    if training and sums is not None:
-        mean = torch.empty_like(scale)
-        rstd = torch.empty_like(scale)
-        _C.check(L.toda_bn_finalize_sums(_p(sums), n, c, _p(gamma), _p(beta), float(eps), float(momentum),
-                                         _p(running_mean), _p(running_var), _p(scale), _p(shift), _p(mean), _p(rstd),
-                                         _stream()), "toda_bn_finalize_sums")
-        _count(1)
-    elif training:
-        mean = torch.empty_like(scale)
-        rstd = torch.empty_like(scale)
-        ws = _workspace("bn", L.toda_bn_workspace_bytes(c), dev)
-        with _timed("bn_stats", n=n, c=c):
-            _C.check(L.toda_bn_stats(_p(y), n, c, _p(gamma), _p(beta), float(eps), float(momentum), _p(running_mean),
-                                     _p(running_var), _p(scale), _p(shift), _p(mean), _p(rstd), _p(ws), ws.numel(),
-                                     _stream()), "toda_bn_stats")
-        _count(2)
-    else:
-        _C.check(L.toda_bn_eval_coeffs(_p(gamma), _p(beta), _p(running_mean), _p(running_var), float(eps), c, _p(scale),
-                                       _p(shift), _stream()), "toda_bn_eval_coeffs")
-        _count(1)
-        mean = running_mean
-        rstd = torch.rsqrt(running_var + eps) if need_grad else None
-    res = residual.contiguous() if residual is not None else None
-    a = torch.empty_like(y)
-    ab = torch.empty(y.shape, dtype=torch.bfloat16, device=dev) if want_bf16 else None
-    if _relu_tape is not None and relu:
-        # pre-activation z, then the recorded / replayed mask (test instrument, see ReluMaskTape)
-        _C.check(L.toda_bn_apply(_p(y), n, c, _p(scale), _p(shift), _p(res), 0, _p(a), None, _stream()), "toda_bn_apply")
-        _count(1)
-        a, ab, mask = _tape_mask(a, want_bf16)
-        return a, ab, y, mean, rstd, mask, None
-    with _timed("bn_apply", n=n, c=c, residual=res is not None):
-        _C.check(L.toda_bn_apply(_p(y), n, c, _p(scale), _p(shift), _p(res), int(relu), _p(a), _p(ab), _stream()),
-                 "toda_bn_apply")
-    _count(1)
-    return a, ab, y, mean, rstd, a, None
-
-
-def _bn_backward_impl(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16, group=None, gsums=None):
-    """-> (dy, dy_bf16, dresidual, dgamma, dbeta).  group / gsums: the process group and the forward's global sums of a
-    synchronized BatchNorm (then da may be None)."""
-    if group is not None:
-        return _run_phases(_bn_backward_phases(da, y, a, gamma, mean, rstd, relu, has_res, want_bf16, gsums), group)
-    n, c = y.shape
-    da = da.contiguous()
-    L = _C.lib()
-    dy = torch.empty_like(y)
-    dyb = torch.empty(y.shape, dtype=torch.bfloat16, device=y.device) if want_bf16 else None
-    dres = torch.empty_like(y) if has_res else None
-    dgamma = torch.empty((c,), dtype=torch.float32, device=y.device)
-    dbeta = torch.empty_like(dgamma)
-    ws = _workspace("bn", L.toda_bn_workspace_bytes(c), y.device)
-    with _timed("bn_bwd", n=n, c=c, residual=has_res):
-        _C.check(L.toda_bn_bwd(_p(da), _p(a), _p(y), n, c, _p(gamma), _p(mean), _p(rstd), int(relu), int(training),
-                               _p(dy), _p(dyb), _p(dres), _p(dgamma), _p(dbeta), _p(ws), ws.numel(), _stream()),
-                 "toda_bn_bwd")
-    _count(3)
+    _C.check(L.toda_bn_bwd_finish(_p(da), _p(a), _p(y), n, c, _p(gamma), _p(mean), _p(rstd), int(relu), 1, _p(red),
+                                  gsums.data_ptr() + 16 * c, _p(dy), _p(dyb), _p(dres), _stream()), "toda_bn_bwd_finish")
     return dy, dyb, dres, dgamma, dbeta
 
 
 class _BNAct(torch.autograd.Function):
     @staticmethod
     def forward(ctx, y, gamma, beta, running_mean, running_var, eps, momentum, training, residual, relu, want_bf16, sums, group):
-        a, ab, y, mean, rstd, a_mask, gsums = _bn_forward_impl(y, gamma, beta, running_mean, running_var, eps, momentum,
-                                                               training, residual, relu, want_bf16, sums,
-                                                               y.requires_grad or gamma.requires_grad, group)
+        a, ab, y, mean, rstd, a_mask, gsums = _run_phases(
+            _bn_forward_phases(y, gamma, beta, running_mean, running_var, eps, momentum, training, residual, relu, want_bf16, sums,
+                        y.requires_grad or gamma.requires_grad, group is not None), group)
         ctx.save_for_backward(y, a_mask, gamma, mean, rstd, gsums)
         ctx.set_materialize_grads(False)      # the bf16 copy is non-differentiable: no zero tensor for it in backward
         ctx.cfg = (bool(training), bool(relu), residual is not None, bool(want_bf16))
@@ -935,8 +859,8 @@ class _BNAct(torch.autograd.Function):
             return (None,) * 13
         y, a, gamma, mean, rstd, gsums = ctx.saved_tensors
         training, relu, has_res, want_bf16 = ctx.cfg
-        dy, dyb, dres, dgamma, dbeta = _bn_backward_impl(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16,
-                                                         ctx.group, gsums)
+        dy, dyb, dres, dgamma, dbeta = _run_phases(_bn_backward_phases(da, y, a, gamma, mean, rstd, training, relu, has_res,
+                                                                       want_bf16, gsums), ctx.group)
         if dyb is not None:
             dy._toda_bf16 = (dyb, dy._version)     # picked up by the producing conv's backward (see _bf16_shadow_of)
         return dy, dgamma, dbeta, None, None, None, None, None, dres, None, None, None, None
@@ -956,51 +880,42 @@ def _layer_forward(x, x_bf16, weight, bias, rb, precision, gamma, beta, running_
                    residual, relu, want_bf16, need_grad=True, group=None):
     """conv -> BN (+residual) (+ReLU).  -> (a, a_bf16, saved) with saved = (x, x_bf16, weight, y, a_mask, gamma, mean, rstd,
     global_sums).  group: the process group of a synchronized BatchNorm (sync_group), else None (global_sums is then None)."""
-    if group is not None:
-        return _run_phases(_layer_forward_phases(x, x_bf16, weight, bias, rb, precision, gamma, beta, running_mean, running_var,
-                                                 eps, momentum, residual, relu, want_bf16, need_grad), group)
-    if not _fused_ok(training, need_grad):
-        y, sums, x, weight, x_bf16 = _conv_forward_impl(x, x_bf16, weight, bias, rb, precision, bool(training))
-        a, ab, y, mean, rstd, a_mask, _ = _bn_forward_impl(y, gamma, beta, running_mean, running_var, eps, momentum, training,
-                                                           residual, relu, want_bf16, sums, need_grad)
-        return a, ab, (x, x_bf16, weight, y, a_mask, gamma, mean, rstd, None)
-    args, tc, x, x_bf16, weight, y, a, ab, small, _keep = _layer_fwd_args(
-        x, x_bf16, weight, bias, rb, precision, gamma, beta, running_mean, running_var, eps, momentum, training, residual, relu,
-        want_bf16)
-    cout, n_out = y.shape[1], y.shape[0]
-    _C.check(_C.lib().toda_layer_fwd(ctypes.byref(args), _stream()), "toda_layer_fwd")
-    _count(2 if (tc and training and n_out > 0) else (3 if tc else 4))
-    mean = small[2 * cout:3 * cout] if training else running_mean
-    rstd = small[3 * cout:4 * cout] if training else None
-    return a, ab, (x, x_bf16, weight, y, a, gamma, mean, rstd, None)
+    return _run_phases(_layer_forward_phases(x, x_bf16, weight, bias, rb, precision, gamma, beta, running_mean, running_var, eps,
+                                             momentum, residual, relu, want_bf16, need_grad, training, group is not None), group)
 
 
 def _layer_forward_phases(x, x_bf16, weight, bias, rb, precision, gamma, beta, running_mean, running_var, eps, momentum,
-                          residual, relu, want_bf16, need_grad=True):
-    """Phase generator (see _run_phases) of _layer_forward in training mode with a synchronized BatchNorm:
-    toda_layer_fwd_stats, yield the local sums (double[2C+1]) for the all-reduce, toda_layer_fwd_apply."""
-    if not _fused_ok(True, need_grad):
-        y, sums, x, weight, x_bf16 = _conv_forward_impl(x, x_bf16, weight, bias, rb, precision, True)
+                          residual, relu, want_bf16, need_grad=True, training=True, sync=True):
+    """Phase generator (see _run_phases) of _layer_forward.  sync: the BatchNorm is synchronized across processes; the local
+    sums (double[2C+1], with the row count) are then yielded for the all-reduce between toda_layer_fwd_stats and
+    toda_layer_fwd_apply (else one toda_layer_fwd call, and global_sums is None)."""
+    if not _fused_ok(training, need_grad):
+        y, sums, x, weight, x_bf16 = _conv_forward_impl(x, x_bf16, weight, bias, rb, precision, bool(training))
         a, ab, y, mean, rstd, a_mask, gsums = yield from _bn_forward_phases(y, gamma, beta, running_mean, running_var, eps,
-                                                                            momentum, residual, relu, want_bf16, sums)
+                                                                            momentum, training, residual, relu, want_bf16, sums,
+                                                                            need_grad, sync)
         return a, ab, (x, x_bf16, weight, y, a_mask, gamma, mean, rstd, gsums)
-    args, tc, x, x_bf16, weight, y, a, ab, small, _keep = _layer_fwd_args(
-        x, x_bf16, weight, bias, rb, precision, gamma, beta, running_mean, running_var, eps, momentum, True, residual, relu,
+    args, x, x_bf16, weight, y, a, ab, small, _keep = _layer_fwd_args(
+        x, x_bf16, weight, bias, rb, precision, gamma, beta, running_mean, running_var, eps, momentum, training, residual, relu,
         want_bf16)
-    n_out, cout = y.shape
+    cout = y.shape[1]
     L = _C.lib()
-    gsums = torch.empty((2 * cout + 1,), dtype=torch.float64, device=y.device)
-    _C.check(L.toda_layer_fwd_stats(ctypes.byref(args), _p(gsums), _stream()), "toda_layer_fwd_stats")
-    _count(2 if tc else (1 if n_out == 0 else 3))
-    yield gsums
-    _C.check(L.toda_layer_fwd_apply(ctypes.byref(args), _p(gsums), _stream()), "toda_layer_fwd_apply")
-    _count(1)
-    return a, ab, (x, x_bf16, weight, y, a, gamma, small[2 * cout:3 * cout], small[3 * cout:4 * cout], gsums)
+    gsums = None
+    if sync:
+        gsums = torch.empty((2 * cout + 1,), dtype=torch.float64, device=y.device)
+        _C.check(L.toda_layer_fwd_stats(ctypes.byref(args), _p(gsums), _stream()), "toda_layer_fwd_stats")
+        yield gsums
+        _C.check(L.toda_layer_fwd_apply(ctypes.byref(args), _p(gsums), _stream()), "toda_layer_fwd_apply")
+    else:
+        _C.check(L.toda_layer_fwd(ctypes.byref(args), _stream()), "toda_layer_fwd")
+    mean = small[2 * cout:3 * cout] if training else running_mean
+    rstd = small[3 * cout:4 * cout] if training else None
+    return a, ab, (x, x_bf16, weight, y, a, gamma, mean, rstd, gsums)
 
 
 def _layer_fwd_args(x, x_bf16, weight, bias, rb, precision, gamma, beta, running_mean, running_var, eps, momentum, training,
                     residual, relu, want_bf16):
-    """Outputs and toda_layer_fwd_args of one fused layer -> (args, tc, x, x_bf16, weight, y, a, a_bf16, small, keep); keep
+    """Outputs and toda_layer_fwd_args of one fused layer -> (args, x, x_bf16, weight, y, a, a_bf16, small, keep); keep
     holds the other tensors the args point to: all of them must stay alive until the layer's calls are enqueued."""
     x = _need(x.contiguous(), torch.float32, "features")
     weight = _need(weight.contiguous(), torch.float32, "weight")
@@ -1033,19 +948,27 @@ def _layer_fwd_args(x, x_bf16, weight, bias, rb, precision, gamma, beta, running
         pl.ngroups if pl else 0, pl.cap if pl else 0, precision, _vp(ws), ws.numel() if ws is not None else 0,
         gamma.data_ptr(), beta.data_ptr(), float(eps), float(momentum), _vp(running_mean), _vp(running_var), int(bool(training)),
         _vp(res), int(bool(relu)), y.data_ptr(), sp + 16 * cout, sp, a.data_ptr(), _vp(ab), bws.data_ptr(), bws.numel())
-    return args, tc, x, x_bf16, weight, y, a, ab, small, (w, wb, ws, bws, res, b)
+    return args, x, x_bf16, weight, y, a, ab, small, (w, wb, ws, bws, res, b)
 
 
 def _layer_backward(da, saved, rb, precision, training, relu, has_res, has_bias, need_dx, need_dw, addend=None, group=None):
     """-> (dx, dw, db, dgamma, dbeta, dres).  addend: a gradient to be ADDED to dx (fused into the dgrad epilogue).
     group: the process group of a synchronized BatchNorm (then da may be None: zeros)."""
-    if group is not None:
-        return _run_phases(_layer_backward_phases(da, saved, rb, precision, relu, has_res, has_bias, need_dx, need_dw, addend),
-                           group)
-    x, xb, weight, y, a_mask, gamma, mean, rstd, _ = saved
+    return _run_phases(_layer_backward_phases(da, saved, rb, precision, relu, has_res, has_bias, need_dx, need_dw, addend,
+                                              training), group)
+
+
+def _layer_backward_phases(da, saved, rb, precision, relu, has_res, has_bias, need_dx, need_dw, addend=None, training=True):
+    """Phase generator of _layer_backward.  With a synchronized BatchNorm (global_sums in `saved`) the local sums of g and
+    g*xhat (double[2C]) are yielded for the all-reduce between toda_layer_bwd_reduce and toda_layer_bwd_finish, and dy uses
+    the forward's global count; dgamma / dbeta are this process's own (as torch.nn.SyncBatchNorm's: the gradient all-reduce
+    averages them)."""
+    x, xb, weight, y, a_mask, gamma, mean, rstd, gsums = saved
+    if da is None:
+        da = torch.zeros_like(y)
     if not _fused_ok(training, True):
-        dy, dyb, dres, dgamma, dbeta = _bn_backward_impl(da, y, a_mask, gamma, mean, rstd, training, relu, has_res,
-                                                         precision == CONV_BF16)
+        dy, dyb, dres, dgamma, dbeta = yield from _bn_backward_phases(da, y, a_mask, gamma, mean, rstd, training, relu, has_res,
+                                                                      precision == CONV_BF16, gsums)
         dx, dw, db = _conv_backward_impl(dy, dyb, x, weight, xb, rb, precision, need_dx, need_dw, has_bias)
         if addend is not None and dx is not None:
             dx = dx + addend
@@ -1053,36 +976,15 @@ def _layer_backward(da, saved, rb, precision, training, relu, has_res, has_bias,
     args, dx, dw, dres, small, _keep = _layer_bwd_args(da, saved, rb, precision, training, relu, has_res, has_bias, need_dx,
                                                        need_dw, addend)
     cout = y.shape[1]
-    _C.check(_C.lib().toda_layer_bwd(ctypes.byref(args), _stream()), "toda_layer_bwd")
-    _count(3 + (1 if need_dx else 0) + (2 if need_dw else 0) + (2 if has_bias else 0))
-    return dx, dw, (small[2 * cout:] if has_bias else None), small[:cout], small[cout:2 * cout], dres
-
-
-def _layer_backward_phases(da, saved, rb, precision, relu, has_res, has_bias, need_dx, need_dw, addend=None):
-    """Phase generator of _layer_backward with a synchronized BatchNorm: toda_layer_bwd_reduce, yield the local sums of g
-    and g*xhat (double[2C]) for the all-reduce, toda_layer_bwd_finish with the forward's global count.  dgamma / dbeta
-    are this process's own (as torch.nn.SyncBatchNorm's; the gradient all-reduce averages them)."""
-    x, xb, weight, y, a_mask, gamma, mean, rstd, gsums = saved
-    if da is None:
-        da = torch.zeros_like(y)
-    if not _fused_ok(True, True):
-        dy, dyb, dres, dgamma, dbeta = yield from _bn_backward_phases(da, y, a_mask, gamma, mean, rstd, relu, has_res,
-                                                                      precision == CONV_BF16, gsums)
-        dx, dw, db = _conv_backward_impl(dy, dyb, x, weight, xb, rb, precision, need_dx, need_dw, has_bias)
-        if addend is not None and dx is not None:
-            dx = dx + addend
-        return dx, dw, db, dgamma, dbeta, dres
-    args, dx, dw, dres, small, _keep = _layer_bwd_args(da, saved, rb, precision, True, relu, has_res, has_bias, need_dx,
-                                                       need_dw, addend)
-    cout = y.shape[1]
     L = _C.lib()
-    red = torch.empty((2 * cout,), dtype=torch.float64, device=y.device)
-    _C.check(L.toda_layer_bwd_reduce(ctypes.byref(args), _p(red), _stream()), "toda_layer_bwd_reduce")
-    _count(2)
-    yield red
-    _C.check(L.toda_layer_bwd_finish(ctypes.byref(args), _p(red), gsums.data_ptr() + 16 * cout, _stream()),
-             "toda_layer_bwd_finish")
-    _count(1 + (1 if need_dx else 0) + (2 if need_dw else 0) + (2 if has_bias else 0))
+    if gsums is None:
+        _C.check(L.toda_layer_bwd(ctypes.byref(args), _stream()), "toda_layer_bwd")
+    else:
+        red = torch.empty((2 * cout,), dtype=torch.float64, device=y.device)
+        _C.check(L.toda_layer_bwd_reduce(ctypes.byref(args), _p(red), _stream()), "toda_layer_bwd_reduce")
+        yield red
+        _C.check(L.toda_layer_bwd_finish(ctypes.byref(args), _p(red), gsums.data_ptr() + 16 * cout, _stream()),
+                 "toda_layer_bwd_finish")
     return dx, dw, (small[2 * cout:] if has_bias else None), small[:cout], small[cout:2 * cout], dres
 
 
@@ -1208,16 +1110,21 @@ class _ResBlock(torch.autograd.Function):
                 None, None)
 
 
+def _bn_call(bn):
+    """-> (training, group) of one call of BatchNorm module `bn` (group: see sync_group); a training call counts the batch
+    in num_batches_tracked, as torch.nn.BatchNorm1d does."""
+    group = sync_group(bn)
+    training = bn.training or bn.running_mean is None
+    if training and bn.running_mean is not None and bn.num_batches_tracked is not None:
+        bn.num_batches_tracked += 1
+    return training, group
+
+
 def res_block(x, x_bf16, conv1_w, conv1_b, bn1, conv2_w, conv2_b, bn2, rb, precision, want_bf16=False):
     """SparseBasicBlock on feature rows; bn1 / bn2 are the nn.BatchNorm1d (or nn.SyncBatchNorm) modules.
     -> (out, out_bf16 or None)"""
-    group1, group2 = sync_group(bn1), sync_group(bn2)
-    training = bn1.training or bn1.running_mean is None
-    if training:
-        for bn in (bn1, bn2):
-            if bn.running_mean is not None and bn.num_batches_tracked is not None:
-                bn.num_batches_tracked += 1
-    assert bn1.eps == bn2.eps and bn1.momentum == bn2.momentum
+    (training, group1), (training2, group2) = _bn_call(bn1), _bn_call(bn2)
+    assert bn1.eps == bn2.eps and bn1.momentum == bn2.momentum and training == training2
     return _ResBlock.apply(x, x_bf16, conv1_w, conv1_b, bn1.weight, bn1.bias, bn1.running_mean, bn1.running_var, conv2_w, conv2_b,
                            bn2.weight, bn2.bias, bn2.running_mean, bn2.running_var, rb, precision, bn1.eps, bn1.momentum, training,
                            want_bf16, group1, group2)
@@ -1226,10 +1133,7 @@ def res_block(x, x_bf16, conv1_w, conv1_b, bn1, conv2_w, conv2_b, bn2, rb, preci
 def conv_bn_act(x, weight, bias, rb, precision, bn: torch.nn.BatchNorm1d, residual=None, relu=True, x_bf16=None, want_bf16=False):
     """Fused-node version of bn_act(sparse_conv(x, ...), bn, residual, relu).  -> (a, a_bf16 or None).  An nn.SyncBatchNorm
     in training mode reduces its statistics over its process group (sync_group)."""
-    group = sync_group(bn)
-    training = bn.training or bn.running_mean is None
-    if training and bn.running_mean is not None and bn.num_batches_tracked is not None:
-        bn.num_batches_tracked += 1
+    training, group = _bn_call(bn)
     return _ConvBNAct.apply(x, x_bf16, weight, bias, rb, precision, bn.weight, bn.bias, bn.running_mean, bn.running_var, bn.eps,
                             bn.momentum, training, residual, relu, want_bf16, group)
 
@@ -1239,10 +1143,7 @@ def bn_act(y, bn: torch.nn.BatchNorm1d, residual=None, relu=True, want_bf16=Fals
     (spconv_backbone.py L23-24, L54-64).  want_bf16: also return the bf16 copy written by the same pass.
     sums: per-channel (sum, sum of squares) of y from the producing convolution's epilogue (skips the statistics pass).
     An nn.SyncBatchNorm in training mode reduces its statistics over its process group (sync_group)."""
-    group = sync_group(bn)
-    training = bn.training or bn.running_mean is None
-    if training and bn.running_mean is not None and bn.num_batches_tracked is not None:
-        bn.num_batches_tracked += 1
+    training, group = _bn_call(bn)
     a, ab = _BNAct.apply(y, bn.weight, bn.bias, bn.running_mean, bn.running_var, bn.eps, bn.momentum, training, residual,
                          relu, want_bf16, sums if training else None, group)
     return (a, ab) if want_bf16 else a
@@ -1261,7 +1162,6 @@ class _BEVScatter(torch.autograd.Function):
         with _timed("bev_scatter_fwd", n=n, c=c, out_elems=out.numel()):
             _C.check(_C.lib().toda_bev_scatter_fwd(_p(features), _p(coords), n, c, batch, d, h, w, _p(out), _stream()),
                      "toda_bev_scatter_fwd")
-        _count(2)
         ctx.save_for_backward(coords)
         ctx.dims = (n, c, batch, d, h, w)
         return out
@@ -1275,7 +1175,6 @@ class _BEVScatter(torch.autograd.Function):
         with _timed("bev_scatter_bwd", n=n, c=c):
             _C.check(_C.lib().toda_bev_scatter_bwd(_p(dout), _p(coords), n, c, batch, d, h, w, _p(df), _stream()),
                      "toda_bev_scatter_bwd")
-        _count(1)
         return df, None, None, None, None, None
 
 
@@ -1291,7 +1190,6 @@ class _GatherRows(torch.autograd.Function):
         n, c = rows.shape[0], x.shape[1]
         out = torch.empty((n, c), dtype=torch.float32, device=x.device)
         _C.check(_C.lib().toda_gather_rows(_p(x), _p(rows), n, c, _p(out), _stream()), "toda_gather_rows")
-        _count(1)
         ctx.save_for_backward(inverse_rows)
         return out
 
@@ -1302,7 +1200,6 @@ class _GatherRows(torch.autograd.Function):
         n, c = inv.shape[0], dout.shape[1]
         dx = torch.empty((n, c), dtype=torch.float32, device=dout.device)
         _C.check(_C.lib().toda_gather_rows(_p(dout), _p(inv), n, c, _p(dx), _stream()), "toda_gather_rows")
-        _count(1)
         return dx, None, None
 
 
