@@ -98,6 +98,29 @@ int toda_points_select(const float *points, int n, int stride, int x_col, const 
                        void *workspace, size_t workspace_bytes, void *stream);
 
 /* ------------------------------------------------------------------------------------------
+ * K0 world augmentations: the point side of DataAugmentor.random_world_flip / random_world_rotation /
+ * random_world_scaling (pcdet/datasets/augmentor/data_augmentor.py L43-80, augmentor_utils.py L8-82; OpenPCDet v0.5.2)
+ * for a whole batch of frames in one elementwise launch.  The random draws are made on the host; each step carries
+ * per-frame parameters, params_host[(step * nb + b) * 2 + {0, 1}] with nb = batch (1 when frame_offsets is NULL):
+ *   TODA_WORLD_FLIP_X  {enabled, -}: negate y (random_flip_along_x)     TODA_WORLD_FLIP_Y  {enabled, -}: negate x
+ *   TODA_WORLD_ROTATE  {cos, sin}: common_utils.rotate_points_along_z with cos / sin of the float32 angle as torch.cos /
+ *        torch.sin give them; the product is rounded as torch.matmul on the CPU rounds it, which depends on the frame's
+ *        row count off[b+1] - off[b]: unfused products and sums from a zero accumulator for <= 44 rows (ATen's naive bmm),
+ *        a chain of fmas for >= 45 (BLAS).  The 0 and 1 entries of the rotation matrix take part in both.
+ *   TODA_WORLD_SCALE   {noise, -}: points[:, :3] *= noise, i.e. x * float32(noise)
+ * Steps apply in list order (n_steps <= 4), float32 op by op, so the result is bit-identical to the reference's.  A
+ * scaling step whose range is narrower than 1e-3 draws nothing in the reference and is left out of the list.
+ *   points [n][stride] fp32, x, y, z at columns x_col..x_col+2; frame_offsets int32[batch+1] device or NULL (one frame),
+ *   batch <= 64; out [n][stride]: every other column copied bit for bit.  No workspace, deterministic.
+ * ------------------------------------------------------------------------------------------ */
+#define TODA_WORLD_FLIP_X 0
+#define TODA_WORLD_FLIP_Y 1
+#define TODA_WORLD_ROTATE 2
+#define TODA_WORLD_SCALE 3
+int toda_points_world_transform(const float *points, int n, int stride, int x_col, const int32_t *frame_offsets, int batch,
+                                int n_steps, const int *kinds_host, const float *params_host, float *out, void *stream);
+
+/* ------------------------------------------------------------------------------------------
  * K1 hard voxelizer.  Replaces spconv.utils.Point2VoxelCPU3d.point_to_voxel as called from
  * pcdet/datasets/processor/data_processor.py L36-42, L54 (VoxelGeneratorWrapper) /
  * L115-143 (transform_points_to_voxels), for a whole batch of frames in one call.

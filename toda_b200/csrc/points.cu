@@ -253,3 +253,134 @@ extern "C" int toda_points_select(const float *points, int n, int stride, int x_
     TODA_LAUNCH_OK();
     return TODA_OK;
 }
+
+// ------------------------------------------------------------------------------------------------
+// World augmentations (DataAugmentor random_world_flip / _rotation / _scaling, augmentor_utils.py L8-82), applied to the
+// points of a whole batch in one elementwise pass.  Each step has per-frame parameters drawn on the host.  The float32
+// arithmetic is the reference's, op by op:
+//   flip x / flip y   points[:, 1] = -points[:, 1] / points[:, 0] = -points[:, 0]: a sign flip
+//   scale             points[:, :3] *= noise: x * float32(noise)
+//   rotate            common_utils.rotate_points_along_z: torch.matmul(xyz, [[c, s, 0], [-s, c, 0], [0, 0, 1]]) on the CPU,
+//                     which for a (1, N, 3) x (1, 3, 3) product takes one of two paths by the frame's row count:
+//                       N <= 44  ATen's naive bmm loop (3 * N * 3 < 400): acc = 0; acc += v[k] * R[k][j], every op rounded
+//                       N >= 45  the BLAS kernel:                          acc = fma(v[k], R[k][j], acc) from acc = 0
+//                     The zero and one entries of R take part, so z' = (x*0 + y*0) + z*1 and x' carries + z*0 (signed zeros,
+//                     inf and NaN come out as torch gives them).
+// Tile of kTfRows rows staged through shared memory: coalesced loads and stores, one thread per row in between.
+namespace {
+
+constexpr int kTfRows = 128;                   // rows per CTA = threads per CTA
+constexpr int kTfMaxSteps = 4;
+constexpr int kTfMaxBatch = 64;
+constexpr int kTfNaiveMaxRows = 44;            // largest frame that torch rotates with the naive loop
+constexpr int kTfUnroll = 8;                   // loads in flight per thread
+
+struct TfParams {
+    int n_steps;
+    int kind[kTfMaxSteps];
+    float2 prm[kTfMaxSteps][kTfMaxBatch];      // flip: (enabled, -); rotate: (cos, sin); scale: (noise, -)
+    float zero, one;                           // the constant entries of R, passed in so that no product with them is folded
+};
+
+__device__ __forceinline__ float neg_bits(float v) { return __int_as_float(__float_as_int(v) ^ 0x80000000); }
+
+// torch.matmul of the row (x, y, z) with column (r0, r1, r2) of the rotation matrix, as one of the two CPU paths rounds it
+__device__ __forceinline__ float rot_dot(bool fused, float x, float y, float z, float r0, float r1, float r2, float zero) {
+    if (fused) return __fmaf_rn(z, r2, __fmaf_rn(y, r1, __fmaf_rn(x, r0, zero)));
+    return __fadd_rn(__fadd_rn(__fadd_rn(zero, __fmul_rn(x, r0)), __fmul_rn(y, r1)), __fmul_rn(z, r2));
+}
+
+__global__ void __launch_bounds__(kTfRows) world_transform_kernel(const float *__restrict__ points, int n, int stride, int x_col,
+                                                                 const int32_t *__restrict__ frame_offsets, int batch,
+                                                                 const TfParams p, float *__restrict__ out) {
+    extern __shared__ float tile[];            // [kTfRows][stride]
+    __shared__ int off_s[kTfMaxBatch + 1];
+    const int row0 = blockIdx.x * kTfRows;
+    const int rows = min(kTfRows, n - row0);
+    const int total = rows * stride;
+    const float *src = points + (size_t)row0 * stride;
+    float *dst = out + (size_t)row0 * stride;
+    if (frame_offsets) {
+        if ((int)threadIdx.x <= batch) off_s[threadIdx.x] = frame_offsets[threadIdx.x];
+    } else if (threadIdx.x == 0) {
+        off_s[0] = 0;
+        off_s[1] = n;
+    }
+    for (int e0 = 0; e0 < total; e0 += kTfRows * kTfUnroll) {
+        float v[kTfUnroll];
+#pragma unroll
+        for (int u = 0; u < kTfUnroll; ++u) {
+            const int e = e0 + u * kTfRows + threadIdx.x;
+            if (e < total) v[u] = __ldg(src + e);
+        }
+#pragma unroll
+        for (int u = 0; u < kTfUnroll; ++u) {
+            const int e = e0 + u * kTfRows + threadIdx.x;
+            if (e < total) tile[e] = v[u];
+        }
+    }
+    __syncthreads();
+    if ((int)threadIdx.x < rows) {
+        const int i = row0 + threadIdx.x;
+        const int nb = frame_offsets ? batch : 1;
+        int lo = 0, hi = nb;                   // frame b: off[b] <= i < off[b+1] (the last such b: empty frames are skipped)
+        while (hi - lo > 1) {
+            const int mid = (lo + hi) >> 1;
+            if (off_s[mid] <= i) lo = mid; else hi = mid;
+        }
+        const bool fused = off_s[lo + 1] - off_s[lo] > kTfNaiveMaxRows;
+        float *r = tile + threadIdx.x * stride + x_col;
+        float x = r[0], y = r[1], z = r[2];
+        for (int s = 0; s < p.n_steps; ++s) {
+            const float2 q = p.prm[s][lo];
+            const int kind = p.kind[s];
+            if (kind == TODA_WORLD_FLIP_X) {
+                if (q.x != 0.f) y = neg_bits(y);
+            } else if (kind == TODA_WORLD_FLIP_Y) {
+                if (q.x != 0.f) x = neg_bits(x);
+            } else if (kind == TODA_WORLD_ROTATE) {
+                const float c = q.x, sn = q.y;
+                const float xr = rot_dot(fused, x, y, z, c, neg_bits(sn), p.zero, p.zero);
+                const float yr = rot_dot(fused, x, y, z, sn, c, p.zero, p.zero);
+                const float zr = rot_dot(fused, x, y, z, p.zero, p.zero, p.one, p.zero);
+                x = xr; y = yr; z = zr;
+            } else {
+                x = __fmul_rn(x, q.x); y = __fmul_rn(y, q.x); z = __fmul_rn(z, q.x);
+            }
+        }
+        r[0] = x; r[1] = y; r[2] = z;
+    }
+    __syncthreads();
+    for (int e = threadIdx.x; e < total; e += kTfRows) dst[e] = tile[e];
+}
+
+}  // namespace
+
+extern "C" int toda_points_world_transform(const float *points, int n, int stride, int x_col, const int32_t *frame_offsets,
+                                           int batch, int n_steps, const int *kinds_host, const float *params_host, float *out,
+                                           void *stream) {
+    TODA_CHECK_ARG(n >= 0 && stride >= 3 && stride <= 63 && x_col >= 0 && x_col + 2 < stride,
+                   "points_world_transform: bad layout n=%d stride=%d x_col=%d", n, stride, x_col);
+    TODA_CHECK_ARG(!frame_offsets || (batch >= 1 && batch <= kTfMaxBatch), "points_world_transform: batch %d outside [1, %d]",
+                   batch, kTfMaxBatch);
+    TODA_CHECK_ARG(n_steps >= 0 && n_steps <= kTfMaxSteps, "points_world_transform: %d steps (at most %d)", n_steps, kTfMaxSteps);
+    TODA_CHECK_ARG(n_steps == 0 || (kinds_host && params_host), "points_world_transform: null step list");
+    TODA_CHECK_ARG(n == 0 || (points && out), "points_world_transform: null pointer");
+    const int nb = frame_offsets ? batch : 1;
+    TfParams p = {};
+    p.n_steps = n_steps;
+    p.zero = 0.f;
+    p.one = 1.f;
+    for (int s = 0; s < n_steps; ++s) {
+        const int k = kinds_host[s];
+        TODA_CHECK_ARG(k >= TODA_WORLD_FLIP_X && k <= TODA_WORLD_SCALE, "points_world_transform: bad step kind %d", k);
+        p.kind[s] = k;
+        for (int b = 0; b < nb; ++b) p.prm[s][b] = make_float2(params_host[2 * (s * nb + b)], params_host[2 * (s * nb + b) + 1]);
+    }
+    if (n == 0) return TODA_OK;
+    const size_t smem = (size_t)kTfRows * stride * sizeof(float);
+    world_transform_kernel<<<ceil_div(n, kTfRows), kTfRows, smem, (cudaStream_t)stream>>>(points, n, stride, x_col, frame_offsets,
+                                                                                          batch, p, out);
+    TODA_LAUNCH_OK();
+    return TODA_OK;
+}

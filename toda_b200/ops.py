@@ -161,6 +161,53 @@ def points_select(points, frame_offsets, mode, params, invert=False, add_batch_c
     return out, out_offsets
 
 
+WORLD_FLIP_X, WORLD_FLIP_Y, WORLD_ROTATE, WORLD_SCALE = 0, 1, 2, 3
+WORLD_MAX_STEPS = 4
+WORLD_MAX_BATCH = 64
+
+
+def points_world_transform(points, frame_offsets, steps, x_col=0):
+    """The point side of pcdet's world augmentations (random_world_flip / _rotation / _scaling) for a batch of frames,
+    bit-identical to the reference's float32 arithmetic (see include/toda_b200.h).  Returns a new (N, stride) tensor.
+
+    points (N, stride) float32 CUDA with x, y, z at x_col..x_col+2; frame_offsets int32 (B+1) CUDA tensor or None (one
+    frame).  steps: at most 4 (kind, per-frame values) pairs applied in order, one value per frame:
+      WORLD_FLIP_X / WORLD_FLIP_Y  whether the flip is enabled
+      WORLD_ROTATE                 (cos, sin) of the float32 angle as torch.cos / torch.sin give them
+      WORLD_SCALE                  the scale factor (rounded to float32)
+    """
+    points = _need(points, torch.float32, "points")
+    if points.dim() != 2:
+        raise ValueError("points must be (N, stride)")
+    n, stride = points.shape
+    if not (0 <= x_col and x_col + 2 < stride <= 63):
+        raise ValueError(f"points_world_transform: x, y, z at columns {x_col}..{x_col + 2} do not fit stride {stride} (<= 63)")
+    batch = 1
+    if frame_offsets is not None:
+        frame_offsets = _need(frame_offsets, torch.int32, "frame_offsets")
+        batch = frame_offsets.numel() - 1
+        if not 1 <= batch <= WORLD_MAX_BATCH:
+            raise ValueError(f"points_world_transform: batch {batch} outside [1, {WORLD_MAX_BATCH}]")
+    if len(steps) > WORLD_MAX_STEPS:
+        raise ValueError(f"points_world_transform: {len(steps)} steps (at most {WORLD_MAX_STEPS})")
+    kinds, params = [], np.zeros((len(steps), batch, 2), np.float32)
+    for s, (kind, values) in enumerate(steps):
+        if kind not in (WORLD_FLIP_X, WORLD_FLIP_Y, WORLD_ROTATE, WORLD_SCALE):
+            raise ValueError(f"points_world_transform: unknown step kind {kind!r}")
+        v = np.asarray(values, dtype=np.float32).reshape(batch, -1)
+        if v.shape[1] != (2 if kind == WORLD_ROTATE else 1):
+            raise ValueError(f"points_world_transform: step {s} needs {2 if kind == WORLD_ROTATE else 1} value(s) per frame for "
+                             f"{batch} frame(s), got {np.shape(values)}")
+        kinds.append(int(kind))
+        params[s, :, :v.shape[1]] = v
+    out = torch.empty_like(points)
+    with _timed("points_world_transform", n=n, stride=stride, steps=len(steps)):
+        _C.check(_C.lib().toda_points_world_transform(_p(points), n, stride, int(x_col), _p(frame_offsets), batch, len(kinds),
+                                                      _C.ints(kinds or [0]), _C.floats(params.reshape(-1).tolist() or [0.0]),
+                                                      _p(out), _stream()), "toda_points_world_transform")
+    return out
+
+
 def gather_point_rows(points, rows):
     """out[i] = points[rows[i]] (numpy `points[idx]`): shuffle_points / mixup prefixes for a given index vector."""
     points = _need(points, torch.float32, "points")

@@ -28,8 +28,11 @@ class _Handle:
 
 
 class InputPipeline:
-    def __init__(self, vfe, backbone, device, reserve_bytes=8 << 30):
-        self.vfe, self.backbone = vfe, backbone
+    def __init__(self, vfe, backbone, device, reserve_bytes=8 << 30, preprocess=None):
+        """preprocess: optional callable batch_dict -> batch_dict run on the side stream after the inputs are staged and
+        before the VFE, e.g. the device augmentations and point pre-steps `lambda bd: pp.forward(aug.forward(bd))`.  Run
+        before submit() instead, those would sit on the main stream behind the previous batch's backward pass."""
+        self.vfe, self.backbone, self.preprocess = vfe, backbone, preprocess
         self.device = torch.device(device)
         lo, hi = torch.cuda.Stream.priority_range()      # (lowest, highest): highest is the numerically smaller one
         self.stream = torch.cuda.Stream(self.device, priority=hi)
@@ -68,6 +71,8 @@ class InputPipeline:
                         staged.append(t)
                     bd[key] = t
             before = set(id(v) for v in bd.values() if torch.is_tensor(v))
+            if self.preprocess is not None:
+                bd = self.preprocess(bd)
             bd = self.vfe(bd)
             plan = None
             if bd.get("voxel_coords_canonical", False):
