@@ -242,9 +242,18 @@ int toda_spconv_fwd_plan(const float *x, const void *x_bf16, int n_in, int cin, 
  * ([cout][kvol*max(cin,16)] bf16), so that a caller that caches them per optimizer step saves the conversion per call. */
 int toda_weight_kmajor_bf16(const float *w, int kvol, int cin, int cout, void *w_bf16, void *stream);
 size_t toda_spconv_wgrad_workspace_bytes(int n_in, int n_out, int kvol, int cin, int cout, int precision);
+/* tile_masks (optional, may be NULL): the toda_table_tile_masks words of `nbr`.  The tensor-core weight gradient then
+ * skips, per 128-row tile, the groups of kernel offsets that have no neighbour there; NULL: every group is computed. */
 int toda_spconv_wgrad(const float *x, const void *x_bf16, int n_in, int cin, const int32_t *nbr, int n_out, int kvol,
-                      const float *dy, const void *dy_bf16, int cout, float *dw_param, void *workspace,
-                      size_t workspace_bytes, int precision, void *stream);
+                      const uint32_t *tile_masks, const float *dy, const void *dy_bf16, int cout, float *dw_param,
+                      void *workspace, size_t workspace_bytes, int precision, void *stream);
+/* How the tensor-core weight gradient splits the rows of one call: it runs groups x splits CTAs (one offset group, one
+ * row range each) and cuts each group's rows into `splits` ranges of whole row chunks (128 rows, 64 when cout = 128)
+ * holding equal shares of the group's live (chunk, offset group) items, computed on the device from tile_masks (NULL:
+ * every item live).  Writes *groups and *splits and, when row_begin (device int32[groups*splits]) is given, the first
+ * row of every range at row_begin[group*splits + split] (a range ends where the next begins, the last at n_out). */
+int toda_spconv_wgrad_row_splits(const uint32_t *tile_masks, int n_out, int kvol, int cin, int cout, int *groups,
+                                 int *splits, int32_t *row_begin, void *stream);
 
 /* ------------------------------------------------------------------------------------------
  * K8 BatchNorm1d(eps, momentum) + ReLU (+ residual) over (N_active, C) rows
@@ -287,13 +296,17 @@ int toda_bn_apply_sums(const float *y, int n, int channels, const double *sums, 
 int toda_bn_bwd_reduce(const float *da, const float *a, const float *y, int n, int channels, const float *save_mean,
                        const float *save_rstd, int relu, double *red, float *dgamma, float *dbeta, void *workspace,
                        size_t workspace_bytes, void *stream);
+/* dbias (optional, may be NULL): sum_rows dy[:,c], the gradient of a bias added before the BatchNorm, summed in the same
+ * pass from fixed-order fp64 partials (workspace: toda_bn_workspace_bytes(channels), needed only with dbias). */
 int toda_bn_bwd_finish(const float *da, const float *a, const float *y, int n, int channels, const float *gamma,
                        const float *save_mean, const float *save_rstd, int relu, int training, const double *red,
-                       const double *count, float *dy, void *dy_bf16, float *dresidual, void *stream);
+                       const double *count, float *dy, void *dy_bf16, float *dresidual, float *dbias, void *workspace,
+                       size_t workspace_bytes, void *stream);
 int toda_bn_bwd(const float *da, const float *a, const float *y, int n, int channels, const float *gamma,
                 const float *save_mean, const float *save_rstd, int relu, int training, float *dy, void *dy_bf16,
-                float *dresidual, float *dgamma, float *dbeta, void *workspace, size_t workspace_bytes, void *stream);
-/* column sums: dbias[c] = sum_rows dy[:,c] */
+                float *dresidual, float *dgamma, float *dbeta, float *dbias, void *workspace, size_t workspace_bytes,
+                void *stream);
+/* column sums: dbias[c] = sum_rows dy[:,c] (the bias gradient of a convolution with no BatchNorm after it) */
 int toda_col_sum(const float *dy, int n, int channels, float *out, void *workspace, size_t workspace_bytes,
                  void *stream);
 
@@ -328,7 +341,8 @@ typedef struct {
     const int32_t *dgrad_out_rows /* optional */; const uint32_t *dgrad_masks /* optional */;
     const uint16_t *dplan_lidx /* optional */; const int32_t *dplan_rows; const int32_t *dplan_cnt; int dplan_groups, dplan_cap;
     const float *addend /* optional */; float *dx;
-    int need_dw; const int32_t *nbr_fwd; float *dw; void *wgrad_ws; size_t wgrad_ws_bytes;
+    int need_dw; const int32_t *nbr_fwd; const uint32_t *fwd_masks /* optional: tile masks of nbr_fwd */; float *dw;
+    void *wgrad_ws; size_t wgrad_ws_bytes;
     int need_db; float *db;
     int precision; void *conv_ws; size_t conv_ws_bytes;
 } toda_layer_bwd_args;

@@ -23,9 +23,9 @@ for n in names[:12] + names[-6:]:
 from toda_b200 import ops
 orig = ops._bn_backward_phases
 log = []
-def spy(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16, gsums=None):
-    out = yield from orig(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16, gsums)
-    dy, dyb, dres, dgamma, dbeta = out
+def spy(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16, gsums=None, want_db=False):
+    out = yield from orig(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16, gsums, want_db)
+    dy, dyb, dres, dgamma, dbeta, _ = out
     g = da * (a > 0) if relu else da
     ref_db = g.double().sum(0)
     xhat = (y.double() - mean.double()) * rstd.double()
@@ -39,9 +39,9 @@ r = PU.run_backbone(net, hc, vf, vc, 2, cot=cot, train=True)
 for l in log[:8]: print(l)
 # ---- compare d(x_conv4) between oracle and GPU
 das = []
-def spy2(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16, gsums=None):
+def spy2(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16, gsums=None, want_db=False):
     das.append((da.detach().cpu().numpy().copy(), a.detach().cpu().numpy().copy()))
-    return (yield from orig(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16, gsums))
+    return (yield from orig(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16, gsums, want_db))
 ops._bn_backward_phases = spy2
 twin, net = PU.build_pair("VoxelResBackBone8x", nf, g["grid_size"], seed=int(g["seed"]))
 net.train(); twin.train()

@@ -57,7 +57,9 @@ SIGNATURES = {
     "toda_layer_bwd_reduce": (c_int, [c_vp, c_vp, c_vp]),
     "toda_layer_bwd_finish": (c_int, [c_vp, c_vp, c_vp, c_vp]),
     "toda_spconv_wgrad_workspace_bytes": (c_sz, [c_int] * 6),
-    "toda_spconv_wgrad": (c_int, [c_vp, c_vp, c_int, c_int, c_vp, c_int, c_int, c_vp, c_vp, c_int, c_vp, c_vp, c_sz, c_int, c_vp]),
+    "toda_spconv_wgrad": (c_int, [c_vp, c_vp, c_int, c_int, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_vp, c_vp, c_sz, c_int,
+                                  c_vp]),
+    "toda_spconv_wgrad_row_splits": (c_int, [c_vp, c_int, c_int, c_int, c_int, _IP, _IP, c_vp, c_vp]),
     "toda_bn_workspace_bytes": (c_sz, [c_int]),
     "toda_bn_local_sums": (c_int, [c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "toda_bn_eval_coeffs": (c_int, [c_vp, c_vp, c_vp, c_vp, c_f32, c_int, c_vp, c_vp, c_vp]),
@@ -65,10 +67,10 @@ SIGNATURES = {
     "toda_bn_apply_sums": (c_int, [c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_f32, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
                                    c_vp, c_int, c_vp, c_vp, c_vp]),
     "toda_bn_bwd": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp,
-                            c_vp, c_sz, c_vp]),
+                            c_vp, c_vp, c_sz, c_vp]),
     "toda_bn_bwd_reduce": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "toda_bn_bwd_finish": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_vp, c_vp, c_vp,
-                                   c_vp]),
+                                   c_vp, c_vp, c_sz, c_vp]),
     "toda_col_sum": (c_int, [c_vp, c_int, c_int, c_vp, c_vp, c_sz, c_vp]),
     "toda_bev_scatter_fwd": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp]),
     "toda_bev_scatter_bwd": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_int, c_int, c_int, c_vp, c_vp]),
@@ -97,7 +99,7 @@ class LayerBwdArgs(ctypes.Structure):
                 ("need_dx", c_int), ("dgrad_nbr", c_vp), ("wt", c_vp), ("wt_bf16", c_vp), ("dgrad_out_rows", c_vp), ("dgrad_masks", c_vp),
                 ("dplan_lidx", c_vp), ("dplan_rows", c_vp), ("dplan_cnt", c_vp), ("dplan_groups", c_int), ("dplan_cap", c_int),
                 ("addend", c_vp), ("dx", c_vp),
-                ("need_dw", c_int), ("nbr_fwd", c_vp), ("dw", c_vp), ("wgrad_ws", c_vp), ("wgrad_ws_bytes", c_sz),
+                ("need_dw", c_int), ("nbr_fwd", c_vp), ("fwd_masks", c_vp), ("dw", c_vp), ("wgrad_ws", c_vp), ("wgrad_ws_bytes", c_sz),
                 ("need_db", c_int), ("db", c_vp),
                 ("precision", c_int), ("conv_ws", c_vp), ("conv_ws_bytes", c_sz)]
 

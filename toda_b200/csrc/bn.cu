@@ -9,6 +9,9 @@ namespace {
 
 constexpr int kThreads = 256;
 constexpr int kPartials = 2 * kNumSMs;  // CTAs in the reduction grids
+// CTAs of a resident streaming grid at most (2048 threads per SM): the backward apply pass leaves one partial column sum
+// per CTA for the bias gradient
+constexpr int kApplyPartials = 2048 / kThreads * kNumSMs;
 
 // per-CTA partial sums of up to two quantities per channel; C % 4 == 0 path: one thread owns 4 channels (float4
 // loads) and walks rows with four independent loads in flight per array.
@@ -128,18 +131,20 @@ static void launch_col_reduce(const float *p0, const float *p1, const float *p2,
 
 // fixed-order sum of the per-CTA partials of one channel: one warp per channel, lanes stride over the partials.
 // All loads of a lane are issued before the first add (the loop used to be a chain of ~10 dependent L2 round trips,
-// which made this tiny kernel take as long as a third of the streaming pass next to it).
+// which made this tiny kernel take as long as a third of the streaming pass next to it).  A CTA left ROWS rows of c
+// partials (quantity q in row q; ss is only summed when ROWS = 2), at most MAX_BLOCKS CTAs.
+template <int MAX_BLOCKS = kPartials, int ROWS = 2>
 __device__ __forceinline__ void warp_sum_partials(const double *__restrict__ partial, int nblocks, int c, int ch, double &s,
                                                   double &ss) {
     const int lane = threadIdx.x & 31;
-    constexpr int kPerLane = (kPartials + 31) / 32;
+    constexpr int kPerLane = (MAX_BLOCKS + 31) / 32;
     double va[kPerLane], vb[kPerLane];
 #pragma unroll
     for (int i = 0; i < kPerLane; ++i) {
         const int j = lane + 32 * i;
         const bool ok = j < nblocks;
-        va[i] = ok ? partial[((size_t)j * 2) * c + ch] : 0.0;
-        vb[i] = ok ? partial[((size_t)j * 2 + 1) * c + ch] : 0.0;
+        va[i] = ok ? partial[((size_t)j * ROWS) * c + ch] : 0.0;
+        vb[i] = ok && ROWS == 2 ? partial[((size_t)j * ROWS + 1) * c + ch] : 0.0;
     }
     double a = 0.0, b = 0.0;
 #pragma unroll
@@ -293,18 +298,27 @@ __global__ void bn_bwd_finalize_kernel(const double *__restrict__ partial, int n
 // C = -A*sum_g/N - B*mean: coefficients are computed once per thread (4 channels), rows stream as float4.
 // The sums are bn_bwd_finalize_kernel's (all-reduced over the processes of a synchronized BatchNorm), rounded to float;
 // N is *count (the global count of a synchronized BatchNorm, device memory) or n when count is NULL.
+// db_partial (optional): the column sums of dy -- the gradient of the bias of the convolution before the BatchNorm -- as
+// fixed-order fp64 partials, one row of c per CTA in dynamic shared memory of kThreads*4 doubles (col_sum_finalize_kernel
+// sums them).  Every thread keeps the same
+// channels over its whole grid-stride loop: VEC, because kThreads is a multiple of c/4; scalar, because the stride is
+// rounded down to a multiple of c (the few threads past it idle).  At most 48 registers: the 5 CTAs per SM this
+// HBM-bound pass had before it also summed dy.
 template <bool VEC>
-__global__ void __launch_bounds__(kThreads) bn_bwd_apply_kernel(const float *__restrict__ da, const float *__restrict__ a,
+__global__ void __launch_bounds__(kThreads, 5) bn_bwd_apply_kernel(const float *__restrict__ da, const float *__restrict__ a,
                                                                 const float *__restrict__ y, long long total, int c, int n,
                                                                 const double *__restrict__ count, const float *__restrict__ gamma,
                                                                 const float *__restrict__ mean, const float *__restrict__ rstd,
                                                                 const double *__restrict__ sums, int relu, int training,
                                                                 float *__restrict__ dy, float *__restrict__ dres,
-                                                                __nv_bfloat16 *__restrict__ dy_bf16) {
+                                                                __nv_bfloat16 *__restrict__ dy_bf16, double *__restrict__ db_partial) {
+    extern __shared__ double s_db[];
+    double db[4] = {0.0, 0.0, 0.0, 0.0};       // this thread's sums of dy (VEC: its 4 channels; scalar: db[0])
     if (count) n = (int)*count;
     auto sum = [&](int i) -> float { return (float)sums[i]; };
     const float inv_n = n > 0 ? 1.0f / (float)n : 0.f;
-    const long long stride = (long long)gridDim.x * blockDim.x;
+    const long long threads = (long long)gridDim.x * blockDim.x;
+    const long long stride = VEC ? threads : threads / c * c;
     long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     if (VEC) {
         const long long tv = total >> 2;
@@ -333,9 +347,10 @@ __global__ void __launch_bounds__(kThreads) bn_bwd_apply_kernel(const float *__r
             o.w = fmaf(A[3], g4.w, fmaf(B[3], y4.w, C[3]));
             if (dy) ((float4 *)dy)[e] = o;
             if (dy_bf16) store_bf16x4(dy_bf16, e, o);
+            if (db_partial) { db[0] += o.x; db[1] += o.y; db[2] += o.z; db[3] += o.w; }
         }
     } else {
-        for (; e < total; e += stride) {
+        for (e = e < stride ? e : total; e < total; e += stride) {
             int ch = (int)(e % c);
             float g = __ldg(da + e);
             if (relu && !(__ldg(a + e) > 0.f)) g = 0.f;
@@ -351,20 +366,42 @@ __global__ void __launch_bounds__(kThreads) bn_bwd_apply_kernel(const float *__r
             }
             if (dy) dy[e] = o;
             if (dy_bf16) dy_bf16[e] = __float2bfloat16_rn(o);
+            if (db_partial) db[0] += o;
         }
+    }
+    if (!db_partial) return;
+    // CTA sum per channel in a fixed order: thread t < c takes channel t's slots
+    constexpr int kSlots = VEC ? 4 : 1;
+#pragma unroll
+    for (int q = 0; q < kSlots; ++q) s_db[threadIdx.x * kSlots + q] = db[q];
+    __syncthreads();
+    if ((int)threadIdx.x < c) {
+        // VEC: thread t holds channels 4*(t % (c/4)) + q; scalar: channel (blockIdx.x*kThreads + t) % c
+        const int units = VEC ? c / 4 : c;
+        const int u = VEC ? (int)threadIdx.x >> 2 : (int)threadIdx.x, q = VEC ? (int)threadIdx.x & 3 : 0;
+        double t = 0.0;
+        for (int j = u; j < kThreads; j += units) t += s_db[j * kSlots + q];
+        const int ch = VEC ? (int)threadIdx.x : (int)(((long long)blockIdx.x * kThreads + threadIdx.x) % c);
+        db_partial[(size_t)blockIdx.x * c + ch] = t;
     }
 }
 
+// out[ch] = the fixed-order sum of the first quantity of the per-CTA partials (col_reduce: two rows per CTA; the
+// backward apply pass's bias sums: one row per CTA)
+template <int MAX_BLOCKS, int ROWS>
 __global__ void col_sum_finalize_kernel(const double *__restrict__ partial, int nblocks, int c, float *out) {
     int ch = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (ch >= c) return;
     double s, unused;
-    warp_sum_partials(partial, nblocks, c, ch, s, unused);
+    warp_sum_partials<MAX_BLOCKS, ROWS>(partial, nblocks, c, ch, s, unused);
     if ((threadIdx.x & 31) == 0) out[ch] = (float)s;
 }
 
-// workspace: the per-CTA partials, then the 2c reduced backward sums of toda_bn_bwd
-size_t partials_bytes(int c) { return (size_t)kPartials * 2 * c * sizeof(double); }
+// workspace: the per-CTA partials (two rows of c per reduction CTA, or one per backward-apply CTA), then the 2c reduced
+// backward sums of toda_bn_bwd
+size_t partials_bytes(int c) {
+    return (size_t)(2 * kPartials > kApplyPartials ? 2 * kPartials : kApplyPartials) * c * sizeof(double);
+}
 size_t bn_ws_bytes(int c) { return align_up(partials_bytes(c) + 2 * c * sizeof(double), 256); }
 
 // Grid of a grid-stride streaming kernel over `items` work items: exactly the CTAs that are resident at once (occupancy x
@@ -467,34 +504,52 @@ extern "C" int toda_bn_bwd_reduce(const float *da, const float *a, const float *
 
 extern "C" int toda_bn_bwd_finish(const float *da, const float *a, const float *y, int n, int c, const float *gamma,
                                   const float *save_mean, const float *save_rstd, int relu, int training, const double *red,
-                                  const double *count, float *dy, void *dy_bf16, float *dresidual, void *stream) {
+                                  const double *count, float *dy, void *dy_bf16, float *dresidual, float *dbias, void *workspace,
+                                  size_t workspace_bytes, void *stream) {
     TODA_CHECK_ARG(n >= 0 && c > 0 && c <= 256, "bn_bwd_finish: unsupported sizes n=%d c=%d", n, c);
     // dy may be NULL when dy_bf16 is given: the fp32 gradient is then not stored (a caller whose consumers -- tensor-core
     // dgrad and wgrad -- only read the bf16 copy saves 4 of the ~30 bytes per element this pass moves)
     TODA_CHECK_ARG(save_mean && save_rstd && (red || !training) && (n == 0 || (da && y && (dy || dy_bf16))) &&
-                   (!relu || a || n == 0), "bn_bwd_finish: null pointer");
-    if (n == 0) return TODA_OK;
-    const long long total = (long long)n * c;
+                   (!relu || a || n == 0) && (!dbias || workspace), "bn_bwd_finish: null pointer");
     cudaStream_t st = (cudaStream_t)stream;
-    if (vec_channels(c))
-        bn_bwd_apply_kernel<true><<<resident_grid<bn_bwd_apply_kernel<true>>(total / 4), kThreads, 0, st>>>(
-            da, a, y, total, c, n, count, gamma, save_mean, save_rstd, red, relu, training, dy, dresidual, (__nv_bfloat16 *)dy_bf16);
-    else
-        bn_bwd_apply_kernel<false><<<resident_grid<bn_bwd_apply_kernel<false>>(total), kThreads, 0, st>>>(
-            da, a, y, total, c, n, count, gamma, save_mean, save_rstd, red, relu, training, dy, dresidual, (__nv_bfloat16 *)dy_bf16);
+    if (dbias && workspace_bytes < bn_ws_bytes(c)) { toda_set_error("bn_bwd_finish: workspace too small"); return TODA_ERR_WORKSPACE; }
+    if (n == 0) {
+        if (dbias) TODA_CUDA_OK(cudaMemsetAsync(dbias, 0, sizeof(float) * c, st));
+        return TODA_OK;
+    }
+    const long long total = (long long)n * c;
+    double *db_partial = dbias ? (double *)workspace : nullptr;
+    const size_t smem = dbias ? kThreads * 4 * sizeof(double) : 0;    // the CTA's column sums, only with a bias gradient
+    int grid;
+    if (vec_channels(c)) {
+        grid = resident_grid<bn_bwd_apply_kernel<true>>(total / 4);
+        grid = grid < kApplyPartials ? grid : kApplyPartials;
+        bn_bwd_apply_kernel<true><<<grid, kThreads, smem, st>>>(da, a, y, total, c, n, count, gamma, save_mean, save_rstd, red, relu,
+                                                               training, dy, dresidual, (__nv_bfloat16 *)dy_bf16, db_partial);
+    } else {
+        grid = resident_grid<bn_bwd_apply_kernel<false>>(total);
+        grid = grid < kApplyPartials ? grid : kApplyPartials;
+        bn_bwd_apply_kernel<false><<<grid, kThreads, smem, st>>>(da, a, y, total, c, n, count, gamma, save_mean, save_rstd, red,
+                                                                relu, training, dy, dresidual, (__nv_bfloat16 *)dy_bf16, db_partial);
+    }
     TODA_LAUNCH_OK();
+    if (dbias) {
+        col_sum_finalize_kernel<kApplyPartials, 1><<<ceil_div(c * 32, 128), 128, 0, st>>>(db_partial, grid, c, dbias);
+        TODA_LAUNCH_OK();
+    }
     return TODA_OK;
 }
 
 extern "C" int toda_bn_bwd(const float *da, const float *a, const float *y, int n, int c, const float *gamma,
                            const float *save_mean, const float *save_rstd, int relu, int training, float *dy, void *dy_bf16,
-                           float *dresidual, float *dgamma, float *dbeta, void *workspace, size_t workspace_bytes, void *stream) {
+                           float *dresidual, float *dgamma, float *dbeta, float *dbias, void *workspace, size_t workspace_bytes,
+                           void *stream) {
     TODA_CHECK_ARG(workspace, "bn_bwd: null workspace");
     double *red = bn_workspace_red(workspace, c);
     int rc = toda_bn_bwd_reduce(da, a, y, n, c, save_mean, save_rstd, relu, red, dgamma, dbeta, workspace, workspace_bytes, stream);
     if (rc) return rc;
     return toda_bn_bwd_finish(da, a, y, n, c, gamma, save_mean, save_rstd, relu, training, red, nullptr, dy, dy_bf16, dresidual,
-                              stream);
+                              dbias, workspace, workspace_bytes, stream);
 }
 
 extern "C" int toda_col_sum(const float *dy, int n, int c, float *out, void *workspace, size_t workspace_bytes, void *stream) {
@@ -504,7 +559,7 @@ extern "C" int toda_col_sum(const float *dy, int n, int c, float *out, void *wor
     double *partial = (double *)workspace;
     launch_col_reduce<2>(dy, nullptr, nullptr, n, c, nullptr, nullptr, 0, partial, st);
     TODA_LAUNCH_OK();
-    col_sum_finalize_kernel<<<ceil_div(c * 32, 128), 128, 0, st>>>(partial, kPartials, c, out);
+    col_sum_finalize_kernel<kPartials, 2><<<ceil_div(c * 32, 128), 128, 0, st>>>(partial, kPartials, c, out);
     TODA_LAUNCH_OK();
     return TODA_OK;
 }

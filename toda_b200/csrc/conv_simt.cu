@@ -12,8 +12,8 @@ int conv_tc_fwd(const float *x, const void *x_bf16, int n_in, int cin, const int
                 cudaStream_t st, const TilePlan *plan, const float *addend, const void *w_bf16);
 size_t conv_tc_fwd_workspace_bytes(int n_in, int cin, int cout, int kvol);
 int conv_tc_wgrad(const float *x, const void *x_bf16, int n_in, int cin, const int32_t *nbr, int n_out, int kvol,
-                  const float *dy, const void *dy_bf16, int cout, float *dw_param, void *workspace, size_t workspace_bytes,
-                  cudaStream_t st);
+                  const uint32_t *tile_masks, const float *dy, const void *dy_bf16, int cout, float *dw_param, void *workspace,
+                  size_t workspace_bytes, cudaStream_t st);
 bool conv_tc_supported(int cin, int cout, int kvol);
 // TODA_CONV_BF16X3 (conv_x3.cu): three bf16 tensor-core launches per product, fp32-class accuracy
 size_t conv_x3_fwd_workspace_bytes(int n_in, int cin, int cout, int kvol);
@@ -21,8 +21,8 @@ int conv_x3_fwd(const float *x, int n_in, int cin, const int32_t *nbr, int n_out
                 float *y, const int32_t *out_rows, const uint32_t *tile_masks, double *bn_sums, void *workspace, size_t workspace_bytes,
                 cudaStream_t st, const TilePlan *plan, const float *addend);
 size_t conv_x3_wgrad_workspace_bytes(int n_in, int n_out, int kvol, int cin, int cout);
-int conv_x3_wgrad(const float *x, int n_in, int cin, const int32_t *nbr, int n_out, int kvol, const float *dy, int cout, float *dw_param,
-                  void *workspace, size_t workspace_bytes, cudaStream_t st);
+int conv_x3_wgrad(const float *x, int n_in, int cin, const int32_t *nbr, int n_out, int kvol, const uint32_t *tile_masks,
+                  const float *dy, int cout, float *dw_param, void *workspace, size_t workspace_bytes, cudaStream_t st);
 bool conv_tc_wgrad_supported(int cin, int cout, int kvol);
 size_t conv_tc_wgrad_workspace_bytes(int n_in, int n_out, int kvol, int cin, int cout);
 
@@ -346,8 +346,8 @@ extern "C" size_t toda_spconv_wgrad_workspace_bytes(int n_in, int n_out, int kvo
 }
 
 extern "C" int toda_spconv_wgrad(const float *x, const void *x_bf16, int n_in, int cin, const int32_t *nbr, int n_out,
-                                 int kvol, const float *dy, const void *dy_bf16, int cout, float *dw_param, void *workspace,
-                                 size_t workspace_bytes, int precision, void *stream) {
+                                 int kvol, const uint32_t *tile_masks, const float *dy, const void *dy_bf16, int cout,
+                                 float *dw_param, void *workspace, size_t workspace_bytes, int precision, void *stream) {
     TODA_CHECK_ARG(n_in >= 0 && n_out >= 0 && cin > 0 && cout > 0 && kvol > 0, "spconv_wgrad: bad sizes");
     TODA_CHECK_ARG(dw_param, "spconv_wgrad: null dw");
     cudaStream_t st = (cudaStream_t)stream;
@@ -359,9 +359,10 @@ extern "C" int toda_spconv_wgrad(const float *x, const void *x_bf16, int n_in, i
     TODA_CHECK_ARG(precision == TODA_CONV_FP32 || precision == TODA_CONV_BF16 || precision == TODA_CONV_BF16X3,
                    "spconv_wgrad: unknown precision %d", precision);
     if (precision == TODA_CONV_BF16X3 && conv_tc_wgrad_supported(cin, cout, kvol))
-        return conv_x3_wgrad(x, n_in, cin, nbr, n_out, kvol, dy, cout, dw_param, workspace, workspace_bytes, st);
+        return conv_x3_wgrad(x, n_in, cin, nbr, n_out, kvol, tile_masks, dy, cout, dw_param, workspace, workspace_bytes, st);
     if (precision == TODA_CONV_BF16 && conv_tc_wgrad_supported(cin, cout, kvol))
-        return conv_tc_wgrad(x, x_bf16, n_in, cin, nbr, n_out, kvol, dy, dy_bf16, cout, dw_param, workspace, workspace_bytes, st);
+        return conv_tc_wgrad(x, x_bf16, n_in, cin, nbr, n_out, kvol, tile_masks, dy, dy_bf16, cout, dw_param, workspace,
+                             workspace_bytes, st);
     int splits = wgrad_splits(n_out, kvol, cin, cout);
     size_t need = (size_t)splits * kvol * cin * cout * sizeof(float);
     if (workspace_bytes < need) {

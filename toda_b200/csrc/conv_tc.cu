@@ -665,15 +665,65 @@ __device__ __forceinline__ uint64_t make_desc_mn_sw128(uint32_t smem_addr, uint3
     return d;
 }
 
+// Live passes (bit ps) of row chunk c (rows c*rows ..) for the npass passes of opp offsets from offset k0: those with a
+// neighbour under one of their offsets in the 128-row tile that encloses the chunk (a 64-row chunk reads its tile's word,
+// which may claim more than the chunk holds but never misses a neighbour).  No masks: every pass.
+__device__ __forceinline__ uint32_t wgrad_live_passes(const uint32_t *__restrict__ tile_masks, int c, int rows, int k0, int npass,
+                                                      int opp) {
+    if (!tile_masks) return (1u << npass) - 1u;
+    const uint32_t om = __ldg(tile_masks + ((c * rows) >> 7)) >> k0;
+    uint32_t lm = 0;
+    for (int ps = 0; ps < npass; ++ps)
+        if ((om >> (ps * opp)) & ((1u << opp) - 1u)) lm |= 1u << ps;
+    return lm;
+}
+
+// Row chunks [c_begin, c_end) of split `split` of one offset group: the group's chunks cut into `splits` contiguous ranges
+// with equal shares of its live items.  Split s starts at the first chunk c whose preceding chunks hold at least
+// floor(s*T/splits) of the T live items (the last split ends at the last chunk).  The boundaries depend only on the
+// masks, so the partition of the fp32 partial sums -- and the result -- is the same on every run.  Called by the whole
+// block; scratch: blockDim.x + 2 ints of shared memory.
+__device__ void wgrad_split_chunks(const uint32_t *__restrict__ tile_masks, int n_out, int rows, int k0, int npass, int opp,
+                                   int split, int splits, int *scratch, int &c_begin, int &c_end) {
+    const int tid = threadIdx.x, nt = blockDim.x;
+    const int nch = (n_out + rows - 1) / rows;
+    const int per = (nch + nt - 1) / nt, c0 = min(nch, tid * per), c1 = min(nch, c0 + per);
+    int local = 0;
+    for (int c = c0; c < c1; ++c) local += __popc(wgrad_live_passes(tile_masks, c, rows, k0, npass, opp));
+    if (tid == 0) scratch[nt] = scratch[nt + 1] = 0;
+    scratch[tid] = local;
+    __syncthreads();
+    for (int off = 1; off < nt; off <<= 1) {           // inclusive scan of the per-thread counts
+        const int v = tid >= off ? scratch[tid - off] : 0;
+        __syncthreads();
+        scratch[tid] += v;
+        __syncthreads();
+    }
+    const long long total = scratch[nt - 1];
+    const long long ta = (long long)split * total / splits, tb = (long long)(split + 1) * total / splits;
+    int run = scratch[tid] - local, na = 0, nb = 0;    // live items before chunk c
+    for (int c = c0; c < c1; ++c) {
+        na += run < ta;
+        nb += run < tb;
+        run += __popc(wgrad_live_passes(tile_masks, c, rows, k0, npass, opp));
+    }
+    if (na) atomicAdd(scratch + nt, na);
+    if (nb) atomicAdd(scratch + nt + 1, nb);
+    __syncthreads();
+    c_begin = split == 0 ? 0 : scratch[nt];
+    c_end = split + 1 == splits ? nch : scratch[nt + 1];
+}
+
 // Roles as in the forward kernel: warps 0-7 produce (gather x rows per pass into the A ring; dy rows once per row
 // chunk into a double-buffered B tile), warp 8 issues the MMAs, warps 9-12 drain TMEM at the end, warp 13 streams
-// the table slice of the next row chunk into shared memory.
+// the table slice of the next row chunk into shared memory.  The row range of the CTA is computed first, by the whole
+// block (wgrad_split_chunks, gridDim.x splits per offset group).
 template <int CIN, int NPAD, int ROWS>
 __global__ void __launch_bounds__(kWgradThreads, 1) conv_tc_wgrad_kernel(const __nv_bfloat16 *__restrict__ xb,
                                                                          const int *__restrict__ nbr, int n_out, int kvol,
                                                                          const __nv_bfloat16 *__restrict__ dyb, int cout,
-                                                                         int rows_per_split, int passes_per_cta,
-                                                                         float *__restrict__ partial) {
+                                                                         const uint32_t *__restrict__ tile_masks /* optional */,
+                                                                         int passes_per_cta, float *__restrict__ partial) {
     using W = WCfg<NPAD, ROWS>;
     constexpr int kOffsPerPass = 128 / CIN;
     constexpr int S = W::kStages;
@@ -698,9 +748,17 @@ __global__ void __launch_bounds__(kWgradThreads, 1) conv_tc_wgrad_kernel(const _
     const int npass = min(passes_per_cta, total_passes - pass0);
     const int k0 = pass0 * kOffsPerPass;                         // first kernel offset of this CTA
     const int noffs = min(npass * kOffsPerPass, kvol - k0);      // offsets this CTA really owns
-    const int r_begin = split * rows_per_split;
-    const int r_end = min(n_out, r_begin + rows_per_split);
-    const int nchunks = r_end > r_begin ? (r_end - r_begin + kRowsW - 1) / kRowsW : 0;
+    int c_begin, c_end;     // scratch: the A ring, which nothing uses before the __syncthreads below
+    wgrad_split_chunks(tile_masks, n_out, kRowsW, k0, npass, kOffsPerPass, split, gridDim.x, (int *)(smem_raw + (base - raw)),
+                       c_begin, c_end);
+    const int r_begin = c_begin * kRowsW;
+    const int r_end = min(n_out, c_end * kRowsW);
+    const int nchunks = c_end - c_begin;
+    // An item = a live (chunk, pass) pair; every role derives the same item sequence from the same mask words, so the
+    // rings stay in step.  Chunks without a live pass are skipped whole (no dy rows, no table slice).
+    auto live_of = [&](int rc) -> uint32_t {
+        return wgrad_live_passes(tile_masks, c_begin + rc, kRowsW, k0, npass, kOffsPerPass);
+    };
 
     if (tid == 0) {
         for (int s = 0; s < S; ++s) {
@@ -738,27 +796,44 @@ __global__ void __launch_bounds__(kWgradThreads, 1) conv_tc_wgrad_kernel(const _
         //   CIN=128: (0, mb*64+p*8)  CIN=64: (mb, p*8)  CIN=32: (2mb + p/4, (p%4)*8)  CIN=16: (4mb + p/2, (p%2)*8)
         const int off_lo = CIN >= 64 ? 0 : p / (CIN / 8);
         const int ci_lo = CIN >= 64 ? p * 8 : (p % (CIN / 8)) * 8;
-        // Completion of item j is signalled kLagW items later (per warp, see the forward kernel).  The dy tile of
-        // chunk rc may only be overwritten once the MMAs of chunk rc-3 are done, and those need the signals of every
-        // item up to (rc-2)*npass-1, the last of which is sent at item (rc-2)*npass-1+kLagW < rc*npass  <=>
-        // kLagW <= 2*npass: holds for npass >= 2; single-pass launches drain at every chunk boundary instead.
-        constexpr int kLagW = W::kLag;       // (2 dy buffers: kLagW <= npass; 3 buffers: kLagW <= 2*npass)
-        int g = 0, signalled = 0;
+        // Completion of item j is signalled kLagW items later (per warp, see the forward kernel); the dy tile of a live
+        // chunk joins the cp.async group of the chunk's first item and is signalled (b_full) with it.
+        // Hang freedom.  (a) A ring: before item g overwrites stage g % S the MMAs of item g-S must be done, and they need
+        // the signals of items <= g-S; signalled are items < g-kLagW, so kLagW <= S-1 suffices (4/2, 8/3), whatever the
+        // chunks.  (b) dy ring: before live chunk lc overwrites dy buffer lc % kBBufsW, the MMA warp must have finished live
+        // chunk lc-kBBufsW, i.e. every item of it must be signalled: signalled >= first item of live chunk
+        // lc-kBBufsW+1.  With a fixed npass items per chunk that held for kLagW <= (kBBufsW-1)*npass; with a variable
+        // number of live passes per chunk it can fail (chunks of one live item), so it is tested here and, where it fails,
+        // the producer drains: waits for all of its copies and signals every pending item before it waits on b_empty.
+        // (c) The table-slice ring involves only the indexer and the producers.
+        constexpr int kLagW = W::kLag;
+        int g = 0, signalled = 0;       // items issued / items signalled
+        int lc = 0, bsig = 0;           // live chunks started / dy tiles signalled
+        int first1 = 0, first2 = 0;     // first item of live chunk lc-1 / lc-2
+        uint32_t pend_first = 0;        // bit i: pending item signalled+i is the first of its chunk (carries its dy tile)
+        auto signal_next = [&]() {
+            if (lane == 0) {
+                if (pend_first & 1u) mbar_arrive(b_full + 8 * (bsig % kBBufsW));
+                mbar_arrive(a_full + 8 * (signalled % S));
+            }
+            bsig += pend_first & 1u;
+            pend_first >>= 1;
+            ++signalled;
+        };
         for (int rc = 0; rc < nchunks; ++rc) {
-            const int ib = rc & 1, use_i = rc >> 1;
-            const int bb = rc % kBBufsW, use_b = rc / kBBufsW;
+            const uint32_t lm = live_of(rc);
+            if (!lm) continue;
+            const int ib = lc & 1, use_i = lc >> 1;
+            const int bb = lc % kBBufsW, use_b = lc / kBBufsW;
             const int row_base = r_begin + rc * kRowsW;
-            if (npass < kLagW) {
+            if (use_b > 0 && signalled < (kBBufsW == 2 ? first1 : first2)) {
                 asm volatile("cp.async.wait_group 0;" ::: "memory");
                 asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
                 __syncwarp();
-                if (lane == 0)
-                    for (; signalled < g; ++signalled) {
-                        if (signalled % npass == 0) mbar_arrive(b_full + 8 * ((signalled / npass) % kBBufsW));
-                        mbar_arrive(a_full + 8 * (signalled % S));
-                    }
-                signalled = g;
+                while (signalled < g) signal_next();
             }
+            first2 = first1;
+            first1 = g;
             // dy rows of this chunk (shared by every pass)
             if (use_b > 0) mbar_wait(b_empty + 8 * bb, (use_b - 1) & 1);
             {
@@ -774,12 +849,12 @@ __global__ void __launch_bounds__(kWgradThreads, 1) conv_tc_wgrad_kernel(const _
                         else st_shared_zero16(dst);
                     }
                 }
-                // no group commit here: the dy copies join the cp.async group of this chunk's first pass and are
-                // signalled (b_full) together with it
             }
             mbar_wait(idx_full + 8 * ib, use_i & 1);
             const uint32_t idx_tile = idx_base + ib * kIdxW + 4 * rbase;
-            for (int ps = 0; ps < npass; ++ps, ++g) {
+            for (uint32_t m = lm; m; m &= m - 1, ++g) {
+                const int ps = __ffs(m) - 1;
+                if (m == lm) pend_first |= 1u << (g - signalled);
                 const int s = g % S, use = g / S;
                 if (use > 0) mbar_wait(a_empty + 8 * s, (use - 1) & 1);
                 const uint32_t a_dst = base + s * kATileW + piece_off;
@@ -803,39 +878,35 @@ __global__ void __launch_bounds__(kWgradThreads, 1) conv_tc_wgrad_kernel(const _
                 }
                 asm volatile("cp.async.commit_group;" ::: "memory");
                 if (g - signalled >= kLagW) {
+                    // the copies of item signalled (= g - kLagW) have landed
                     asm volatile("cp.async.wait_group %0;" ::"n"(kLagW) : "memory");
                     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
                     __syncwarp();
-                    const int j = signalled;                     // item whose copies have landed (= g - kLagW)
-                    if (lane == 0) {
-                        if (j % npass == 0) mbar_arrive(b_full + 8 * ((j / npass) % kBBufsW));   // its chunk's dy tile came with it
-                        mbar_arrive(a_full + 8 * (j % S));
-                    }
-                    ++signalled;
+                    signal_next();
                 }
             }
             mbar_arrive(idx_empty + 8 * ib);
+            ++lc;
         }
         asm volatile("cp.async.wait_group 0;" ::: "memory");
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
         __syncwarp();
-        if (lane == 0)
-            for (int j = signalled; j < g; ++j) {
-                if (j % npass == 0) mbar_arrive(b_full + 8 * ((j / npass) % kBBufsW));
-                mbar_arrive(a_full + 8 * (j % S));
-            }
+        while (signalled < g) signal_next();
     } else if (warp == 8) {
         // ------------------------------------------------------------------ MMA issuer (warp-uniform loop, one elected lane issues)
         if (nchunks > 0) {
             // D = A(MN-major) x B(MN-major): bits 15 / 16 of the instruction descriptor select MN-major operands
             constexpr uint32_t idesc = make_idesc_bf16(128, NPAD) | (1u << 15) | (1u << 16);
-            int g = 0;
-            uint32_t ready = 0;
+            int g = 0, lc = 0;
+            uint32_t ready = 0, started = 0;     // bit ps: pass ps's accumulator holds its first live item
             for (int rc = 0; rc < nchunks; ++rc) {
-                const int ib = rc % kBBufsW;
-                mbar_wait(b_full + 8 * ib, (rc / kBBufsW) & 1);
+                const uint32_t lm = live_of(rc);
+                if (!lm) continue;
+                const int ib = lc % kBBufsW;
+                mbar_wait(b_full + 8 * ib, (lc / kBBufsW) & 1);
                 const uint32_t b_tile = b_base + ib * kBTileW;
-                for (int ps = 0; ps < npass; ++ps, ++g) {
+                for (uint32_t m = lm; m; m &= m - 1, ++g) {
+                    const int ps = __ffs(m) - 1;
                     const int s = g % S, use = g / S;
                     if (!ready) mbar_wait(a_full + 8 * s, use & 1);
                     ready = mbar_test(a_full + 8 * ((g + 1) % S), ((g + 1) / S) & 1);   // look one stage ahead
@@ -845,23 +916,29 @@ __global__ void __launch_bounds__(kWgradThreads, 1) conv_tc_wgrad_kernel(const _
 #pragma unroll
                         // UMMA K = 16 rows = 2 swizzle atoms of 8 rows = 2048 B: a K-step adds 128 to the start-address field
                         const uint64_t ad0 = make_desc_mn_sw128(a_tile, kRowsW * 128), bd0 = make_desc_mn_sw128(b_tile, kRowsW * 128);
-                        umma_bf16(tmem_base + ps * NPAD, ad0, bd0, idesc, rc != 0);
+                        umma_bf16(tmem_base + ps * NPAD, ad0, bd0, idesc, (started >> ps) & 1u);
                         for (int j = 1; j < kRowsW / 16; ++j)
                             umma_bf16(tmem_base + ps * NPAD, ad0 + 128 * j, bd0 + 128 * j, idesc, 1u);
                         umma_commit(a_empty + 8 * s);
                     }
                     __syncwarp();
                 }
-                if (elect_one()) umma_commit(b_empty + 8 * ib);      // dy tile reusable once every pass of this chunk has read it
+                started |= lm;
+                if (elect_one()) umma_commit(b_empty + 8 * ib);      // dy tile reusable once every live pass of this chunk has read it
+                __syncwarp();
+                ++lc;
+            }
+            if (g > 0) {
+                if (elect_one()) umma_commit(accum_bar);
                 __syncwarp();
             }
-            if (elect_one()) umma_commit(accum_bar);
-            __syncwarp();
         }
     } else if (warp < 13) {
         // ------------------------------------------------------------------ epilogue: TMEM lane = M slot (offset, ci)
         const int q = warp & 3;
-        if (nchunks > 0) {
+        uint32_t used = 0;                                       // passes with at least one live item (written TMEM)
+        for (int rc = 0; rc < nchunks; ++rc) used |= live_of(rc);
+        if (used) {
             mbar_wait(accum_bar, 0);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         }
@@ -872,7 +949,7 @@ __global__ void __launch_bounds__(kWgradThreads, 1) conv_tc_wgrad_kernel(const _
             const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + ps * NPAD;
             for (int n0 = 0; n0 < cout; n0 += 16) {
                 uint32_t v[16];
-                if (nchunks > 0) {
+                if ((used >> ps) & 1u) {
                     asm volatile(
                         "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
                         : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
@@ -881,7 +958,7 @@ __global__ void __launch_bounds__(kWgradThreads, 1) conv_tc_wgrad_kernel(const _
                     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
                 } else {
 #pragma unroll
-                    for (int qq = 0; qq < 16; ++qq) v[qq] = 0u;      // this split has no rows: its partial is zero
+                    for (int qq = 0; qq < 16; ++qq) v[qq] = 0u;      // no live item of this pass in this split: its partial is zero
                 }
                 if (k < kvol) {
 #pragma unroll
@@ -894,8 +971,10 @@ __global__ void __launch_bounds__(kWgradThreads, 1) conv_tc_wgrad_kernel(const _
         asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     } else {
         // ------------------------------------------------------------------ indexer (warp 13)
-        for (int rc = 0; rc < nchunks; ++rc) {
-            const int ib = rc & 1, use = rc >> 1;
+        for (int rc = 0, lc = 0; rc < nchunks; ++rc) {
+            if (!live_of(rc)) continue;
+            const int ib = lc & 1, use = lc >> 1;
+            ++lc;
             if (use > 0) mbar_wait(idx_empty + 8 * ib, (use - 1) & 1);
             const uint32_t dst0 = idx_base + ib * kIdxW;
             const int row_base = r_begin + rc * kRowsW;
@@ -940,7 +1019,7 @@ __global__ void __launch_bounds__(256) wgrad_tc_reduce_kernel(const float *__res
 }
 
 struct WgradPlan {
-    int passes_per_cta, groups, splits, rows_per_split;
+    int passes_per_cta, groups, splits, rows;
     size_t xb_bytes, dyb_bytes, partial_bytes;
 };
 
@@ -957,16 +1036,43 @@ WgradPlan wgrad_plan(int n_in, int n_out, int kvol, int cin, int cout) {
     int max_by_rows = (n_out + 4 * kRowsW - 1) / (4 * kRowsW);
     p.splits = want < max_by_rows ? want : max_by_rows;
     if (p.splits < 1) p.splits = 1;
-    int rps = (n_out + p.splits - 1) / p.splits;
-    p.rows_per_split = (rps + kRowsW - 1) / kRowsW * kRowsW;
-    if (p.rows_per_split < kRowsW) p.rows_per_split = kRowsW;
+    p.rows = kRowsW;
     p.xb_bytes = align_up((size_t)n_in * cin * 2 + 16, 256);
     p.dyb_bytes = align_up((size_t)n_out * cout * 2 + 16, 256);
     p.partial_bytes = align_up((size_t)p.splits * kvol * cin * cout * 4, 256);
     return p;
 }
 
+// first row of every (offset group, split) of a wgrad launch: row_begin[group * splits + split]
+__global__ void __launch_bounds__(kWgradThreads) wgrad_row_splits_kernel(const uint32_t *__restrict__ tile_masks, int n_out,
+                                                                         int kvol, int opp, int rows, int passes_per_cta,
+                                                                         int32_t *__restrict__ row_begin) {
+    __shared__ int scratch[kWgradThreads + 2];
+    const int total_passes = (kvol + opp - 1) / opp, pass0 = blockIdx.y * passes_per_cta;
+    int c_begin, c_end;
+    wgrad_split_chunks(tile_masks, n_out, rows, pass0 * opp, min(passes_per_cta, total_passes - pass0), opp, blockIdx.x, gridDim.x,
+                       scratch, c_begin, c_end);
+    if (threadIdx.x == 0) row_begin[blockIdx.y * gridDim.x + blockIdx.x] = min(n_out, c_begin * rows);
+}
+
 }  // namespace
+
+bool conv_tc_wgrad_supported(int cin, int cout, int kvol);
+
+extern "C" int toda_spconv_wgrad_row_splits(const uint32_t *tile_masks, int n_out, int kvol, int cin, int cout, int *groups,
+                                            int *splits, int32_t *row_begin, void *stream) {
+    TODA_CHECK_ARG(n_out > 0 && kvol > 0 && kvol <= kMaxKvol && groups && splits && conv_tc_wgrad_supported(cin, cout, kvol),
+                   "spconv_wgrad_row_splits: bad args");
+    const int cp = pad16(cin);
+    WgradPlan p = wgrad_plan(0, n_out, kvol, cp, cout);
+    *groups = p.groups;
+    *splits = p.splits;
+    if (!row_begin) return TODA_OK;
+    wgrad_row_splits_kernel<<<dim3(p.splits, p.groups), kWgradThreads, 0, (cudaStream_t)stream>>>(tile_masks, n_out, kvol, 128 / cp,
+                                                                                                  p.rows, p.passes_per_cta, row_begin);
+    TODA_LAUNCH_OK();
+    return TODA_OK;
+}
 
 bool conv_tc_wgrad_supported(int cin, int cout, int kvol) {
     // (the kernel's shared-memory table slice holds at most 32 offsets: larger kernels take the fp32 wgrad)
@@ -979,8 +1085,8 @@ size_t conv_tc_wgrad_workspace_bytes(int n_in, int n_out, int kvol, int cin, int
 }
 
 int conv_tc_wgrad(const float *x, const void *x_bf16, int n_in, int cin, const int32_t *nbr, int n_out, int kvol,
-                  const float *dy, const void *dy_bf16, int cout, float *dw_param, void *workspace, size_t workspace_bytes,
-                  cudaStream_t st) {
+                  const uint32_t *tile_masks, const float *dy, const void *dy_bf16, int cout, float *dw_param, void *workspace,
+                  size_t workspace_bytes, cudaStream_t st) {
     const int cin_real = cin;
     cin = pad16(cin);
     WgradPlan p = wgrad_plan(n_in, n_out, kvol, cin, cout);
@@ -1020,7 +1126,7 @@ int conv_tc_wgrad(const float *x, const void *x_bf16, int n_in, int cin, const i
             TODA_CUDA_OK(cudaFuncSetAttribute(conv_tc_wgrad_kernel<CI, NP, RW>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
             attr_set = true;                                                                                               \
         }                                                                                                                  \
-        conv_tc_wgrad_kernel<CI, NP, RW><<<grid, kWgradThreads, smem, st>>>(xb, nbr, n_out, kvol, dyb, cout, p.rows_per_split,  \
+        conv_tc_wgrad_kernel<CI, NP, RW><<<grid, kWgradThreads, smem, st>>>(xb, nbr, n_out, kvol, dyb, cout, tile_masks,       \
                                                                            p.passes_per_cta, partial);                      \
     } while (0)
     const bool wide = cout > 64;

@@ -15,8 +15,8 @@ int conv_tc_fwd(const float *x, const void *x_bf16, int n_in, int cin, const int
                 cudaStream_t st, const TilePlan *plan, const float *addend, const void *w_bf16);
 size_t conv_tc_fwd_workspace_bytes(int n_in, int cin, int cout, int kvol);
 int conv_tc_wgrad(const float *x, const void *x_bf16, int n_in, int cin, const int32_t *nbr, int n_out, int kvol,
-                  const float *dy, const void *dy_bf16, int cout, float *dw_param, void *workspace, size_t workspace_bytes,
-                  cudaStream_t st);
+                  const uint32_t *tile_masks, const float *dy, const void *dy_bf16, int cout, float *dw_param, void *workspace,
+                  size_t workspace_bytes, cudaStream_t st);
 size_t conv_tc_wgrad_workspace_bytes(int n_in, int n_out, int kvol, int cin, int cout);
 
 namespace {
@@ -131,8 +131,8 @@ size_t conv_x3_wgrad_workspace_bytes(int n_in, int n_out, int kvol, int cin, int
     return 2 * l.x_bytes + 2 * l.dy_bytes + 3 * l.t_bytes + l.inner + 256;
 }
 
-int conv_x3_wgrad(const float *x, int n_in, int cin, const int32_t *nbr, int n_out, int kvol, const float *dy, int cout, float *dw_param,
-                  void *workspace, size_t workspace_bytes, cudaStream_t st) {
+int conv_x3_wgrad(const float *x, int n_in, int cin, const int32_t *nbr, int n_out, int kvol, const uint32_t *tile_masks,
+                  const float *dy, int cout, float *dw_param, void *workspace, size_t workspace_bytes, cudaStream_t st) {
     const size_t need = conv_x3_wgrad_workspace_bytes(n_in, n_out, kvol, cin, cout);
     if (!workspace || workspace_bytes < need) {
         toda_set_error("spconv_wgrad(bf16x3): workspace %zu < required %zu bytes", workspace_bytes, need);
@@ -149,11 +149,11 @@ int conv_x3_wgrad(const float *x, int n_in, int cin, const int32_t *nbr, int n_o
     TODA_LAUNCH_OK();
     split_rows_kernel<<<wave_grid((int64_t)n_out * cout, 256), 256, 0, st>>>(dy, n_out, cout, cout, dh, dl);
     TODA_LAUNCH_OK();
-    int rc = conv_tc_wgrad(x, xh, n_in, cp, nbr, n_out, kvol, dy, dh, cout, t1, inner, l.inner, st);
+    int rc = conv_tc_wgrad(x, xh, n_in, cp, nbr, n_out, kvol, tile_masks, dy, dh, cout, t1, inner, l.inner, st);
     if (rc) return rc;
-    rc = conv_tc_wgrad(x, xh, n_in, cp, nbr, n_out, kvol, dy, dl, cout, t2, inner, l.inner, st);
+    rc = conv_tc_wgrad(x, xh, n_in, cp, nbr, n_out, kvol, tile_masks, dy, dl, cout, t2, inner, l.inner, st);
     if (rc) return rc;
-    rc = conv_tc_wgrad(x, xl, n_in, cp, nbr, n_out, kvol, dy, dh, cout, t3, inner, l.inner, st);
+    rc = conv_tc_wgrad(x, xl, n_in, cp, nbr, n_out, kvol, tile_masks, dy, dh, cout, t3, inner, l.inner, st);
     if (rc) return rc;
     const size_t rows = (size_t)cout * kvol;
     sum3_unpad_kernel<<<wave_grid((int64_t)rows * cin, 256), 256, 0, st>>>(t1, t2, t3, rows, cp, cin, dw_param);

@@ -64,15 +64,16 @@ static int layer_bwd_empty(const toda_layer_bwd_args *p, bool bn_grads, cudaStre
 }
 
 // The fp32 copy of the gradient between BatchNorm and the convolution is only written when something reads it: the
-// tensor-core dgrad / wgrad take the bf16 copy the same pass writes (4 of ~30 bytes per element of this HBM-bound pass).
+// tensor-core dgrad / wgrad take the bf16 copy the same pass writes (4 of ~30 bytes per element of this HBM-bound pass),
+// and the bias gradient is summed by that pass itself.
 static bool layer_bwd_reads_dy_f32(const toda_layer_bwd_args *p) {
     const int c = p->cout;
-    return p->need_db || !p->dy_bf16 || p->precision != TODA_CONV_BF16 ||
+    return !p->dy_bf16 || p->precision != TODA_CONV_BF16 ||
            (p->need_dx && !toda_spconv_uses_tensor_cores(c, p->cin, p->kvol, p->precision)) ||
            (p->need_dw && !toda_spconv_wgrad_uses_tensor_cores(p->cin, c, p->kvol, p->precision));
 }
 
-// The convolution's part of the layer backward, from dy: dgrad (+ residual-branch addend), wgrad, bias gradient.
+// The convolution's part of the layer backward, from dy: dgrad (+ residual-branch addend), wgrad.
 static int layer_bwd_conv(const toda_layer_bwd_args *p, void *stream) {
     const int c = p->cout, n = p->n_out;
     int rc;
@@ -85,12 +86,8 @@ static int layer_bwd_conv(const toda_layer_bwd_args *p, void *stream) {
         if (rc) return rc;
     }
     if (p->need_dw) {
-        rc = toda_spconv_wgrad(p->x, p->x_bf16, p->n_in, p->cin, p->nbr_fwd, n, p->kvol, p->dy, p->dy_bf16, c, p->dw, p->wgrad_ws,
-                               p->wgrad_ws_bytes, p->precision, stream);
-        if (rc) return rc;
-    }
-    if (p->need_db) {
-        rc = toda_col_sum(p->dy, n, c, p->db, p->bn_ws, p->bn_ws_bytes, stream);
+        rc = toda_spconv_wgrad(p->x, p->x_bf16, p->n_in, p->cin, p->nbr_fwd, n, p->kvol, p->fwd_masks, p->dy, p->dy_bf16, c, p->dw,
+                               p->wgrad_ws, p->wgrad_ws_bytes, p->precision, stream);
         if (rc) return rc;
     }
     return TODA_OK;
@@ -101,13 +98,14 @@ static int layer_bwd_reduce(const toda_layer_bwd_args *p, double *red, void *str
                               p->bn_ws, p->bn_ws_bytes, stream);
 }
 
-// The layer backward from the BatchNorm's reduced sums on: dy (+ dres) from `red` and the row count (`count`, or n_out
-// when NULL), then the convolution's part.
+// The layer backward from the BatchNorm's reduced sums on: dy (+ dres, + the bias gradient) from `red` and the row count
+// (`count`, or n_out when NULL), then the convolution's part.
 static int layer_bwd_finish(const toda_layer_bwd_args *p, const double *red, const double *count, void *stream) {
     const int c = p->cout, n = p->n_out;
     if (n == 0) return layer_bwd_empty(p, false, (cudaStream_t)stream);   // dgamma / dbeta: written by the reduce phase
     int rc = toda_bn_bwd_finish(p->da, p->a_mask, p->y, n, c, p->gamma, p->mean, p->rstd, p->relu, p->training, red, count,
-                                layer_bwd_reads_dy_f32(p) ? p->dy : nullptr, p->dy_bf16, p->dres, stream);
+                                layer_bwd_reads_dy_f32(p) ? p->dy : nullptr, p->dy_bf16, p->dres, p->need_db ? p->db : nullptr,
+                                p->bn_ws, p->bn_ws_bytes, stream);
     return rc ? rc : layer_bwd_conv(p, stream);
 }
 

@@ -698,8 +698,9 @@ def _conv_backward_impl(dy, dyb, x, weight, xb, rb, precision, need_dx, need_dw,
         ws = _workspace("wgrad", ws_bytes, dy.device)
         with _timed("conv_wgrad", n_in=rb.n_in, n_out=rb.n_out, cin=cin, cout=cout, kvol=rb.kvol, precision=precision,
                     rb=id(rb)):
-            _C.check(L.toda_spconv_wgrad(_p(x), _p(xb), rb.n_in, cin, _p(rb.nbr_fwd), rb.n_out, rb.kvol, _p(dy), _p(dyb),
-                                         cout, _p(dw), _p(ws), ws.numel(), precision, _stream()), "toda_spconv_wgrad")
+            _C.check(L.toda_spconv_wgrad(_p(x), _p(xb), rb.n_in, cin, _p(rb.nbr_fwd), rb.n_out, rb.kvol, _p(rb.tile_masks),
+                                         _p(dy), _p(dyb), cout, _p(dw), _p(ws), ws.numel(), precision, _stream()),
+                     "toda_spconv_wgrad")
     if need_db:
         db = col_sum(dy)
     return dx, dw, db
@@ -859,11 +860,12 @@ def _bn_forward_phases(y, gamma, beta, running_mean, running_var, eps, momentum,
     return a, ab, y, mean, rstd, a, gsums
 
 
-def _bn_backward_phases(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16, gsums=None):
-    """Phase generator of the backward of _bn_forward_phases -> (dy, dy_bf16, dresidual, dgamma, dbeta).  gsums: the forward's
-    global sums of a synchronized BatchNorm: the local sums of g and g*xhat (and this process's dgamma / dbeta) are then
-    yielded for the all-reduce, and dy follows from the global sums and the forward's global count.  da None = zeros (a
-    rank must join the collective even when no gradient reached it)."""
+def _bn_backward_phases(da, y, a, gamma, mean, rstd, training, relu, has_res, want_bf16, gsums=None, want_db=False):
+    """Phase generator of the backward of _bn_forward_phases -> (dy, dy_bf16, dresidual, dgamma, dbeta, dbias).  gsums: the
+    forward's global sums of a synchronized BatchNorm: the local sums of g and g*xhat (and this process's dgamma / dbeta) are
+    then yielded for the all-reduce, and dy follows from the global sums and the forward's global count.  da None = zeros (a
+    rank must join the collective even when no gradient reached it).  want_db: dbias = the column sums of dy (the gradient
+    of the preceding convolution's bias), summed by the pass that writes dy; else None."""
     n, c = y.shape
     da = da.contiguous() if da is not None else torch.zeros_like(y)
     L = _C.lib()
@@ -871,19 +873,22 @@ def _bn_backward_phases(da, y, a, gamma, mean, rstd, training, relu, has_res, wa
     dyb = torch.empty(y.shape, dtype=torch.bfloat16, device=y.device) if want_bf16 else None
     dres = torch.empty_like(y) if has_res else None
     dgamma, dbeta = torch.empty((2, c), dtype=torch.float32, device=y.device).unbind(0)
+    db = torch.empty((c,), dtype=torch.float32, device=y.device) if want_db else None
     ws = _workspace("bn", L.toda_bn_workspace_bytes(c), y.device)
     if gsums is None:
         with _timed("bn_bwd", n=n, c=c, residual=has_res):
             _C.check(L.toda_bn_bwd(_p(da), _p(a), _p(y), n, c, _p(gamma), _p(mean), _p(rstd), int(relu), int(training),
-                                   _p(dy), _p(dyb), _p(dres), _p(dgamma), _p(dbeta), _p(ws), ws.numel(), _stream()), "toda_bn_bwd")
-        return dy, dyb, dres, dgamma, dbeta
+                                   _p(dy), _p(dyb), _p(dres), _p(dgamma), _p(dbeta), _p(db), _p(ws), ws.numel(), _stream()),
+                     "toda_bn_bwd")
+        return dy, dyb, dres, dgamma, dbeta, db
     red = torch.empty((2 * c,), dtype=torch.float64, device=y.device)
     _C.check(L.toda_bn_bwd_reduce(_p(da), _p(a), _p(y), n, c, _p(mean), _p(rstd), int(relu), _p(red), _p(dgamma), _p(dbeta),
                                   _p(ws), ws.numel(), _stream()), "toda_bn_bwd_reduce")
     yield red
     _C.check(L.toda_bn_bwd_finish(_p(da), _p(a), _p(y), n, c, _p(gamma), _p(mean), _p(rstd), int(relu), 1, _p(red),
-                                  gsums.data_ptr() + 16 * c, _p(dy), _p(dyb), _p(dres), _stream()), "toda_bn_bwd_finish")
-    return dy, dyb, dres, dgamma, dbeta
+                                  gsums.data_ptr() + 16 * c, _p(dy), _p(dyb), _p(dres), _p(db), _p(ws), ws.numel(), _stream()),
+             "toda_bn_bwd_finish")
+    return dy, dyb, dres, dgamma, dbeta, db
 
 
 class _BNAct(torch.autograd.Function):
@@ -906,8 +911,8 @@ class _BNAct(torch.autograd.Function):
             return (None,) * 13
         y, a, gamma, mean, rstd, gsums = ctx.saved_tensors
         training, relu, has_res, want_bf16 = ctx.cfg
-        dy, dyb, dres, dgamma, dbeta = _run_phases(_bn_backward_phases(da, y, a, gamma, mean, rstd, training, relu, has_res,
-                                                                       want_bf16, gsums), ctx.group)
+        dy, dyb, dres, dgamma, dbeta, _ = _run_phases(_bn_backward_phases(da, y, a, gamma, mean, rstd, training, relu, has_res,
+                                                                          want_bf16, gsums), ctx.group)
         if dyb is not None:
             dy._toda_bf16 = (dyb, dy._version)     # picked up by the producing conv's backward (see _bf16_shadow_of)
         return dy, dgamma, dbeta, None, None, None, None, None, dres, None, None, None, None
@@ -1014,9 +1019,9 @@ def _layer_backward_phases(da, saved, rb, precision, relu, has_res, has_bias, ne
     if da is None:
         da = torch.zeros_like(y)
     if not _fused_ok(training, True):
-        dy, dyb, dres, dgamma, dbeta = yield from _bn_backward_phases(da, y, a_mask, gamma, mean, rstd, training, relu, has_res,
-                                                                      precision == CONV_BF16, gsums)
-        dx, dw, db = _conv_backward_impl(dy, dyb, x, weight, xb, rb, precision, need_dx, need_dw, has_bias)
+        dy, dyb, dres, dgamma, dbeta, db = yield from _bn_backward_phases(da, y, a_mask, gamma, mean, rstd, training, relu,
+                                                                          has_res, precision == CONV_BF16, gsums, has_bias)
+        dx, dw, _ = _conv_backward_impl(dy, dyb, x, weight, xb, rb, precision, need_dx, need_dw, False)
         if addend is not None and dx is not None:
             dx = dx + addend
         return dx, dw, db, dgamma, dbeta, dres
@@ -1083,7 +1088,7 @@ def _layer_bwd_args(da, saved, rb, precision, training, relu, has_res, has_bias,
         int(bool(need_dx)), _vp(nbr), _vp(wt), _vp(wtb), _vp(out_rows), _vp(masks),
         _vp(pl.lidx) if pl else None, _vp(pl.rows) if pl else None, _vp(pl.cnt) if pl else None, pl.ngroups if pl else 0,
         pl.cap if pl else 0, _vp(addend) if need_dx else None, _vp(dx),
-        int(bool(need_dw)), rb.nbr_fwd.data_ptr(), _vp(dw), _vp(wws), wws.numel() if wws is not None else 0,
+        int(bool(need_dw)), rb.nbr_fwd.data_ptr(), _vp(rb.tile_masks), _vp(dw), _vp(wws), wws.numel() if wws is not None else 0,
         int(bool(has_bias)), sp + 8 * cout, precision, _vp(ws), ws.numel() if ws is not None else 0)
     return args, dx, dw, dres, small, (da, dy, dyb, addend, wt, wtb, ws, wws, bws)
 
