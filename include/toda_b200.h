@@ -199,45 +199,45 @@ int toda_parity_order(const int32_t *coords, int n, const int *stride_host, cons
 int toda_weight_repack(const float *w_param, int kvol, int cin, int cout, int transpose, int mirror_k, float *w_out,
                        void *stream);
 size_t toda_spconv_fwd_workspace_bytes(int n_in, int cin, int cout, int kvol, int precision);
-/* x_bf16 / dy_bf16 (optional, may be NULL): an existing bf16 copy of x / dy ([rows][channels], same values rounded to
- * nearest) that the TODA_CONV_BF16 kernels use instead of converting x / dy themselves. */
-/* bn_sums (optional, may be NULL; tensor-core kernel only, see toda_spconv_uses_tensor_cores): double[2*cout] receiving
- * sum(y) and sum(y*y) per output channel, accumulated in the epilogue, for toda_bn_apply_sums -- the BatchNorm that
- * follows the convolution (spconv_backbone.py L23-24) then needs no statistics pass over y. */
-/* out_rows (optional, may be NULL): int32[n_out]; output row o of this call is written to y[out_rows[o], :] instead of
- * y[o, :].  Used by the dgrad of strided convolutions: with stride s only the offsets k = (in + pad) mod s (per axis) can
- * reach an input voxel, so its rows are processed in s_z*s_y*s_x parity classes, each with the compact table of its own
- * 1..kvol offsets: the caller sorts the rows (and the table's columns) by class and they are scattered back to
- * canonical rows here; with tile_masks the K blocks that are structurally empty for a class are skipped (in canonical
- * order every tile mixes all classes and the [27] table is ~85 % structural padding).
- * tile_masks (optional, may be NULL): uint32[ceil(n_out/128)] from toda_table_tile_masks -- bit k set when some row of
- * that 128-row tile has a neighbour under offset k; the tensor-core kernel then walks only the K blocks that hold data
- * (the FFMA kernel tests this per tile itself). */
+/* tile_masks: uint32[ceil(n_out/128)], bit k set when some row of that 128-row tile has a neighbour under offset k. */
 int toda_table_tile_masks(const int32_t *nbr, int n_out, int kvol, uint32_t *masks, void *stream);
 int toda_spconv_uses_tensor_cores(int cin, int cout, int kvol, int precision);
 /* the same question for toda_spconv_wgrad */
 int toda_spconv_wgrad_uses_tensor_cores(int cin, int cout, int kvol, int precision);
-int toda_spconv_fwd(const float *x, const void *x_bf16, int n_in, int cin, const int32_t *nbr, int n_out, int kvol,
-                    const float *w, int cout, const float *bias, float *y, const int32_t *out_rows,
-                    const uint32_t *tile_masks, double *bn_sums, int precision, void *workspace, size_t workspace_bytes,
-                    void *stream);
 /* Tile plan (row cache of the TODA_CONV_BF16 kernel): for every 128-row tile of a neighbour table and every group of
  * kvol/ngroups consecutive offsets (ngroups = kz: the neighbours of one group lie in one z plane), the ascending list of
  * DISTINCT input rows the tile gathers (`rows`: int32, `cap` entries reserved per (tile, group); `cnt`: int32 per
  * (tile, group), entries used) and the table rewritten as 16-bit slots into that list (`lidx`: uint16
- * [tiles][kvol][128]; 0xFFFF = no neighbour, 0xFFFE = not in the list, read the row through `nbr`).  With a plan the
- * convolution loads each distinct row once per tile into shared memory and feeds tcgen05.mma's A operand from tensor
- * memory.  cap = toda_tile_plan_capacity(channels of the gathered rows) (<= 512).  toda_spconv_fwd_plan is
- * toda_spconv_fwd with the plan and an optional `addend` ([n_out][cout] fp32, added to y in the epilogue: the
- * residual-branch gradient in SparseBasicBlock's backward, spconv_backbone.py L63). */
+ * [tiles][kvol][128]; 0xFFFF = no neighbour, 0xFFFE = not in the list, read the row through `nbr`).
+ * cap = toda_tile_plan_capacity(channels of the gathered rows) (<= 512). */
 int toda_tile_plan_capacity(int channels);
 int toda_table_tile_plan(const int32_t *nbr, int n_out, int kvol, int ngroups, int cap, uint16_t *lidx, int32_t *rows,
                          int32_t *cnt, void *stream);
-int toda_spconv_fwd_plan(const float *x, const void *x_bf16, int n_in, int cin, const int32_t *nbr, int n_out, int kvol,
-                         const float *w, int cout, const float *bias, const float *addend, float *y,
-                         const int32_t *out_rows, const uint32_t *tile_masks, const uint16_t *plan_lidx,
-                         const int32_t *plan_rows, const int32_t *plan_cnt, int plan_groups, int plan_cap, double *bn_sums,
-                         const void *w_bf16, int precision, void *workspace, size_t workspace_bytes, void *stream);
+/* The convolution.  Every argument below is optional (NULL, or plan_lidx NULL for no plan):
+ * x_bf16 / dy_bf16: an existing bf16 copy of x / dy ([rows][channels], same values rounded to nearest) that the
+ *   TODA_CONV_BF16 kernels use instead of converting x / dy themselves.
+ * addend: [n_out][cout] fp32, added to y in the epilogue (every kernel): the residual-branch gradient in
+ *   SparseBasicBlock's backward, spconv_backbone.py L63.
+ * out_rows: int32[n_out]; output row o of this call is written to y[out_rows[o], :] instead of y[o, :].  Used by the
+ *   dgrad of strided convolutions: with stride s only the offsets k = (in + pad) mod s (per axis) can reach an input
+ *   voxel, so its rows are processed in s_z*s_y*s_x parity classes, each with the compact table of its own 1..kvol
+ *   offsets: the caller sorts the rows (and the table's columns) by class and they are scattered back to canonical rows
+ *   here; with tile_masks the K blocks that are structurally empty for a class are skipped (in canonical order every
+ *   tile mixes all classes and the [27] table is ~85 % structural padding).
+ * tile_masks: the toda_table_tile_masks words of `nbr`; the tensor-core kernels then walk only the K blocks that hold
+ *   data (the FFMA kernel tests this per tile itself).
+ * plan_lidx / plan_rows / plan_cnt / plan_groups / plan_cap: a tile plan of `nbr` (toda_table_tile_plan).  With a plan
+ *   the tensor-core convolution loads each distinct row once per tile into shared memory and feeds tcgen05.mma's A
+ *   operand from tensor memory; the FFMA kernel ignores it.
+ * bn_sums (tensor-core kernels only, see toda_spconv_uses_tensor_cores): double[2*cout] receiving sum(y) and sum(y*y)
+ *   per output channel, accumulated in the epilogue, for toda_bn_apply_sums -- the BatchNorm that follows the
+ *   convolution (spconv_backbone.py L23-24) then needs no statistics pass over y.
+ * w_bf16: see toda_weight_kmajor_bf16. */
+int toda_spconv_fwd(const float *x, const void *x_bf16, int n_in, int cin, const int32_t *nbr, int n_out, int kvol,
+                    const float *w, int cout, const float *bias, const float *addend, float *y,
+                    const int32_t *out_rows, const uint32_t *tile_masks, const uint16_t *plan_lidx,
+                    const int32_t *plan_rows, const int32_t *plan_cnt, int plan_groups, int plan_cap, double *bn_sums,
+                    const void *w_bf16, int precision, void *workspace, size_t workspace_bytes, void *stream);
 /* w_bf16 (optional, may be NULL): the weights already converted for the tensor-core kernels by toda_weight_kmajor_bf16
  * ([cout][kvol*max(cin,16)] bf16), so that a caller that caches them per optimizer step saves the conversion per call. */
 int toda_weight_kmajor_bf16(const float *w, int kvol, int cin, int cout, void *w_bf16, void *stream);

@@ -1,4 +1,4 @@
-"""The C-ABI library loads and exports every symbol include/toda_b200.h declares (no GPU needed)."""
+"""The C-ABI library loads and exports exactly the symbols include/toda_b200.h declares (no GPU needed)."""
 import os
 import re
 import subprocess
@@ -27,7 +27,7 @@ def test_every_declared_symbol_is_exported_and_bound(built):
     assert len(syms) >= 31
     out = subprocess.check_output(["nm", "-D", "--defined-only", built.LIB_PATH], text=True)
     exported = set(re.findall(r" T (toda_[a-z0-9_]+)", out))
-    assert set(syms) <= exported, sorted(set(syms) - exported)
+    assert set(syms) == exported, (sorted(set(syms) - exported), sorted(exported - set(syms)))
     assert set(syms) == set(built.SIGNATURES), (sorted(set(syms) ^ set(built.SIGNATURES)))
     lib = built.lib()
     for s in syms:
@@ -45,11 +45,12 @@ def test_size_queries_work_without_a_gpu(built):
     assert lib.toda_voxelize_workspace_bytes(1200000, 4, grid, 10, 120000) > 0
 
 
-def test_argument_errors_are_reported_not_ignored(built):
+def test_argument_errors_of_the_entry_points_are_reported(built):
     lib = built.lib()
     rc = lib.toda_mean_vfe_fwd(None, None, 0, 10, 0, 5, None, None)
     assert rc == -1 and b"mean_vfe_fwd" in lib.toda_last_error()
-    rc = lib.toda_spconv_fwd(None, None, 0, 0, None, 5, 27, None, 16, None, None, None, None, None, 0, None, 0, None)
+    rc = lib.toda_spconv_fwd(None, None, 0, 0, None, 5, 27, None, 16, None, None, None, None, None, None, None, None, 0, 0, None,
+                             None, 0, None, 0, None)
     assert rc == -1
 
 

@@ -1,4 +1,4 @@
-"""Row-cache / TMEM-operand convolution kernel (csrc/conv_ts.cu, toda_spconv_fwd_plan) against the round-1 tensor-core
+"""Row-cache / TMEM-operand convolution kernel (csrc/conv_ts.cu, toda_spconv_fwd with a tile plan) against the round-1 tensor-core
 kernels on the same tables: same bf16 operands, same K order, fp32 accumulation in TMEM => bit-identical outputs and
 BatchNorm sums.  Covers every conv geometry of VoxelResBackBone8x (SubM, stride-2 forward, parity-sorted dgrad with
 out_rows, the (3,1,1) conv_out), the 4/5-channel input layer, ragged tails and plans that overflow the slab

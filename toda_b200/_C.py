@@ -43,12 +43,10 @@ SIGNATURES = {
     "toda_parity_order_workspace_bytes": (c_sz, [c_int]),
     "toda_parity_order": (c_int, [c_vp, c_int, _IP, _IP, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "toda_table_tile_masks": (c_int, [c_vp, c_int, c_int, c_vp, c_vp]),
-    "toda_spconv_fwd": (c_int, [c_vp, c_vp, c_int, c_int, c_vp, c_int, c_int, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_vp,
-                                c_sz, c_vp]),
     "toda_tile_plan_capacity": (c_int, [c_int]),
     "toda_table_tile_plan": (c_int, [c_vp, c_int, c_int, c_int, c_int, c_vp, c_vp, c_vp, c_vp]),
-    "toda_spconv_fwd_plan": (c_int, [c_vp, c_vp, c_int, c_int, c_vp, c_int, c_int, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
-                                     c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_int, c_vp, c_sz, c_vp]),
+    "toda_spconv_fwd": (c_int, [c_vp, c_vp, c_int, c_int, c_vp, c_int, c_int, c_vp, c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp,
+                                c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_int, c_vp, c_sz, c_vp]),
     "toda_weight_kmajor_bf16": (c_int, [c_vp, c_int, c_int, c_int, c_vp, c_vp]),
     "toda_layer_fwd": (c_int, [c_vp, c_vp]),
     "toda_layer_bwd": (c_int, [c_vp, c_vp]),

@@ -279,39 +279,19 @@ extern "C" size_t toda_spconv_fwd_workspace_bytes(int n_in, int cin, int cout, i
     return 0;
 }
 
-static int spconv_fwd_impl(const float *x, const void *x_bf16, int n_in, int cin, const int32_t *nbr, int n_out, int kvol,
-                           const float *w, int cout, const float *bias, float *y, const int32_t *out_rows,
-                           const uint32_t *tile_masks, double *bn_sums, int precision, void *workspace, size_t workspace_bytes,
-                           void *stream, const TilePlan *plan, const float *addend, const void *w_bf16);
-
 extern "C" int toda_spconv_fwd(const float *x, const void *x_bf16, int n_in, int cin, const int32_t *nbr, int n_out, int kvol,
-                               const float *w, int cout, const float *bias, float *y, const int32_t *out_rows,
-                               const uint32_t *tile_masks, double *bn_sums, int precision,
-                               void *workspace, size_t workspace_bytes, void *stream) {
-    return spconv_fwd_impl(x, x_bf16, n_in, cin, nbr, n_out, kvol, w, cout, bias, y, out_rows, tile_masks, bn_sums, precision, workspace,
-                           workspace_bytes, stream, nullptr, nullptr, nullptr);
-}
-
-extern "C" int toda_spconv_fwd_plan(const float *x, const void *x_bf16, int n_in, int cin, const int32_t *nbr, int n_out, int kvol,
-                                    const float *w, int cout, const float *bias, const float *addend, float *y,
-                                    const int32_t *out_rows, const uint32_t *tile_masks, const uint16_t *plan_lidx,
-                                    const int32_t *plan_rows, const int32_t *plan_cnt, int plan_groups, int plan_cap, double *bn_sums,
-                                    const void *w_bf16, int precision, void *workspace, size_t workspace_bytes, void *stream) {
-    TilePlan plan{plan_lidx, plan_rows, plan_cnt, plan_groups, plan_cap};
-    return spconv_fwd_impl(x, x_bf16, n_in, cin, nbr, n_out, kvol, w, cout, bias, y, out_rows, tile_masks, bn_sums, precision, workspace,
-                           workspace_bytes, stream, plan_lidx ? &plan : nullptr, addend, w_bf16);
-}
-
-static int spconv_fwd_impl(const float *x, const void *x_bf16, int n_in, int cin, const int32_t *nbr, int n_out, int kvol,
-                           const float *w, int cout, const float *bias, float *y, const int32_t *out_rows,
-                           const uint32_t *tile_masks, double *bn_sums, int precision, void *workspace, size_t workspace_bytes,
-                           void *stream, const TilePlan *plan, const float *addend, const void *w_bf16) {
+                               const float *w, int cout, const float *bias, const float *addend, float *y,
+                               const int32_t *out_rows, const uint32_t *tile_masks, const uint16_t *plan_lidx,
+                               const int32_t *plan_rows, const int32_t *plan_cnt, int plan_groups, int plan_cap, double *bn_sums,
+                               const void *w_bf16, int precision, void *workspace, size_t workspace_bytes, void *stream) {
     TODA_CHECK_ARG(n_in >= 0 && n_out >= 0 && cin > 0 && cout > 0 && kvol > 0, "spconv_fwd: bad sizes");
     if (n_out == 0) return TODA_OK;
     TODA_CHECK_ARG(x && nbr && w && y, "spconv_fwd: null pointer");
     cudaStream_t st = (cudaStream_t)stream;
     TODA_CHECK_ARG(precision == TODA_CONV_FP32 || precision == TODA_CONV_BF16 || precision == TODA_CONV_BF16X3,
                    "spconv_fwd: unknown precision %d", precision);
+    const TilePlan plan_data{plan_lidx, plan_rows, plan_cnt, plan_groups, plan_cap};
+    const TilePlan *plan = plan_lidx ? &plan_data : nullptr;
     if (precision == TODA_CONV_BF16X3 && conv_tc_supported(cin, cout, kvol))
         return conv_x3_fwd(x, n_in, cin, nbr, n_out, kvol, w, cout, bias, y, out_rows, tile_masks, bn_sums, workspace, workspace_bytes, st,
                            plan, addend);

@@ -18,7 +18,6 @@
 // input-stationary table with transposed weights.
 #include <cuda.h>
 #include <cuda_bf16.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "conv_ts.cuh"
@@ -171,8 +170,7 @@ __global__ void __launch_bounds__(kFwdThreads, 1) conv_tc_fwd_kernel(const __nv_
                                                                      float *__restrict__ y,
                                                                      const int *__restrict__ out_rows /* optional */,
                                                                      const uint32_t *__restrict__ tile_masks /* optional */,
-                                                                     double *__restrict__ bn_sums, int num_tiles,
-                                                                     long long *__restrict__ dbg) {
+                                                                     double *__restrict__ bn_sums, int num_tiles) {
     static_assert(COUT % 16 == 0 && COUT >= 16 && COUT <= 128, "UMMA N");
     static_assert(CIN == 16 || CIN == 32 || CIN == 64 || CIN == 128, "row = 32..256 bytes of bf16");
     using C = FwdCfg<COUT, KB>;
@@ -252,10 +250,7 @@ __global__ void __launch_bounds__(kFwdThreads, 1) conv_tc_fwd_kernel(const __nv_
         int g = 0, it = 0;              // global chunk counter (stage ring position), tile counter
         for (int t = blockIdx.x; t < num_tiles; t += gridDim.x, ++it) {
             const int ib = it & 1;
-            if (dbg && blockIdx.x == 0 && tid == 0 && it < 256) dbg[0 * 256 + it] = clock64();      // tile start (before the slice wait)
             mbar_wait(idx_full + 8 * ib, (it >> 1) & 1);
-            if (dbg && blockIdx.x == 0 && tid == 0 && it < 256) dbg[1 * 256 + it] = clock64();      // slice there
-            if (dbg && blockIdx.x == 0 && tid == 0 && it < 255) dbg[7 * 256 + it] = g;              // first chunk index of the tile
             const uint32_t idx_tile = idx_lane + ib * kIdxBytes;
             for (unsigned long long cm = chunk_mask_of(t); cm; cm &= cm - 1, ++g) {
                 const int c = __ffsll((long long)cm) - 1;
@@ -302,7 +297,6 @@ __global__ void __launch_bounds__(kFwdThreads, 1) conv_tc_fwd_kernel(const __nv_
                     __syncwarp();
                     if (lane == 0) mbar_arrive(full_bar + 8 * ((g - kLag) % S));
                 }
-                if (dbg && blockIdx.x == 0 && tid == 0 && g < 256) dbg[3 * 256 + g] = clock64();
             }
             mbar_arrive(idx_empty + 8 * ib);   // this tile's table slice has been consumed
         }
@@ -329,9 +323,7 @@ __global__ void __launch_bounds__(kFwdThreads, 1) conv_tc_fwd_kernel(const __nv_
                 for (unsigned long long cm = chunk_mask_of(t); cm; cm &= cm - 1, ++g) {
                     const int c = __ffsll((long long)cm) - 1;
                     const int s = g % S, use = g / S;
-                    if (dbg && blockIdx.x == 0 && lane == 0 && g < 256) dbg[4 * 256 + g] = clock64();
                     if (!ready) mbar_wait(full_bar + 8 * s, use & 1);
-                    if (dbg && blockIdx.x == 0 && lane == 0 && g < 256) dbg[5 * 256 + g] = clock64();
                     const int sn = (g + 1) % S, usen = (g + 1) / S;
                     ready = mbar_test(full_bar + 8 * sn, usen & 1);            // look one stage ahead
                     // (the producers fence their generic-proxy zero stores before signalling; no proxy fence needed here)
@@ -351,7 +343,6 @@ __global__ void __launch_bounds__(kFwdThreads, 1) conv_tc_fwd_kernel(const __nv_
                     }
                     accumulate = 1u;
                     __syncwarp();
-                    if (dbg && blockIdx.x == 0 && lane == 0 && g < 256) dbg[6 * 256 + g] = clock64();
                 }
                 if (elect_one()) umma_commit(acc_full + 8 * ab);            // accumulator of this tile complete
                 __syncwarp();
@@ -411,7 +402,6 @@ __global__ void __launch_bounds__(kFwdThreads, 1) conv_tc_fwd_kernel(const __nv_
             }
             asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
             mbar_arrive(acc_empty + 8 * ab);
-            if (dbg && blockIdx.x == 0 && q == 1 && lane == 0 && it < 256) dbg[2 * 256 + it] = clock64();   // tile drained
         }
         if (bn_sums && !(lane & 1)) {
             // lane l (even) owns column n0 + ((l >> 1) & 15); one fp64 atomic per CTA-warp and channel
@@ -513,14 +503,6 @@ int conv_tma_fwd(const void *xb, int n_in, int cin, const int32_t *nbr, int n_ou
                  const float *bias, const float *addend, float *y, const int32_t *out_rows, const uint32_t *tile_masks, double *bn_sums,
                  cudaStream_t st);
 
-// development aid: device buffer (8 x 256 int64: clock64 samples per chunk / per tile) filled by CTA 0 of the cp.async forward kernel
-static long long *g_dbg_timeline = nullptr;
-extern "C" void toda_debug_set_timeline(long long *buf) { g_dbg_timeline = buf; }
-long long *conv_tc_debug_timeline() { return g_dbg_timeline; }
-static int g_dbg_mode = 0;
-extern "C" void toda_debug_set_mode(int m) { g_dbg_mode = m; }
-int conv_tc_debug_mode() { return g_dbg_mode; }
-
 // w [kvol][cin][cout] fp32 -> [cout][kvol*max(cin,16)] bf16, the B operand of the tensor-core kernels (cacheable by the caller)
 extern "C" int toda_weight_kmajor_bf16(const float *w, int kvol, int cin, int cout, void *w_bf16, void *stream) {
     TODA_CHECK_ARG(w && w_bf16 && kvol > 0 && cin > 0 && cout > 0, "weight_kmajor_bf16: bad args");
@@ -573,18 +555,13 @@ int conv_tc_fwd(const float *x, const void *x_bf16, int n_in, int cin, const int
     }
     cin = cp;
     if (bn_sums) TODA_CUDA_OK(cudaMemsetAsync(bn_sums, 0, 2 * (size_t)cout * sizeof(double), st));
-    // operand feed, chosen by shape from measurements on B200 (profiles/r01_feed_ab.md): TMA (gather4 rows + tiled
-    // weights, conv_tma.cu) wins when rows are 256 bytes (Cin = Cout = 128); gather4 costs ~20-50 cycles per instruction
-    // whatever the row width, so the cp.async producers below are faster for narrower rows.
-    // TODA_TC_FEED=tma|cpasync forces one of them (A/B measurements).
-    static int feed = -1;
-    if (feed < 0) { const char *e = getenv("TODA_TC_FEED"); feed = !e ? 2 : (e[0] == 'c' ? 0 : (e[0] == 't' && e[1] == 'm' ? 1 : 2)); }
     // with a tile plan (toda_table_tile_plan) the row-cache / TMEM-operand kernel takes every supported shape
-    // (TODA_TC_FEED=tma|cpasync keeps the round-1 kernels for A/B measurements)
-    if (feed == 2 && conv_ts_supported(cin, cout, kvol, plan))
+    if (conv_ts_supported(cin, cout, kvol, plan))
         return conv_ts_fwd(xb, n_in, cin, nbr, n_out, kvol, *plan, wb, cout, bias, addend, y, out_rows, tile_masks, bn_sums, st);
-    if (feed == 1 || (feed == 2 && cin == 128 && cout == 128))
-        {
+    // otherwise the operand feed is chosen by shape from measurements on B200 (profiles/r01_feed_ab.md): TMA (gather4 rows +
+    // tiled weights, conv_tma.cu) wins when rows are 256 bytes (Cin = Cout = 128); gather4 costs ~20-50 cycles per
+    // instruction whatever the row width, so the cp.async producers below are faster for narrower rows.
+    if (cin == 128 && cout == 128) {
         // (raster-order masks skip ~17 % of the 128-channel chunks but measured slower on this kernel -- the skipped chunks
         // unbalance the round-robin of its four issuing warps; class-sorted dgrad rows, where most chunks vanish, keep them)
         return conv_tma_fwd(xb, n_in, cin, nbr, n_out, kvol, wb, cout, bias, addend, y, out_rows, out_rows ? tile_masks : nullptr, bn_sums, st);
@@ -604,7 +581,7 @@ int conv_tc_fwd(const float *x, const void *x_bf16, int n_in, int cin, const int
             TODA_CUDA_OK(cudaFuncSetAttribute(conv_tc_fwd_kernel<CI, CO, KB_>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); \
             attr_set = true;                                                                                                 \
         }                                                                                                                    \
-        conv_tc_fwd_kernel<CI, CO, KB_><<<grid, kFwdThreads, smem, st>>>(xb, nbr, n_out, kvol, map_w, bias, addend, y, out_rows, tile_masks, bn_sums, num_tiles, g_dbg_timeline); \
+        conv_tc_fwd_kernel<CI, CO, KB_><<<grid, kFwdThreads, smem, st>>>(xb, nbr, n_out, kvol, map_w, bias, addend, y, out_rows, tile_masks, bn_sums, num_tiles); \
     } while (0)
 #define LAUNCH_TC_CO(CI)                                                                                 \
     switch (cout) {                                                                                      \
@@ -618,7 +595,14 @@ int conv_tc_fwd(const float *x, const void *x_bf16, int n_in, int cin, const int
         case 16: LAUNCH_TC_CO(16); break;
         case 32: LAUNCH_TC_CO(32); break;
         case 64: LAUNCH_TC_CO(64); break;
-        case 128: LAUNCH_TC_CO(128); break;
+        case 128:                       // (Cout = 128 went to conv_tma_fwd above)
+            switch (cout) {
+                case 16: LAUNCH_TC(128, 16); break;
+                case 32: LAUNCH_TC(128, 32); break;
+                case 64: LAUNCH_TC(128, 64); break;
+                default: toda_set_error("conv_tc_fwd: unsupported cout %d", cout); return TODA_ERR_UNSUPPORTED;
+            }
+            break;
         default: toda_set_error("conv_tc_fwd: unsupported cin %d", cin); return TODA_ERR_UNSUPPORTED;
     }
 #undef LAUNCH_TC_CO

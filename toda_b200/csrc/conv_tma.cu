@@ -400,26 +400,15 @@ int conv_tma_make_map(CUtensorMap *m, const void *ptr, uint64_t rows, uint64_t c
     return make_map(m, ptr, rows, cols, box_rows, box_cols);
 }
 
-// xb: bf16 [n_in][cin], wb: bf16 [cout][kvol*cin]; cin, cout in {16,32,64,128}
+// xb: bf16 [n_in][128], wb: bf16 [128][kvol*128].  Only Cin = Cout = 128 is built: narrower rows go to conv_tc.cu's
+// cp.async producers, which are faster for them (profiles/r01_feed_ab.md).
 int conv_tma_fwd(const void *xb, int n_in, int cin, const int32_t *nbr, int n_out, int kvol, const void *wb, int cout,
                  const float *bias, const float *addend, float *y, const int32_t *out_rows, const uint32_t *tile_masks, double *bn_sums,
                  cudaStream_t st) {
-    const __nv_bfloat16 *x = (const __nv_bfloat16 *)xb, *w = (const __nv_bfloat16 *)wb;
-#define CASE_CO(CI)                                                                                    \
-    switch (cout) {                                                                                    \
-        case 16: return launch<CI, 16>(x, n_in, nbr, n_out, kvol, w, bias, addend, y, out_rows, tile_masks, bn_sums, st);                     \
-        case 32: return launch<CI, 32>(x, n_in, nbr, n_out, kvol, w, bias, addend, y, out_rows, tile_masks, bn_sums, st);                     \
-        case 64: return launch<CI, 64>(x, n_in, nbr, n_out, kvol, w, bias, addend, y, out_rows, tile_masks, bn_sums, st);                     \
-        case 128: return launch<CI, 128>(x, n_in, nbr, n_out, kvol, w, bias, addend, y, out_rows, tile_masks, bn_sums, st);                   \
-    }                                                                                                  \
-    break;
-    switch (cin) {
-        case 16: CASE_CO(16)
-        case 32: CASE_CO(32)
-        case 64: CASE_CO(64)
-        case 128: CASE_CO(128)
+    if (cin != 128 || cout != 128) {
+        toda_set_error("conv_tma_fwd: only cin=cout=128 is built, got cin=%d cout=%d", cin, cout);
+        return TODA_ERR_UNSUPPORTED;
     }
-#undef CASE_CO
-    toda_set_error("conv_tma_fwd: unsupported cin=%d cout=%d", cin, cout);
-    return TODA_ERR_UNSUPPORTED;
+    return launch<128, 128>((const __nv_bfloat16 *)xb, n_in, nbr, n_out, kvol, (const __nv_bfloat16 *)wb, bias, addend, y, out_rows,
+                            tile_masks, bn_sums, st);
 }

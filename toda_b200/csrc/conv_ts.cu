@@ -43,7 +43,6 @@ constexpr uint32_t kLidxGlobal = 0xFFFEu;         // neighbour exists but is not
 // Same bytes in flight per SM either way; the second is ahead for 256-byte rows, the first for the narrow layers.
 // the warp scheduler favours high warp ids: the latency-critical gather warps get them
 constexpr int kWarpMma = 4, kWarpLoader = 5, kWarpB = 6, kWarpLoader2 = 7, kWarpGather0 = 8;
-constexpr int kLoaders = 2;   // slab loader warps (2: even / odd blocks)
 // A ring: pair slots of 2 x 32 TMEM columns (2 x 64 K elements) behind the two accumulators
 // Pair gp is produced by warpgroup gp % 4 into slot gp % kSlots.  Its barriers are NOT per slot but per pair index modulo
 // 16 (a_full / a_empty[gp & 15]): every barrier is then waited on by one warpgroup only, which sees each of its phases in turn
@@ -59,14 +58,8 @@ __device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
 }
 // A lost arrival must not hang the GPU box: a wait gives up (trap) after 2^26 probes (seconds; generous, because the first
 // NCCL all-reduce of a multi-GPU run can stall every kernel on the device for hundreds of milliseconds).  (A wall-clock limit read from %globaltimer cost registers in every inlined
-// wait and 10 % of the kernel's speed; -DTODA_TS_VERBOSE_TIMEOUT compiles in the printf that names the barrier, lists every
-// stuck waiter before trapping, and records each role's progress in shared memory.)
-#ifdef TODA_TS_VERBOSE_TIMEOUT
-__shared__ int ts_prog[32];
-#define TS_PROG(v) do { } while (0)
-#else
-#define TS_PROG(v) do { } while (0)
-#endif
+// wait and 10 % of the kernel's speed; -DTODA_TS_VERBOSE_TIMEOUT compiles in the printf that names the barrier and lists
+// every stuck waiter before trapping.)
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
     uint32_t done = 0, spins = 0;
     while (!done) {
@@ -82,11 +75,8 @@ __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
             : "memory");
         if (!done && ++spins > (1u << 26)) {
 #ifdef TODA_TS_VERBOSE_TIMEOUT
-            if ((threadIdx.x & 31) == 0) {
-                volatile int *pg = ts_prog;
-                printf("conv_ts: mbarrier timeout smem=0x%x parity=%u block=%d warp=%d | prog mma %x L0 %x L1 %x B %x g8 %x g12 %x g16 %x g20 %x me %x\n", bar, parity, (int)blockIdx.x,
-                       (int)(threadIdx.x >> 5), pg[4], pg[5], pg[7], pg[6], pg[8], pg[12], pg[16], pg[20], pg[threadIdx.x >> 5]);
-            }
+            if ((threadIdx.x & 31) == 0)
+                printf("conv_ts: mbarrier timeout smem=0x%x parity=%u block=%d warp=%d\n", bar, parity, (int)blockIdx.x, (int)(threadIdx.x >> 5));
             if (spins < (1u << 26) + (1u << 25)) { spins += (1u << 24); continue; }
 #endif
             __trap();
@@ -250,7 +240,7 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
                                                                   const float *__restrict__ bias, const float *__restrict__ addend,
                                                                   float *__restrict__ y, const int *__restrict__ out_rows,
                                                                   const uint32_t *__restrict__ tile_masks,
-                                                                  double *__restrict__ bn_sums, int num_tiles, long long *__restrict__ dbg, int xmode) {
+                                                                  double *__restrict__ bn_sums, int num_tiles) {
     using C = TsCfg<CIN, COUT>;
     constexpr int NB = C::kNB, SB = C::kSB, PARTS = C::kParts, PV = C::kPV;
     constexpr bool BRES = C::kBRes;
@@ -353,12 +343,6 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem_base = *tmem_slot_ptr;
-    // development aid (scripts/debug_timeline_ts.py): clock64 samples of CTA 0, 16 rows x 256 entries
-#ifdef TODA_TS_TIMELINE
-#define TS_DBG(cond, rowi, idx) do { if (dbg && blockIdx.x == 0 && (cond) && (idx) < 256) dbg[(rowi) * 256 + (idx)] = clock64(); } while (0)
-#else
-#define TS_DBG(cond, rowi, idx) do { } while (0)
-#endif
 
     if (warp >= kWarpGather0) {
         // ------------------------------------------------------------------ gather warps: thread = tile row = TMEM lane
@@ -373,19 +357,13 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
         const uint32_t ugs = (uint32_t)gs, ugs2 = (uint32_t)gs2, ukvol = (uint32_t)kvol;
         uint32_t gpbase = 0, it = 0;                    // global index of this tile's first pair
         uint32_t uq = 0, ur = 0;                        // the tile's first (tile, group) unit is number uq * NB + ur of this CTA
-#ifdef TODA_TS_TIMELINE
-        int gbase = 0;
-#endif
         uint32_t om_next = load_om(blockIdx.x);
         for (int t = blockIdx.x; t < num_tiles; t += gridDim.x, ++it) {
             const uint32_t ib = it & 1u;
             const uint32_t om = om_next;
             om_next = load_om(t + gridDim.x);
-            TS_DBG(tid == 256, 22, it);
             mbar_wait(lidx_full + 8 * ib, (it >> 1) & 1u);
-            TS_DBG(tid == 256, 23, it);
             const uint32_t lidx_tile = lidx_base + ib * kLidxBytes + 2u * row;
-            TS_PROG((int)((it << 12) | (uq << 4) | ur));
             // slab buffer, barrier offset and phase parity of the tile's (up to three) offset groups
             uint32_t sbuf[3], sbar[3], spar[3];
 #pragma unroll
@@ -479,20 +457,13 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
             const uint32_t nact = (uint32_t)__popcll(cm), npairs = (nact + 1u) >> 1;
             int kl0, kl1;
             kb_list(cm, kl0, kl1);
-#ifdef TODA_TS_TIMELINE
-            if (dbg && blockIdx.x == 0 && tid == 256 && it < 256) dbg[10 * 256 + it] = gbase;
-#endif
             // this warpgroup's pairs of the tile: global pair index gp = gpbase + pj with gp % kWGs == wg (kWGs is 2 or 4)
             for (uint32_t pj = (wg - gpbase) & (uint32_t)(C::kWGs - 1); pj < npairs; pj += (uint32_t)C::kWGs) {
                 const uint32_t kbA = (uint32_t)kb_at(kl0, kl1, (int)(2u * pj));
                 const uint32_t kbB = (uint32_t)kb_at(kl0, kl1, (int)((2u * pj + 1u) & 63u));
                 const bool two = 2u * pj + 1u < nact;
-#ifdef TODA_TS_TIMELINE
-                const int gA = gbase + 2 * (int)pj;
-#endif
                 const uint32_t gp = gpbase + pj;        // global pair index: A slot gp % kASlots (two 32-column blocks)
                 const uint32_t aslot = gp % (uint32_t)kASlots;
-                TS_DBG((tid & 127) == 0, 0, gA);
                 uint32_t liA[PARTS], liB[PARTS];
                 load_li(kbA, true, liA);
                 load_li(kbB, two, liB);
@@ -502,7 +473,6 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
                 const uint32_t k_last = min(CIN == 128 ? (kb_last >> 1) : kb_last * PARTS + PARTS - 1, ukvol - 1u);
                 const uint32_t g_last = (k_last >= ugs ? 1u : 0u) + (k_last >= ugs2 ? 1u : 0u);
                 release_below(g_first);                 // slabs of earlier groups are no longer read by this warp
-                TS_DBG((tid & 127) == 0, 1, gA);
                 // With two slab buffers (256-byte rows) groups 0 and 2 of a tile share a buffer: a pair whose blocks lie in
                 // those two groups (group 1 fully masked out) cannot have both resident -- it is walked one block at a time,
                 // the first group handed back in between.  (Waiting for both deadlocked the CTA on such a tile.)
@@ -519,7 +489,6 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
                         mbar_wait(a_empty + 8u * (pg & (kABars - 1)), (pg / kABars) & 1u);
                         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                     }
-                    TS_DBG((tid & 127) == 0, 12, gA);
                     if (__any_sync(0xffffffffu, fixA || fixB)) {
                         fix_block(kbA, liA, va);
                         fix_block(kbB, liB, vb);
@@ -533,7 +502,6 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
                         mbar_wait(a_empty + 8u * (pg & (kABars - 1)), (pg / kABars) & 1u);
                         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                     }
-                    TS_DBG((tid & 127) == 0, 12, gA);
                     if (__any_sync(0xffffffffu, fixA)) fix_block(kbA, liA, va);
                     __syncwarp();
                     TS_STTM_X32(t_lane + aslot * 64u, va);
@@ -548,21 +516,13 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
                         TS_STTM_X32(t_lane + aslot * 64u + 32u, va);
                     }
                 }
-                TS_DBG((tid & 127) == 0, 2, gA);
                 asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
                 asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
                 __syncwarp();
                 if (lane == 0) mbar_arrive(a_full + 8u * (gp & (kABars - 1)));
-                TS_DBG((tid & 127) == 0, 3, gA);
-                TS_DBG(lane == 0, 16 + (warp - kWarpGather0), gA);
             }
-#ifdef TODA_TS_TIMELINE
-            gbase += (int)nact;
-#endif
             gpbase += npairs;
-            TS_DBG(tid == 256, 20, it);
             release_below((uint32_t)ngroups);
-            TS_DBG(tid == 256, 21, it);
             ur += (uint32_t)ngroups;
             while (ur >= (uint32_t)NB) { ur -= (uint32_t)NB; ++uq; }
             __syncwarp();
@@ -595,7 +555,7 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
                 float o[16];
 #pragma unroll
                 for (int j = 0; j < 16; ++j) o[j] = __uint_as_float(v[j]) + (bias ? __ldg(bias + n0 + j) : 0.f);
-                if (row < n_out && !(xmode & 16)) {
+                if (row < n_out) {
                     if (addend) {
                         const float4 *ad = (const float4 *)(addend + (size_t)orow * COUT + n0);
 #pragma unroll
@@ -644,9 +604,7 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
             const int ab = it & 1, ause = it >> 1;
             const uint32_t om = om_next;
             om_next = load_om(t + gridDim.x);
-            TS_DBG(lane == 0, 14, it);
             if (ause > 0) mbar_wait(acc_empty + 8 * ab, (ause - 1) & 1);   // epilogue has drained this accumulator
-            TS_DBG(lane == 0, 15, it);
             const uint32_t d_tmem = tmem_base + ab * COUT;
             uint32_t accumulate = 0;
             const unsigned long long cm = kb_mask_from(om);
@@ -665,13 +623,11 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
                     m32 &= m32 - 1u;
                 }
                 const int aslot = gp % kASlots;
-                TS_PROG((it << 12) | gp);
                 mbar_wait(a_full + 8 * (gp & (kABars - 1)), (gp / kABars) & 1);
                 if (!BRES) {
                     mbar_wait(b_full + 8 * (gA % SB), (gA / SB) & 1);
                     if (n == 2) mbar_wait(b_full + 8 * ((gA + 1) % SB), ((gA + 1) / SB) & 1);
                 }
-                TS_DBG(lane == 0, 4, gA);
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                 if (elect_one()) {
 #pragma unroll
@@ -681,11 +637,9 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
                             const int stage = BRES ? kb : g % SB;
                             const uint64_t bd0 = make_desc_k_sw128(base + stage * C::kBStage);
                             const uint32_t a0 = tmem_base + kACol0 + aslot * 64 + i * 32;
-                            if (!(xmode & 4)) {
-                                umma_bf16_ts(d_tmem, a0, bd0, idesc, accumulate);
+                            umma_bf16_ts(d_tmem, a0, bd0, idesc, accumulate);
 #pragma unroll
-                                for (int jj = 1; jj < 4; ++jj) umma_bf16_ts(d_tmem, a0 + 8 * jj, bd0 + 2 * jj, idesc, 1u);   // K = 16: 8 columns / 32 bytes
-                            }
+                            for (int jj = 1; jj < 4; ++jj) umma_bf16_ts(d_tmem, a0 + 8 * jj, bd0 + 2 * jj, idesc, 1u);   // K = 16: 8 columns / 32 bytes
                             accumulate = 1u;
                             if (!BRES) umma_commit(b_empty + 8 * stage);
                         }
@@ -694,20 +648,18 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
                 }
                 accumulate = 1u;
                 __syncwarp();
-                TS_DBG(lane == 0, 5, gA);
                 ++gp;
             }
             gbase += nact;
             if (elect_one()) umma_commit(acc_full + 8 * ab);
             __syncwarp();
         }
-    } else if (warp == kWarpLoader || (warp == kWarpLoader2 && kLoaders == 2)) {
+    } else if (warp == kWarpLoader || warp == kWarpLoader2) {
         // ------------------------------------------------------------------ loaders (two warps: even / odd blocks; issuing a TMA costs
         // ~65 cycles): table slice + row slabs, up to NB groups ahead.
         // One TMA box copy (16 rows, hardware-swizzled) per cached block, lane i issuing block i of the unit.  The block list of
         // unit u+1 is fetched while unit u is issued (a list read is two dependent L2 round trips).
         const int L = warp == kWarpLoader ? 0 : 1;
-        const bool idle_loader = L == 1 && (xmode & 256);   // TODA_TS_LOADERS=1: the first loader warp fetches every block
         int bid_n = -1, nb_n = 0;
         auto fetch_unit = [&](int t, int grp) {
             if (t < num_tiles) {
@@ -717,20 +669,17 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
         };
         fetch_unit(blockIdx.x, 0);
         int it = 0;
-        for (int t = blockIdx.x; t < num_tiles && !idle_loader; t += gridDim.x, ++it) {
+        for (int t = blockIdx.x; t < num_tiles; t += gridDim.x, ++it) {
             const int ib = it & 1;
-            TS_PROG((it << 4) | 5);
-            if (L == 0 && lane == 0 && !(xmode & 64)) {
+            if (L == 0 && lane == 0) {
                 if (it >= 2) mbar_wait(lidx_empty + 8 * ib, ((it >> 1) - 1) & 1);
                 const uint32_t bytes = (uint32_t)kvol * (kTileM * 2);
                 mbar_arrive_expect_tx(lidx_full + 8 * ib, bytes);
                 bulk_copy_g2s(lidx_base + ib * kLidxBytes, lidx + (size_t)t * kvol * kTileM, bytes, lidx_full + 8 * ib);
             }
             __syncwarp();
-            for (int grp = 0; grp < ngroups && !(xmode & 32); ++grp) {
+            for (int grp = 0; grp < ngroups; ++grp) {
                 const int u = it * ngroups + grp, buf = u % NB, use = u / NB;
-                TS_PROG((u << 4) | 1);
-                TS_DBG(L == 0 && lane == 0, 7, u);
                 const int bid = bid_n, nb = nb_n;
                 if (grp + 1 < ngroups) fetch_unit(t, grp + 1);
                 else fetch_unit(t + gridDim.x, 0);
@@ -741,26 +690,20 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
                 if (L == 0) {
                     if (use > 0) mbar_wait(slab_empty + 8 * buf, (use - 1) & 1);
                     if (lane == 0) {
-                        if (nb > 0 && !(xmode & 8)) mbar_arrive_expect_tx(slab_full + 8 * buf, (uint32_t)nb * 16u * C::kRowBytes);
+                        if (nb > 0) mbar_arrive_expect_tx(slab_full + 8 * buf, (uint32_t)nb * 16u * C::kRowBytes);
                         else mbar_arrive(slab_full + 8 * buf);
                     }
                 }
-                TS_PROG((u << 4) | 2);
-                TS_DBG(L == 0 && lane == 0, 8, u);
                 __syncwarp();
-                if (kLoaders == 2 && !(xmode & 256)) asm volatile("barrier.sync 1, 64;" ::: "memory");
-                if (bid >= 0 && (kLoaders == 1 || (xmode & 256) || (lane & 1) == L) && !(xmode & 8)) {
+                asm volatile("barrier.sync 1, 64;" ::: "memory");
+                if (bid >= 0 && (lane & 1) == L) {
                     const uint32_t dst = slab_base + buf * C::kSlab + lane * (16 * C::kRB);
 #pragma unroll
                     for (int h = 0; h < C::kHalves; ++h)
                         tma_load_2d(dst + h * C::kHalfSlab, &map_x, h * 64, bid * 16, slab_full + 8 * buf);
                 }
-                TS_PROG((u << 4) | 3);
-                TS_DBG(L == 0 && lane == 0, 9, u);
             }
-            TS_PROG((it << 4) | 4);
         }
-        TS_PROG(0xfffff);
     } else if (warp == kWarpB) {
         // ------------------------------------------------------------------ weight producer (the warp walks the tiles together: the
         // K-block mask is a warp-collective; lane 0 issues the TMA copies)
@@ -780,7 +723,6 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
                         const int kb = __ffsll((long long)cm) - 1;
                         const int stage = gg % SB, use = gg / SB;
                         if (use > 0) mbar_wait_relaxed(b_empty + 8 * stage, (use - 1) & 1);
-                        TS_DBG(true, 13, gg);
                         mbar_arrive_expect_tx(b_full + 8 * stage, C::kBStage);
                         tma_load_2d(base + stage * C::kBStage, &map_w, kb * 64, 0, b_full + 8 * stage);
                     }
@@ -889,13 +831,6 @@ __global__ void __launch_bounds__(128) tile_plan_kernel(const int *__restrict__ 
     }
 }
 
-// TODA_TS_LOADERS=1: one slab-loader warp instead of two (A/B switch)
-static int ts_env_mode() {
-    static int m = -1;
-    if (m < 0) { const char *e = getenv("TODA_TS_LOADERS"); m = (e && e[0] == '1') ? 256 : 0; }
-    return m;
-}
-
 template <int CIN, int COUT>
 int launch_ts(const __nv_bfloat16 *xb, int n_in, const int32_t *nbr, int n_out, int kvol, const TilePlan &plan, const __nv_bfloat16 *wb,
               const float *bias, const float *addend, float *y, const int32_t *out_rows, const uint32_t *tile_masks, double *bn_sums,
@@ -917,7 +852,7 @@ int launch_ts(const __nv_bfloat16 *xb, int n_in, const int32_t *nbr, int n_out, 
     }
     conv_ts_fwd_kernel<CIN, COUT><<<grid, C::kThreads, C::kSmem, st>>>(xb, nbr, n_out, kvol, plan.lidx, plan.rows, plan.cnt, plan.ngroups,
                                                                    plan.cap, map_x, map_w, bias, addend, y, out_rows, tile_masks, bn_sums,
-                                                                   num_tiles, conv_tc_debug_timeline(), conv_tc_debug_mode() | ts_env_mode());
+                                                                   num_tiles);
     TODA_LAUNCH_OK();
     return TODA_OK;
 }

@@ -22,6 +22,3 @@ int conv_ts_fwd(const void *xb, int n_in, int cin, const int32_t *nbr, int n_out
                 double *bn_sums, cudaStream_t st);
 // 2-D bf16 row-major tensor map [rows][cols] with box [box_rows][box_cols], swizzle by box row bytes (conv_tma.cu)
 int conv_tma_make_map(CUtensorMap *m, const void *ptr, uint64_t rows, uint64_t cols, uint32_t box_rows, uint32_t box_cols);
-// development aid: device buffer for clock64 timelines (set through toda_debug_set_timeline), or nullptr
-long long *conv_tc_debug_timeline();
-int conv_tc_debug_mode();

@@ -6,9 +6,9 @@
 #include "common.cuh"
 
 static int layer_conv(const toda_layer_fwd_args *p, double *bn_sums, void *stream) {
-    return toda_spconv_fwd_plan(p->x, p->x_bf16, p->n_in, p->cin, p->nbr, p->n_out, p->kvol, p->w, p->cout, p->bias, nullptr, p->y,
-                                nullptr, p->tile_masks, p->plan_lidx, p->plan_rows, p->plan_cnt, p->plan_groups, p->plan_cap,
-                                bn_sums, p->w_bf16, p->precision, p->conv_ws, p->conv_ws_bytes, stream);
+    return toda_spconv_fwd(p->x, p->x_bf16, p->n_in, p->cin, p->nbr, p->n_out, p->kvol, p->w, p->cout, p->bias, nullptr, p->y,
+                           nullptr, p->tile_masks, p->plan_lidx, p->plan_rows, p->plan_cnt, p->plan_groups, p->plan_cap,
+                           bn_sums, p->w_bf16, p->precision, p->conv_ws, p->conv_ws_bytes, stream);
 }
 
 // Training forward up to the BatchNorm's statistics: the convolution, then sum(y) | sum(y*y) of its output in `sums` (in
@@ -80,9 +80,9 @@ static int layer_bwd_conv(const toda_layer_bwd_args *p, void *stream) {
     if (p->need_dx) {
         // dgrad = the forward kernel on the input-stationary table with transposed (SubM: mirrored) weights; `addend` is the
         // gradient that reaches the same tensor through the block's residual branch (spconv_backbone.py L63)
-        rc = toda_spconv_fwd_plan(p->dy, p->dy_bf16, n, c, p->dgrad_nbr, p->n_in, p->kvol, p->wt, p->cin, nullptr, p->addend, p->dx,
-                                  p->dgrad_out_rows, p->dgrad_masks, p->dplan_lidx, p->dplan_rows, p->dplan_cnt, p->dplan_groups,
-                                  p->dplan_cap, nullptr, p->wt_bf16, p->precision, p->conv_ws, p->conv_ws_bytes, stream);
+        rc = toda_spconv_fwd(p->dy, p->dy_bf16, n, c, p->dgrad_nbr, p->n_in, p->kvol, p->wt, p->cin, nullptr, p->addend, p->dx,
+                             p->dgrad_out_rows, p->dgrad_masks, p->dplan_lidx, p->dplan_rows, p->dplan_cnt, p->dplan_groups,
+                             p->dplan_cap, nullptr, p->wt_bf16, p->precision, p->conv_ws, p->conv_ws_bytes, stream);
         if (rc) return rc;
     }
     if (p->need_dw) {

@@ -7,7 +7,7 @@
 // Full tiles take the fast path: a running pointer and ROWS/32 coalesced 128-byte cp.async per offset, ~3 instructions
 // per copy.  (The first version recomputed k, r, the bounds test and a 64-bit address per element, ~15 instructions; on
 // 16-channel layers the single indexer warp then took longer per tile than the eight producer warps and they stalled
-// ~4 k cycles at every tile boundary -- scripts/debug_timeline.py 16 16.)
+// ~4 k cycles at every tile boundary: the "indexer fix" of profiles/r01_feed_ab.md.)
 template <int ROWS>
 __device__ __forceinline__ void load_table_slice(uint32_t dst0, const int *__restrict__ nbr_k0, int n_out, int row_base, int r_end,
                                                  int noffs, int lane) {

@@ -18,7 +18,6 @@ ORDER_CANONICAL = 1
 CONV_FP32 = 0
 CONV_BF16 = 1
 CONV_BF16X3 = 2      # split-bf16, three tensor-core launches per product: fp32-class accuracy (csrc/conv_x3.cu)
-_TC_PRECISIONS = (CONV_BF16, CONV_BF16X3)
 
 # launches of this library's kernels since the last reset (bench.py reports it as gpu_launches): counted inside the
 # library, at every launch site (toda_launch_count)
@@ -424,6 +423,15 @@ class Rulebook:
     def kvol(self):
         return self.ksize[0] * self.ksize[1] * self.ksize[2]
 
+    def dgrad_table(self):
+        """-> (nbr, out_rows, tile_masks, plan) of the dgrad: SubM walks nbr_fwd (with mirrored weights); a strided conv
+        walks nbr_bwd, in parity-class order when there is one (rows written back to canonical order through out_rows)."""
+        if self.subm:
+            return self.nbr_fwd, None, self.tile_masks, self.plan
+        if self.dgrad_order is None:
+            return self.nbr_bwd, None, None, self.dgrad_plan
+        return self.nbr_bwd_sorted, self.dgrad_order, self.dgrad_tile_masks, self.dgrad_plan
+
 
 @dataclass
 class TilePlan:
@@ -622,38 +630,19 @@ def _bf16_shadow_of(t):
 
 def _conv_call(x, xb, cin, nbr, n_out, kvol, w, cout, bias, precision, what="conv_fwd", rb=None, bn_sums=None, y=None,
                out_rows=None, tile_masks=None, plan=None, addend=None, w_bf16=None):
-    """addend (optional, (n_out, cout) fp32): added to the result in the kernel's epilogue; only with a usable plan
-    (see conv_plan_usable), otherwise the caller adds it."""
+    """addend (optional, (n_out, cout) fp32): added to the result in the kernel's epilogue."""
     if y is None:
         y = torch.empty((n_out, cout), dtype=torch.float32, device=x.device)
     L = _C.lib()
     ws_bytes = L.toda_spconv_fwd_workspace_bytes(x.shape[0], cin, cout, kvol, precision)
     ws = _workspace("conv", ws_bytes, x.device) if ws_bytes else None
-    if precision not in _TC_PRECISIONS:
-        plan = None
     with _timed(what, n_in=x.shape[0], n_out=n_out, cin=cin, cout=cout, kvol=kvol, precision=precision, rb=id(rb)):
-        if plan is None and addend is None and w_bf16 is None:
-            _C.check(L.toda_spconv_fwd(_p(x), _p(xb), x.shape[0], cin, _p(nbr), n_out, kvol, _p(w), cout, _p(bias), _p(y),
-                                       _p(out_rows), _p(tile_masks), _p(bn_sums), precision, _p(ws), ws.numel() if ws is not None else 0,
-                                       _stream()), "toda_spconv_fwd")
-        else:
-            pl = plan
-            _C.check(L.toda_spconv_fwd_plan(_p(x), _p(xb), x.shape[0], cin, _p(nbr), n_out, kvol, _p(w), cout, _p(bias),
-                                            _p(addend), _p(y), _p(out_rows), _p(tile_masks), _p(pl.lidx) if pl else None,
-                                            _p(pl.rows) if pl else None, _p(pl.cnt) if pl else None, pl.ngroups if pl else 0,
-                                            pl.cap if pl else 0, _p(bn_sums), _p(w_bf16), precision, _p(ws),
-                                            ws.numel() if ws is not None else 0, _stream()), "toda_spconv_fwd_plan")
+        _C.check(L.toda_spconv_fwd(_p(x), _p(xb), x.shape[0], cin, _p(nbr), n_out, kvol, _p(w), cout, _p(bias), _p(addend), _p(y),
+                                   _p(out_rows), _p(tile_masks), _p(plan.lidx) if plan else None,
+                                   _p(plan.rows) if plan else None, _p(plan.cnt) if plan else None,
+                                   plan.ngroups if plan else 0, plan.cap if plan else 0, _p(bn_sums), _p(w_bf16), precision,
+                                   _p(ws), ws.numel() if ws is not None else 0, _stream()), "toda_spconv_fwd")
     return y
-
-
-def conv_plan_usable(plan, cin, cout, kvol, precision):
-    """True when toda_spconv_fwd_plan will run the row-cache kernel for this call (and can therefore fuse an addend)."""
-    if plan is None or precision not in _TC_PRECISIONS or _os.environ.get("TODA_TC_FEED", "ts")[:1] in ("c",) or \
-            _os.environ.get("TODA_TC_FEED", "ts")[:2] == "tm":
-        return False
-    cp = max(16, cin)
-    return (cp in (16, 32, 64, 128) and cout in (16, 32, 64, 128) and kvol <= 27
-            and plan.cap <= _C.lib().toda_tile_plan_capacity(cp))
 
 
 def _conv_forward_impl(x, x_bf16, weight, bias, rb, precision, want_stats):
@@ -682,16 +671,9 @@ def _conv_backward_impl(dy, dyb, x, weight, xb, rb, precision, need_dx, need_dw,
     if need_dx:
         # dgrad = the same gather-GEMM on the input-stationary table with transposed weights
         wt = _repack(weight, True, rb.subm)
-        if rb.subm:
-            dx = _conv_call(dy, dyb, cout, rb.nbr_fwd, rb.n_in, rb.kvol, wt, cin, None, precision, "conv_dgrad", rb,
-                            tile_masks=rb.tile_masks, plan=rb.plan)
-        elif rb.dgrad_order is None:
-            dx = _conv_call(dy, dyb, cout, rb.nbr_bwd, rb.n_in, rb.kvol, wt, cin, None, precision, "conv_dgrad", rb,
-                            plan=rb.dgrad_plan)
-        else:
-            # strided conv: rows in parity-class order (empty K blocks are skipped), written back to canonical rows
-            dx = _conv_call(dy, dyb, cout, rb.nbr_bwd_sorted, rb.n_in, rb.kvol, wt, cin, None, precision, "conv_dgrad",
-                            rb, out_rows=rb.dgrad_order, tile_masks=rb.dgrad_tile_masks, plan=rb.dgrad_plan)
+        nbr, out_rows, masks, plan = rb.dgrad_table()
+        dx = _conv_call(dy, dyb, cout, nbr, rb.n_in, rb.kvol, wt, cin, None, precision, "conv_dgrad", rb,
+                        out_rows=out_rows, tile_masks=masks, plan=plan)
     if need_dw:
         dw = torch.empty_like(weight)
         ws_bytes = L.toda_spconv_wgrad_workspace_bytes(rb.n_in, rb.n_out, rb.kvol, cin, cout, precision)
@@ -992,7 +974,7 @@ def _layer_fwd_args(x, x_bf16, weight, bias, rb, precision, gamma, beta, running
     bws = _workspace("bn", L.toda_bn_workspace_bytes(cout), dev)
     res = residual.contiguous() if residual is not None else None
     b = bias.contiguous() if bias is not None else None
-    pl = rb.plan if precision in _TC_PRECISIONS else None
+    pl = rb.plan
     sp = small.data_ptr()
     args = _C.LayerFwdArgs(
         x.data_ptr(), _vp(x_bf16), x.shape[0], cin, rb.nbr_fwd.data_ptr(), n_out, kvol, w.data_ptr(), _vp(wb), cout, _vp(b),
@@ -1063,14 +1045,7 @@ def _layer_bwd_args(da, saved, rb, precision, training, relu, has_res, has_bias,
             wt, wtb = _repack(weight, True, rb.subm, True)
         else:
             wt = _repack(weight, True, rb.subm)
-        if rb.subm:
-            nbr, masks, pl = rb.nbr_fwd, rb.tile_masks, rb.plan
-        elif rb.dgrad_order is None:
-            nbr, pl = rb.nbr_bwd, rb.dgrad_plan
-        else:
-            nbr, out_rows, masks, pl = rb.nbr_bwd_sorted, rb.dgrad_order, rb.dgrad_tile_masks, rb.dgrad_plan
-        if precision not in _TC_PRECISIONS:
-            pl = None
+        nbr, out_rows, masks, pl = rb.dgrad_table()
         dx = torch.empty((rb.n_in, cin), dtype=torch.float32, device=dev)
         if addend is not None:
             addend = addend.contiguous()
