@@ -121,6 +121,42 @@ int toda_points_world_transform(const float *points, int n, int stride, int x_co
                                 int n_steps, const int *kinds_host, const float *params_host, float *out, void *stream);
 
 /* ------------------------------------------------------------------------------------------
+ * K0 gt_sampling: the device side of DataBaseSampler.__call__ / add_sampled_boxes_to_scene
+ * (pcdet/datasets/augmentor/database_sampler.py; OpenPCDet v0.5.2) for a whole batch of frames.  The database samples
+ * are drawn on the host; the collision test, the scene-point removal and the paste run on `stream` in four launches
+ * without a host synchronisation.
+ *
+ * toda_gt_sampling_pack_boxes (host only): boxes_host float32 [n][7] (x, y, z, dx, dy, dz, heading) ->
+ * packed_host float32 [n][16] = {x, y, z, dx, dy, dz, cosf(h), sinf(h), cosf(-h), sinf(-h), dx + w0, dy + w1, dz + w2, 0,
+ * 0, 0} with libm cosf / sinf (what the compiled ops iou3d_cpu.cpp / roiaware_pool3d.cpp evaluate) and the enlarged sizes
+ * of box_utils.enlarge_box3d in float32 (w = extra_width_host[3], or 0 when it is NULL).
+ *
+ * toda_gt_sampling:
+ *   points [n][stride] fp32 frames back to back, frame_offsets int32[batch+1] device, batch <= 64; x_col 0 (raw frames)
+ *     or 1 (collated, column 0 = batch index); stride = x_col + db_features.
+ *   exist_boxes packed [E][16]: every frame's unmasked gt_boxes, frame b at exist_offsets_host[b..b+1).
+ *   samp_boxes packed [S][16] (enlarged by REMOVE_EXTRA_WIDTH): frame by frame, within a frame class by class in
+ *     SAMPLE_GROUPS order; group_sizes_host[b * n_groups + g] samples of group g in frame b (n_groups <= 16, at most 1024
+ *     samples per frame, else TODA_ERR_UNSUPPORTED).
+ *   samp_rows int64 [S][2] (first row, row count) of each sample's object points in db_points [R][db_features];
+ *   samp_shift float64 [S][3]: the database box centre box3d_lidar[:3]; shift_f64 != 0 when the database stores float64
+ *     boxes (object xyz = float32(double(p) + c)), 0 for float32 boxes (float32 add).
+ * A sample is accepted iff every iou_bev against the frame's gt boxes, the samples accepted for earlier classes and
+ * the other samples of its class is exactly 0 (boxes_bev_iou_cpu, iou1.max + iou2.max == 0); accepted int32 [S] gets
+ * 1 / 0.  Scene rows inside an accepted box (points_in_boxes_cpu with the enlarged box) are removed.  out [>= n + sum of
+ * the sample row counts][stride]: frame b = the object rows of its accepted samples in sample order, xyz shifted by the box
+ * centre (batch column = b when x_col == 1), then its kept scene rows in input order; out_offsets int32[batch+1].
+ * Deterministic, no atomics.  The workspace is toda_gt_sampling_workspace_bytes(n, batch, S) bytes.
+ * ------------------------------------------------------------------------------------------ */
+int toda_gt_sampling_pack_boxes(const float *boxes_host, int n, const float *extra_width_host, float *packed_host);
+size_t toda_gt_sampling_workspace_bytes(int n, int batch, int n_samples);
+int toda_gt_sampling(const float *points, int n, int stride, int x_col, const int32_t *frame_offsets, int batch,
+                     const float *exist_boxes, const int *exist_offsets_host, const float *samp_boxes, const int *group_sizes_host,
+                     int n_groups, const float *db_points, int db_features, const int64_t *samp_rows, const double *samp_shift,
+                     int shift_f64, float *out, int32_t *out_offsets, int32_t *accepted, void *workspace, size_t workspace_bytes,
+                     void *stream);
+
+/* ------------------------------------------------------------------------------------------
  * K1 hard voxelizer.  Replaces spconv.utils.Point2VoxelCPU3d.point_to_voxel as called from
  * pcdet/datasets/processor/data_processor.py L36-42, L54 (VoxelGeneratorWrapper) /
  * L115-143 (transform_points_to_voxels), for a whole batch of frames in one call.

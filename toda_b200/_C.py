@@ -28,6 +28,10 @@ SIGNATURES = {
     "toda_points_select": (c_int, [c_vp, c_int, c_int, c_int, c_vp, c_int, c_int, ctypes.POINTER(ctypes.c_double), c_int, c_int,
                                    c_vp, c_vp, c_vp, c_sz, c_vp]),
     "toda_points_world_transform": (c_int, [c_vp, c_int, c_int, c_int, c_vp, c_int, c_int, _IP, _FP, c_vp, c_vp]),
+    "toda_gt_sampling_pack_boxes": (c_int, [c_vp, c_int, c_vp, c_vp]),
+    "toda_gt_sampling_workspace_bytes": (c_sz, [c_int, c_int, c_int]),
+    "toda_gt_sampling": (c_int, [c_vp, c_int, c_int, c_int, c_vp, c_int, c_vp, _IP, c_vp, _IP, c_int, c_vp, c_int, c_vp, c_vp,
+                                 c_int, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "toda_voxelize_workspace_bytes": (c_sz, [c_i64, c_int, _IP, c_int, c_int]),
     "toda_voxelize_hard": (c_int, [c_vp, c_i64, c_int, c_int, c_int, c_int, c_vp, c_int, _FP, _FP, _IP, c_int, c_int,
                                    c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),

@@ -61,8 +61,20 @@ __device__ __forceinline__ bool sel_keep(const SelParams &p, float x, float y, f
     return k != (p.invert != 0);
 }
 
-__global__ void __launch_bounds__(kSelThreads) select_flag_kernel(const float *__restrict__ points, int n, int stride, int x_col,
-                                                                  SelParams p, uint32_t *__restrict__ words,
+// the predicate of toda_points_select: one of the four modes above on the row's x, y (and z)
+struct SelKeep {
+    const float *points;
+    int stride, x_col;
+    SelParams p;
+    __device__ __forceinline__ bool operator()(int i) const {
+        const float *row = points + (size_t)i * stride + x_col;
+        return sel_keep(p, __ldg(row), __ldg(row + 1), p.mode == 3 ? __ldg(row + 2) : 0.f);
+    }
+};
+
+// launch 1 of the compaction: ballot words and per-tile counts of rows i < n for which keep(i) holds
+template <class Keep>
+__global__ void __launch_bounds__(kSelThreads) select_flag_kernel(int n, const Keep keep, uint32_t *__restrict__ words,
                                                                   int *__restrict__ tile_counts) {
     __shared__ int warp_cnt[kSelThreads / 32];
     const int tile0 = blockIdx.x * kSelTile;
@@ -71,11 +83,7 @@ __global__ void __launch_bounds__(kSelThreads) select_flag_kernel(const float *_
 #pragma unroll
     for (int j = 0; j < kSelTile / kSelThreads; ++j) {
         const int i = tile0 + j * kSelThreads + threadIdx.x;      // a warp covers 32 consecutive points = one word
-        bool k = false;
-        if (i < n) {
-            const float *row = points + (size_t)i * stride + x_col;
-            k = sel_keep(p, __ldg(row), __ldg(row + 1), p.mode == 3 ? __ldg(row + 2) : 0.f);
-        }
+        const bool k = i < n && keep(i);
         const uint32_t w = __ballot_sync(0xffffffffu, k);
         if (lane == 0) {
             words[(tile0 >> 5) + j * (kSelThreads / 32) + warp] = w;
@@ -96,13 +104,15 @@ __global__ void __launch_bounds__(kSelThreads) select_copy_kernel(const float *_
                                                                   const uint32_t *__restrict__ words,
                                                                   const int *__restrict__ tile_counts,
                                                                   const int32_t *__restrict__ frame_offsets, int batch,
-                                                                  int add_batch_col, float *__restrict__ out,
-                                                                  int32_t *__restrict__ out_offsets) {
+                                                                  int add_batch_col, const int *__restrict__ frame_lead,
+                                                                  float *__restrict__ out, int32_t *__restrict__ out_offsets) {
     __shared__ int warp_sums[kSelThreads / 32];
     __shared__ int tile_offset_s;
     __shared__ int word_prefix[kSelTile / 32 + 1];
     __shared__ int frame_lo[65];               // frame_offsets (batch <= 64)
+    __shared__ int lead_lo[65];                // rows written in front of the kept rows of the frames before b
     __shared__ int kept_rows[kSelTile];
+    __shared__ unsigned char kept_frame[kSelTile];
     __shared__ uint32_t word_s[kSelTile / 32];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     int part = 0;
@@ -111,6 +121,14 @@ __global__ void __launch_bounds__(kSelThreads) select_copy_kernel(const float *_
     for (int o = 16; o > 0; o >>= 1) part += __shfl_xor_sync(0xffffffffu, part, o);
     if (lane == 0) warp_sums[warp] = part;
     if (frame_offsets && (int)threadIdx.x <= batch) frame_lo[threadIdx.x] = frame_offsets[threadIdx.x];
+    if (frame_lead && threadIdx.x == 0) {
+        int t = 0;
+        for (int q = 0; q < batch; ++q) {
+            lead_lo[q] = t;
+            t += frame_lead[q];
+        }
+        lead_lo[batch] = t;
+    }
     __syncthreads();
     const int tile0 = blockIdx.x * kSelTile;
     if (warp == 0) {
@@ -150,23 +168,33 @@ __global__ void __launch_bounds__(kSelThreads) select_copy_kernel(const float *_
                         const int rel = fo - tile0, w = rel >> 5, b = rel & 31;
                         v = tile_offset + word_prefix[w] + __popc(word_s[w] & ((1u << b) - 1u));
                     }
-                    out_offsets[threadIdx.x] = v;
+                    out_offsets[threadIdx.x] = v + (frame_lead ? lead_lo[threadIdx.x] : 0);
                 }
             }
         } else if (threadIdx.x == 0 && (tile0 + kSelTile >= n)) {
             out_offsets[0] = tile_offset + word_prefix[kSelTile / 32];
         }
     }
-    // kept rows of this tile, in order, as a list in shared memory; then the tile's output range
-    // [tile_offset, tile_offset + count) x out_stride is written element by element: stores are fully coalesced and the
-    // loads walk neighbouring rows
+    // kept rows of this tile, in order, as a list in shared memory (with their frame where it is needed); then the
+    // tile's output range [tile_offset, tile_offset + count) x out_stride is written element by element: stores are
+    // fully coalesced and the loads walk neighbouring rows.  With frame_lead, the rows of frame b move down by the
+    // frame_lead rows of frames 0..b (a gap in front of each frame's rows, filled by the caller).
     const int out_stride = stride + (add_batch_col ? 1 : 0);
+    const bool need_frame = frame_offsets && (add_batch_col || frame_lead);
 #pragma unroll
     for (int j = 0; j < kSelTile / kSelThreads; ++j) {
         const int i = tile0 + j * kSelThreads + threadIdx.x;
         const int wi = j * (kSelThreads / 32) + warp;
         const uint32_t w = word_s[wi];
-        if ((w >> lane) & 1u) kept_rows[word_prefix[wi] + __popc(w & ((1u << lane) - 1u))] = i;
+        if ((w >> lane) & 1u) {
+            const int r = word_prefix[wi] + __popc(w & ((1u << lane) - 1u));
+            kept_rows[r] = i;
+            if (need_frame) {
+                int b = 0;
+                for (int q = 1; q < batch; ++q) b += (i >= frame_lo[q]) ? 1 : 0;   // frame of point i (batch is small)
+                kept_frame[r] = (unsigned char)b;
+            }
+        }
     }
     __syncthreads();
     const int count = word_prefix[kSelTile / 32];
@@ -180,17 +208,15 @@ __global__ void __launch_bounds__(kSelThreads) select_copy_kernel(const float *_
         float v;
         if (add_batch_col) {
             if (c == 0) {
-                int b = 0;
-                if (frame_offsets)
-                    for (int q = 1; q < batch; ++q) b += (i >= frame_lo[q]) ? 1 : 0;   // frame of point i (batch is small)
-                v = (float)b;
+                v = frame_offsets ? (float)kept_frame[r] : 0.f;
             } else {
                 v = __ldg(points + (size_t)i * stride + c - 1);
             }
         } else {
             v = __ldg(points + (size_t)i * stride + c);
         }
-        o[e] = v;
+        if (frame_lead) o[e + (size_t)lead_lo[kept_frame[r] + 1] * out_stride] = v;
+        else o[e] = v;
     }
 }
 
@@ -246,10 +272,10 @@ extern "C" int toda_points_select(const float *points, int n, int stride, int x_
     const int tiles = ceil_div(n > 0 ? n : 1, kSelTile);
     uint32_t *words = (uint32_t *)workspace;
     int *tile_counts = (int *)((char *)workspace + align_up((size_t)tiles * (kSelTile / 32) * sizeof(uint32_t), 256));
-    select_flag_kernel<<<tiles, kSelThreads, 0, st>>>(points, n, stride, x_col, p, words, tile_counts);
+    select_flag_kernel<<<tiles, kSelThreads, 0, st>>>(n, SelKeep{points, stride, x_col, p}, words, tile_counts);
     TODA_LAUNCH_OK();
     select_copy_kernel<<<tiles, kSelThreads, 0, st>>>(points, n, stride, words, tile_counts, frame_offsets, batch, add_batch_col,
-                                                      out, out_offsets);
+                                                      nullptr, out, out_offsets);
     TODA_LAUNCH_OK();
     return TODA_OK;
 }
@@ -382,5 +408,460 @@ extern "C" int toda_points_world_transform(const float *points, int n, int strid
     world_transform_kernel<<<ceil_div(n, kTfRows), kTfRows, smem, (cudaStream_t)stream>>>(points, n, stride, x_col, frame_offsets,
                                                                                           batch, p, out);
     TODA_LAUNCH_OK();
+    return TODA_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// gt_sampling (DataBaseSampler.__call__ / add_sampled_boxes_to_scene, pcdet/datasets/augmentor/database_sampler.py;
+// OpenPCDet v0.5.2) for a whole batch: the sampled database boxes are drawn on the host, the rest runs here in four
+// launches on the stream, with no host synchronisation:
+//   1 gts_accept_kernel   one CTA per frame.  Classes in SAMPLE_GROUPS order; every sample of a class is tested against
+//                         the frame's gt boxes, the boxes accepted for earlier classes (shared memory) and the other
+//                         samples of its class, all pairs of a class in parallel.  A sample is accepted iff every iou_bev
+//                         is exactly 0 (boxes_bev_iou_cpu, iou1.max + iou2.max == 0).  Writes the accepted flags, the
+//                         accepted boxes enlarged by REMOVE_EXTRA_WIDTH, and where each accepted sample's object rows go.
+//   2 select_flag_kernel  (K0 compaction, launch 1) scene rows outside every accepted box of their frame
+//                         (remove_points_in_boxes3d / points_in_boxes_cpu semantics); the frame by binary search.
+//   3 select_copy_kernel  (K0 compaction, launch 2) kept rows, each frame moved down by its object rows.
+//   4 gts_paste_kernel    one CTA per sample: the object rows of the accepted samples in front of their frame's rows,
+//                         shifted by the database box centre.
+// The float32 arithmetic is that of the compiled ops, op by op without FMA (iou3d_cpu.cpp box_overlap, roiaware_pool3d.cpp
+// check_pt_in_box3d_cpu); cos / sin of the headings come from the host (toda_gt_sampling_pack_boxes, libm cosf / sinf),
+// and point_cmp's atan2f is the fdlibm float algorithm that glibc's libm implements, restated below.
+namespace {
+
+constexpr int kGtsThreads = 256;
+constexpr int kGtsMaxSamples = 1024;           // sampled boxes per frame (shared memory of gts_accept_kernel)
+constexpr int kGtsMaxGroups = 16;
+constexpr int kGtsMaxBatch = 64;
+constexpr int kGtsBoxFloats = 16;              // packed box: see include/toda_b200.h
+
+struct GtsFrames {
+    int n_groups;
+    int exist_off[kGtsMaxBatch + 1];           // gt boxes of frame b: [exist_off[b], exist_off[b+1])
+    int samp_off[kGtsMaxBatch + 1];            // sampled boxes of frame b, grouped by class in SAMPLE_GROUPS order
+    unsigned short group_size[kGtsMaxBatch][kGtsMaxGroups];
+};
+
+struct BevBox { float cx, cy, dx, dy, ca, sa, cna, sna; };   // cos / sin of rz and of -rz
+
+__device__ __forceinline__ BevBox load_bev(const float4 *__restrict__ boxes, int i) {
+    const float4 u = __ldg(boxes + 4 * i), v = __ldg(boxes + 4 * i + 1), w = __ldg(boxes + 4 * i + 2);
+    return BevBox{u.x, u.y, u.w, v.x, v.z, v.w, w.x, w.y};
+}
+
+// ---- atan2f as glibc's libm computes it (sysdeps/ieee754/flt-32/e_atan2f.c, s_atanf.c: the fdlibm float algorithm)
+__device__ __forceinline__ float ref_atanf(float x) {
+    const float atanhi[4] = {4.6364760399e-01f, 7.8539812565e-01f, 9.8279368877e-01f, 1.5707962513e+00f};
+    const float atanlo[4] = {5.0121582440e-09f, 3.7748947079e-08f, 3.4473217170e-08f, 7.5497894159e-08f};
+    const int hx = __float_as_int(x), ix = hx & 0x7fffffff;
+    int id;
+    if (ix >= 0x4c000000) {                    // |x| >= 2^25
+        if (ix > 0x7f800000) return __fadd_rn(x, x);
+        return hx > 0 ? __fadd_rn(atanhi[3], atanlo[3]) : __fsub_rn(-atanhi[3], atanlo[3]);
+    }
+    if (ix < 0x3ee00000) {                     // |x| < 0.4375
+        if (ix < 0x31000000) return x;         // |x| < 2^-29
+        id = -1;
+    } else {
+        x = fabsf(x);
+        if (ix < 0x3f980000) {
+            if (ix < 0x3f300000) { id = 0; x = __fdiv_rn(__fsub_rn(__fmul_rn(2.0f, x), 1.0f), __fadd_rn(2.0f, x)); }
+            else { id = 1; x = __fdiv_rn(__fsub_rn(x, 1.0f), __fadd_rn(x, 1.0f)); }
+        } else {
+            if (ix < 0x401c0000) { id = 2; x = __fdiv_rn(__fsub_rn(x, 1.5f), __fadd_rn(1.0f, __fmul_rn(1.5f, x))); }
+            else { id = 3; x = __fdiv_rn(-1.0f, x); }
+        }
+    }
+    const float z = __fmul_rn(x, x), w = __fmul_rn(z, z);
+    const float s1 = __fmul_rn(z, __fadd_rn(3.3333334327e-01f, __fmul_rn(w, __fadd_rn(1.4285714924e-01f, __fmul_rn(w,
+                     __fadd_rn(9.0908870101e-02f, __fmul_rn(w, __fadd_rn(6.6610731184e-02f, __fmul_rn(w,
+                     __fadd_rn(4.9768779427e-02f, __fmul_rn(w, 1.6285819933e-02f)))))))))));
+    const float s2 = __fmul_rn(w, __fadd_rn(-2.0000000298e-01f, __fmul_rn(w, __fadd_rn(-1.1111110449e-01f, __fmul_rn(w,
+                     __fadd_rn(-7.6918758452e-02f, __fmul_rn(w, __fadd_rn(-5.8335702866e-02f, __fmul_rn(w, -3.6531571299e-02f)))))))));
+    if (id < 0) return __fsub_rn(x, __fmul_rn(x, __fadd_rn(s1, s2)));
+    const float r = __fsub_rn(atanhi[id], __fsub_rn(__fsub_rn(__fmul_rn(x, __fadd_rn(s1, s2)), atanlo[id]), x));
+    return hx < 0 ? -r : r;
+}
+
+__device__ __forceinline__ float ref_atan2f(float y, float x) {
+    const float tiny = 1.0e-30f, pi_o_4 = 7.8539818525e-01f, pi_o_2 = 1.5707963705e+00f, pi = 3.1415927410e+00f,
+                pi_lo = -8.7422776573e-08f;
+    const int hx = __float_as_int(x), ix = hx & 0x7fffffff, hy = __float_as_int(y), iy = hy & 0x7fffffff;
+    if (ix > 0x7f800000 || iy > 0x7f800000) return __fadd_rn(x, y);
+    if (hx == 0x3f800000) return ref_atanf(y);
+    const int m = ((hy >> 31) & 1) | ((hx >> 30) & 2);
+    if (iy == 0) {
+        if (m < 2) return y;
+        return m == 2 ? __fadd_rn(pi, tiny) : __fsub_rn(-pi, tiny);
+    }
+    if (ix == 0) return hy < 0 ? __fsub_rn(-pi_o_2, tiny) : __fadd_rn(pi_o_2, tiny);
+    if (ix == 0x7f800000) {
+        if (iy == 0x7f800000) {
+            if (m == 0) return __fadd_rn(pi_o_4, tiny);
+            if (m == 1) return __fsub_rn(-pi_o_4, tiny);
+            if (m == 2) return __fadd_rn(__fmul_rn(3.0f, pi_o_4), tiny);
+            return __fsub_rn(__fmul_rn(-3.0f, pi_o_4), tiny);
+        }
+        if (m == 0) return 0.0f;
+        if (m == 1) return -0.0f;
+        return m == 2 ? __fadd_rn(pi, tiny) : __fsub_rn(-pi, tiny);
+    }
+    if (iy == 0x7f800000) return hy < 0 ? __fsub_rn(-pi_o_2, tiny) : __fadd_rn(pi_o_2, tiny);
+    const int k = (iy - ix) >> 23;
+    float z;
+    if (k > 60) z = __fadd_rn(pi_o_2, __fmul_rn(0.5f, pi_lo));
+    else if (hx < 0 && k < -60) z = 0.0f;
+    else z = ref_atanf(fabsf(__fdiv_rn(y, x)));
+    if (m == 0) return z;
+    if (m == 1) return __int_as_float(__float_as_int(z) ^ 0x80000000);
+    if (m == 2) return __fsub_rn(pi, __fsub_rn(z, pi_lo));
+    return __fsub_rn(__fsub_rn(z, pi_lo), pi);
+}
+
+// ---- iou3d_cpu.cpp, float32 op by op
+__device__ __forceinline__ float ref_min(float a, float b) { return a > b ? b : a; }
+__device__ __forceinline__ float ref_max(float a, float b) { return a > b ? a : b; }
+
+__device__ __forceinline__ float cross3(float2 p1, float2 p2, float2 p0) {      // cross(p1, p2, p0)
+    return __fsub_rn(__fmul_rn(__fsub_rn(p1.x, p0.x), __fsub_rn(p2.y, p0.y)), __fmul_rn(__fsub_rn(p2.x, p0.x), __fsub_rn(p1.y, p0.y)));
+}
+
+__device__ __forceinline__ bool check_rect_cross(float2 p1, float2 p2, float2 q1, float2 q2) {
+    return ref_min(p1.x, p2.x) <= ref_max(q1.x, q2.x) && ref_min(q1.x, q2.x) <= ref_max(p1.x, p2.x) &&
+           ref_min(p1.y, p2.y) <= ref_max(q1.y, q2.y) && ref_min(q1.y, q2.y) <= ref_max(p1.y, p2.y);
+}
+
+__device__ __forceinline__ bool check_in_box2d(const BevBox &b, float2 p) {
+    const float sx = __fsub_rn(p.x, b.cx), sy = __fsub_rn(p.y, b.cy);
+    const float rx = __fadd_rn(__fmul_rn(sx, b.cna), __fmul_rn(sy, -b.sna));
+    const float ry = __fadd_rn(__fmul_rn(sx, b.sna), __fmul_rn(sy, b.cna));
+    return fabsf(rx) < __fadd_rn(__fdiv_rn(b.dx, 2.0f), 1e-2f) && fabsf(ry) < __fadd_rn(__fdiv_rn(b.dy, 2.0f), 1e-2f);
+}
+
+__device__ __forceinline__ bool intersection(float2 p1, float2 p0, float2 q1, float2 q0, float2 &ans) {
+    if (!check_rect_cross(p0, p1, q0, q1)) return false;
+    const float s1 = cross3(q0, p1, p0), s2 = cross3(p1, q1, p0), s3 = cross3(p0, q1, q0), s4 = cross3(q1, p1, q0);
+    if (!(__fmul_rn(s1, s2) > 0.f && __fmul_rn(s3, s4) > 0.f)) return false;
+    const float s5 = cross3(q1, p1, p0);
+    const float d = __fsub_rn(s5, s1);
+    if (fabsf(d) > 1e-8f) {
+        ans.x = __fdiv_rn(__fsub_rn(__fmul_rn(s5, q0.x), __fmul_rn(s1, q1.x)), d);
+        ans.y = __fdiv_rn(__fsub_rn(__fmul_rn(s5, q0.y), __fmul_rn(s1, q1.y)), d);
+    } else {
+        const float a0 = __fsub_rn(p0.y, p1.y), b0 = __fsub_rn(p1.x, p0.x);
+        const float c0 = __fsub_rn(__fmul_rn(p0.x, p1.y), __fmul_rn(p1.x, p0.y));
+        const float a1 = __fsub_rn(q0.y, q1.y), b1 = __fsub_rn(q1.x, q0.x);
+        const float c1 = __fsub_rn(__fmul_rn(q0.x, q1.y), __fmul_rn(q1.x, q0.y));
+        const float D = __fsub_rn(__fmul_rn(a0, b1), __fmul_rn(a1, b0));
+        ans.x = __fdiv_rn(__fsub_rn(__fmul_rn(b0, c1), __fmul_rn(b1, c0)), D);
+        ans.y = __fdiv_rn(__fsub_rn(__fmul_rn(a1, c0), __fmul_rn(a0, c1)), D);
+    }
+    return true;
+}
+
+__device__ __forceinline__ float2 rotate_around_center(float2 c, float cs, float sn, float2 p) {
+    const float sx = __fsub_rn(p.x, c.x), sy = __fsub_rn(p.y, c.y);
+    return make_float2(__fadd_rn(__fadd_rn(__fmul_rn(sx, cs), __fmul_rn(sy, -sn)), c.x),
+                       __fadd_rn(__fadd_rn(__fmul_rn(sx, sn), __fmul_rn(sy, cs)), c.y));
+}
+
+__device__ __forceinline__ float box_overlap(const BevBox &a, const BevBox &b) {
+    const float adx = __fdiv_rn(a.dx, 2.0f), ady = __fdiv_rn(a.dy, 2.0f), bdx = __fdiv_rn(b.dx, 2.0f), bdy = __fdiv_rn(b.dy, 2.0f);
+    const float ax1 = __fsub_rn(a.cx, adx), ay1 = __fsub_rn(a.cy, ady), ax2 = __fadd_rn(a.cx, adx), ay2 = __fadd_rn(a.cy, ady);
+    const float bx1 = __fsub_rn(b.cx, bdx), by1 = __fsub_rn(b.cy, bdy), bx2 = __fadd_rn(b.cx, bdx), by2 = __fadd_rn(b.cy, bdy);
+    const float2 ca = make_float2(a.cx, a.cy), cb = make_float2(b.cx, b.cy);
+    float2 pa[5], pb[5];
+    pa[0] = make_float2(ax1, ay1); pa[1] = make_float2(ax2, ay1); pa[2] = make_float2(ax2, ay2); pa[3] = make_float2(ax1, ay2);
+    pb[0] = make_float2(bx1, by1); pb[1] = make_float2(bx2, by1); pb[2] = make_float2(bx2, by2); pb[3] = make_float2(bx1, by2);
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        pa[k] = rotate_around_center(ca, a.ca, a.sa, pa[k]);
+        pb[k] = rotate_around_center(cb, b.ca, b.sa, pb[k]);
+    }
+    pa[4] = pa[0];
+    pb[4] = pb[0];
+    float2 pts[16];
+    float2 center = make_float2(0.f, 0.f);
+    int cnt = 0;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            float2 q;
+            if (intersection(pa[i + 1], pa[i], pb[j + 1], pb[j], q)) {
+                center = make_float2(__fadd_rn(center.x, q.x), __fadd_rn(center.y, q.y));
+                pts[cnt++] = q;
+            }
+        }
+    }
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        if (check_in_box2d(a, pb[k])) {
+            center = make_float2(__fadd_rn(center.x, pb[k].x), __fadd_rn(center.y, pb[k].y));
+            pts[cnt++] = pb[k];
+        }
+        if (check_in_box2d(b, pa[k])) {
+            center = make_float2(__fadd_rn(center.x, pa[k].x), __fadd_rn(center.y, pa[k].y));
+            pts[cnt++] = pa[k];
+        }
+    }
+    if (cnt < 2) return 0.f;                   // the reference's area loop does not run: fabs(0) / 2
+    center.x = __fdiv_rn(center.x, (float)cnt);
+    center.y = __fdiv_rn(center.y, (float)cnt);
+    // point_cmp's bubble sort; the angle of a point depends only on the point, so it is computed once per point
+    float ang[16];
+    for (int k = 0; k < cnt; ++k) ang[k] = ref_atan2f(__fsub_rn(pts[k].y, center.y), __fsub_rn(pts[k].x, center.x));
+    for (int j = 0; j < cnt - 1; ++j) {
+        for (int i = 0; i < cnt - j - 1; ++i) {
+            if (ang[i] > ang[i + 1]) {
+                const float2 t = pts[i]; pts[i] = pts[i + 1]; pts[i + 1] = t;
+                const float ta = ang[i]; ang[i] = ang[i + 1]; ang[i + 1] = ta;
+            }
+        }
+    }
+    float area = 0.f;
+    for (int k = 0; k < cnt - 1; ++k) {
+        const float d0x = __fsub_rn(pts[k].x, pts[0].x), d0y = __fsub_rn(pts[k].y, pts[0].y);
+        const float d1x = __fsub_rn(pts[k + 1].x, pts[0].x), d1y = __fsub_rn(pts[k + 1].y, pts[0].y);
+        area = __fadd_rn(area, __fsub_rn(__fmul_rn(d0x, d1y), __fmul_rn(d0y, d1x)));
+    }
+    return (float)(fabs((double)area) / 2.0);
+}
+
+__device__ __forceinline__ float iou_bev(const BevBox &a, const BevBox &b) {
+    const float sa = __fmul_rn(a.dx, a.dy), sb = __fmul_rn(b.dx, b.dy);
+    const float s = box_overlap(a, b);
+    return __fdiv_rn(s, fmaxf(__fsub_rn(__fadd_rn(sa, sb), s), 1e-8f));
+}
+
+__global__ void __launch_bounds__(kGtsThreads, 1) gts_accept_kernel(const float4 *__restrict__ exist, const float4 *__restrict__ samp,
+                                                                 const long long *__restrict__ samp_rows, const GtsFrames f,
+                                                                 int32_t *__restrict__ accepted, float4 *__restrict__ rm_boxes,
+                                                                 int *__restrict__ frame_stats, int *__restrict__ obj_dst) {
+    extern __shared__ BevBox acc_s[];          // boxes accepted so far in this frame (they join existed_boxes)
+    __shared__ int rej_s[kGtsMaxSamples];
+    __shared__ int n_acc_s, rows_s;
+    const int b = blockIdx.x, batch = gridDim.x;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int e0 = f.exist_off[b], ne = f.exist_off[b + 1] - e0;
+    if (threadIdx.x == 0) {
+        n_acc_s = 0;
+        rows_s = 0;
+    }
+    int s_begin = f.samp_off[b];
+    for (int g = 0; g < f.n_groups; ++g) {
+        const int ns = f.group_size[b][g];
+        if (ns == 0) continue;
+        for (int t = threadIdx.x; t < ns; t += kGtsThreads) rej_s[t] = 0;
+        __syncthreads();
+        const int na = n_acc_s;
+        const int others = ne + na + ns;       // iou1 columns (gt boxes, then accepted samples), then iou2 columns
+        for (int q = threadIdx.x; q < ns * others; q += kGtsThreads) {
+            const int i = q / others, j = q - i * others;
+            if (j == ne + na + i) continue;    // iou2's diagonal is zeroed
+            const BevBox a = load_bev(samp, s_begin + i);
+            const BevBox o = j < ne ? load_bev(exist, e0 + j) : j < ne + na ? acc_s[j - ne] : load_bev(samp, s_begin + j - ne - na);
+            if (!(iou_bev(a, o) == 0.f)) rej_s[i] = 1;   // a NaN iou rejects too (numpy's max propagates it)
+        }
+        __syncthreads();
+        if (warp == 0) {
+            int na2 = na, rows = rows_s;
+            for (int c = 0; c < ns; c += 32) {
+                const int k = c + lane, s = s_begin + k;
+                const bool ok = k < ns && rej_s[k] == 0;
+                const uint32_t m = __ballot_sync(0xffffffffu, ok);
+                const int cnt = ok ? (int)samp_rows[2 * s + 1] : 0;
+                int incl = cnt;
+#pragma unroll
+                for (int o = 1; o < 32; o <<= 1) {
+                    const int t = __shfl_up_sync(0xffffffffu, incl, o);
+                    if (lane >= o) incl += t;
+                }
+                if (k < ns) {
+                    accepted[s] = ok ? 1 : 0;
+                    obj_dst[s] = ok ? rows + incl - cnt : -1;
+                }
+                if (ok) {
+                    const int slot = na2 + __popc(m & ((1u << lane) - 1u));
+                    acc_s[slot] = load_bev(samp, s);
+                    const float4 u = __ldg(samp + 4 * s), v = __ldg(samp + 4 * s + 1), w = __ldg(samp + 4 * s + 2),
+                                 x = __ldg(samp + 4 * s + 3);
+                    rm_boxes[2 * (f.samp_off[b] + slot)] = make_float4(u.x, u.y, u.z, w.x);       // cx, cy, cz, cos(-rz)
+                    rm_boxes[2 * (f.samp_off[b] + slot) + 1] = make_float4(w.y, w.z, w.w, x.x);   // sin(-rz), enlarged dx, dy, dz
+                }
+                na2 += __popc(m);
+                rows += __shfl_sync(0xffffffffu, incl, 31);
+            }
+            if (lane == 0) {
+                n_acc_s = na2;
+                rows_s = rows;
+            }
+        }
+        __syncthreads();
+        s_begin += ns;
+    }
+    if (threadIdx.x == 0) {
+        frame_stats[b] = n_acc_s;
+        frame_stats[batch + b] = rows_s;
+        frame_stats[2 * batch + b] = f.samp_off[b];
+    }
+}
+
+// the predicate of the scene-point removal: the row lies in none of its frame's accepted boxes (check_pt_in_box3d_cpu:
+// the z test and the half sizes plus margin in double, the local coordinates in float32)
+struct GtsOutsideBoxes {
+    const float *points;
+    int stride, x_col, batch;
+    const int32_t *frame_offsets;
+    const float4 *rm_boxes;
+    const int *frame_stats;
+    __device__ __forceinline__ bool operator()(int i) const {
+        int lo = 0, hi = batch;                // frame b: off[b] <= i < off[b+1] (the last such b: empty frames are skipped)
+        while (hi - lo > 1) {
+            const int mid = (lo + hi) >> 1;
+            if (__ldg(frame_offsets + mid) <= i) lo = mid; else hi = mid;
+        }
+        const int nb = __ldg(frame_stats + lo), r0 = __ldg(frame_stats + 2 * batch + lo);
+        const float *row = points + (size_t)i * stride + x_col;
+        const float x = __ldg(row), y = __ldg(row + 1), z = __ldg(row + 2);
+        for (int k = 0; k < nb; ++k) {
+            const float4 u = __ldg(rm_boxes + 2 * (r0 + k)), v = __ldg(rm_boxes + 2 * (r0 + k) + 1);
+            if ((double)fabsf(__fsub_rn(z, u.z)) > (double)v.w / 2.0) continue;
+            const float sx = __fsub_rn(x, u.x), sy = __fsub_rn(y, u.y);
+            const float lx = __fadd_rn(__fmul_rn(sx, u.w), __fmul_rn(sy, -v.x));
+            const float ly = __fadd_rn(__fmul_rn(sx, v.x), __fmul_rn(sy, u.w));
+            if ((double)fabsf(lx) < __dadd_rn((double)v.y / 2.0, (double)1e-2f) &&
+                (double)fabsf(ly) < __dadd_rn((double)v.z / 2.0, (double)1e-2f))
+                return false;
+        }
+        return true;
+    }
+};
+
+__global__ void __launch_bounds__(kGtsThreads) gts_paste_kernel(const float *__restrict__ db_points, int feat,
+                                                                const long long *__restrict__ samp_rows,
+                                                                const double *__restrict__ samp_shift, int shift_f64,
+                                                                const int32_t *__restrict__ accepted,
+                                                                const int *__restrict__ obj_dst, const GtsFrames f, int batch,
+                                                                int x_col, const int32_t *__restrict__ out_offsets,
+                                                                float *__restrict__ out) {
+    const int s = blockIdx.x;
+    if (!accepted[s]) return;
+    int b = 0;
+    while (b + 1 < batch && f.samp_off[b + 1] <= s) ++b;
+    const long long first = samp_rows[2 * s];
+    const int cnt = (int)samp_rows[2 * s + 1];
+    const int out_stride = x_col + feat;
+    const double sh[3] = {samp_shift[3 * s], samp_shift[3 * s + 1], samp_shift[3 * s + 2]};
+    float *o = out + ((size_t)out_offsets[b] + obj_dst[s]) * out_stride;
+    const float *src = db_points + (size_t)first * feat;
+    for (int e = threadIdx.x; e < cnt * out_stride; e += kGtsThreads) {
+        const int r = e / out_stride, c = e - r * out_stride - x_col;
+        float v;
+        if (c < 0) {
+            v = (float)b;                      // the batch column of collate_batch
+        } else {
+            v = __ldg(src + (size_t)r * feat + c);
+            if (c < 3)                         // obj_points[:, :3] += box3d_lidar[:3], in the database box's dtype
+                v = shift_f64 ? (float)__dadd_rn((double)v, sh[c]) : __fadd_rn(v, (float)sh[c]);
+        }
+        o[e] = v;
+    }
+}
+
+}  // namespace
+
+extern "C" int toda_gt_sampling_pack_boxes(const float *boxes_host, int n, const float *extra_width_host, float *packed_host) {
+    TODA_CHECK_ARG(n >= 0 && (n == 0 || (boxes_host && packed_host)), "gt_sampling_pack_boxes: bad arguments (n=%d)", n);
+    for (int i = 0; i < n; ++i) {
+        const float *g = boxes_host + 7 * i;
+        float *q = packed_host + kGtsBoxFloats * i;
+        for (int k = 0; k < 6; ++k) q[k] = g[k];
+        // libm cosf / sinf of the float32 heading, as the compiled ops call cos / sin on a float
+        q[6] = cosf(g[6]);
+        q[7] = sinf(g[6]);
+        q[8] = cosf(-g[6]);
+        q[9] = sinf(-g[6]);
+        for (int k = 0; k < 3; ++k) q[10 + k] = extra_width_host ? g[3 + k] + extra_width_host[k] : g[3 + k];   // enlarge_box3d
+        q[13] = q[14] = q[15] = 0.f;
+    }
+    return TODA_OK;
+}
+
+extern "C" size_t toda_gt_sampling_workspace_bytes(int n, int batch, int n_samples) {
+    if (n < 0 || batch < 0 || n_samples < 0) return 0;
+    return toda_points_select_workspace_bytes(n) + align_up((size_t)n_samples * 2 * sizeof(float4), 256) +
+           align_up((size_t)n_samples * sizeof(int), 256) + align_up((size_t)batch * 3 * sizeof(int), 256);
+}
+
+extern "C" int toda_gt_sampling(const float *points, int n, int stride, int x_col, const int32_t *frame_offsets, int batch,
+                                const float *exist_boxes, const int *exist_offsets_host, const float *samp_boxes,
+                                const int *group_sizes_host, int n_groups, const float *db_points, int db_features,
+                                const int64_t *samp_rows, const double *samp_shift, int shift_f64, float *out,
+                                int32_t *out_offsets, int32_t *accepted, void *workspace, size_t workspace_bytes, void *stream) {
+    TODA_CHECK_ARG(n >= 0 && (x_col == 0 || x_col == 1) && db_features >= 3 && stride == x_col + db_features && stride <= 63,
+                   "gt_sampling: bad layout n=%d stride=%d x_col=%d features=%d", n, stride, x_col, db_features);
+    TODA_CHECK_ARG(batch >= 1 && batch <= kGtsMaxBatch, "gt_sampling: batch %d outside [1, %d]", batch, kGtsMaxBatch);
+    TODA_CHECK_ARG(n_groups >= 1 && n_groups <= kGtsMaxGroups, "gt_sampling: %d sample groups (at most %d)", n_groups, kGtsMaxGroups);
+    TODA_CHECK_ARG(exist_offsets_host && group_sizes_host && frame_offsets && out_offsets && accepted && workspace &&
+                   (n == 0 || (points && out)), "gt_sampling: null pointer");
+    GtsFrames f = {};
+    f.n_groups = n_groups;
+    int max_frame = 0;
+    for (int b = 0; b < batch; ++b) {
+        TODA_CHECK_ARG(exist_offsets_host[b] >= 0 && exist_offsets_host[b + 1] >= exist_offsets_host[b],
+                       "gt_sampling: gt box offsets are not ascending at frame %d", b);
+        f.exist_off[b] = exist_offsets_host[b];
+        int frame = 0;
+        for (int g = 0; g < n_groups; ++g) {
+            const int k = group_sizes_host[b * n_groups + g];
+            TODA_CHECK_ARG(k >= 0, "gt_sampling: negative group size");
+            frame += k;
+            if (frame > kGtsMaxSamples) {
+                toda_set_error("gt_sampling: frame %d has more than %d sampled boxes", b, kGtsMaxSamples);
+                return TODA_ERR_UNSUPPORTED;
+            }
+            f.group_size[b][g] = (unsigned short)k;
+        }
+        f.samp_off[b + 1] = f.samp_off[b] + frame;
+        max_frame = frame > max_frame ? frame : max_frame;
+    }
+    f.exist_off[batch] = exist_offsets_host[batch];
+    const int n_samples = f.samp_off[batch];
+    TODA_CHECK_ARG(n_samples == 0 || (samp_boxes && db_points && samp_rows && samp_shift), "gt_sampling: null sample table");
+    TODA_CHECK_ARG(f.exist_off[batch] == 0 || exist_boxes, "gt_sampling: null gt box table");
+    if (workspace_bytes < toda_gt_sampling_workspace_bytes(n, batch, n_samples)) {
+        toda_set_error("gt_sampling: workspace %zu < required %zu bytes", workspace_bytes,
+                       toda_gt_sampling_workspace_bytes(n, batch, n_samples));
+        return TODA_ERR_WORKSPACE;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int tiles = ceil_div(n > 0 ? n : 1, kSelTile);
+    char *ws = (char *)workspace;
+    uint32_t *words = (uint32_t *)ws;
+    int *tile_counts = (int *)(ws + align_up((size_t)tiles * (kSelTile / 32) * sizeof(uint32_t), 256));
+    ws += toda_points_select_workspace_bytes(n);
+    float4 *rm_boxes = (float4 *)ws;
+    ws += align_up((size_t)n_samples * 2 * sizeof(float4), 256);
+    int *obj_dst = (int *)ws;
+    ws += align_up((size_t)n_samples * sizeof(int), 256);
+    int *frame_stats = (int *)ws;              // [3][batch]: accepted boxes, object rows, first removal box
+
+    gts_accept_kernel<<<batch, kGtsThreads, (size_t)max_frame * sizeof(BevBox), st>>>(
+        (const float4 *)exist_boxes, (const float4 *)samp_boxes, (const long long *)samp_rows, f, accepted, rm_boxes,
+        frame_stats, obj_dst);
+    TODA_LAUNCH_OK();
+    select_flag_kernel<<<tiles, kSelThreads, 0, st>>>(
+        n, GtsOutsideBoxes{points, stride, x_col, batch, frame_offsets, rm_boxes, frame_stats}, words, tile_counts);
+    TODA_LAUNCH_OK();
+    select_copy_kernel<<<tiles, kSelThreads, 0, st>>>(points, n, stride, words, tile_counts, frame_offsets, batch, 0,
+                                                      frame_stats + batch, out, out_offsets);
+    TODA_LAUNCH_OK();
+    if (n_samples > 0) {
+        gts_paste_kernel<<<n_samples, kGtsThreads, 0, st>>>(db_points, db_features, (const long long *)samp_rows, samp_shift,
+                                                            shift_f64, accepted, obj_dst, f, batch, x_col, out_offsets, out);
+        TODA_LAUNCH_OK();
+    }
     return TODA_OK;
 }

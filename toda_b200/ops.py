@@ -207,6 +207,87 @@ def points_world_transform(points, frame_offsets, steps, x_col=0):
     return out
 
 
+GTS_MAX_BATCH = 64
+GTS_MAX_GROUPS = 16
+GTS_MAX_SAMPLES_PER_FRAME = 1024
+
+
+def gt_sampling_pack_boxes(boxes, extra_width=None):
+    """(n, 7+) boxes -> float32 (n, 16) table of the device's box format (include/toda_b200.h), made by the library's host
+    code: the first 7 columns cast to float32, libm cosf / sinf of the heading and of its negation, and the sizes
+    enlarged by extra_width in float32."""
+    b = np.ascontiguousarray(np.asarray(boxes)[:, :7], dtype=np.float32)
+    out = np.zeros((b.shape[0], 16), np.float32)
+    w = None if extra_width is None else np.ascontiguousarray(extra_width, dtype=np.float32)
+    _C.check(_C.lib().toda_gt_sampling_pack_boxes(b.ctypes.data, b.shape[0], None if w is None else w.ctypes.data,
+                                                  out.ctypes.data), "toda_gt_sampling_pack_boxes")
+    return out
+
+
+def gt_sampling(points, frame_offsets, gt_boxes, sampled_boxes, group_sizes, db_points, sample_rows, sample_centres,
+                centres_f64, extra_width, x_col=0):
+    """The device side of pcdet's gt_sampling for a batch of frames (collision test, scene-point removal, paste; see
+    include/toda_b200.h).  One host-to-device copy of the box tables and one device-to-host copy of the accepted flags
+    and the new frame offsets, which is the only host synchronisation.
+
+    points (N, x_col + F) float32 CUDA, frame_offsets int32 (B+1) CUDA.  gt_boxes: B host arrays (M_b, 7+), each frame's
+    unmasked gt boxes.  sampled_boxes (S, 7+) host, frame by frame and within a frame group by group; group_sizes (B, G)
+    host ints.  db_points (R, F) float32 CUDA; sample_rows (S, 2) host: first row and row count of each sample's object
+    points; sample_centres (S, 3) host: box3d_lidar[:3] of each sample (float64 values of the database's box dtype);
+    centres_f64: the database stores float64 boxes.  extra_width: REMOVE_EXTRA_WIDTH.
+    Returns (points, frame_offsets, accepted) with accepted a host bool array (S,).
+    """
+    points = _need(points, torch.float32, "points")
+    frame_offsets = _need(frame_offsets, torch.int32, "frame_offsets")
+    db_points = _need(db_points, torch.float32, "db_points")
+    if points.dim() != 2 or db_points.dim() != 2:
+        raise ValueError("gt_sampling: points and db_points must be 2-D")
+    n, stride = points.shape
+    feat = db_points.shape[1]
+    batch = frame_offsets.numel() - 1
+    if x_col not in (0, 1) or stride != x_col + feat:
+        raise ValueError(f"gt_sampling: points have {stride} columns, the database {feat} features (x_col={x_col})")
+    if not 1 <= batch <= GTS_MAX_BATCH or len(gt_boxes) != batch:
+        raise ValueError(f"gt_sampling: {batch} frames and {len(gt_boxes)} gt_boxes arrays (at most {GTS_MAX_BATCH} frames)")
+    group_sizes = np.asarray(group_sizes, np.int32).reshape(batch, -1)
+    n_groups = group_sizes.shape[1]
+    if not 1 <= n_groups <= GTS_MAX_GROUPS:
+        raise ValueError(f"gt_sampling: {n_groups} sample groups (at most {GTS_MAX_GROUPS})")
+    s = int(group_sizes.sum())
+    if np.asarray(sampled_boxes).shape[0] != s or np.asarray(sample_rows).shape != (s, 2):
+        raise ValueError(f"gt_sampling: the group sizes add up to {s} samples, the tables do not")
+    exist = [gt_sampling_pack_boxes(g) for g in gt_boxes]
+    exist_off = np.cumsum([0] + [e.shape[0] for e in exist]).astype(np.int32)
+    rows = np.ascontiguousarray(sample_rows, dtype=np.int64)
+    # one pinned staging buffer, one upload: gt box table | sample box table | sample rows | sample centres
+    parts = [np.concatenate(exist) if exist_off[-1] else np.zeros((0, 16), np.float32),
+             gt_sampling_pack_boxes(sampled_boxes, extra_width), rows, np.ascontiguousarray(sample_centres, dtype=np.float64)]
+    offs, total = [], 0
+    for p in parts:
+        offs.append(total)
+        total += (p.nbytes + 255) // 256 * 256
+    staging = torch.empty(max(total, 256), dtype=torch.uint8, pin_memory=True)
+    host = staging.numpy()
+    for p, o in zip(parts, offs):
+        host[o:o + p.nbytes] = np.frombuffer(p.tobytes(), np.uint8)
+    dev = points.device
+    tables = staging.to(dev, non_blocking=True)
+    base = tables.data_ptr()
+    L = _C.lib()
+    ws = _workspace("gt_sampling", L.toda_gt_sampling_workspace_bytes(n, batch, s), dev)
+    out = torch.empty((n + int(rows[:, 1].sum()), stride), dtype=torch.float32, device=dev)
+    res = torch.empty((s + batch + 1,), dtype=torch.int32, device=dev)          # accepted flags | new frame offsets
+    with _timed("gt_sampling", n=n, stride=stride, samples=s):
+        _C.check(L.toda_gt_sampling(_p(points), n, stride, int(x_col), _p(frame_offsets), batch, ctypes.c_void_p(base + offs[0]),
+                                    _C.ints(exist_off), ctypes.c_void_p(base + offs[1]), _C.ints(group_sizes.reshape(-1)),
+                                    n_groups, _p(db_points), feat, ctypes.c_void_p(base + offs[2]),
+                                    ctypes.c_void_p(base + offs[3]), int(bool(centres_f64)), _p(out), _p(res[s:]), _p(res),
+                                    _p(ws), ws.numel(), _stream()), "toda_gt_sampling")
+    back = res.cpu()
+    new_offsets = res[s:]
+    return out[:int(back[-1])], new_offsets, back[:s].numpy().astype(bool)
+
+
 def gather_point_rows(points, rows):
     """out[i] = points[rows[i]] (numpy `points[idx]`): shuffle_points / mixup prefixes for a given index vector."""
     points = _need(points, torch.float32, "points")
