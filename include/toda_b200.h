@@ -157,6 +157,44 @@ int toda_gt_sampling(const float *points, int n, int stride, int x_col, const in
                      void *stream);
 
 /* ------------------------------------------------------------------------------------------
+ * K0 rotate-paste: PolarMix's rotate-pasting (rotate_copy and the instance paste, Xiao et al., NeurIPS 2022; TODA's
+ * inter_domain_point_polarmix.py L153-191) for a whole batch of frames, adapted to boxes with gt_sampling's collision
+ * rule.  For frame b, the instance boxes of the source frame are copied, rotated about z by each of the frame's angles
+ * (drawn by the caller; [0, w1, w2] gives PolarMix's unrotated copy and two rotated ones); the copies that collide are
+ * dropped, and the source rows inside the instance box of each surviving copy are appended, rotated by its angle.
+ *   src [n_src][stride], dst [n_dst][stride] fp32 frames back to back (the same stride; they may be the same buffer),
+ *     src_offsets / dst_offsets int32[batch+1] device, batch <= 64; x_col 0 (raw frames) or 1 (collated, column 0 = batch
+ *     index), x, y, z at x_col..x_col+2.
+ *   dst_boxes packed [E][16] (toda_gt_sampling_pack_boxes without extra width): frame b's destination boxes at
+ *     dst_box_offsets_host[b..b+1).
+ *   inst_boxes packed [I][16]: frame b's instance boxes at inst_offsets_host[b..b+1) (inst_offsets_host[0] = 0), M_b each.
+ *   angle_counts_host[b] = A_b angles (at most 16); cos_sin double [sum A_b][2] device: (cos w, sin w) in double, frame by
+ *     frame.
+ *   cand_boxes packed [sum A_b * M_b][16]: frame by frame, angle by angle, each angle's copies of the instance boxes in
+ *     order (candidate (b, a, j)); at most 1024 instance boxes and 1024 candidates per frame, else TODA_ERR_UNSUPPORTED.
+ * A candidate is accepted iff its iou_bev is exactly 0 against every destination box of its frame, every candidate
+ * accepted under an earlier angle and every other candidate of its angle (toda_gt_sampling's rule, angles as the
+ * classes).  The instance rows of box j are the source rows of the frame inside the unrotated box (points_in_boxes_cpu,
+ * check_pt_in_box3d_cpu); a row inside two boxes is copied for each.  Output frame b = its destination rows in input order,
+ * then the instance rows of every accepted candidate in candidate order, rotated: each coordinate is
+ * float32((x*R[0][k] + y*R[1][k]) + z*R[2][k]) in double without FMA, R = [[c, s, 0], [-s, c, 0], [0, 0, 1]]; every other
+ * column is copied bit for bit, and the batch column is b when x_col == 1.
+ * After the collision test, result_host int32 [C + 2*batch] (C = sum A_b * M_b) receives the accepted flags (1 / 0),
+ * then per frame the accepted candidates and the pasted rows: this device-to-host copy is the call's only host
+ * synchronisation.  alloc_out(rows, alloc_ctx) is then called once for the output, [rows][stride] fp32 with rows = n_dst +
+ * the pasted rows (it may return NULL when rows is 0); out_offsets int32[batch+1] device receives the new frame offsets.
+ * Deterministic, no atomics.  The workspace is toda_rotate_paste_workspace_bytes(n_src, batch, max M_b, C) bytes.
+ * ------------------------------------------------------------------------------------------ */
+typedef void *(*toda_alloc_fn)(size_t rows, void *ctx);
+size_t toda_rotate_paste_workspace_bytes(int n_src, int batch, int max_inst, int n_cand);
+int toda_rotate_paste(const float *src, int n_src, const int32_t *src_offsets, const float *dst, int n_dst,
+                      const int32_t *dst_offsets, int stride, int x_col, int batch, const float *dst_boxes,
+                      const int *dst_box_offsets_host, const float *inst_boxes, const int *inst_offsets_host,
+                      const float *cand_boxes, const double *cos_sin, const int *angle_counts_host, int32_t *result_host,
+                      toda_alloc_fn alloc_out, void *alloc_ctx, int32_t *out_offsets, void *workspace, size_t workspace_bytes,
+                      void *stream);
+
+/* ------------------------------------------------------------------------------------------
  * K1 hard voxelizer.  Replaces spconv.utils.Point2VoxelCPU3d.point_to_voxel as called from
  * pcdet/datasets/processor/data_processor.py L36-42, L54 (VoxelGeneratorWrapper) /
  * L115-143 (transform_points_to_voxels), for a whole batch of frames in one call.

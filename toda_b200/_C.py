@@ -11,6 +11,8 @@ LIB_PATH = os.path.join(_HERE, "lib", "libtoda_b200.so")
 c_int, c_i64, c_f32, c_vp, c_sz = ctypes.c_int, ctypes.c_int64, ctypes.c_float, ctypes.c_void_p, ctypes.c_size_t
 _IP = ctypes.POINTER(ctypes.c_int)
 _FP = ctypes.POINTER(ctypes.c_float)
+# toda_alloc_fn: (rows, ctx) -> device pointer of the output the library asks for once it knows its size
+ALLOC_FN = ctypes.CFUNCTYPE(c_vp, c_sz, c_vp)
 
 # name -> (restype, argtypes); must list every symbol include/toda_b200.h declares
 SIGNATURES = {
@@ -32,6 +34,9 @@ SIGNATURES = {
     "toda_gt_sampling_workspace_bytes": (c_sz, [c_int, c_int, c_int]),
     "toda_gt_sampling": (c_int, [c_vp, c_int, c_int, c_int, c_vp, c_int, c_vp, _IP, c_vp, _IP, c_int, c_vp, c_int, c_vp, c_vp,
                                  c_int, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
+    "toda_rotate_paste_workspace_bytes": (c_sz, [c_int] * 4),
+    "toda_rotate_paste": (c_int, [c_vp, c_int, c_vp, c_vp, c_int, c_vp, c_int, c_int, c_int, c_vp, _IP, c_vp, _IP, c_vp, c_vp, _IP,
+                                  c_vp, ALLOC_FN, c_vp, c_vp, c_vp, c_sz, c_vp]),
     "toda_voxelize_workspace_bytes": (c_sz, [c_i64, c_int, _IP, c_int, c_int]),
     "toda_voxelize_hard": (c_int, [c_vp, c_i64, c_int, c_int, c_int, c_int, c_vp, c_int, _FP, _FP, _IP, c_int, c_int,
                                    c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),

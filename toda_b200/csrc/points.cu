@@ -708,8 +708,19 @@ __global__ void __launch_bounds__(kGtsThreads, 1) gts_accept_kernel(const float4
     }
 }
 
-// the predicate of the scene-point removal: the row lies in none of its frame's accepted boxes (check_pt_in_box3d_cpu:
-// the z test and the half sizes plus margin in double, the local coordinates in float32)
+// roiaware_pool3d.cpp check_pt_in_box3d_cpu: the z test and the half sizes plus margin in double, the local coordinates in
+// float32; ca / sa = cosf(-rz) / sinf(-rz) of the box heading rz
+__device__ __forceinline__ bool pt_in_box3d(float x, float y, float z, float cx, float cy, float cz, float ca, float sa,
+                                            float dx, float dy, float dz) {
+    if ((double)fabsf(__fsub_rn(z, cz)) > (double)dz / 2.0) return false;
+    const float sx = __fsub_rn(x, cx), sy = __fsub_rn(y, cy);
+    const float lx = __fadd_rn(__fmul_rn(sx, ca), __fmul_rn(sy, -sa));
+    const float ly = __fadd_rn(__fmul_rn(sx, sa), __fmul_rn(sy, ca));
+    return (double)fabsf(lx) < __dadd_rn((double)dx / 2.0, (double)1e-2f) &&
+           (double)fabsf(ly) < __dadd_rn((double)dy / 2.0, (double)1e-2f);
+}
+
+// the predicate of the scene-point removal: the row lies in none of its frame's accepted boxes
 struct GtsOutsideBoxes {
     const float *points;
     int stride, x_col, batch;
@@ -727,13 +738,7 @@ struct GtsOutsideBoxes {
         const float x = __ldg(row), y = __ldg(row + 1), z = __ldg(row + 2);
         for (int k = 0; k < nb; ++k) {
             const float4 u = __ldg(rm_boxes + 2 * (r0 + k)), v = __ldg(rm_boxes + 2 * (r0 + k) + 1);
-            if ((double)fabsf(__fsub_rn(z, u.z)) > (double)v.w / 2.0) continue;
-            const float sx = __fsub_rn(x, u.x), sy = __fsub_rn(y, u.y);
-            const float lx = __fadd_rn(__fmul_rn(sx, u.w), __fmul_rn(sy, -v.x));
-            const float ly = __fadd_rn(__fmul_rn(sx, v.x), __fmul_rn(sy, u.w));
-            if ((double)fabsf(lx) < __dadd_rn((double)v.y / 2.0, (double)1e-2f) &&
-                (double)fabsf(ly) < __dadd_rn((double)v.z / 2.0, (double)1e-2f))
-                return false;
+            if (pt_in_box3d(x, y, z, u.x, u.y, u.z, u.w, v.x, v.y, v.z, v.w)) return false;
         }
         return true;
     }
@@ -861,6 +866,390 @@ extern "C" int toda_gt_sampling(const float *points, int n, int stride, int x_co
     if (n_samples > 0) {
         gts_paste_kernel<<<n_samples, kGtsThreads, 0, st>>>(db_points, db_features, (const long long *)samp_rows, samp_shift,
                                                             shift_f64, accepted, obj_dst, f, batch, x_col, out_offsets, out);
+        TODA_LAUNCH_OK();
+    }
+    return TODA_OK;
+}
+
+// ------------------------------------------------------------------------------------------------
+// PolarMix rotate-pasting (rotate_copy and the instance paste of Xiao et al., NeurIPS 2022; TODA's
+// inter_domain_point_polarmix.py L153-191) for a whole batch, adapted to boxes with gt_sampling's collision rule.  The
+// candidate boxes (every instance box rotated by every angle of its frame) are made on the host; five launches and one
+// device-to-host copy:
+//   1 rp_member_kernel    one CTA per 1024 source rows of a frame (tiles start at frame starts): for every instance box
+//                         of the frame, ballot words and per-tile counts of the rows inside the unrotated, unenlarged box
+//                         (check_pt_in_box3d_cpu, pt_in_box3d above).  Each row is tested once per box, not per angle.
+//   2 rp_box_rows_kernel  one CTA per instance box: its row count, written as the row count of each of its candidates.
+//   3 gts_accept_kernel   gt_sampling's collision test with the angles as the sample groups: a candidate is accepted iff
+//                         its iou_bev is exactly 0 against the destination boxes, the candidates accepted under earlier
+//                         angles and the other candidates of its angle.
+//     then the accepted flags and per-frame totals are copied to the host (the call's only synchronisation), which sizes
+//     the output through the caller's allocator.
+//   4 rp_copy_dst_kernel  the destination rows to their new frame starts; the new frame offsets.
+//   5 rp_paste_kernel     one CTA per instance box: its rows (ranked by popcount from launch 1's words) rotated by each
+//                         accepted angle, written after the destination rows of the frame in candidate order.
+// Rotation: column j of R = [[c, s, 0], [-s, c, 0], [0, 0, 1]] (c, s: cos / sin of the angle in double), each coordinate
+// float32((x*R[0][j] + y*R[1][j]) + z*R[2][j]) in double without FMA; every other column is copied bit for bit.
+namespace {
+
+constexpr int kRpThreads = 256;
+constexpr int kRpTile = 1024;                  // source rows per membership tile = 4 per thread = 32 ballot words
+
+struct RpFrames {
+    int inst_off[kGtsMaxBatch + 1];            // instance boxes of frame b: [inst_off[b], inst_off[b+1])
+    int cand_off[kGtsMaxBatch + 1];            // candidates of frame b, angle by angle, instance boxes in order
+    int ang_off[kGtsMaxBatch + 1];             // angles of frame b: rows [ang_off[b], ang_off[b+1]) of the cos / sin table
+};
+
+struct RpBox { float cx, cy, cz, ca, sa, dx, dy, dz; };
+
+// first membership tile of every source frame (a frame of N rows has ceil(N / 1024) tiles); tile_lo[batch] = all tiles
+__device__ void rp_tile_starts(const int32_t *__restrict__ off, int batch, int *tile_lo) {
+    int t = 0;
+    for (int q = 0; q < batch; ++q) {
+        tile_lo[q] = t;
+        t += (__ldg(off + q + 1) - __ldg(off + q) + kRpTile - 1) / kRpTile;
+    }
+    tile_lo[batch] = t;
+}
+
+// the frame of instance box g (uniform across the CTA)
+__device__ __forceinline__ int rp_box_frame(const RpFrames &f, int g) {
+    int b = 0;
+    while (f.inst_off[b + 1] <= g) ++b;
+    return b;
+}
+
+__global__ void __launch_bounds__(kRpThreads) rp_member_kernel(const float *__restrict__ src, int stride, int x_col,
+                                                               const int32_t *__restrict__ src_off, int batch,
+                                                               const float4 *__restrict__ inst, const RpFrames f, int tiles,
+                                                               uint32_t *__restrict__ words, int *__restrict__ tile_counts) {
+    extern __shared__ RpBox box_s[];           // the frame's instance boxes, then per-warp counts [box][warp] as bytes
+    __shared__ int tile_lo[kGtsMaxBatch + 1];
+    __shared__ int frame_s;
+    const int t = blockIdx.x;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (threadIdx.x == 0) {
+        rp_tile_starts(src_off, batch, tile_lo);
+        int b = 0;
+        while (b < batch && tile_lo[b + 1] <= t) ++b;
+        frame_s = b;
+    }
+    __syncthreads();
+    const int b = frame_s;
+    if (b >= batch) return;                    // the grid is sized for ceil(n / 1024) + batch tiles
+    const int i0 = f.inst_off[b], m = f.inst_off[b + 1] - i0;
+    if (m == 0) return;
+    unsigned char *cnt_s = (unsigned char *)(box_s + m);
+    for (int k = threadIdx.x; k < m; k += kRpThreads) {
+        const float4 u = __ldg(inst + 4 * (i0 + k)), v = __ldg(inst + 4 * (i0 + k) + 1), w = __ldg(inst + 4 * (i0 + k) + 2);
+        box_s[k] = RpBox{u.x, u.y, u.z, w.x, w.y, u.w, v.x, v.y};      // packed: cosf(-rz), sinf(-rz) at 8, 9
+    }
+    const int row0 = __ldg(src_off + b) + (t - tile_lo[b]) * kRpTile, row_end = __ldg(src_off + b + 1);
+    float x[kRpTile / kRpThreads], y[kRpTile / kRpThreads], z[kRpTile / kRpThreads];
+    bool valid[kRpTile / kRpThreads];
+#pragma unroll
+    for (int j = 0; j < kRpTile / kRpThreads; ++j) {
+        const int i = row0 + j * kRpThreads + threadIdx.x;   // a warp covers 32 consecutive rows = one word
+        valid[j] = i < row_end;
+        const float *row = src + (size_t)(valid[j] ? i : row0) * stride + x_col;
+        x[j] = __ldg(row);
+        y[j] = __ldg(row + 1);
+        z[j] = __ldg(row + 2);
+    }
+    __syncthreads();
+    for (int k = 0; k < m; ++k) {
+        const RpBox q = box_s[k];
+        int cnt = 0;
+#pragma unroll
+        for (int j = 0; j < kRpTile / kRpThreads; ++j) {
+            const bool in = valid[j] && pt_in_box3d(x[j], y[j], z[j], q.cx, q.cy, q.cz, q.ca, q.sa, q.dx, q.dy, q.dz);
+            const uint32_t w = __ballot_sync(0xffffffffu, in);
+            if (lane == 0) {
+                words[((size_t)k * tiles + t) * (kRpTile / 32) + j * (kRpThreads / 32) + warp] = w;
+                cnt += __popc(w);
+            }
+        }
+        if (lane == 0) cnt_s[k * (kRpThreads / 32) + warp] = (unsigned char)cnt;     // <= 128
+    }
+    __syncthreads();
+    for (int k = threadIdx.x; k < m; k += kRpThreads) {
+        int s = 0;
+#pragma unroll
+        for (int w = 0; w < kRpThreads / 32; ++w) s += cnt_s[k * (kRpThreads / 32) + w];
+        tile_counts[(size_t)k * tiles + t] = s;
+    }
+}
+
+__global__ void __launch_bounds__(128) rp_box_rows_kernel(const int32_t *__restrict__ src_off, int batch, const RpFrames f,
+                                                          int tiles, const int *__restrict__ tile_counts,
+                                                          long long *__restrict__ cand_rows) {
+    __shared__ int tile_lo[kGtsMaxBatch + 1];
+    __shared__ int part[4];
+    const int g = blockIdx.x, b = rp_box_frame(f, g);
+    const int j = g - f.inst_off[b], m = f.inst_off[b + 1] - f.inst_off[b];
+    if (threadIdx.x == 0) rp_tile_starts(src_off, batch, tile_lo);
+    __syncthreads();
+    int s = 0;
+    for (int t = tile_lo[b] + threadIdx.x; t < tile_lo[b + 1]; t += 128) s += tile_counts[(size_t)j * tiles + t];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+    if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = s;
+    __syncthreads();
+    if ((int)threadIdx.x < f.ang_off[b + 1] - f.ang_off[b]) {
+        const int c = f.cand_off[b] + threadIdx.x * m + j;
+        cand_rows[2 * c] = 0;                  // (first row, row count) as gts_accept_kernel reads its samples' rows
+        cand_rows[2 * c + 1] = part[0] + part[1] + part[2] + part[3];
+    }
+}
+
+__global__ void __launch_bounds__(kRpThreads) rp_copy_dst_kernel(const float *__restrict__ dst, int n, int stride,
+                                                                 const int32_t *__restrict__ dst_off, int batch,
+                                                                 const int *__restrict__ frame_stats, float *__restrict__ out,
+                                                                 int32_t *__restrict__ out_off) {
+    __shared__ long long off_e[kGtsMaxBatch + 1];   // frame starts in elements
+    __shared__ long long shift_e[kGtsMaxBatch];     // pasted rows of the frames before b, in elements
+    if (threadIdx.x == 0) {
+        long long p = 0;
+        for (int q = 0; q <= batch; ++q) {
+            const int o = __ldg(dst_off + q);
+            off_e[q] = (long long)o * stride;
+            if (q < batch) shift_e[q] = p * stride;
+            if (blockIdx.x == 0) out_off[q] = o + (int)p;
+            if (q < batch) p += frame_stats[batch + q];
+        }
+    }
+    __syncthreads();
+    const long long e0 = (long long)blockIdx.x * kRpTile * stride;
+    const long long e1 = min((long long)n * stride, e0 + (long long)kRpTile * stride);
+    int b = 0;                                 // frame of element e: the last b with off_e[b] <= e (empty frames skipped)
+    for (long long e = e0 + threadIdx.x; e < e1; e += kRpThreads) {
+        while (b + 1 < batch && off_e[b + 1] <= e) ++b;
+        out[e + shift_e[b]] = __ldg(dst + e);
+    }
+}
+
+// coordinate k of (x, y, z) times the rotation matrix of (c, s); the 0 and 1 entries are passed in so that no product
+// with them is folded
+__device__ __forceinline__ float rp_rotate(int k, float x, float y, float z, double c, double s, double zero, double one) {
+    double r0, r1, r2;
+    if (k == 0) { r0 = c; r1 = -s; r2 = zero; }
+    else if (k == 1) { r0 = s; r1 = c; r2 = zero; }
+    else { r0 = zero; r1 = zero; r2 = one; }
+    return __double2float_rn(__dadd_rn(__dadd_rn(__dmul_rn((double)x, r0), __dmul_rn((double)y, r1)), __dmul_rn((double)z, r2)));
+}
+
+__global__ void __launch_bounds__(kRpThreads) rp_paste_kernel(const float *__restrict__ src, int stride, int x_col,
+                                                              const int32_t *__restrict__ src_off,
+                                                              const int32_t *__restrict__ dst_off, int batch, const RpFrames f,
+                                                              int tiles, const uint32_t *__restrict__ words,
+                                                              const int *__restrict__ tile_counts,
+                                                              const double2 *__restrict__ cos_sin,
+                                                              const int *__restrict__ obj_dst, const int32_t *__restrict__ out_off,
+                                                              double zero, double one, float *__restrict__ out) {
+    __shared__ int tile_lo[kGtsMaxBatch + 1];
+    __shared__ int dst_row_s[kGtsMaxGroups];   // first output row of each accepted copy of this box
+    __shared__ double2 cs_s[kGtsMaxGroups];    // and its angle's cos / sin
+    __shared__ int n_copies_s, n_list_s;
+    __shared__ int list_t[32], list_p[32];     // tiles with rows in the box (frame-local index) and the box's rows before each
+    __shared__ uint32_t word_s[kRpTile / 32];
+    __shared__ int word_prefix[kRpTile / 32 + 1];
+    __shared__ int rows_s[kRpTile];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int g = blockIdx.x, b = rp_box_frame(f, g);
+    const int j = g - f.inst_off[b], m = f.inst_off[b + 1] - f.inst_off[b];
+    if (threadIdx.x == 0) {
+        rp_tile_starts(src_off, batch, tile_lo);
+        const int base = out_off[b] + __ldg(dst_off + b + 1) - __ldg(dst_off + b);
+        int nc = 0;
+        for (int a = 0; a < f.ang_off[b + 1] - f.ang_off[b]; ++a) {
+            const int d = obj_dst[f.cand_off[b] + a * m + j];          // -1 when the candidate was rejected
+            if (d >= 0) {
+                dst_row_s[nc] = base + d;
+                cs_s[nc] = cos_sin[f.ang_off[b] + a];
+                ++nc;
+            }
+        }
+        n_copies_s = nc;
+    }
+    __syncthreads();
+    const int nc = n_copies_s;
+    if (nc == 0) return;
+    const int t_lo = tile_lo[b], n_t = tile_lo[b + 1] - t_lo, row_base = __ldg(src_off + b);
+    const uint32_t *wbox = words + ((size_t)j * tiles + t_lo) * (kRpTile / 32);
+    const int *cbox = tile_counts + (size_t)j * tiles + t_lo;
+    int done = 0;                              // rows of the box in the tiles before t0 (warp 0)
+    for (int t0 = 0; t0 < n_t; t0 += 32) {
+        if (warp == 0) {
+            const int c = t0 + lane < n_t ? cbox[t0 + lane] : 0;
+            int incl = c;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int v = __shfl_up_sync(0xffffffffu, incl, o);
+                if (lane >= o) incl += v;
+            }
+            const uint32_t nz = __ballot_sync(0xffffffffu, c > 0);
+            if (c > 0) {
+                const int slot = __popc(nz & ((1u << lane) - 1u));
+                list_t[slot] = t0 + lane;
+                list_p[slot] = done + incl - c;
+            }
+            if (lane == 0) n_list_s = __popc(nz);
+            done += __shfl_sync(0xffffffffu, incl, 31);
+        }
+        __syncthreads();
+        for (int q = 0; q < n_list_s; ++q) {
+            const int tl = list_t[q], p = list_p[q];
+            if (warp == 0) {
+                const uint32_t w = wbox[(size_t)tl * (kRpTile / 32) + lane];
+                word_s[lane] = w;
+                const int c = __popc(w);
+                int incl = c;
+#pragma unroll
+                for (int o = 1; o < 32; o <<= 1) {
+                    const int v = __shfl_up_sync(0xffffffffu, incl, o);
+                    if (lane >= o) incl += v;
+                }
+                word_prefix[lane] = incl - c;
+                if (lane == 31) word_prefix[kRpTile / 32] = incl;
+            }
+            __syncthreads();
+#pragma unroll
+            for (int jj = 0; jj < kRpTile / kRpThreads; ++jj) {
+                const int wi = jj * (kRpThreads / 32) + warp;
+                const uint32_t w = word_s[wi];
+                if ((w >> lane) & 1u) rows_s[word_prefix[wi] + __popc(w & ((1u << lane) - 1u))] = row_base + tl * kRpTile + jj * kRpThreads + threadIdx.x;
+            }
+            __syncthreads();
+            const int total = word_prefix[kRpTile / 32] * stride;
+            for (int a = 0; a < nc; ++a) {
+                const double2 cs = cs_s[a];
+                float *o = out + (size_t)(dst_row_s[a] + p) * stride;
+                for (int e = threadIdx.x; e < total; e += kRpThreads) {
+                    const int r = e / stride, c = e - r * stride, k = c - x_col;
+                    const float *row = src + (size_t)rows_s[r] * stride;
+                    float v;
+                    if (k < 0) v = (float)b;   // the batch column of collate_batch
+                    else if (k < 3) v = rp_rotate(k, __ldg(row + x_col), __ldg(row + x_col + 1), __ldg(row + x_col + 2), cs.x, cs.y, zero, one);
+                    else v = __ldg(row + c);
+                    o[e] = v;
+                }
+            }
+            __syncthreads();
+        }
+        __syncthreads();
+    }
+}
+
+}  // namespace
+
+extern "C" size_t toda_rotate_paste_workspace_bytes(int n_src, int batch, int max_inst, int n_cand) {
+    if (n_src < 0 || batch < 0 || max_inst < 0 || n_cand < 0) return 0;
+    const size_t slots = (size_t)max_inst * ((size_t)ceil_div(n_src, kRpTile) + batch);   // (box, tile) pairs
+    return align_up(slots * (kRpTile / 32) * sizeof(uint32_t), 256) + align_up(slots * sizeof(int), 256) +
+           align_up((size_t)n_cand * 2 * sizeof(long long), 256) + align_up((size_t)n_cand * 2 * sizeof(float4), 256) +
+           align_up((size_t)n_cand * sizeof(int), 256) + align_up(((size_t)n_cand + 3 * (size_t)batch) * sizeof(int), 256);
+}
+
+extern "C" int toda_rotate_paste(const float *src, int n_src, const int32_t *src_offsets, const float *dst, int n_dst,
+                                 const int32_t *dst_offsets, int stride, int x_col, int batch, const float *dst_boxes,
+                                 const int *dst_box_offsets_host, const float *inst_boxes, const int *inst_offsets_host,
+                                 const float *cand_boxes, const double *cos_sin, const int *angle_counts_host,
+                                 int32_t *result_host, toda_alloc_fn alloc_out, void *alloc_ctx, int32_t *out_offsets,
+                                 void *workspace, size_t workspace_bytes, void *stream) {
+    TODA_CHECK_ARG(n_src >= 0 && n_dst >= 0 && (x_col == 0 || x_col == 1) && stride >= x_col + 3 && stride <= 63,
+                   "rotate_paste: bad layout n_src=%d n_dst=%d stride=%d x_col=%d", n_src, n_dst, stride, x_col);
+    TODA_CHECK_ARG(dst_box_offsets_host && inst_offsets_host && angle_counts_host && inst_offsets_host[0] == 0,
+                   "rotate_paste: null box table offsets, or instance box offsets that do not start at 0");
+    if (batch < 1 || batch > kGtsMaxBatch) {
+        toda_set_error("rotate_paste: batch %d outside [1, %d]", batch, kGtsMaxBatch);
+        return batch < 1 ? TODA_ERR_INVALID : TODA_ERR_UNSUPPORTED;
+    }
+    GtsFrames gf = {};
+    RpFrames rf = {};
+    int max_inst = 0, max_cand = 0;
+    for (int b = 0; b < batch; ++b) {
+        const int ne = dst_box_offsets_host[b + 1] - dst_box_offsets_host[b], m = inst_offsets_host[b + 1] - inst_offsets_host[b];
+        const int na = angle_counts_host[b];
+        TODA_CHECK_ARG(dst_box_offsets_host[b] >= 0 && ne >= 0 && inst_offsets_host[b] >= 0 && m >= 0 && na >= 0,
+                       "rotate_paste: box offsets or angle counts of frame %d are not ascending", b);
+        if (na > kGtsMaxGroups) {
+            toda_set_error("rotate_paste: frame %d has %d angles (at most %d)", b, na, kGtsMaxGroups);
+            return TODA_ERR_UNSUPPORTED;
+        }
+        if (m > kGtsMaxSamples || na * m > kGtsMaxSamples) {
+            toda_set_error("rotate_paste: frame %d has %d instance boxes and %d candidates (at most %d each)", b, m, na * m,
+                           kGtsMaxSamples);
+            return TODA_ERR_UNSUPPORTED;
+        }
+        gf.exist_off[b] = dst_box_offsets_host[b];
+        gf.samp_off[b + 1] = gf.samp_off[b] + na * m;
+        for (int a = 0; a < na; ++a) gf.group_size[b][a] = (unsigned short)m;
+        gf.n_groups = na > gf.n_groups ? na : gf.n_groups;
+        rf.inst_off[b + 1] = rf.inst_off[b] + m;
+        rf.ang_off[b + 1] = rf.ang_off[b] + na;
+        max_inst = m > max_inst ? m : max_inst;
+        max_cand = na * m > max_cand ? na * m : max_cand;
+    }
+    gf.exist_off[batch] = dst_box_offsets_host[batch];
+    for (int b = 0; b <= batch; ++b) rf.cand_off[b] = gf.samp_off[b];
+    const int n_inst = rf.inst_off[batch], n_cand = gf.samp_off[batch];
+    TODA_CHECK_ARG(src_offsets && dst_offsets && out_offsets && result_host && alloc_out && workspace &&
+                   (n_src == 0 || src) && (n_dst == 0 || dst) && (gf.exist_off[batch] == 0 || dst_boxes) &&
+                   (n_inst == 0 || inst_boxes) && (n_cand == 0 || (cand_boxes && cos_sin)), "rotate_paste: null pointer");
+    const size_t need = toda_rotate_paste_workspace_bytes(n_src, batch, max_inst, n_cand);
+    if (workspace_bytes < need) {
+        toda_set_error("rotate_paste: workspace %zu < required %zu bytes", workspace_bytes, need);
+        return TODA_ERR_WORKSPACE;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const int tiles = ceil_div(n_src, kRpTile) + batch;
+    const size_t slots = (size_t)max_inst * tiles;
+    char *ws = (char *)workspace;
+    uint32_t *words = (uint32_t *)ws;
+    ws += align_up(slots * (kRpTile / 32) * sizeof(uint32_t), 256);
+    int *tile_counts = (int *)ws;
+    ws += align_up(slots * sizeof(int), 256);
+    long long *cand_rows = (long long *)ws;
+    ws += align_up((size_t)n_cand * 2 * sizeof(long long), 256);
+    float4 *rm_boxes = (float4 *)ws;           // written by gts_accept_kernel, not used here
+    ws += align_up((size_t)n_cand * 2 * sizeof(float4), 256);
+    int *obj_dst = (int *)ws;
+    ws += align_up((size_t)n_cand * sizeof(int), 256);
+    int32_t *accepted = (int32_t *)ws;         // accepted flags, then frame_stats [3][batch]: accepted, pasted rows, first
+    int *frame_stats = accepted + n_cand;
+
+    if (n_inst > 0) {
+        rp_member_kernel<<<tiles, kRpThreads, (size_t)max_inst * (sizeof(RpBox) + kRpThreads / 32), st>>>(
+            src, stride, x_col, src_offsets, batch, (const float4 *)inst_boxes, rf, tiles, words, tile_counts);
+        TODA_LAUNCH_OK();
+        rp_box_rows_kernel<<<n_inst, 128, 0, st>>>(src_offsets, batch, rf, tiles, tile_counts, cand_rows);
+        TODA_LAUNCH_OK();
+    }
+    gts_accept_kernel<<<batch, kGtsThreads, (size_t)max_cand * sizeof(BevBox), st>>>(
+        (const float4 *)dst_boxes, (const float4 *)cand_boxes, cand_rows, gf, accepted, rm_boxes, frame_stats, obj_dst);
+    TODA_LAUNCH_OK();
+    TODA_CUDA_OK(cudaMemcpyAsync(result_host, accepted, ((size_t)n_cand + 2 * batch) * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    TODA_CUDA_OK(cudaStreamSynchronize(st));
+    long long rows = n_dst, pasted = 0;
+    for (int b = 0; b < batch; ++b) pasted += result_host[n_cand + batch + b];
+    rows += pasted;
+    if (rows > 0x7fffffffLL) {
+        toda_set_error("rotate_paste: %lld output rows (at most 2^31 - 1)", rows);
+        return TODA_ERR_UNSUPPORTED;
+    }
+    float *out = (float *)alloc_out((size_t)rows, alloc_ctx);
+    if (!out && rows > 0) {
+        toda_set_error("rotate_paste: the allocator returned no memory for %lld rows", rows);
+        return TODA_ERR_INVALID;
+    }
+    rp_copy_dst_kernel<<<ceil_div(n_dst > 0 ? n_dst : 1, kRpTile), kRpThreads, 0, st>>>(dst, n_dst, stride, dst_offsets, batch,
+                                                                                       frame_stats, out, out_offsets);
+    TODA_LAUNCH_OK();
+    if (pasted > 0) {
+        rp_paste_kernel<<<n_inst, kRpThreads, 0, st>>>(src, stride, x_col, src_offsets, dst_offsets, batch, rf, tiles, words,
+                                                       tile_counts, (const double2 *)cos_sin, obj_dst, out_offsets, 0.0, 1.0,
+                                                       out);
         TODA_LAUNCH_OK();
     }
     return TODA_OK;

@@ -288,6 +288,89 @@ def gt_sampling(points, frame_offsets, gt_boxes, sampled_boxes, group_sizes, db_
     return out[:int(back[-1])], new_offsets, back[:s].numpy().astype(bool)
 
 
+RP_MAX_BATCH = GTS_MAX_BATCH
+RP_MAX_ANGLES = GTS_MAX_GROUPS
+RP_MAX_CANDIDATES_PER_FRAME = GTS_MAX_SAMPLES_PER_FRAME
+
+
+def rotate_paste(dst_points, dst_offsets, src_points, src_offsets, dst_boxes, inst_boxes, cand_boxes, rotations, x_col=0):
+    """PolarMix's rotate-pasting for a batch of frames (collision test of the rotated instance copies and the paste of
+    their points; see include/toda_b200.h).  One pinned host-to-device copy of the box tables and the angles' cos / sin,
+    and one device-to-host copy of the accepted flags and the per-frame totals, which is the only host synchronisation.
+
+    dst_points / src_points (N, x_col + F) float32 CUDA with the same columns (they may be the same tensor); dst_offsets /
+    src_offsets int32 (B+1) CUDA.  Per frame, host arrays: dst_boxes[b] (E_b, 7+) destination boxes, inst_boxes[b]
+    (M_b, 7+) instance boxes, rotations[b] (A_b, 2) float64 (cos w, sin w) of the A_b angles, cand_boxes[b] (A_b * M_b, 7+)
+    the instance boxes rotated by each angle, angle by angle.  Returns (points, frame_offsets, accepted) with accepted a host bool array of the candidates,
+    frame by frame.
+    """
+    dst_points = _need(dst_points, torch.float32, "dst_points")
+    src_points = _need(src_points, torch.float32, "src_points")
+    dst_offsets = _need(dst_offsets, torch.int32, "dst_offsets")
+    src_offsets = _need(src_offsets, torch.int32, "src_offsets")
+    if dst_points.dim() != 2 or src_points.dim() != 2:
+        raise ValueError("rotate_paste: points must be (N, stride)")
+    n_dst, stride = dst_points.shape
+    if src_points.shape[1] != stride:
+        raise ValueError(f"rotate_paste: source rows have {src_points.shape[1]} columns, destination rows {stride}")
+    if x_col not in (0, 1) or not x_col + 3 <= stride <= 63:
+        raise ValueError(f"rotate_paste: x, y, z at columns {x_col}..{x_col + 2} do not fit stride {stride} (<= 63)")
+    batch = dst_offsets.numel() - 1
+    if src_offsets.numel() - 1 != batch or not 1 <= batch <= RP_MAX_BATCH:
+        raise ValueError(f"rotate_paste: {batch} destination and {src_offsets.numel() - 1} source frames "
+                         f"(at most {RP_MAX_BATCH})")
+    if not len(dst_boxes) == len(inst_boxes) == len(cand_boxes) == len(rotations) == batch:
+        raise ValueError(f"rotate_paste: {batch} frames need {batch} box tables and rotation tables")
+    rotations = [np.asarray(r, np.float64).reshape(-1, 2) for r in rotations]
+    counts = np.array([r.shape[0] for r in rotations], np.int32)
+    inst = [np.asarray(m).reshape(-1, np.shape(m)[-1]) for m in inst_boxes]
+    for b, (a, m, c) in enumerate(zip(counts, inst, cand_boxes)):
+        if a > RP_MAX_ANGLES:
+            raise ValueError(f"rotate_paste: frame {b} has {a} angles (at most {RP_MAX_ANGLES})")
+        if m.shape[0] > RP_MAX_CANDIDATES_PER_FRAME or a * m.shape[0] > RP_MAX_CANDIDATES_PER_FRAME:
+            raise ValueError(f"rotate_paste: frame {b} has {m.shape[0]} instance boxes and {a * m.shape[0]} candidates "
+                             f"(at most {RP_MAX_CANDIDATES_PER_FRAME} each)")
+        if np.shape(c)[0] != a * m.shape[0]:
+            raise ValueError(f"rotate_paste: frame {b} has {np.shape(c)[0]} candidate boxes, not {a} x {m.shape[0]}")
+    packs = [[gt_sampling_pack_boxes(np.asarray(x).reshape(-1, np.shape(x)[-1])) for x in xs]
+             for xs in (dst_boxes, inst, cand_boxes)]
+    dst_off = np.cumsum([0] + [p.shape[0] for p in packs[0]]).astype(np.int32)
+    inst_off = np.cumsum([0] + [p.shape[0] for p in packs[1]]).astype(np.int32)
+    n_cand = sum(p.shape[0] for p in packs[2])
+    # one pinned staging buffer, one upload: destination boxes | instance boxes | candidate boxes | cos / sin
+    parts = [np.concatenate(p) for p in packs] + [np.concatenate(rotations)]
+    offs, total = [], 0
+    for p in parts:
+        offs.append(total)
+        total += (p.nbytes + 255) // 256 * 256
+    staging = torch.empty(max(total, 256), dtype=torch.uint8, pin_memory=True)
+    host = staging.numpy()
+    for p, o in zip(parts, offs):
+        host[o:o + p.nbytes] = np.frombuffer(p.tobytes(), np.uint8)
+    dev = dst_points.device
+    tables = staging.to(dev, non_blocking=True)
+    base = tables.data_ptr()
+    L = _C.lib()
+    n_src = src_points.shape[0]
+    ws = _workspace("rotate_paste", L.toda_rotate_paste_workspace_bytes(n_src, batch, max(p.shape[0] for p in packs[1]),
+                                                                         n_cand), dev)
+    result = torch.empty(n_cand + 2 * batch, dtype=torch.int32, pin_memory=True)
+    out_offsets = torch.empty(batch + 1, dtype=torch.int32, device=dev)
+    out = []
+
+    def alloc(rows, _ctx):
+        out.append(torch.empty((rows, stride), dtype=torch.float32, device=dev))
+        return out[0].data_ptr() if rows else None
+    alloc_fn = _C.ALLOC_FN(alloc)
+    with _timed("rotate_paste", n_src=n_src, n_dst=n_dst, stride=stride, candidates=n_cand):
+        _C.check(L.toda_rotate_paste(_p(src_points), n_src, _p(src_offsets), _p(dst_points), n_dst, _p(dst_offsets), stride,
+                                     int(x_col), batch, ctypes.c_void_p(base + offs[0]), _C.ints(dst_off),
+                                     ctypes.c_void_p(base + offs[1]), _C.ints(inst_off), ctypes.c_void_p(base + offs[2]),
+                                     ctypes.c_void_p(base + offs[3]), _C.ints(counts), _p(result), alloc_fn, None,
+                                     _p(out_offsets), _p(ws), ws.numel(), _stream()), "toda_rotate_paste")
+    return out[0], out_offsets, result[:n_cand].numpy().astype(bool)
+
+
 def gather_point_rows(points, rows):
     """out[i] = points[rows[i]] (numpy `points[idx]`): shuffle_points / mixup prefixes for a given index vector."""
     points = _need(points, torch.float32, "points")

@@ -121,6 +121,66 @@ def polar_swap_points(pt1, pt2, start_angle, end_angle, dis_th=None, dis_less=Tr
     return torch.cat([keep1, take2], dim=0)
 
 
+def rotation_cos_sin(angles):
+    """(A, 2) float64 (cos w, sin w) of each angle, as PolarMix's rot_mat takes them (np.cos / np.sin of the scalar)."""
+    return np.array([[np.cos(w), np.sin(w)] for w in np.asarray(angles, np.float64).reshape(-1)], np.float64).reshape(-1, 2)
+
+
+def rotate_boxes_about_z(boxes, cos_sin, angle):
+    """Boxes (M, 7 / 9 / 10) rotated about z: x, y as float32((x*R[0][j] + y*R[1][j]) + z*R[2][j]) in float64 without FMA
+    with R = [[c, s, 0], [-s, c, 0], [0, 0, 1]], z unchanged, heading + angle in float32 (no period wrap), the velocity
+    columns 7, 8 by the same 2x2 expression, any other column copied.  Returns float32 (M, C)."""
+    src = np.asarray(boxes)
+    out = src.astype(np.float32, copy=True)
+    c, s = float(cos_sin[0]), float(cos_sin[1])
+    r = np.array([[c, s, 0.0], [-s, c, 0.0], [0.0, 0.0, 1.0]])
+    x, y, z = (out[:, k].astype(np.float64) for k in range(3))
+    for k in range(2):
+        out[:, k] = ((x * r[0, k] + y * r[1, k]) + z * r[2, k]).astype(np.float32)
+    out[:, 6] = out[:, 6] + np.float32(angle)
+    if out.shape[1] >= 9:
+        vx, vy = out[:, 7].astype(np.float64), out[:, 8].astype(np.float64)
+        out[:, 7] = (vx * r[0, 0] + vy * r[1, 0]).astype(np.float32)
+        out[:, 8] = (vx * r[0, 1] + vy * r[1, 1]).astype(np.float32)
+    return out
+
+
+def rotate_paste_points(dst_points, dst_offsets, src_points, src_offsets, gt_boxes, gt_names, inst_boxes, inst_names, angles,
+                        x_col=0):
+    """PolarMix's rotate-pasting (rotate_copy + paste, inter_domain_point_polarmix.py L153-191) for a batch of frames,
+    adapted to boxes: frame b's instance boxes inst_boxes[b] (M_b, 7 / 9 / 10 columns, already filtered by class) are
+    copied, rotated about z by each angle of angles[b] (drawn by the caller; [0, w1, w2] reproduces PolarMix's
+    `[pts_inst] + rotated copies`), the copies whose BEV IoU with a box already in the scene is not exactly 0 are dropped
+    (gt_sampling's rule, angle by angle, see include/toda_b200.h), and the source points inside the instance box of each
+    surviving copy are appended to the destination frame, rotated by its angle.
+
+    dst_points / src_points (N, x_col + F) float32 CUDA with frame offsets int32 (B+1) CUDA (src may be dst).  gt_boxes,
+    gt_names: the destination frames' boxes and names (per-frame host arrays); inst_names: the names of the instance boxes.
+    Returns (points, frame_offsets, boxes, names): boxes[b] / names[b] are the destination boxes / names followed by those
+    of the accepted copies, in angle order and, within an angle, instance order.
+    """
+    batch = len(gt_boxes)
+    inst = [np.asarray(m).reshape(-1, np.shape(m)[-1]) for m in inst_boxes]
+    for b, m in enumerate(inst):
+        if m.shape[1] not in (7, 9, 10) or np.shape(gt_boxes[b])[-1] != m.shape[1]:
+            raise ValueError(f"rotate_paste_points: frame {b} has instance boxes of {m.shape[1]} columns and destination "
+                             f"boxes of {np.shape(gt_boxes[b])[-1]} (7, 9 or 10, the same on both sides)")
+    if not len(gt_names) == len(inst) == len(inst_names) == len(angles) == batch:
+        raise ValueError(f"rotate_paste_points: {batch} frames need {batch} name arrays, instance tables and angle lists")
+    rotations = [rotation_cos_sin(a) for a in angles]
+    cands = [np.concatenate([rotate_boxes_about_z(m, cs, w) for cs, w in zip(r, np.asarray(a, np.float64).reshape(-1))])
+             if len(r) else np.zeros((0, m.shape[1]), np.float32) for m, r, a in zip(inst, rotations, angles)]
+    points, offsets, accepted = ops.rotate_paste(dst_points, dst_offsets, src_points, src_offsets, gt_boxes, inst, cands,
+                                                 rotations, x_col=x_col)
+    boxes, names, lo = [], [], 0
+    for b in range(batch):
+        ok = accepted[lo:lo + cands[b].shape[0]]
+        lo += cands[b].shape[0]
+        boxes.append(np.concatenate([np.asarray(gt_boxes[b]), cands[b][ok]], axis=0))
+        names.append(np.concatenate([np.asarray(gt_names[b]), np.tile(np.asarray(inst_names[b]), len(rotations[b]))[ok]]))
+    return points, offsets, boxes, names
+
+
 def mixup_points(points_1, points_2, lam, shuffle_idx_1, shuffle_idx_2):
     """Prefixes int(N1*lam) / int(N2*(1-lam)) of the two shuffled frames."""
     def prefix(points, idx, frac):
