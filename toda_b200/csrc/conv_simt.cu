@@ -4,27 +4,7 @@
 // No scatter, no atomics: every output row is written exactly once (deterministic).
 // The tcgen05 path (conv_tc.cu) has the same structure with the accumulator in TMEM.
 #include "common.cuh"
-#include "conv_ts.cuh"
-
-int conv_tc_fwd(const float *x, const void *x_bf16, int n_in, int cin, const int32_t *nbr, int n_out, int kvol, const float *w,
-                int cout, const float *bias, float *y, const int32_t *out_rows, const uint32_t *tile_masks, double *bn_sums,
-                void *workspace, size_t workspace_bytes,
-                cudaStream_t st, const TilePlan *plan, const float *addend, const void *w_bf16);
-size_t conv_tc_fwd_workspace_bytes(int n_in, int cin, int cout, int kvol);
-int conv_tc_wgrad(const float *x, const void *x_bf16, int n_in, int cin, const int32_t *nbr, int n_out, int kvol,
-                  const uint32_t *tile_masks, const float *dy, const void *dy_bf16, int cout, float *dw_param, void *workspace,
-                  size_t workspace_bytes, cudaStream_t st);
-bool conv_tc_supported(int cin, int cout, int kvol);
-// TODA_CONV_BF16X3 (conv_x3.cu): three bf16 tensor-core launches per product, fp32-class accuracy
-size_t conv_x3_fwd_workspace_bytes(int n_in, int cin, int cout, int kvol);
-int conv_x3_fwd(const float *x, int n_in, int cin, const int32_t *nbr, int n_out, int kvol, const float *w, int cout, const float *bias,
-                float *y, const int32_t *out_rows, const uint32_t *tile_masks, double *bn_sums, void *workspace, size_t workspace_bytes,
-                cudaStream_t st, const TilePlan *plan, const float *addend);
-size_t conv_x3_wgrad_workspace_bytes(int n_in, int n_out, int kvol, int cin, int cout);
-int conv_x3_wgrad(const float *x, int n_in, int cin, const int32_t *nbr, int n_out, int kvol, const uint32_t *tile_masks,
-                  const float *dy, int cout, float *dw_param, void *workspace, size_t workspace_bytes, cudaStream_t st);
-bool conv_tc_wgrad_supported(int cin, int cout, int kvol);
-size_t conv_tc_wgrad_workspace_bytes(int n_in, int n_out, int kvol, int cin, int cout);
+#include "conv.cuh"
 
 namespace {
 

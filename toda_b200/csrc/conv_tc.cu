@@ -20,9 +20,10 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
-#include "conv_ts.cuh"
+#include "conv.cuh"
 #include "epilogue.cuh"
 #include "table_slice.cuh"
+#include "tcgen05.cuh"
 
 namespace {
 
@@ -36,99 +37,14 @@ constexpr int kBBytesMax = 128 * kChunkK * 2;     // 16 KB (Cout <= 128)
 constexpr int kStageBytes = kABytes + kBBytesMax;
 constexpr int kMaxKvol = 27;
 constexpr int kIdxBytes = kMaxKvol * kTileM * 4;  // this tile's slice of the neighbour table (13.5 KB)
+constexpr uint32_t kMaxSpins = 1u << 24;          // mbarrier probes before a wait traps (tcgen05.cuh)
 
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t done = 0;
-    uint32_t spins = 0;
-    while (!done) {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(done)
-            : "r"(bar), "r"(parity)
-            : "memory");
-        if (!done && ++spins > (1u << 24)) __trap();   // a lost arrival must not hang the GPU box
-    }
-}
-// non-blocking probe of a barrier phase (used to look one stage ahead while the current MMAs are being issued)
-__device__ __forceinline__ uint32_t mbar_test(uint32_t bar, uint32_t parity) {
-    uint32_t done;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(done)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    return done;
-}
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "elect.sync _|p, 0xffffffff;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(pred));
-    return pred != 0;
-}
 __device__ __forceinline__ void cp_async_16(uint32_t dst, const void *src, uint32_t src_bytes) {
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(src_bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap *map, int c0, int c1, uint32_t bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-        ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(bar)
-        : "memory");
 }
 __device__ __forceinline__ void st_shared_zero16(uint32_t dst) {
     asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(dst), "r"(0u) : "memory");
 }
-__device__ __forceinline__ void cp_async_arrive_noinc(uint32_t bar) {
-    asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-
-// K-major, SWIZZLE_128B shared-memory matrix descriptor (cute::UMMA::SmemDescriptor bit layout):
-//   [0,14) start address >> 4 | [16,30) leading byte offset >> 4 (1 for swizzled K-major) |
-//   [32,46) stride byte offset >> 4 (8 rows x 128 B = 1024 B between 8-row groups) | [46,48) version = 1 (sm_100) |
-//   [61,64) layout type = 2 (SWIZZLE_128B)
-__device__ __forceinline__ uint64_t make_desc_k_sw128(uint32_t smem_addr) {
-    uint64_t d = 0;
-    d |= (uint64_t)((smem_addr >> 4) & 0x3fff);
-    d |= (uint64_t)1 << 16;
-    d |= (uint64_t)(1024 >> 4) << 32;
-    d |= (uint64_t)1 << 46;
-    d |= (uint64_t)2 << 61;
-    return d;
-}
-
-// instruction descriptor (cute::UMMA::InstrDescriptor): D=f32, A=B=bf16, both K-major, M=128, N=n
-__host__ __device__ constexpr uint32_t make_idesc_bf16(int m, int n) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
-}
-
-// byte offset of 16-byte piece `p` of row `r` inside a [rows][64 bf16] SWIZZLE_128B tile
-__device__ __forceinline__ uint32_t sw128_offset(int r, int p) { return (uint32_t)(r * 128 + ((p ^ (r & 7)) << 4)); }
-
 // ---- forward / dgrad kernel: persistent, warp-specialised --------------------------------------------------
 //   warps 0-7   producers : gather A + copy B for every K chunk into the stage ring (cp.async, SWIZZLE_128B)
 //   warp  8     MMA       : one thread issues tcgen05.mma; accumulators double-buffered in TMEM
@@ -154,13 +70,6 @@ template <int COUT, int KB> struct FwdCfg {
     static constexpr int kTmemCols = 2 * COUT < 32 ? 32 : 2 * COUT;
     static_assert(kStages >= 3, "need at least 3 stages");
 };
-
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void cp_async_4(uint32_t dst, const void *src) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(dst), "l"(src) : "memory");
-}
 
 template <int CIN, int COUT, int KB>
 __global__ void __launch_bounds__(kFwdThreads, 1) conv_tc_fwd_kernel(const __nv_bfloat16 *__restrict__ xb,
@@ -224,10 +133,7 @@ __global__ void __launch_bounds__(kFwdThreads, 1) conv_tc_fwd_kernel(const __nv_
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (warp == 8) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "n"(C::kTmemCols) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 8) tmem_alloc<C::kTmemCols>(tmem_slot);
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
@@ -250,12 +156,12 @@ __global__ void __launch_bounds__(kFwdThreads, 1) conv_tc_fwd_kernel(const __nv_
         int g = 0, it = 0;              // global chunk counter (stage ring position), tile counter
         for (int t = blockIdx.x; t < num_tiles; t += gridDim.x, ++it) {
             const int ib = it & 1;
-            mbar_wait(idx_full + 8 * ib, (it >> 1) & 1);
+            mbar_wait<kMaxSpins>(idx_full + 8 * ib, (it >> 1) & 1);
             const uint32_t idx_tile = idx_lane + ib * kIdxBytes;
             for (unsigned long long cm = chunk_mask_of(t); cm; cm &= cm - 1, ++g) {
                 const int c = __ffsll((long long)cm) - 1;
                 const int s = g % S, use = g / S;
-                if (use > 0) mbar_wait(empty_bar + 8 * s, (use - 1) & 1);
+                if (use > 0) mbar_wait<kMaxSpins>(empty_bar + 8 * s, (use - 1) & 1);
                 const uint32_t a_dst0 = base + s * C::kStage + piece_off;
 #pragma unroll
                 for (int kb = 0; kb < KB; ++kb) {
@@ -317,13 +223,13 @@ __global__ void __launch_bounds__(kFwdThreads, 1) conv_tc_fwd_kernel(const __nv_
             uint32_t ready = 0;
             for (int t = blockIdx.x; t < num_tiles; t += gridDim.x, ++it) {
                 const int ab = it & 1, ause = it >> 1;
-                if (ause > 0) mbar_wait(acc_empty + 8 * ab, (ause - 1) & 1);   // epilogue has drained this accumulator
+                if (ause > 0) mbar_wait<kMaxSpins>(acc_empty + 8 * ab, (ause - 1) & 1);   // epilogue has drained this accumulator
                 const uint32_t d_tmem = tmem_base + ab * COUT;
                 uint32_t accumulate = 0;
                 for (unsigned long long cm = chunk_mask_of(t); cm; cm &= cm - 1, ++g) {
                     const int c = __ffsll((long long)cm) - 1;
                     const int s = g % S, use = g / S;
-                    if (!ready) mbar_wait(full_bar + 8 * s, use & 1);
+                    if (!ready) mbar_wait<kMaxSpins>(full_bar + 8 * s, use & 1);
                     const int sn = (g + 1) % S, usen = (g + 1) / S;
                     ready = mbar_test(full_bar + 8 * sn, usen & 1);            // look one stage ahead
                     // (the producers fence their generic-proxy zero stores before signalling; no proxy fence needed here)
@@ -357,78 +263,23 @@ __global__ void __launch_bounds__(kFwdThreads, 1) conv_tc_fwd_kernel(const __nv_
         int it = 0;
         for (int t = blockIdx.x; t < num_tiles; t += gridDim.x, ++it) {
             const int ab = it & 1;
-            mbar_wait(acc_full + 8 * ab, (it >> 1) & 1);
+            mbar_wait<kMaxSpins>(acc_full + 8 * ab, (it >> 1) & 1);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             const int row = t * kTileM + q * 32 + lane;          // TMEM lane = tile row
-            // row of y this tile row is written to (class-sorted dgrad launches scatter back to canonical rows)
-            const int orow = (out_rows && row < n_out) ? __ldg(out_rows + row) : row;
-            const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + ab * COUT;
-#pragma unroll
-            for (int n0 = 0; n0 < COUT; n0 += 16) {
-                uint32_t v[16];
-                asm volatile(
-                    "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                    : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-                      "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-                    : "r"(taddr + n0));
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                float o[16];
-#pragma unroll
-                for (int j = 0; j < 16; ++j) o[j] = __uint_as_float(v[j]) + (bias ? __ldg(bias + n0 + j) : 0.f);
-                if (row < n_out) {
-                    if (addend) {
-                        const float4 *ad = (const float4 *)(addend + (size_t)orow * COUT + n0);
-#pragma unroll
-                        for (int qq = 0; qq < 4; ++qq) {
-                            const float4 a4 = __ldg(ad + qq);
-                            o[4 * qq] += a4.x; o[4 * qq + 1] += a4.y; o[4 * qq + 2] += a4.z; o[4 * qq + 3] += a4.w;
-                        }
-                    }
-                    float4 *dst = (float4 *)(y + (size_t)orow * COUT + n0);
-#pragma unroll
-                    for (int qq = 0; qq < 4; ++qq) dst[qq] = make_float4(o[4 * qq], o[4 * qq + 1], o[4 * qq + 2], o[4 * qq + 3]);
-                }
-                if (bn_sums) {
-                    // statistics of the rows just produced, for the BatchNorm that follows: no second pass over y
-                    float sq[16];
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) {
-                        o[j] = row < n_out ? o[j] : 0.f;
-                        sq[j] = o[j] * o[j];
-                    }
-                    acc_s[n0 / 16] += warp_colsum16(o, lane);
-                    acc_q[n0 / 16] += warp_colsum16(sq, lane);
-                }
-            }
+            drain_accumulator<COUT>(tmem_base + ((uint32_t)(q * 32) << 16), ab, row, n_out, out_rows, bias, addend, y, bn_sums, acc_s,
+                                    acc_q, lane);
             asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
             mbar_arrive(acc_empty + 8 * ab);
         }
-        if (bn_sums && !(lane & 1)) {
-            // lane l (even) owns column n0 + ((l >> 1) & 15); one fp64 atomic per CTA-warp and channel
-            const int col = (lane >> 1) & 15;
-#pragma unroll
-            for (int i = 0; i < COUT / 16; ++i) {
-                atomicAdd(bn_sums + i * 16 + col, (double)acc_s[i]);
-                atomicAdd(bn_sums + COUT + i * 16 + col, (double)acc_q[i]);
-            }
-        }
+        flush_bn_sums<COUT>(bn_sums, acc_s, acc_q, lane);
     } else {
         // ------------------------------------------------------------------ indexer (warp 13)
-        int it = 0;
-        for (int t = blockIdx.x; t < num_tiles; t += gridDim.x, ++it) {
-            const int ib = it & 1, use = it >> 1;
-            if (use > 0) mbar_wait(idx_empty + 8 * ib, (use - 1) & 1);
-            const uint32_t dst0 = idx_base + ib * kIdxBytes;
-            const int row0 = t * kTileM;
-            load_table_slice<kTileM>(dst0, nbr, n_out, row0, n_out, kvol, lane);
-            cp_async_arrive_noinc(idx_full + 8 * ib);
-            mbar_arrive(idx_full + 8 * ib);
-        }
+        index_tiles<kTileM, kMaxSpins>(idx_base, kIdxBytes, idx_full, idx_empty, nbr, n_out, kvol, num_tiles, lane);
     }
     __syncthreads();
     if (warp == 8) {
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(C::kTmemCols) : "memory");
+        tmem_dealloc<C::kTmemCols>(tmem_base);
     }
 }
 
@@ -497,16 +348,10 @@ extern "C" int toda_table_tile_masks(const int32_t *nbr, int n_out, int kvol, ui
     return TODA_OK;
 }
 
-static inline int pad16(int c) { return c < 16 ? 16 : c; }
-
-int conv_tma_fwd(const void *xb, int n_in, int cin, const int32_t *nbr, int n_out, int kvol, const void *wb, int cout,
-                 const float *bias, const float *addend, float *y, const int32_t *out_rows, const uint32_t *tile_masks, double *bn_sums,
-                 cudaStream_t st);
-
 // w [kvol][cin][cout] fp32 -> [cout][kvol*max(cin,16)] bf16, the B operand of the tensor-core kernels (cacheable by the caller)
 extern "C" int toda_weight_kmajor_bf16(const float *w, int kvol, int cin, int cout, void *w_bf16, void *stream) {
     TODA_CHECK_ARG(w && w_bf16 && kvol > 0 && cin > 0 && cout > 0, "weight_kmajor_bf16: bad args");
-    const int cp = cin < 16 ? 16 : cin;
+    const int cp = pad16(cin);
     weight_to_kmajor_bf16_kernel<<<wave_grid((int64_t)kvol * cp * cout, 256), 256, 0, (cudaStream_t)stream>>>(w, kvol, cin, cp, cout,
                                                                                                             (__nv_bfloat16 *)w_bf16);
     TODA_LAUNCH_OK();
@@ -569,7 +414,7 @@ int conv_tc_fwd(const float *x, const void *x_bf16, int n_in, int cin, const int
     int num_tiles = ceil_div(n_out, kTileM);
     int grid = num_tiles < kNumSMs ? num_tiles : kNumSMs;   // persistent: one CTA per SM walks the tiles
     CUtensorMap map_w;
-    if (int rc = conv_tma_make_map(&map_w, wb, (uint64_t)cout, (uint64_t)kvol * cin, (uint32_t)cout, kChunkK)) return rc;
+    if (int rc = make_tensor_map_bf16(&map_w, wb, (uint64_t)cout, (uint64_t)kvol * cin, (uint32_t)cout, kChunkK)) return rc;
     // K blocks per chunk: 2 for Cout <= 64 (8 MMAs per barrier round trip), 1 for Cout = 128 (more stages); the A/B is in
     // profiles/r01_feed_ab.md
 #define LAUNCH_TC(CI, CO)                                                                                                    \
@@ -819,7 +664,7 @@ __global__ void __launch_bounds__(kWgradThreads, 1) conv_tc_wgrad_kernel(const _
             first2 = first1;
             first1 = g;
             // dy rows of this chunk (shared by every pass)
-            if (use_b > 0) mbar_wait(b_empty + 8 * bb, (use_b - 1) & 1);
+            if (use_b > 0) mbar_wait<kMaxSpins>(b_empty + 8 * bb, (use_b - 1) & 1);
             {
                 const uint32_t b_dst = b_base + bb * kBTileW + piece_off;
 #pragma unroll
@@ -834,13 +679,13 @@ __global__ void __launch_bounds__(kWgradThreads, 1) conv_tc_wgrad_kernel(const _
                     }
                 }
             }
-            mbar_wait(idx_full + 8 * ib, use_i & 1);
+            mbar_wait<kMaxSpins>(idx_full + 8 * ib, use_i & 1);
             const uint32_t idx_tile = idx_base + ib * kIdxW + 4 * rbase;
             for (uint32_t m = lm; m; m &= m - 1, ++g) {
                 const int ps = __ffs(m) - 1;
                 if (m == lm) pend_first |= 1u << (g - signalled);
                 const int s = g % S, use = g / S;
-                if (use > 0) mbar_wait(a_empty + 8 * s, (use - 1) & 1);
+                if (use > 0) mbar_wait<kMaxSpins>(a_empty + 8 * s, (use - 1) & 1);
                 const uint32_t a_dst = base + s * kATileW + piece_off;
 #pragma unroll
                 for (int mb = 0; mb < 2; ++mb) {
@@ -887,12 +732,12 @@ __global__ void __launch_bounds__(kWgradThreads, 1) conv_tc_wgrad_kernel(const _
                 const uint32_t lm = live_of(rc);
                 if (!lm) continue;
                 const int ib = lc % kBBufsW;
-                mbar_wait(b_full + 8 * ib, (lc / kBBufsW) & 1);
+                mbar_wait<kMaxSpins>(b_full + 8 * ib, (lc / kBBufsW) & 1);
                 const uint32_t b_tile = b_base + ib * kBTileW;
                 for (uint32_t m = lm; m; m &= m - 1, ++g) {
                     const int ps = __ffs(m) - 1;
                     const int s = g % S, use = g / S;
-                    if (!ready) mbar_wait(a_full + 8 * s, use & 1);
+                    if (!ready) mbar_wait<kMaxSpins>(a_full + 8 * s, use & 1);
                     ready = mbar_test(a_full + 8 * ((g + 1) % S), ((g + 1) / S) & 1);   // look one stage ahead
                     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                     const uint32_t a_tile = base + s * kATileW;
@@ -923,7 +768,7 @@ __global__ void __launch_bounds__(kWgradThreads, 1) conv_tc_wgrad_kernel(const _
         uint32_t used = 0;                                       // passes with at least one live item (written TMEM)
         for (int rc = 0; rc < nchunks; ++rc) used |= live_of(rc);
         if (used) {
-            mbar_wait(accum_bar, 0);
+            mbar_wait<kMaxSpins>(accum_bar, 0);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
         }
         const int m = q * 32 + lane;
@@ -959,7 +804,7 @@ __global__ void __launch_bounds__(kWgradThreads, 1) conv_tc_wgrad_kernel(const _
             if (!live_of(rc)) continue;
             const int ib = lc & 1, use = lc >> 1;
             ++lc;
-            if (use > 0) mbar_wait(idx_empty + 8 * ib, (use - 1) & 1);
+            if (use > 0) mbar_wait<kMaxSpins>(idx_empty + 8 * ib, (use - 1) & 1);
             const uint32_t dst0 = idx_base + ib * kIdxW;
             const int row_base = r_begin + rc * kRowsW;
             load_table_slice<ROWS>(dst0, nbr + (size_t)k0 * n_out, n_out, row_base, r_end, noffs, lane);
@@ -1040,8 +885,6 @@ __global__ void __launch_bounds__(kWgradThreads) wgrad_row_splits_kernel(const u
 }
 
 }  // namespace
-
-bool conv_tc_wgrad_supported(int cin, int cout, int kvol);
 
 extern "C" int toda_spconv_wgrad_row_splits(const uint32_t *tile_masks, int n_out, int kvol, int cin, int cout, int *groups,
                                             int *splits, int32_t *row_begin, void *stream) {

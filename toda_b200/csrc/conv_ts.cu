@@ -24,8 +24,9 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
-#include "conv_ts.cuh"
+#include "conv.cuh"
 #include "epilogue.cuh"
+#include "tcgen05.cuh"
 
 namespace {
 
@@ -51,38 +52,8 @@ constexpr int kWarpMma = 4, kWarpLoader = 5, kWarpB = 6, kWarpLoader2 = 7, kWarp
 template <int COUT> struct ARing { static constexpr int kSlots = COUT <= 64 ? 6 : 4; static constexpr int kCol0 = COUT <= 64 ? 128 : 256; };
 constexpr int kABars = 16;
 constexpr int kPlanWindow = 32768;                // block-id window of the plan kernel's bitmap
+constexpr uint32_t kMaxSpins = 1u << 26;          // mbarrier probes before a wait traps (tcgen05.cuh)
 
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
-}
-// A lost arrival must not hang the GPU box: a wait gives up (trap) after 2^26 probes (seconds; generous, because the first
-// NCCL all-reduce of a multi-GPU run can stall every kernel on the device for hundreds of milliseconds).  (A wall-clock limit read from %globaltimer cost registers in every inlined
-// wait and 10 % of the kernel's speed; -DTODA_TS_VERBOSE_TIMEOUT compiles in the printf that names the barrier and lists
-// every stuck waiter before trapping.)
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t done = 0, spins = 0;
-    while (!done) {
-        // (plain try_wait: the form with a suspend-time hint -- "sleep in hardware until the phase completes or the time
-        // is up" -- was used here until the end of round 2 and is implicated in the kernel's deadlocks: with it the stage-2
-        // workload hung in 10 of 12 runs, without it in 0 of 8; profiles/r02_conv_ts.md section 5)
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(done)
-            : "r"(bar), "r"(parity)
-            : "memory");
-        if (!done && ++spins > (1u << 26)) {
-#ifdef TODA_TS_VERBOSE_TIMEOUT
-            if ((threadIdx.x & 31) == 0)
-                printf("conv_ts: mbarrier timeout smem=0x%x parity=%u block=%d warp=%d\n", bar, parity, (int)blockIdx.x, (int)(threadIdx.x >> 5));
-            if (spins < (1u << 26) + (1u << 25)) { spins += (1u << 24); continue; }
-#endif
-            __trap();
-        }
-    }
-}
 // wait of a role that is not on the critical path (epilogue, weight producer): probe, then really sleep -- a spinning warp
 // takes issue slots from the gather warp it shares a scheduler with (the epilogue's wait alone was 12 % of all instructions)
 __device__ __forceinline__ void mbar_wait_relaxed(uint32_t bar, uint32_t parity) {
@@ -97,7 +68,7 @@ __device__ __forceinline__ void mbar_wait_relaxed(uint32_t bar, uint32_t parity)
             : "memory");
         if (done) break;
         __nanosleep(256);
-        if (++spins > (1u << 26)) {
+        if (++spins > kMaxSpins) {
 #ifdef TODA_TS_VERBOSE_TIMEOUT
             printf("conv_ts: mbarrier timeout (relaxed) smem=0x%x parity=%u block=%d warp=%d\n", bar, parity, (int)blockIdx.x, (int)(threadIdx.x >> 5));
 #endif
@@ -105,40 +76,10 @@ __device__ __forceinline__ void mbar_wait_relaxed(uint32_t bar, uint32_t parity)
         }
     }
 }
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "elect.sync _|p, 0xffffffff;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(pred));
-    return pred != 0;
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void cp_async_16(uint32_t dst, const void *src) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async_arrive_noinc(uint32_t bar) {
-    asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(bar) : "memory");
-}
 __device__ __forceinline__ void bulk_copy_g2s(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar) {
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src),
                  "r"(bytes), "r"(bar)
                  : "memory");
-}
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap *map, int c0, int c1, uint32_t bar) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-        ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(bar)
-        : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
 // D[tmem] (+)= A[tmem] * B[smem]: A = 128 lanes x 8 columns (16 bf16 per lane), B = K-major SWIZZLE_128B descriptor
 __device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
@@ -148,19 +89,6 @@ __device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, u
         "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
         ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
         : "memory");
-}
-// K-major SWIZZLE_128B shared-memory matrix descriptor (cute::UMMA::SmemDescriptor, see conv_tc.cu)
-__device__ __forceinline__ uint64_t make_desc_k_sw128(uint32_t smem_addr) {
-    uint64_t d = 0;
-    d |= (uint64_t)((smem_addr >> 4) & 0x3fff);
-    d |= (uint64_t)1 << 16;
-    d |= (uint64_t)(1024 >> 4) << 32;
-    d |= (uint64_t)1 << 46;
-    d |= (uint64_t)2 << 61;
-    return d;
-}
-__host__ __device__ constexpr uint32_t make_idesc_bf16(int m, int n) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
 }
 __device__ __forceinline__ void lds128(uint32_t addr, uint32_t &a, uint32_t &b, uint32_t &c, uint32_t &d) {
     asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(a), "=r"(b), "=r"(c), "=r"(d) : "r"(addr));
@@ -332,10 +260,7 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (warp == kWarpMma) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 512;" ::"r"(tmem_slot) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == kWarpMma) tmem_alloc<512>(tmem_slot);
     if (warp == kWarpB && lane == 0) asm volatile("prefetch.tensormap [%0];" ::"l"(&map_w) : "memory");
     if (tid < 16) asm volatile("st.shared.v4.b32 [%0], {%1, %1, %1, %1};" ::"r"(zero_base + tid * 16), "r"(0u) : "memory");
     if (warp == kWarpLoader && lane == 0) asm volatile("prefetch.tensormap [%0];" ::"l"(&map_x) : "memory");
@@ -362,7 +287,7 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
             const uint32_t ib = it & 1u;
             const uint32_t om = om_next;
             om_next = load_om(t + gridDim.x);
-            mbar_wait(lidx_full + 8 * ib, (it >> 1) & 1u);
+            mbar_wait<kMaxSpins>(lidx_full + 8 * ib, (it >> 1) & 1u);
             const uint32_t lidx_tile = lidx_base + ib * kLidxBytes + 2u * row;
             // slab buffer, barrier offset and phase parity of the tile's (up to three) offset groups
             uint32_t sbuf[3], sbar[3], spar[3];
@@ -380,7 +305,7 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
                 if (gwait > grp) return;
 #pragma unroll
                 for (int g = 0; g < 3; ++g)
-                    if ((uint32_t)g >= gwait && (uint32_t)g <= grp) mbar_wait(slab_full + sbar[g], spar[g]);
+                    if ((uint32_t)g >= gwait && (uint32_t)g <= grp) mbar_wait<kMaxSpins>(slab_full + sbar[g], spar[g]);
                 gwait = grp + 1u;
             };
             auto release_below = [&](uint32_t grp_end) {
@@ -392,7 +317,7 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
                 for (int g = 0; g < 3; ++g)
                     if ((uint32_t)g >= gdone && (uint32_t)g < grp_end) {
                         if ((uint32_t)g >= gwait) {
-                            mbar_wait(slab_full + sbar[g], spar[g]);
+                            mbar_wait<kMaxSpins>(slab_full + sbar[g], spar[g]);
                             gwait = (uint32_t)g + 1u;
                         }
                         __syncwarp();
@@ -486,7 +411,7 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
                     bool fixB = load_data(kbB, liB, vb);
                     if (gp >= (uint32_t)kASlots) {      // the pair that used this slot before (gp - kASlots) has been consumed
                         const uint32_t pg = gp - (uint32_t)kASlots;
-                        mbar_wait(a_empty + 8u * (pg & (kABars - 1)), (pg / kABars) & 1u);
+                        mbar_wait<kMaxSpins>(a_empty + 8u * (pg & (kABars - 1)), (pg / kABars) & 1u);
                         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                     }
                     if (__any_sync(0xffffffffu, fixA || fixB)) {
@@ -499,7 +424,7 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
                 } else {
                     if (gp >= (uint32_t)kASlots) {
                         const uint32_t pg = gp - (uint32_t)kASlots;
-                        mbar_wait(a_empty + 8u * (pg & (kABars - 1)), (pg / kABars) & 1u);
+                        mbar_wait<kMaxSpins>(a_empty + 8u * (pg & (kABars - 1)), (pg / kABars) & 1u);
                         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                     }
                     if (__any_sync(0xffffffffu, fixA)) fix_block(kbA, liA, va);
@@ -540,71 +465,26 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
             mbar_wait_relaxed(acc_full + 8 * ab, (it >> 1) & 1);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
             const int row = t * kTileM + q * 32 + lane;          // TMEM lane = tile row
-            // row of y this tile row is written to (class-sorted dgrad launches scatter back to canonical rows)
-            const int orow = (out_rows && row < n_out) ? __ldg(out_rows + row) : row;
-            const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + ab * COUT;
-#pragma unroll
-            for (int n0 = 0; n0 < COUT; n0 += 16) {
-                uint32_t v[16];
-                asm volatile(
-                    "tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                    : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-                      "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-                    : "r"(taddr + n0));
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                float o[16];
-#pragma unroll
-                for (int j = 0; j < 16; ++j) o[j] = __uint_as_float(v[j]) + (bias ? __ldg(bias + n0 + j) : 0.f);
-                if (row < n_out) {
-                    if (addend) {
-                        const float4 *ad = (const float4 *)(addend + (size_t)orow * COUT + n0);
-#pragma unroll
-                        for (int qq = 0; qq < 4; ++qq) {
-                            const float4 a4 = __ldg(ad + qq);
-                            o[4 * qq] += a4.x; o[4 * qq + 1] += a4.y; o[4 * qq + 2] += a4.z; o[4 * qq + 3] += a4.w;
-                        }
-                    }
-                    float4 *dst = (float4 *)(y + (size_t)orow * COUT + n0);
-#pragma unroll
-                    for (int qq = 0; qq < 4; ++qq) dst[qq] = make_float4(o[4 * qq], o[4 * qq + 1], o[4 * qq + 2], o[4 * qq + 3]);
-                }
-                if (bn_sums) {
-                    float sq[16];
-#pragma unroll
-                    for (int j = 0; j < 16; ++j) {
-                        o[j] = row < n_out ? o[j] : 0.f;
-                        sq[j] = o[j] * o[j];
-                    }
-                    acc_s[n0 / 16] += warp_colsum16(o, lane);
-                    acc_q[n0 / 16] += warp_colsum16(sq, lane);
-                }
-            }
+            drain_accumulator<COUT>(tmem_base + ((uint32_t)(q * 32) << 16), ab, row, n_out, out_rows, bias, addend, y, bn_sums, acc_s,
+                                    acc_q, lane);
             asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
             __syncwarp();
             if (lane == 0) mbar_arrive(acc_empty + 8 * ab);
         }
-        if (bn_sums && !(lane & 1)) {
-            // lane l (even) owns column n0 + ((l >> 1) & 15); one fp64 atomic per CTA-warp and channel
-            const int col = (lane >> 1) & 15;
-#pragma unroll
-            for (int i = 0; i < COUT / 16; ++i) {
-                atomicAdd(bn_sums + i * 16 + col, (double)acc_s[i]);
-                atomicAdd(bn_sums + COUT + i * 16 + col, (double)acc_q[i]);
-            }
-        }
+        flush_bn_sums<COUT>(bn_sums, acc_s, acc_q, lane);
     } else if (warp == kWarpMma) {
         // ------------------------------------------------------------------ MMA issuer.  The single issuing thread is the serial
         // resource of the kernel (a tcgen05.mma costs ~45 cycles of issue whatever its N: scripts/ubench/commit_lat.cu), so the
         // loop around it is kept minimal: ONE full-barrier per pair of K blocks, warp-uniform waits, 8 MMAs + 1-2 commits.
         constexpr uint32_t idesc = make_idesc_bf16(kTileM, COUT);
-        if (BRES) mbar_wait(b_full, 0);
+        if (BRES) mbar_wait<kMaxSpins>(b_full, 0);
         int gbase = 0, gp = 0, it = 0;
         uint32_t om_next = load_om(blockIdx.x);
         for (int t = blockIdx.x; t < num_tiles; t += gridDim.x, ++it) {
             const int ab = it & 1, ause = it >> 1;
             const uint32_t om = om_next;
             om_next = load_om(t + gridDim.x);
-            if (ause > 0) mbar_wait(acc_empty + 8 * ab, (ause - 1) & 1);   // epilogue has drained this accumulator
+            if (ause > 0) mbar_wait<kMaxSpins>(acc_empty + 8 * ab, (ause - 1) & 1);   // epilogue has drained this accumulator
             const uint32_t d_tmem = tmem_base + ab * COUT;
             uint32_t accumulate = 0;
             const unsigned long long cm = kb_mask_from(om);
@@ -623,10 +503,10 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
                     m32 &= m32 - 1u;
                 }
                 const int aslot = gp % kASlots;
-                mbar_wait(a_full + 8 * (gp & (kABars - 1)), (gp / kABars) & 1);
+                mbar_wait<kMaxSpins>(a_full + 8 * (gp & (kABars - 1)), (gp / kABars) & 1);
                 if (!BRES) {
-                    mbar_wait(b_full + 8 * (gA % SB), (gA / SB) & 1);
-                    if (n == 2) mbar_wait(b_full + 8 * ((gA + 1) % SB), ((gA + 1) / SB) & 1);
+                    mbar_wait<kMaxSpins>(b_full + 8 * (gA % SB), (gA / SB) & 1);
+                    if (n == 2) mbar_wait<kMaxSpins>(b_full + 8 * ((gA + 1) % SB), ((gA + 1) / SB) & 1);
                 }
                 asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
                 if (elect_one()) {
@@ -672,7 +552,7 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
         for (int t = blockIdx.x; t < num_tiles; t += gridDim.x, ++it) {
             const int ib = it & 1;
             if (L == 0 && lane == 0) {
-                if (it >= 2) mbar_wait(lidx_empty + 8 * ib, ((it >> 1) - 1) & 1);
+                if (it >= 2) mbar_wait<kMaxSpins>(lidx_empty + 8 * ib, ((it >> 1) - 1) & 1);
                 const uint32_t bytes = (uint32_t)kvol * (kTileM * 2);
                 mbar_arrive_expect_tx(lidx_full + 8 * ib, bytes);
                 bulk_copy_g2s(lidx_base + ib * kLidxBytes, lidx + (size_t)t * kvol * kTileM, bytes, lidx_full + 8 * ib);
@@ -688,7 +568,7 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
                 // block to fetch completed without it; that warp could then fall two uses of a buffer behind, where its
                 // parity wait never passes again: a deadlock seen a few times in ten runs on one rank's frames.)
                 if (L == 0) {
-                    if (use > 0) mbar_wait(slab_empty + 8 * buf, (use - 1) & 1);
+                    if (use > 0) mbar_wait<kMaxSpins>(slab_empty + 8 * buf, (use - 1) & 1);
                     if (lane == 0) {
                         if (nb > 0) mbar_arrive_expect_tx(slab_full + 8 * buf, (uint32_t)nb * 16u * C::kRowBytes);
                         else mbar_arrive(slab_full + 8 * buf);
@@ -735,7 +615,7 @@ __global__ void __launch_bounds__((TsCfg<CIN, COUT>::kThreads), 1) conv_ts_fwd_k
     __syncthreads();
     if (warp == kWarpMma) {
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem_base) : "memory");
+        tmem_dealloc<512>(tmem_base);
     }
 }
 
@@ -841,8 +721,8 @@ int launch_ts(const __nv_bfloat16 *xb, int n_in, const int32_t *nbr, int n_out, 
         return TODA_ERR_INVALID;
     }
     CUtensorMap map_w, map_x;
-    if (int rc = conv_tma_make_map(&map_w, wb, (uint64_t)COUT, (uint64_t)kvol * CIN, (uint32_t)COUT, 64)) return rc;
-    if (int rc = conv_tma_make_map(&map_x, xb, (uint64_t)n_in, (uint64_t)CIN, 16u, (uint32_t)(CIN < 64 ? CIN : 64))) return rc;
+    if (int rc = make_tensor_map_bf16(&map_w, wb, (uint64_t)COUT, (uint64_t)kvol * CIN, (uint32_t)COUT, 64)) return rc;
+    if (int rc = make_tensor_map_bf16(&map_x, xb, (uint64_t)n_in, (uint64_t)CIN, 16u, (uint32_t)(CIN < 64 ? CIN : 64))) return rc;
     const int num_tiles = ceil_div(n_out, kTileM);
     const int grid = num_tiles < kNumSMs ? num_tiles : kNumSMs;
     static bool attr_set = false;      // per <CIN, COUT> instantiation
@@ -860,7 +740,7 @@ int launch_ts(const __nv_bfloat16 *xb, int n_in, const int32_t *nbr, int n_out, 
 }  // namespace
 
 int conv_ts_slab_capacity(int cin) {
-    switch (cin <= 16 ? 16 : cin) {
+    switch (pad16(cin)) {
         case 16: return TsCfg<16, 16>::kCap;
         case 32: return TsCfg<32, 32>::kCap;
         case 64: return TsCfg<64, 64>::kCap;
@@ -872,7 +752,7 @@ int conv_ts_slab_capacity(int cin) {
 bool conv_ts_supported(int cin, int cout, int kvol, const TilePlan *plan) {
     if (!plan || !plan->lidx || !plan->rows || !plan->cnt) return false;
     if (plan->ngroups < 1 || plan->ngroups > 3 || kvol % plan->ngroups != 0 || kvol / plan->ngroups > 9 || kvol > kMaxKvol) return false;
-    const int cp = cin <= 16 ? 16 : cin;
+    const int cp = pad16(cin);
     if (!(cp == 16 || cp == 32 || cp == 64 || cp == 128)) return false;
     if (!(cout == 16 || cout == 32 || cout == 64 || cout == 128)) return false;
     return plan->cap >= 1 && plan->cap <= conv_ts_slab_capacity(cp);

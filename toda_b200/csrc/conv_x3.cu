@@ -7,21 +7,9 @@
 #include <cuda_bf16.h>
 
 #include "common.cuh"
-#include "conv_ts.cuh"
-
-int conv_tc_fwd(const float *x, const void *x_bf16, int n_in, int cin, const int32_t *nbr, int n_out, int kvol, const float *w,
-                int cout, const float *bias, float *y, const int32_t *out_rows, const uint32_t *tile_masks, double *bn_sums,
-                void *workspace, size_t workspace_bytes,
-                cudaStream_t st, const TilePlan *plan, const float *addend, const void *w_bf16);
-size_t conv_tc_fwd_workspace_bytes(int n_in, int cin, int cout, int kvol);
-int conv_tc_wgrad(const float *x, const void *x_bf16, int n_in, int cin, const int32_t *nbr, int n_out, int kvol,
-                  const uint32_t *tile_masks, const float *dy, const void *dy_bf16, int cout, float *dw_param, void *workspace,
-                  size_t workspace_bytes, cudaStream_t st);
-size_t conv_tc_wgrad_workspace_bytes(int n_in, int n_out, int kvol, int cin, int cout);
+#include "conv.cuh"
 
 namespace {
-
-static inline int pad16(int c) { return c < 16 ? 16 : c; }
 
 __device__ __forceinline__ void split_bf16(float v, __nv_bfloat16 &hi, __nv_bfloat16 &lo) {
     hi = __float2bfloat16_rn(v);

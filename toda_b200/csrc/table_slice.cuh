@@ -2,6 +2,8 @@
 #pragma once
 #include <cstdint>
 
+#include "tcgen05.cuh"
+
 // One warp copies nbr[k][row_base .. row_base + ROWS) for k = 0..noffs-1 (`nbr_k0` points at offset 0 of the slice,
 // rows of the table are `n_out` ints apart) to dst0 as [noffs][ROWS] int32.  Rows >= r_end are written as -1.
 // Full tiles take the fast path: a running pointer and ROWS/32 coalesced 128-byte cp.async per offset, ~3 instructions
@@ -30,5 +32,22 @@ __device__ __forceinline__ void load_table_slice(uint32_t dst0, const int *__res
                     asm volatile("st.shared.b32 [%0], %1;" ::"r"(dst + 128u * j), "r"(-1) : "memory");
             }
         }
+    }
+}
+
+// The indexer warp of the forward kernels (conv_tc.cu, conv_tma.cu): for every tile t of this CTA, the slice of the
+// [kvol][n_out] table for the tile's ROWS rows goes into buffer ib = it & 1 (idx_bytes apart from idx_base), one tile ahead of
+// the producers.  idx_empty[ib] is waited for before the buffer is reused; idx_full[ib] (expected count 64: the warp's
+// cp.async completions and its plain arrivals) completes once the slice has landed.
+template <int ROWS, uint32_t kMaxSpins>
+__device__ __forceinline__ void index_tiles(uint32_t idx_base, int idx_bytes, uint32_t idx_full, uint32_t idx_empty,
+                                            const int *__restrict__ nbr, int n_out, int kvol, int num_tiles, int lane) {
+    int it = 0;
+    for (int t = blockIdx.x; t < num_tiles; t += gridDim.x, ++it) {
+        const int ib = it & 1, use = it >> 1;
+        if (use > 0) mbar_wait<kMaxSpins>(idx_empty + 8 * ib, (use - 1) & 1);
+        load_table_slice<ROWS>(idx_base + ib * idx_bytes, nbr, n_out, t * ROWS, n_out, kvol, lane);
+        cp_async_arrive_noinc(idx_full + 8 * ib);
+        mbar_arrive(idx_full + 8 * ib);
     }
 }
