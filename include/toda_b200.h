@@ -220,6 +220,21 @@ int toda_voxelize_hard(const float *points, int64_t n_points, int point_stride, 
                        float *voxels, int32_t *coords, int32_t *num_points, int32_t *voxel_counts, void *workspace,
                        size_t workspace_bytes, void *stream);
 
+/* K1 dynamic voxelization + per-voxel mean: pcdet/models/backbones_3d/vfe/dynamic_mean_vfe.py (DynamicMeanVFE.forward,
+ * OpenPCDet v0.5.2) for a whole batch, without torch_scatter.  Same inputs, cell arithmetic and argument limits as
+ * toda_voxelize_hard (a point outside [0,grid) on any axis, or with a NaN coordinate, is dropped), but no caps: every
+ * distinct (b,z,y,x) of a kept point is a voxel and every kept point counts.
+ *   features[v][f] = (fp32 sum of column feat_col+f over the voxel's points, added in ascending point index starting
+ *                     from +0.0) / (float)count, IEEE division: bit-exact and independent of scheduling.
+ *   coords[v] = (b,z,y,x); rows in canonical (b,z,y,x) order (the reference sorts by (b,x,y,z); each row's values are
+ *   the same).  voxel_counts int32[batch+1] = per-frame V_b then V.
+ * Outputs are caller-owned and sized for n_points rows (V <= n_points); no allocation, no host synchronisation. */
+size_t toda_voxelize_dynamic_workspace_bytes(int64_t n_points, int batch, const int *grid_host);
+int toda_voxelize_dynamic(const float *points, int64_t n_points, int point_stride, int xyz_col, int feat_col,
+                          int num_features, const int32_t *frame_offsets, int batch, const float *range_host,
+                          const float *vsize_host, const int *grid_host, float *features, int32_t *coords,
+                          int32_t *voxel_counts, void *workspace, size_t workspace_bytes, void *stream);
+
 /* K2 MeanVFE.  pcdet/models/backbones_3d/vfe/mean_vfe.py L25-29: sum over all K slots / max(num,1).
  * num_points is int32 when num_is_float == 0, float32 otherwise (load_data_to_gpu casts it,
  * pcdet/models/__init__.py L34). */

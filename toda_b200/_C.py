@@ -40,6 +40,9 @@ SIGNATURES = {
     "toda_voxelize_workspace_bytes": (c_sz, [c_i64, c_int, _IP, c_int, c_int]),
     "toda_voxelize_hard": (c_int, [c_vp, c_i64, c_int, c_int, c_int, c_int, c_vp, c_int, _FP, _FP, _IP, c_int, c_int,
                                    c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_sz, c_vp]),
+    "toda_voxelize_dynamic_workspace_bytes": (c_sz, [c_i64, c_int, _IP]),
+    "toda_voxelize_dynamic": (c_int, [c_vp, c_i64, c_int, c_int, c_int, c_int, c_vp, c_int, _FP, _FP, _IP, c_vp, c_vp, c_vp,
+                                      c_vp, c_sz, c_vp]),
     "toda_mean_vfe_fwd": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_int, c_vp, c_vp]),
     "toda_mean_vfe_bwd": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_int, c_vp, c_vp]),
     "toda_rulebook_subm": (c_int, [c_vp, c_int, c_int, c_int, c_int, c_vp, c_int, _IP, c_vp, c_vp]),

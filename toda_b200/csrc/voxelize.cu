@@ -1,4 +1,4 @@
-// K1 hard voxelizer + K2 MeanVFE (see include/toda_b200.h).
+// K1 hard voxelizer + K2 MeanVFE, and the uncapped dynamic voxelizer + mean of DynamicMeanVFE (see include/toda_b200.h).
 //
 // The reference is a sequential loop (SURVEY.md Appendix C.1).  Its parallel-equivalent definition:
 //   first[v]  = min{ i : cell(i) = v }                      (per frame)
@@ -267,20 +267,24 @@ __global__ void vox_write_kernel(const float *__restrict__ points, int stride, i
     }
 }
 
+// (b,z,y,x) of an index cell id
+__device__ __forceinline__ int4 cell_coords(const GridIndex &gi, long long cell) {
+    long long hw = (long long)gi.H * gi.W;
+    int b = (int)(cell / gi.frame_stride);
+    long long r = cell - (long long)b * gi.frame_stride;
+    int z = (int)(r / hw);
+    int rem = (int)(r - (long long)z * hw);
+    return make_int4(b, z, rem / gi.W, rem % gi.W);
+}
+
 __global__ void vox_meta_kernel(GridIndex gi, const uint32_t *__restrict__ cid_cell, const int *__restrict__ counts,
                                 const int *__restrict__ row_of_cid, const int *__restrict__ slots, int K,
                                 int4 *__restrict__ coords, int *__restrict__ num_points) {
     int vall = counts[0];
-    long long hw = (long long)gi.H * gi.W;
     for (int c = blockIdx.x * blockDim.x + threadIdx.x; c < vall; c += gridDim.x * blockDim.x) {
         int row = row_of_cid[c];
         if (row < 0) continue;
-        long long cell = cid_cell[c];
-        int b = (int)(cell / gi.frame_stride);
-        long long r = cell - (long long)b * gi.frame_stride;
-        int z = (int)(r / hw);
-        int rem = (int)(r - (long long)z * hw);
-        coords[row] = make_int4(b, z, rem / gi.W, rem % gi.W);
+        coords[row] = cell_coords(gi, cid_cell[c]);
         const int *s = slots + (long long)row * K;
         int cnt = 0;
         for (int k = 0; k < K; ++k) cnt += (s[k] != kEmpty);
@@ -322,6 +326,214 @@ __global__ void mean_vfe_bwd_kernel(const float *__restrict__ dout, const void *
         int f = (int)(e % F);
         float nrm = kNumIsFloat ? ((const float *)num)[v] : (float)((const int *)num)[v];
         dvoxels[e] = __ldg(dout + v * F + f) / fmaxf(nrm, 1.0f);
+    }
+}
+
+// --- dynamic voxelization + mean (pcdet DynamicMeanVFE) --------------------------------------------
+// No caps: every kept point belongs to its voxel, every voxel is a row, and the rows are the cids (canonical order).
+//   cells, build, frames, release : the K1 passes above; coords through cell_coords, as vox_meta_kernel writes them
+//   count : cid per point, cnt[cid] += 1                       (warp-aggregated integer atomics)
+//   scan  : seg[cid] = exclusive prefix of cnt
+//   place : members[seg[cid] + slot] = point index, slot from an atomic cursor: seg[cid] ends as the segment's end
+//   short : one thread per voxel: its coords; with <= kShortSeg members, the members in ascending order by selection,
+//           ordered fp32 sum, divide; longer voxels are appended to a list
+//   long  : one CTA per listed voxel: its members in ascending order through a shared-memory bitmap over its frame's
+//           rows, then the ordered sum with the member rows staged in shared memory
+// The fp32 sum adds the members in ascending point index from +0.0, so the result does not depend on scheduling.
+constexpr int kShortSeg = 32;
+constexpr int kShortF = 8;                        // short path: feature columns summed per pass
+constexpr int kSegWinWords = 8192;                // long path: 32 KB bitmap window = 2^18 point indices
+constexpr int kLongGrid = 2 * kNumSMs;
+
+struct DynWork {
+    GridIndex gi;
+    uint32_t *pt_cell;   // [n] cell id, then cid; the long path reuses it for its ordered member lists
+    uint32_t *cid_cell;  // [n] cell id of each cid
+    int *cnt;            // [n] members per cid (zeroed per call)
+    int *seg;            // [n+1] segment start per cid, the segment end once the place pass has run
+    int *members;        // [n] point indices grouped by cid
+    int *long_cids;      // [n/(kShortSeg+1)+1] voxels left to the long path
+    int *scan_tmp;
+    int *counts;         // as VoxWork::counts, then the length of long_cids
+    size_t bytes;
+};
+
+size_t layout_dynamic(DynWork *w, void *base, int64_t n, int batch, const int *grid) {
+    char *p = (char *)base;
+    GridIndex *gp = w ? &w->gi : nullptr;
+    size_t off = align_up(index_layout(gp, base, batch, grid[2], grid[1], grid[0]), 256);
+    auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; };
+    size_t o_ptcell = take((size_t)n * 4);
+    size_t o_cidcell = take((size_t)n * 4);
+    size_t o_cnt = take((size_t)n * 4);
+    size_t o_seg = take((size_t)(n + 1) * 4);
+    size_t o_members = take((size_t)n * 4);
+    size_t o_long = take((size_t)(n / (kShortSeg + 1) + 1) * 4);
+    size_t o_tmp = take((size_t)(n / kScanTile + 2) * 4);
+    size_t o_counts = take((size_t)(3 * batch + 9) * 4);
+    if (w) {
+        w->pt_cell = (uint32_t *)(p + o_ptcell);
+        w->cid_cell = (uint32_t *)(p + o_cidcell);
+        w->cnt = (int *)(p + o_cnt);
+        w->seg = (int *)(p + o_seg);
+        w->members = (int *)(p + o_members);
+        w->long_cids = (int *)(p + o_long);
+        w->scan_tmp = (int *)(p + o_tmp);
+        w->counts = (int *)(p + o_counts);
+        w->bytes = off;
+    }
+    return off;
+}
+
+__global__ void dyn_count_kernel(GridIndex gi, uint32_t *__restrict__ pt_cell, long long n, int *__restrict__ cnt) {
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        uint32_t cell = pt_cell[i];
+        if (cell == kNoCell) continue;
+        int cid = index_lookup(gi, (long long)cell);
+        pt_cell[i] = (uint32_t)cid;
+        unsigned peers = __match_any_sync(__activemask(), cid);
+        if ((int)(threadIdx.x & 31) == __ffs(peers) - 1) atomicAdd(cnt + cid, __popc(peers));
+    }
+}
+
+__global__ void dyn_place_kernel(const uint32_t *__restrict__ pt_cid, long long n, int *__restrict__ seg,
+                                 int *__restrict__ members) {
+    int lane = threadIdx.x & 31;
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        uint32_t cid = pt_cid[i];
+        if (cid == kNoCell) continue;
+        unsigned peers = __match_any_sync(__activemask(), cid);
+        int leader = __ffs(peers) - 1;
+        int base = 0;
+        if (lane == leader) base = atomicAdd(seg + cid, __popc(peers));
+        base = __shfl_sync(peers, base, leader);
+        members[base + __popc(peers & ((1u << lane) - 1u))] = (int)i;
+    }
+}
+
+__global__ void dyn_mean_short_kernel(const float *__restrict__ points, int stride, int feat_col, int F, GridIndex gi,
+                                      const uint32_t *__restrict__ cid_cell, const int *__restrict__ counts,
+                                      const int *__restrict__ cnt, const int *__restrict__ seg_end,
+                                      const int *__restrict__ members, int *__restrict__ long_cids,
+                                      int *__restrict__ n_long, float *__restrict__ features, int4 *__restrict__ coords) {
+    int vall = counts[0];
+    for (int c = blockIdx.x * blockDim.x + threadIdx.x; c < vall; c += gridDim.x * blockDim.x) {
+        coords[c] = cell_coords(gi, cid_cell[c]);
+        int L = cnt[c];
+        int e = seg_end[c], s = e - L;
+        if (L > kShortSeg) {
+            long_cids[atomicAdd(n_long, 1)] = c;
+            continue;
+        }
+        // members in ascending order by repeated selection of the next larger index (read-only, O(L^2) L1 hits),
+        // kShortF feature columns per pass in registers
+        for (int f0 = 0; f0 < F; f0 += kShortF) {
+            float acc[kShortF];
+#pragma unroll
+            for (int u = 0; u < kShortF; ++u) acc[u] = 0.0f;
+            int prev = -1;
+            for (int r = 0; r < L; ++r) {
+                int m = 0x7fffffff;
+                for (int j = s; j < e; ++j) {
+                    int x = __ldg(members + j);
+                    if (x > prev && x < m) m = x;
+                }
+                prev = m;
+                const float *row = points + (long long)m * stride + feat_col + f0;
+#pragma unroll
+                for (int u = 0; u < kShortF; ++u)
+                    if (f0 + u < F) acc[u] = __fadd_rn(acc[u], __ldg(row + u));
+            }
+#pragma unroll
+            for (int u = 0; u < kShortF; ++u)
+                if (f0 + u < F) features[(long long)c * F + f0 + u] = __fdiv_rn(acc[u], (float)L);
+        }
+    }
+}
+
+// exclusive prefix of v over the CTA (blockDim.x == kBlock); *total = the CTA's sum.  Ends with a barrier.
+__device__ __forceinline__ int block_exclusive_sum(int v, int *warp_sums, int *total) {
+    int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int incl = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        int t = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += t;
+    }
+    if (lane == 31) warp_sums[warp] = incl;
+    __syncthreads();
+    int woff = 0, tot = 0;
+#pragma unroll
+    for (int w = 0; w < kBlock / 32; ++w) {
+        int ws = warp_sums[w];
+        woff += w < warp ? ws : 0;
+        tot += ws;
+    }
+    *total = tot;
+    __syncthreads();
+    return woff + incl - v;
+}
+
+__global__ void __launch_bounds__(kBlock) dyn_mean_long_kernel(const float *__restrict__ points, int stride, int feat_col,
+                                                               int F, GridIndex gi, const uint32_t *__restrict__ cid_cell,
+                                                               const int *__restrict__ frame_off, int batch, long long n,
+                                                               const int *__restrict__ cnt,
+                                                               const int *__restrict__ seg_end,
+                                                               const int *__restrict__ members,
+                                                               const int *__restrict__ long_cids,
+                                                               const int *__restrict__ n_long, int *ordered,
+                                                               float *__restrict__ features) {
+    __shared__ unsigned win[kSegWinWords];     // member bitmap of one index window, then staged feature rows
+    __shared__ int red[kBlock / 32];
+    float *stage = (float *)win;
+    int nl = *n_long;
+    for (int k = blockIdx.x; k < nl; k += gridDim.x) {
+        int c = long_cids[k];
+        int L = cnt[c];
+        int s = seg_end[c] - L;
+        // the members lie in their frame's rows [lo, hi], as vox_cells_kernel assigns rows to frames
+        int b = (int)((long long)cid_cell[c] / gi.frame_stride);
+        int lo = b == 0 ? 0 : __ldg(frame_off + b);
+        int hi = b == batch - 1 ? (int)(n - 1) : __ldg(frame_off + b + 1) - 1;
+        // ascending member list: one window of 32*kSegWinWords indices at a time, bits extracted in word order
+        int done = 0;
+        for (long long w0 = lo; w0 <= hi; w0 += 32ll * kSegWinWords) {
+            int nw = (int)min((long long)kSegWinWords, ((hi - w0) >> 5) + 1);
+            for (int j = threadIdx.x; j < nw; j += kBlock) win[j] = 0u;
+            __syncthreads();
+            for (int j = threadIdx.x; j < L; j += kBlock) {
+                long long d = members[s + j] - w0;
+                if (d >= 0 && d < 32ll * nw) atomicOr(win + (d >> 5), 1u << (d & 31));
+            }
+            __syncthreads();
+            int per = (nw + kBlock - 1) / kBlock;
+            int wa = min(nw, (int)threadIdx.x * per), wb = min(nw, wa + per);
+            int mine = 0;
+            for (int w = wa; w < wb; ++w) mine += __popc(win[w]);
+            int tot;
+            int pos = s + done + block_exclusive_sum(mine, red, &tot);
+            for (int w = wa; w < wb; ++w) {
+                for (unsigned bits = win[w]; bits; bits &= bits - 1u)
+                    ordered[pos++] = (int)(w0 + 32ll * w + (__ffs(bits) - 1));
+            }
+            done += tot;
+            __syncthreads();
+        }
+        // ordered sum: thread f < F adds column f of the staged rows, in member order
+        int rows_per = kSegWinWords / F;
+        float acc = 0.0f;
+        for (int j0 = 0; j0 < L; j0 += rows_per) {
+            int rows = min(rows_per, L - j0);
+            for (int t = threadIdx.x; t < rows * F; t += kBlock) {
+                int r = t / F;
+                stage[t] = __ldg(points + (long long)ordered[s + j0 + r] * stride + feat_col + (t - r * F));
+            }
+            __syncthreads();
+            if ((int)threadIdx.x < F)
+                for (int r = 0; r < rows; ++r) acc = __fadd_rn(acc, stage[r * F + threadIdx.x]);
+            __syncthreads();
+        }
+        if ((int)threadIdx.x < F) features[(long long)c * F + threadIdx.x] = __fdiv_rn(acc, (float)L);
     }
 }
 
@@ -405,6 +617,72 @@ extern "C" int toda_voxelize_hard(const float *points, int64_t n, int stride, in
         TODA_LAUNCH_OK();
         vox_meta_kernel<<<g_v, kBlock, 0, st>>>(w.gi, w.cid_cell, w.counts, w.row_of_cid, w.slots, K, (int4 *)coords,
                                                 num_points);
+        TODA_LAUNCH_OK();
+        vox_release_kernel<<<g_v, kBlock, 0, st>>>(w.gi, w.cid_cell, w.counts);
+        TODA_LAUNCH_OK();
+    }
+    return TODA_OK;
+}
+
+extern "C" size_t toda_voxelize_dynamic_workspace_bytes(int64_t n_points, int batch, const int *grid) {
+    if (n_points < 0 || batch <= 0 || !grid) return 0;
+    return layout_dynamic(nullptr, nullptr, n_points > 0 ? n_points : 1, batch, grid);
+}
+
+extern "C" int toda_voxelize_dynamic(const float *points, int64_t n, int stride, int xyz_col, int feat_col, int F,
+                                     const int32_t *frame_offsets, int batch, const float *range, const float *vsize,
+                                     const int *grid, float *features, int32_t *coords, int32_t *voxel_counts,
+                                     void *workspace, size_t workspace_bytes, void *stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    TODA_CHECK_ARG(n >= 0 && n < (1ll << 31) - 64, "voxelize_dynamic: n_points=%lld out of range", (long long)n);
+    TODA_CHECK_ARG(batch > 0 && batch <= 1024 && frame_offsets, "voxelize_dynamic: bad batch/frame_offsets");
+    TODA_CHECK_ARG(range && vsize && grid, "voxelize_dynamic: bad geometry args");
+    TODA_CHECK_ARG(stride >= 3 && xyz_col >= 0 && xyz_col + 3 <= stride && feat_col >= 0 && F > 0 &&
+                       feat_col + F <= stride, "voxelize_dynamic: column layout does not fit point_stride=%d", stride);
+    TODA_CHECK_ARG(features && coords && voxel_counts && workspace, "voxelize_dynamic: null output/workspace");
+    for (int a = 0; a < 3; ++a)
+        TODA_CHECK_ARG(grid[a] > 0 && vsize[a] > 0.f, "voxelize_dynamic: bad grid/vsize on axis %d", a);
+    long long cells = index_frame_stride(grid[2], grid[1], grid[0]) * batch;
+    TODA_CHECK_ARG(cells < (1ll << 32) - 1, "voxelize_dynamic: %lld cells exceed the 32-bit cell id range", cells);
+    size_t smem = (size_t)kBlock * stride * sizeof(float) + 16;
+    TODA_CHECK_ARG(smem <= 48 * 1024, "voxelize_dynamic: point_stride %d too large", stride);
+    int64_t n_eff = n > 0 ? n : 1;
+    DynWork w;
+    size_t need = layout_dynamic(&w, workspace, n_eff, batch, grid);
+    if (workspace_bytes < need) {
+        toda_set_error("voxelize_dynamic: workspace %zu < required %zu bytes", workspace_bytes, need);
+        return TODA_ERR_WORKSPACE;
+    }
+    VoxGeom geo;
+    for (int a = 0; a < 3; ++a) { geo.lo[a] = range[a]; geo.vs[a] = vsize[a]; geo.grid[a] = grid[a]; }
+    int *n_long = w.counts + 3 * batch + 8;
+
+    size_t zero_bytes = (size_t)((char *)w.gi.rank0 - (char *)w.gi.bits0);
+    TODA_CUDA_OK(cudaMemsetAsync(w.gi.bits0, 0, zero_bytes, st));
+    TODA_CUDA_OK(cudaMemsetAsync(w.cnt, 0, (size_t)n_eff * 4, st));
+    TODA_CUDA_OK(cudaMemsetAsync(n_long, 0, sizeof(int), st));
+    if (n > 0) {
+        vox_cells_kernel<<<wave_grid(n, kBlock), kBlock, smem, st>>>(points, n, stride, xyz_col, frame_offsets, batch, geo,
+                                                                    w.gi, w.pt_cell);
+        TODA_LAUNCH_OK();
+    }
+    // every voxel is kept, so the canonical rank (cid) is the output row
+    if (int rc = index_build_ranks(w.gi, nullptr, (int)n_eff, w.cid_cell, w.counts, st)) return rc;
+    vox_frames_kernel<<<1, 32, 0, st>>>(w.counts, batch, 0x7fffffff, voxel_counts);
+    TODA_LAUNCH_OK();
+    if (n > 0) {
+        int g_v = wave_grid(n, kBlock);
+        dyn_count_kernel<<<g_v, kBlock, 0, st>>>(w.gi, w.pt_cell, n, w.cnt);
+        TODA_LAUNCH_OK();
+        if (int rc = scan_exclusive(LoadInt{w.cnt}, (int)n, w.seg, w.scan_tmp, nullptr, st)) return rc;
+        dyn_place_kernel<<<g_v, kBlock, 0, st>>>(w.pt_cell, n, w.seg, w.members);
+        TODA_LAUNCH_OK();
+        dyn_mean_short_kernel<<<g_v, kBlock, 0, st>>>(points, stride, feat_col, F, w.gi, w.cid_cell, w.counts, w.cnt, w.seg,
+                                                      w.members, w.long_cids, n_long, features, (int4 *)coords);
+        TODA_LAUNCH_OK();
+        dyn_mean_long_kernel<<<kLongGrid, kBlock, 0, st>>>(points, stride, feat_col, F, w.gi, w.cid_cell, frame_offsets, batch,
+                                                          n, w.cnt, w.seg, w.members, w.long_cids, n_long, (int *)w.pt_cell,
+                                                          features);
         TODA_LAUNCH_OK();
         vox_release_kernel<<<g_v, kBlock, 0, st>>>(w.gi, w.cid_cell, w.counts);
         TODA_LAUNCH_OK();

@@ -433,6 +433,58 @@ def voxelize(points, frame_offsets, pc_range, voxel_size, max_points, max_voxels
     return voxels, coords, num, counts
 
 
+def voxelize_dynamic(points, frame_offsets, pc_range, voxel_size, grid=None, xyz_col=1, feat_col=1):
+    """Uncapped voxelization and per-voxel mean of a batch of frames (pcdet DynamicMeanVFE.forward, OpenPCDet v0.5.2,
+    without torch_scatter).
+
+    points: (N, stride) float32 CUDA, frames back to back, x,y,z at xyz_col..xyz_col+2; frame_offsets: int32 (B+1) CUDA
+    tensor or list.  Every point inside [0, grid) on all three axes counts; the features are all columns from feat_col
+    on, averaged over each voxel's points with an fp32 sum in ascending point order.  Returns features (V, F) float32,
+    coords (V, 4) = [b, z, y, x] int32 in canonical order and counts (B+1,) int32 (per-frame V_b, then V).  One host
+    sync (the voxel count).
+    """
+    if not torch.is_tensor(points):
+        raise TypeError("voxelize_dynamic: points must be a torch tensor")
+    points = _need(points, torch.float32, "points")
+    if points.dim() != 2:
+        raise ValueError(f"voxelize_dynamic: points must be (N, stride), got shape {tuple(points.shape)}")
+    n, stride = points.shape
+    dev = points.device
+    if not torch.is_tensor(frame_offsets):
+        frame_offsets = torch.tensor(list(frame_offsets), dtype=torch.int32, device=dev)
+    frame_offsets = _need(frame_offsets, torch.int32, "frame_offsets")
+    if frame_offsets.dim() != 1 or frame_offsets.numel() < 2:
+        raise ValueError("voxelize_dynamic: frame_offsets must be a (B+1,) vector with B >= 1")
+    batch = frame_offsets.numel() - 1
+    xyz_col, feat_col = int(xyz_col), int(feat_col)
+    if not (0 <= xyz_col and xyz_col + 3 <= stride and 0 <= feat_col < stride):
+        raise ValueError(f"voxelize_dynamic: xyz_col={xyz_col} / feat_col={feat_col} do not fit point stride {stride}")
+    f = stride - feat_col
+    pc_range = np.asarray(pc_range, dtype=np.float32).reshape(-1)
+    voxel_size = np.asarray(voxel_size, dtype=np.float32).reshape(-1)
+    if pc_range.size != 6 or voxel_size.size != 3 or not (voxel_size > 0).all():
+        raise ValueError("voxelize_dynamic: pc_range needs 6 values and voxel_size 3 positive values")
+    grid = grid_size_xyz(pc_range, voxel_size) if grid is None else np.asarray(grid).reshape(-1)
+    if grid.size != 3 or not (grid > 0).all():
+        raise ValueError(f"voxelize_dynamic: grid must be 3 positive sizes (x, y, z), got {grid}")
+    grid_c = _C.ints(grid)
+    L = _C.lib()
+    ws_bytes = L.toda_voxelize_dynamic_workspace_bytes(n, batch, grid_c)
+    if ws_bytes == 0:
+        raise RuntimeError("toda_voxelize_dynamic_workspace_bytes rejected the arguments")
+    ws = _workspace("vox", ws_bytes, dev)
+    features = torch.empty((max(n, 1), f), dtype=torch.float32, device=dev)
+    coords = torch.empty((max(n, 1), 4), dtype=torch.int32, device=dev)
+    counts = torch.empty((batch + 1,), dtype=torch.int32, device=dev)
+    with _timed("voxelize_dynamic", n_points=n, batch=batch, F=f):
+        rc = L.toda_voxelize_dynamic(_p(points), n, stride, xyz_col, feat_col, f, _p(frame_offsets), batch,
+                                     _C.floats(pc_range), _C.floats(voxel_size), grid_c, _p(features), _p(coords),
+                                     _p(counts), _p(ws), ws.numel(), _stream())
+    _C.check(rc, "toda_voxelize_dynamic")
+    v = int(counts[batch].item())
+    return features[:v], coords[:v], counts
+
+
 class _MeanVFE(torch.autograd.Function):
     @staticmethod
     def forward(ctx, voxels, num_points):

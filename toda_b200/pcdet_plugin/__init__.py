@@ -18,6 +18,18 @@ VoxelResBackBone8x = _classes["VoxelResBackBone8x"]
 SparseBasicBlock = _classes["SparseBasicBlock"]
 
 
+def frame_offsets(batch_dict):
+    """int32 (B+1) row offsets of the frames of batch_dict['points']: `point_frame_offsets` when present, otherwise found
+    from the batch column, since collate_batch stores the frames back to back (dataset.py L173-178)."""
+    offsets = batch_dict.get("point_frame_offsets")
+    if offsets is None:
+        points = batch_dict["points"]
+        bidx = points[:, 0].contiguous()
+        bounds = torch.arange(int(batch_dict["batch_size"]) + 1, device=points.device, dtype=torch.float32)
+        offsets = torch.searchsorted(bidx, bounds).int()
+    return offsets
+
+
 class MeanVFE(nn.Module):
     """pcdet/models/backbones_3d/vfe/mean_vfe.py; constructor as detector3d_template.py L56-63 calls it.
 
@@ -49,13 +61,7 @@ class MeanVFE(nn.Module):
 
     def voxelize(self, batch_dict):
         points = batch_dict["points"]                       # (N, 1+F): [b, x, y, z, ...]
-        batch_size = int(batch_dict["batch_size"])
-        offsets = batch_dict.get("point_frame_offsets")
-        if offsets is None:
-            # frames are stored back to back by collate_batch (dataset.py L173-178)
-            bidx = points[:, 0].contiguous()
-            bounds = torch.arange(batch_size + 1, device=points.device, dtype=torch.float32)
-            offsets = torch.searchsorted(bidx, bounds).int()
+        offsets = frame_offsets(batch_dict)
         mode = "train" if self.training else "test"
         max_voxels = self._cfg("MAX_NUMBER_OF_VOXELS")
         max_voxels = max_voxels[mode] if hasattr(max_voxels, "__getitem__") and not isinstance(max_voxels, int) else max_voxels
@@ -71,6 +77,36 @@ class MeanVFE(nn.Module):
         if "voxels" not in batch_dict:
             batch_dict = self.voxelize(batch_dict)
         batch_dict["voxel_features"] = ops.mean_vfe(batch_dict["voxels"], batch_dict["voxel_num_points"])
+        return batch_dict
+
+
+class DynamicMeanVFE(nn.Module):
+    """pcdet/models/backbones_3d/vfe/dynamic_mean_vfe.py (OpenPCDet v0.5.2), without torch_scatter.
+
+    Reads `points` [b, x, y, z, ...] (the `transform_points_to_voxels_placeholder` path) and voxelizes with no caps:
+    every point inside [0, grid_size) on all three axes counts, and each voxel's feature is the mean of columns 1..F of
+    its points (fp32 sum in ascending point order).  Differences from the reference, by design: rows come in canonical
+    (b, z, y, x) order instead of sorted (b, x, y, z) keys (each row's values are the same), points with a NaN coordinate
+    are dropped, and the voxel key has no int32 wrap.  Like the reference's forward, nothing here carries a gradient.
+    """
+
+    def __init__(self, model_cfg, num_point_features, voxel_size, grid_size, point_cloud_range, **kwargs):
+        super().__init__()
+        self.model_cfg = model_cfg
+        self.num_point_features = num_point_features
+        self.voxel_size = voxel_size
+        self.grid_size = grid_size
+        self.point_cloud_range = point_cloud_range
+
+    def get_output_feature_dim(self):
+        return self.num_point_features
+
+    @torch.no_grad()
+    def forward(self, batch_dict, **kwargs):
+        features, coords, _ = ops.voxelize_dynamic(batch_dict["points"].contiguous(), frame_offsets(batch_dict),
+                                                   self.point_cloud_range, self.voxel_size, grid=self.grid_size)
+        batch_dict["voxel_features"], batch_dict["voxel_coords"] = features, coords
+        batch_dict["voxel_coords_canonical"] = True
         return batch_dict
 
 
@@ -91,7 +127,7 @@ class HeightCompression(nn.Module):
         return batch_dict
 
 
-VFE = {"MeanVFE": MeanVFE}
+VFE = {"MeanVFE": MeanVFE, "DynamicMeanVFE": DynamicMeanVFE}
 BACKBONES_3D = {"VoxelBackBone8x": VoxelBackBone8x, "VoxelResBackBone8x": VoxelResBackBone8x}
 MAP_TO_BEV = {"HeightCompression": HeightCompression}
 
